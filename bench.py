@@ -6,6 +6,7 @@
                                                                  (oracle/_ref, one process per core; oracle port if absent)
   python bench.py --config c1|c2|c4|c5|c3-<1M|10M|100M>-<coh|incoh>-<closest|any>
   python bench.py --scaling strong                               N > 1: a FIXED --spp-per-step per step, split over the ranks
+  python bench.py ... --dump-outputs DIR                         also writes what the last timed step computed (dump_outputs)
 
 Path-tracing configs (c1, c2, c4, c5).  A "step" renders `--spp-per-step` iterations (samples per pixel) of the frame:
 [extend -> shade -> connect] x depth -> accumulate, one pass of the hot path over one batch of width*height*spp path samples.
@@ -77,7 +78,11 @@ def parse_args(argv=None):
     ap.add_argument("--no-ncu", action="store_true")
     ap.add_argument("--no-probes", action="store_true")
     ap.add_argument("--ncu-child", action="store_true", help=argparse.SUPPRESS)
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what the last timed step computed as DIR/<name>.npy (see dump_outputs)")
     args = ap.parse_args(argv)
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs writes the outputs of the GPU arm (--impl b200)")
     if not args.config.startswith("c3"):
         if args.config not in CONFIGS:
             ap.error("unknown --config " + args.config)
@@ -186,6 +191,27 @@ class ClockSampler(threading.Thread):
         return {"sm_mhz": sm[len(sm) // 2] if sm else None, "sm_min_mhz": sm[0] if sm else None,
                 "sm_max_mhz": max(r[1] for r in self.rows) if self.rows else None, "reasons": sorted(reasons),
                 "power_w_max": max(power) if power else None, "samples": len(self.rows), "source": self.source}
+
+
+DUMP_LIMIT = 64 * 10 ** 6          # bytes of array data that --dump-outputs writes at most
+
+
+def dump_outputs(directory, outputs):
+    """--dump-outputs: writes every array of `outputs` ({name: array}) as directory/<name>.npy, float32 arrays as they are and
+    integer arrays as float64 (exact for 32-bit values), so that two builds run with the same arguments can be compared output
+    for output.  When the arrays together exceed DUMP_LIMIT, each keeps the same fixed, seeded sample of its first-axis rows
+    (frame rows, or rays), in order."""
+    import numpy as np
+    size = {name: a.size * (a.itemsize if a.dtype.kind == "f" else 8) for name, a in outputs.items()}
+    total = sum(size.values())
+    os.makedirs(directory, exist_ok=True)
+    for name, a in outputs.items():
+        if total > DUMP_LIMIT:
+            keep = max(1, len(a) * DUMP_LIMIT // total)
+            a = a[np.unique(np.random.default_rng(0).integers(0, len(a), keep))]
+        if a.dtype.kind != "f":
+            a = a.astype(np.float64)
+        np.save(os.path.join(directory, name + ".npy"), np.ascontiguousarray(a))
 
 
 def measured_peak():
@@ -526,6 +552,9 @@ def main():
         combine()
         reduce_ms = ctx.timer_stop()            # on each rank: waiting for the slowest rank + the transfer
     stamps.append(time.time())
+    outputs = None
+    if args.dump_outputs and rank == 0:         # the frame after the last timed step (in a group: the mean over the ranks)
+        outputs = {"frame": (combined if dist is not None else frame).cpu().numpy().reshape(h, w, 4)}
     barrier()
     sampler.stop_flag.set()
     sampler.join()
@@ -675,6 +704,8 @@ def main():
             line["parity_detail"] = parity
         if n == 1 and not args.no_cpu_baseline:
             line["cpu_baseline"] = cpu_baseline_block(args, "Msamples/s")
+        if outputs is not None:
+            dump_outputs(args.dump_outputs, outputs)
         print(json.dumps(line), flush=True)
     app.close()
     if dist is not None:
@@ -860,6 +891,13 @@ def run_rays(args, rank, local_rank, world):
         trace()
     ms = ctx.timer_stop()
     barrier()
+    outputs = None
+    if args.dump_outputs and rank == 0:         # the hits (or occlusion flags) of the last timed step
+        if mode == "closest":
+            hits = ctx.download(d_out, core.HIT_DTYPE, nrays)
+            outputs = {"hit_t": hits["t"], "hit_u": hits["u"], "hit_v": hits["v"], "hit_instance": hits["inst"], "hit_primitive": hits["prim"]}
+        else:
+            outputs = {"occluded": ctx.download(d_out, np.uint32, nrays)}
     sampler.stop_flag.set()
     sampler.join()
     t = torch.tensor([ms], dtype=torch.float64, device="cuda")
@@ -920,6 +958,8 @@ def run_rays(args, rank, local_rank, world):
                              "per_ray": {"nodes": counts.nodes / max(counts.rays, 1), "tris": counts.tris / max(counts.rays, 1), "bytes": per_ray, "flops": flops_ray}}}
         if n == 1 and not args.no_cpu_baseline and ntris <= 10 ** 6:
             line["cpu_baseline"] = rays_cpu(args, ntris, kind, mode, rays)
+        if outputs is not None:
+            dump_outputs(args.dump_outputs, outputs)
         print(json.dumps(line), flush=True)
     ctx.close()
     if dist is not None:

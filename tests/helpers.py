@@ -116,13 +116,40 @@ def random_rgbe(w, h, seed):
     return img
 
 
-def write_rgbe_hdr(path, rgbe):
-    """Flat (not run-length encoded) Radiance .hdr file, top row first, from RGBE bytes [h, w, 4]."""
+def write_rgbe_hdr(path, rgbe, rle=False):
+    """Radiance .hdr file, top row first, from RGBE bytes [h, w, 4]: flat, or with rle=True adaptive run-length encoded
+    scanlines (each channel as runs of one repeated byte and literal stretches)."""
     h, w = rgbe.shape[:2]
+    rgbe = np.ascontiguousarray(rgbe, dtype=np.uint8)
     with open(path, "wb") as f:
         f.write(b"#?RADIANCE\nFORMAT=32-bit_rle_rgbe\n\n-Y %d +X %d\n" % (h, w))
-        f.write(np.ascontiguousarray(rgbe, dtype=np.uint8).tobytes())
+        if not rle:
+            f.write(rgbe.tobytes())
+        else:
+            for row in rgbe:
+                f.write(bytes((2, 2, w >> 8, w & 255)))
+                for c in range(4):
+                    f.write(_rle_bytes(row[:, c].tolist()))
     return path
+
+
+def _rle_bytes(vals):
+    """One channel of a scanline: a run of n >= 3 equal bytes is (128 + n, byte), anything else literal (n, n bytes)."""
+    out, i, n = bytearray(), 0, len(vals)
+    while i < n:
+        run = 1
+        while i + run < n and run < 127 and vals[i + run] == vals[i]:
+            run += 1
+        if run >= 3:
+            out += bytes((128 + run, vals[i]))
+            i += run
+            continue
+        j = i
+        while j < n and j - i < 128 and not (j + 2 < n and vals[j] == vals[j + 1] == vals[j + 2]):
+            j += 1
+        out += bytes([j - i] + vals[i:j])
+        i = j
+    return bytes(out)
 
 
 PORTABLE_MATH_SRC = r"""

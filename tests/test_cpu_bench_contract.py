@@ -38,6 +38,32 @@ def test_reference_arm_is_silent_on_other_ranks(built):
     assert out.returncode == 0 and not [l for l in out.stdout.splitlines() if l.startswith("{")]
 
 
+def test_dump_outputs_writes_float_arrays_within_the_limit(tmp_path, monkeypatch):
+    """--dump-outputs: float32 arrays as they are, integer arrays as float64; over the limit, every array keeps the same seeded
+    sample of its rows, identical from run to run."""
+    import numpy as np
+    import pytest
+    sys.path.insert(0, H.ROOT)
+    import bench
+    with pytest.raises(SystemExit):
+        bench.parse_args(["--impl", "reference", "--dump-outputs", str(tmp_path)])
+    t = np.arange(4000, dtype=np.float32) * np.float32(0.25)
+    prim = np.arange(4000, dtype=np.uint32) + np.uint32(4000000000)
+    bench.dump_outputs(str(tmp_path / "all"), {"hit_t": t, "hit_primitive": prim})
+    assert np.load(str(tmp_path / "all" / "hit_t.npy")).tobytes() == t.tobytes()
+    whole = np.load(str(tmp_path / "all" / "hit_primitive.npy"))
+    assert whole.dtype == np.float64 and np.array_equal(whole, prim)
+    monkeypatch.setattr(bench, "DUMP_LIMIT", 12000)
+    for run in ("a", "b"):
+        bench.dump_outputs(str(tmp_path / run), {"hit_t": t, "hit_primitive": prim})
+    got = {name: np.load(str(tmp_path / "a" / (name + ".npy"))) for name in ("hit_t", "hit_primitive")}
+    assert sum(a.nbytes for a in got.values()) <= 12000 and len(got["hit_t"]) > 500
+    assert np.array_equal(got["hit_t"] * 4, got["hit_primitive"] - 4000000000)          # the same rows of both arrays
+    assert np.all(np.diff(got["hit_t"]) > 0)                                             # in order, no row twice
+    for name, a in got.items():
+        assert np.load(str(tmp_path / "b" / (name + ".npy"))).tobytes() == a.tobytes()
+
+
 def test_clock_sampler_without_a_gpu():
     sys.path.insert(0, H.ROOT)
     import bench

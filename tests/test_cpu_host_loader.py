@@ -1,7 +1,6 @@
 """Host side (no GPU): tokenizer, the two description formats, tessellators, index semantics, tile partition."""
 import ctypes as C
 import os
-import sys
 
 import numpy as np
 import pytest
@@ -276,12 +275,14 @@ def test_environment_cdf_equals_reference_golden(built, tmp_path, key):
         assert any(np.array_equal(row, equal) for row in cdf_u)
 
 
-def test_environment_cdf_equals_live_reference(built, tmp_path):
-    """Container only: the same comparison against oracle/_ref/libreftex.so built from /root/reference right now."""
-    if not os.path.isdir("/root/reference/apps/rtigo3/src"):
-        pytest.skip("/root/reference is not mounted here")
-    sys.path.insert(0, os.path.join(H.ROOT, "tests", "golden"))
-    import make_golden_envcdf
-    texels, cdf_u, cdf_v, integral = _env_case(tmp_path, "random_48x24")
-    u, v, i = make_golden_envcdf.reference_cdf(texels)
+def test_environment_cdf_of_a_run_length_encoded_hdr_equals_reference_golden(built, tmp_path):
+    """The random map of the test above written with run-length encoded scanlines: the reader's RLE path must give the same
+    texels, and the CDFs must equal what the reference's own function returned for them (tests/golden/reference_envcdf.npz)."""
+    gold = np.load(os.path.join(H.ROOT, "tests", "golden", "reference_envcdf.npz"))
+    spec = H.write_rgbe_hdr(os.path.join(str(tmp_path), "random_rle.hdr"), H.random_rgbe(48, 24, 20261018), rle=True)
+    app = load(tmp_path, name="rtigo3_geometry", miss=2, envMap=spec, resolution="8 8")
+    texels, cdf_u, cdf_v, integral = app.environment()
+    app.close()
+    assert texels.tobytes() == gold["random_48x24_texels"].tobytes()
+    u, v, i = gold["random_48x24_cdf_u"], gold["random_48x24_cdf_v"], gold["random_48x24_integral"]
     assert cdf_u.tobytes() == u.tobytes() and cdf_v.tobytes() == v.tobytes() and np.float32(integral).tobytes() == np.float32(i).tobytes()
