@@ -18,10 +18,10 @@ all: core host oracle
 
 core: $(LIB)/librtcore.so
 
-$(LIB)/kernels_trace.o: $(CSRC)/kernels_trace.cu $(CSRC)/trace.cuh $(CSRC)/trace_pool.cuh $(CSRC)/rtc_internal.h include/rtc_core.h include/rtigo3_abi.h
+$(LIB)/kernels_trace.o: $(CSRC)/kernels_trace.cu $(CSRC)/trace.cuh $(CSRC)/rtc_internal.h include/rtc_core.h include/rtigo3_abi.h
 	$(NVCC) $(NVFLAGS) $(TRACE_DEFS) -c $< -o $@
 # shading: FMA contraction off, IEEE division/sqrt -- bit-exact against the scalar oracle
-$(LIB)/kernels_shade.o: $(CSRC)/kernels_shade.cu $(CSRC)/shade.cuh $(CSRC)/trace.cuh $(CSRC)/trace_pool.cuh $(CSRC)/trace_packet.cuh $(CSRC)/schedule_tuner.h $(CSRC)/rtc_internal.h include/rtc_core.h include/rtigo3_abi.h include/rt_portable_math.h
+$(LIB)/kernels_shade.o: $(CSRC)/kernels_shade.cu $(CSRC)/shade.cuh $(CSRC)/trace.cuh $(CSRC)/schedule_tuner.h $(CSRC)/rtc_internal.h include/rtc_core.h include/rtigo3_abi.h include/rt_portable_math.h
 	$(NVCC) $(NVFLAGS) $(TRACE_DEFS) -fmad=false -prec-div=true -prec-sqrt=true -c $< -o $@
 $(LIB)/probes.o: $(CSRC)/probes.cu $(CSRC)/rtc_internal.h include/rtc_core.h
 	$(NVCC) $(NVFLAGS) -c $< -o $@

@@ -84,13 +84,6 @@ typedef struct {
   uint64_t nodes, tris, instances, rays;
 } rtc_trace_counts;
 
-/* How the ray pool of the traversal kernels (csrc/trace_pool.cuh) spent its passes during launches made with countWork:
- * passes[p] warp-level passes of phase p and lanes[p] the ray slots they processed (<= 32 per pass), p = 0 node visit,
- * 1 triangle tests, 2 instance entry, 3 store + fetch.  lanes / (32 * passes) is the SIMD occupancy of the phase. */
-typedef struct {
-  uint64_t passes[4], lanes[4];
-} rtc_pass_stats;
-
 enum { RTC_RAYGEN_FULL_FRAME = 0,      /* __raygen__path_tracer            (raygeneration.cu:167) */
        RTC_RAYGEN_LOCAL_COPY = 1 };    /* __raygen__path_tracer_local_copy (raygeneration.cu:259) */
 
@@ -237,8 +230,6 @@ int rtc_trace_schedule_set(rtc_context* ctx, int schedule);
 /* Work counters of the launches made with countWork since the last reset: [0] extend (radiance rays), [1] connect (shadow rays). */
 int rtc_launch_counts_get(rtc_context* ctx, rtc_trace_counts out[2]);
 int rtc_launch_counts_reset(rtc_context* ctx);
-/* Pass statistics of the same launches: [0] extend, [1] connect. */
-int rtc_launch_pass_stats_get(rtc_context* ctx, rtc_pass_stats out[2]);
 
 /* Device-side timing on the context stream (CUDA events). */
 int rtc_timer_start(rtc_context* ctx);

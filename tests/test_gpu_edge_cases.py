@@ -52,9 +52,9 @@ def test_more_paths_than_one_batch(cuda_device, tmp_path, monkeypatch):
     assert a.tobytes() == b.tobytes()
 
 
-def test_roofline_probes_and_pass_statistics(cuda_device):
+def test_roofline_probes(cuda_device):
     """The denominators bench.py reports fractions against are measured by kernels of this library: they must be in the range
-    a B200 can deliver, and the pass statistics of the (optional) ray-pool driver stay zero under the default driver."""
+    a B200 can deliver."""
     from tweeker_raytracer_b200 import core
     ctx = core.Context(0)
     try:
@@ -64,8 +64,6 @@ def test_roofline_probes_and_pass_statistics(cuda_device):
         assert 500.0 < l2 < 20000.0          # GB/s of random 16-byte gathers out of L2
         assert 20.0 < fp32 < 90.0            # TFLOP/s: 148 SMs x 128 lanes x 2 x ~1.9 GHz = 72
         assert 400.0 < issue < 1300.0        # 1e9 warp instructions per second: 148 SMs x 4 schedulers x ~1.9 GHz = 1125
-        ext, con = ctx.launch_pass_stats()
-        assert all(v[0] == 0 for v in ext.values()) and all(v[0] == 0 for v in con.values())
     finally:
         ctx.close()
 

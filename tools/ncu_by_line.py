@@ -40,7 +40,7 @@ def main():
     tot = sum(v[0] for v in byline.values())
     tots = sum(v[2] for v in byline.values())
     src = {}
-    for f in ("trace.cuh", "trace_pool.cuh", "kernels_trace.cu", "shade.cuh", "kernels_shade.cu"):
+    for f in ("trace.cuh", "kernels_trace.cu", "shade.cuh", "kernels_shade.cu"):
         try:
             src[f] = open(ROOT + "/tweeker_raytracer_b200/csrc/" + f).read().split("\n")
         except OSError:

@@ -29,7 +29,7 @@ SYMBOLS = [
     "rtc_launch", "rtc_launch_ex", "rtc_launch_counts_get", "rtc_launch_counts_reset", "rtc_timer_start", "rtc_timer_stop",
     "rtc_profile_enable", "rtc_profile_get", "rtc_trace_closest", "rtc_trace_any", "rtc_trace_count", "rtc_generate_primary",
     "rtc_composite", "rtc_tonemap", "rtc_stats_get", "rtc_stats_reset",
-    "rtc_launch_pass_stats_get", "rtc_probe_gather", "rtc_probe_pipes", "rtc_scene_export", "rtc_gas_info", "rtc_gas_export",
+    "rtc_probe_gather", "rtc_probe_pipes", "rtc_scene_export", "rtc_gas_info", "rtc_gas_export",
     "rtc_probe_math",
     "rtc_host_gas_build", "rtc_host_ias_build", "rtc_host_accel_info", "rtc_host_accel_export", "rtc_host_accel_destroy",
     "rtc_trace_schedule_get", "rtc_trace_schedule_set",
@@ -59,10 +59,6 @@ SCHEDULE_NAMES = ["group", "one_tri", "two_tri"]
 class TraceSchedule(C.Structure):
     _fields_ = [("schedule", C.c_int), ("decided", C.c_int), ("measured", C.c_int), ("pathsPerBatch", C.c_uint64),
                 ("groupMs", C.c_float * 2), ("oneTriMs", C.c_float), ("twoTriMs", C.c_float)]
-
-
-class PassStats(C.Structure):
-    _fields_ = [("passes", C.c_uint64 * 4), ("lanes", C.c_uint64 * 4)]
 
 
 KERNEL_CLASSES = ["generate", "extend", "shade", "connect", "accumulate", "other"]
@@ -128,7 +124,6 @@ def lib():
         L.rtc_scene_export.argtypes = [C.c_void_p, C.c_uint64, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]
         L.rtc_gas_info.argtypes = [C.c_void_p, C.c_uint32, C.POINTER(C.c_uint64), C.POINTER(C.c_uint64)]
         L.rtc_gas_export.argtypes = [C.c_void_p, C.c_uint32, C.c_void_p, C.c_void_p]
-        L.rtc_launch_pass_stats_get.argtypes = [C.c_void_p, C.POINTER(PassStats)]
         L.rtc_probe_gather.argtypes = [C.c_void_p, C.c_uint64, C.c_uint32, C.POINTER(C.c_double)]
         L.rtc_probe_pipes.argtypes = [C.c_void_p, C.c_int, C.POINTER(C.c_double)]
         L.rtc_probe_math.argtypes = [C.c_void_p, C.c_int, C.c_void_p, C.c_void_p, C.c_void_p, C.c_uint32]
@@ -359,13 +354,6 @@ class Context:
     def set_trace_schedule(self, schedule):
         """schedule: "group", "one_tri", "two_tri", or "auto" (measure again)."""
         _check(self.L.rtc_trace_schedule_set(self.h, {"group": 0, "one_tri": 1, "two_tri": 2, "auto": -1}[schedule]))
-
-    def launch_pass_stats(self):
-        """(extend, connect): {phase: (passes, slots processed, mean lanes per pass)} of the ray pool during count_work launches."""
-        out = (PassStats * 2)()
-        _check(self.L.rtc_launch_pass_stats_get(self.h, out))
-        names = ["node", "triangle", "instance", "fetch"]
-        return tuple({n: (int(o.passes[k]), int(o.lanes[k]), o.lanes[k] / max(o.passes[k], 1)) for k, n in enumerate(names)} for o in out)
 
     def probe_gather(self, nbytes, loads_per_thread=256):
         """GB/s of random 16-byte gathers over a working set of nbytes (L2-resident when it fits)."""

@@ -13,8 +13,7 @@
 #include "shade.cuh"
 // the primary-ray extend kernel generates its rays with the shading arithmetic of this translation unit (see ExtendPrimary)
 #define RTC_STACK_OVERFLOW_COUNTER g_rtcStackOverflowsPrimary
-#include "trace_pool.cuh"
-#include "trace_packet.cuh"
+#include "trace.cuh"
 #include "schedule_tuner.h"
 
 #include <cstdlib>
@@ -228,35 +227,6 @@ struct ExtendPrimary
 };
 
 constexpr int kPrimaryBlock = 128;
-#ifndef RTC_TRACE_MIN_BLOCKS
-#define RTC_TRACE_MIN_BLOCKS 8
-#endif
-#ifndef RTC_POOL_BLOCKS
-#define RTC_POOL_BLOCKS 4
-#endif
-
-template <bool COUNT>
-__global__ void __launch_bounds__(kPrimaryBlock, RTC_POOL_BLOCKS)
-k_extend_primary_pool(const SceneDesc sc, const ExtendPrimary policy, uint32_t n, uint32_t* __restrict__ cursor, unsigned long long* __restrict__ counts,
-                      uint2* __restrict__ overflow)
-{
-  extern __shared__ uint32_t poolWords[];
-  const uint32_t warp = threadIdx.x >> 5;
-  const size_t warpGlobal = (size_t)blockIdx.x * (kPrimaryBlock / 32) + warp;
-  rtpool::trace_pool<false, COUNT, false>(sc, n, cursor, policy, poolWords + warp * rtpool::warp_words(false, false), overflow + warpGlobal * rtpool::kOverflowPerWarp, counts);
-}
-constexpr size_t kPrimaryPoolSmem = (size_t)(kPrimaryBlock / 32) * rtpool::warp_bytes(false, false);
-
-// Packet traversal of the primary rays (trace_packet.cuh): a warp = one 8x4 pixel tile = one shared traversal.
-#ifndef RTC_PACKET_BLOCKS
-#define RTC_PACKET_BLOCKS 4
-#endif
-__global__ void __launch_bounds__(kPrimaryBlock, RTC_PACKET_BLOCKS)
-k_extend_primary_packet(const SceneDesc sc, const ExtendPrimary policy, uint32_t n, uint32_t* __restrict__ cursor)
-{
-  __shared__ uint2 stacks[(kPrimaryBlock / 32) * RTC_PACKET_STACK];
-  trace_packets(sc, n, cursor, policy, stacks + (threadIdx.x >> 5) * RTC_PACKET_STACK);
-}
 
 template <bool COUNT, int TRICAP = 0>
 __global__ void __launch_bounds__(kPrimaryBlock, RTC_TRACE_MIN_BLOCKS)
@@ -946,32 +916,27 @@ void launch_shade_class(rtc_context* ctx, cudaStream_t stream, int grid, const W
 
 // The seven class kernels of one depth only share the output queues (atomic appends): the diffuse class, the largest, stays on
 // the context stream, the other six fork onto side streams after k_bin and join before the next stage, so the small ones fill
-// the tails of the large ones instead of each running alone.  RTC_SHADE_STREAMS=0 keeps everything on the context stream.
+// the tails of the large ones instead of each running alone.
 int launch_shade_classes(rtc_context* ctx, int grid, const WfArgs& a, const SceneDesc& sc, uint32_t* bins, uint32_t binStride, uint32_t* binCounts,
                          uint32_t* qOut, uint32_t* countOut, uint32_t* shadowQueue, uint32_t* shadowCount, bool tex, bool deferRR, bool primary)
 {
-  static const bool concurrent = []() { const char* e = getenv("RTC_SHADE_STREAMS"); return !(e && atoi(e) == 0); }();
-  cudaStream_t s[7];
-  for (int k = 0; k < 7; ++k) s[k] = ctx->stream;
-  if (concurrent)
+  if (!ctx->shadeFork)
   {
-    if (!ctx->shadeFork)
+    RTC_CUDA(cudaEventCreateWithFlags(&ctx->shadeFork, cudaEventDisableTiming));
+    for (int k = 0; k < 6; ++k)
     {
-      RTC_CUDA(cudaEventCreateWithFlags(&ctx->shadeFork, cudaEventDisableTiming));
-      for (int k = 0; k < 6; ++k)
-      {
-        RTC_CUDA(cudaStreamCreateWithFlags(&ctx->shadeStreams[k], cudaStreamNonBlocking));
-        RTC_CUDA(cudaEventCreateWithFlags(&ctx->shadeJoin[k], cudaEventDisableTiming));
-      }
+      RTC_CUDA(cudaStreamCreateWithFlags(&ctx->shadeStreams[k], cudaStreamNonBlocking));
+      RTC_CUDA(cudaEventCreateWithFlags(&ctx->shadeJoin[k], cudaEventDisableTiming));
     }
-    RTC_CUDA(cudaEventRecord(ctx->shadeFork, ctx->stream));
-    int side = 0;
-    for (int k = 0; k < 7; ++k)
-    {
-      if (k == SHADE_BRDF_DIFFUSE) continue;
-      s[k] = ctx->shadeStreams[side++];
-      RTC_CUDA(cudaStreamWaitEvent(s[k], ctx->shadeFork, 0));
-    }
+  }
+  RTC_CUDA(cudaEventRecord(ctx->shadeFork, ctx->stream));
+  cudaStream_t s[7];
+  int side = 0;
+  for (int k = 0; k < 7; ++k)
+  {
+    if (k == SHADE_BRDF_DIFFUSE) { s[k] = ctx->stream; continue; }
+    s[k] = ctx->shadeStreams[side++];
+    RTC_CUDA(cudaStreamWaitEvent(s[k], ctx->shadeFork, 0));
   }
   launch_shade_class<SHADE_MISS>(ctx, s[SHADE_MISS], grid, a, sc, bins, binStride, binCounts, qOut, countOut, shadowQueue, shadowCount, tex, deferRR, primary);
   launch_shade_class<SHADE_BRDF_DIFFUSE>(ctx, s[SHADE_BRDF_DIFFUSE], grid, a, sc, bins, binStride, binCounts, qOut, countOut, shadowQueue, shadowCount, tex, deferRR, primary);
@@ -981,13 +946,10 @@ int launch_shade_classes(rtc_context* ctx, int grid, const WfArgs& a, const Scen
   launch_shade_class<SHADE_BSDF_GGX>(ctx, s[SHADE_BSDF_GGX], grid, a, sc, bins, binStride, binCounts, qOut, countOut, shadowQueue, shadowCount, tex, deferRR, primary);
   launch_shade_class<SHADE_OTHER>(ctx, s[SHADE_OTHER], grid, a, sc, bins, binStride, binCounts, qOut, countOut, shadowQueue, shadowCount, tex, deferRR, primary);
   RTC_CUDA(cudaGetLastError());      // a failed launch surfaces here, not in an unrelated later call
-  if (concurrent)
+  for (int k = 0; k < 6; ++k)
   {
-    for (int k = 0; k < 6; ++k)
-    {
-      RTC_CUDA(cudaEventRecord(ctx->shadeJoin[k], ctx->shadeStreams[k]));
-      RTC_CUDA(cudaStreamWaitEvent(ctx->stream, ctx->shadeJoin[k], 0));
-    }
+    RTC_CUDA(cudaEventRecord(ctx->shadeJoin[k], ctx->shadeStreams[k]));
+    RTC_CUDA(cudaStreamWaitEvent(ctx->stream, ctx->shadeJoin[k], 0));
   }
   return 0;
 }
@@ -1004,14 +966,6 @@ int ensure_cutout_buffers(rtc_context* ctx, uint64_t capacity)
   char* b = static_cast<char*>(base);
   wf.cutBase = base; wf.cutCapacity = capacity;
   wf.cutQueue[0] = (uint32_t*)b; wf.cutQueue[1] = (uint32_t*)(b + q); wf.cutCounters = (uint32_t*)(b + 2 * q);
-  return 0;
-}
-
-// reads one device counter back (host-synchronised rounds, RTC_CUTOUT_GRAPH=0)
-int read_counter(rtc_context* ctx, const uint32_t* d_counter, uint32_t* out)
-{
-  RTC_CUDA(cudaMemcpyAsync(out, d_counter, sizeof(uint32_t), cudaMemcpyDeviceToHost, ctx->stream));
-  RTC_CUDA(cudaStreamSynchronize(ctx->stream));
   return 0;
 }
 
@@ -1116,42 +1070,19 @@ int ensure_cutout_graph(rtc_context* ctx, const SceneRecord* scene, const WfArgs
   return 0;
 }
 
-bool cutout_graph_enabled()
-{
-  static const bool on = []() { const char* e = getenv("RTC_CUTOUT_GRAPH"); return !(e && atoi(e) == 0); }();      // RTC_CUTOUT_GRAPH=0: host-synchronised rounds
-  return on;
-}
-
 // After extend: play __anyhit__radiance_cutout on the closest candidates, re-trace the ignored ones, repeat until none is ignored.
 int resolve_radiance_candidates(rtc_context* ctx, const SceneRecord* scene, const WfArgs& a, int grid, const uint32_t* queue, const uint32_t* count)
 {
   const WavefrontBuffers& wf = ctx->wf;
-  if (cutout_graph_enabled())
-  {
-    if (int rc = ensure_cutout_graph(ctx, scene, a, grid)) return rc;
-    RTC_CUDA(cudaMemsetAsync(wf.cutCounters + 0, 0, sizeof(uint32_t), ctx->stream));
-    if (int rc = profile_begin(ctx, RTC_KERNEL_SHADE)) return rc;
-    k_cutout_radiance<<<grid, kBlock, 0, ctx->stream>>>(a, scene->desc, queue, count, wf.cutQueue[0], wf.cutCounters + 0);
-    if (int rc = profile_end(ctx)) return rc;
-    if (int rc = profile_begin(ctx, RTC_KERNEL_EXTEND)) return rc;       // the whole loop (re-traces dominate) as one span
-    RTC_CUDA(cudaGraphLaunch(static_cast<CutoutGraph*>(ctx->cutoutGraph)->radiance, ctx->stream));
-    ctx->kernelLaunches += 6;                                            // one body execution; further rounds are not counted
-    return profile_end(ctx);
-  }
-  for (int round = 0;; ++round)
-  {
-    const int o = round & 1;
-    RTC_CUDA(cudaMemsetAsync(wf.cutCounters + o, 0, sizeof(uint32_t), ctx->stream));
-    if (int rc = profile_begin(ctx, RTC_KERNEL_SHADE)) return rc;
-    k_cutout_radiance<<<grid, kBlock, 0, ctx->stream>>>(a, scene->desc, queue, count, wf.cutQueue[o], wf.cutCounters + o);
-    ctx->kernelLaunches++;
-    if (int rc = profile_end(ctx)) return rc;
-    uint32_t ignored = 0;
-    if (int rc = read_counter(ctx, wf.cutCounters + o, &ignored)) return rc;
-    if (ignored == 0) return 0;
-    if (int rc = launch_extend_after(ctx, &scene->desc, wf, wf.cutQueue[o], wf.cutCounters + o, wf.cutCounters + 2)) return rc;
-    queue = wf.cutQueue[o]; count = wf.cutCounters + o;
-  }
+  if (int rc = ensure_cutout_graph(ctx, scene, a, grid)) return rc;
+  RTC_CUDA(cudaMemsetAsync(wf.cutCounters + 0, 0, sizeof(uint32_t), ctx->stream));
+  if (int rc = profile_begin(ctx, RTC_KERNEL_SHADE)) return rc;
+  k_cutout_radiance<<<grid, kBlock, 0, ctx->stream>>>(a, scene->desc, queue, count, wf.cutQueue[0], wf.cutCounters + 0);
+  if (int rc = profile_end(ctx)) return rc;
+  if (int rc = profile_begin(ctx, RTC_KERNEL_EXTEND)) return rc;       // the whole loop (re-traces dominate) as one span
+  RTC_CUDA(cudaGraphLaunch(static_cast<CutoutGraph*>(ctx->cutoutGraph)->radiance, ctx->stream));
+  ctx->kernelLaunches += 6;                                            // one body execution; further rounds are not counted
+  return profile_end(ctx);
 }
 
 // Instead of connect: shadow rays as ordered closest-hit queries with __anyhit__shadow / __anyhit__shadow_cutout per candidate.
@@ -1162,32 +1093,15 @@ int resolve_shadow_candidates(rtc_context* ctx, const SceneRecord* scene, const 
   const uint32_t* queue = wf.shadowQueue; const uint32_t* count = shadowCount;
   k_set_cutout_next<<<1, 1, 0, ctx->stream>>>(cutout_next(wf), queueNext, countNext);
   if (int rc = launch_connect_closest(ctx, &scene->desc, wf, queue, count, wf.cutCounters + 2, false)) return rc;
-  if (cutout_graph_enabled())
-  {
-    if (int rc = ensure_cutout_graph(ctx, scene, a, grid)) return rc;
-    RTC_CUDA(cudaMemsetAsync(wf.cutCounters + 0, 0, sizeof(uint32_t), ctx->stream));
-    if (int rc = profile_begin(ctx, RTC_KERNEL_SHADE)) return rc;
-    k_cutout_shadow<<<grid, kBlock, 0, ctx->stream>>>(a, scene->desc, queue, count, wf.cutQueue[0], wf.cutCounters + 0, cutout_next(wf));
-    if (int rc = profile_end(ctx)) return rc;
-    if (int rc = profile_begin(ctx, RTC_KERNEL_CONNECT)) return rc;
-    RTC_CUDA(cudaGraphLaunch(static_cast<CutoutGraph*>(ctx->cutoutGraph)->shadow, ctx->stream));
-    ctx->kernelLaunches += 7;
-    return profile_end(ctx);
-  }
-  for (int round = 0;; ++round)
-  {
-    const int o = round & 1;
-    RTC_CUDA(cudaMemsetAsync(wf.cutCounters + o, 0, sizeof(uint32_t), ctx->stream));
-    if (int rc = profile_begin(ctx, RTC_KERNEL_SHADE)) return rc;
-    k_cutout_shadow<<<grid, kBlock, 0, ctx->stream>>>(a, scene->desc, queue, count, wf.cutQueue[o], wf.cutCounters + o, cutout_next(wf));
-    ctx->kernelLaunches++;
-    if (int rc = profile_end(ctx)) return rc;
-    uint32_t ignored = 0;
-    if (int rc = read_counter(ctx, wf.cutCounters + o, &ignored)) return rc;
-    if (ignored == 0) return 0;
-    if (int rc = launch_connect_closest(ctx, &scene->desc, wf, wf.cutQueue[o], wf.cutCounters + o, wf.cutCounters + 2, true)) return rc;
-    queue = wf.cutQueue[o]; count = wf.cutCounters + o;
-  }
+  if (int rc = ensure_cutout_graph(ctx, scene, a, grid)) return rc;
+  RTC_CUDA(cudaMemsetAsync(wf.cutCounters + 0, 0, sizeof(uint32_t), ctx->stream));
+  if (int rc = profile_begin(ctx, RTC_KERNEL_SHADE)) return rc;
+  k_cutout_shadow<<<grid, kBlock, 0, ctx->stream>>>(a, scene->desc, queue, count, wf.cutQueue[0], wf.cutCounters + 0, cutout_next(wf));
+  if (int rc = profile_end(ctx)) return rc;
+  if (int rc = profile_begin(ctx, RTC_KERNEL_CONNECT)) return rc;
+  RTC_CUDA(cudaGraphLaunch(static_cast<CutoutGraph*>(ctx->cutoutGraph)->shadow, ctx->stream));
+  ctx->kernelLaunches += 7;
+  return profile_end(ctx);
 }
 
 } // namespace
@@ -1245,7 +1159,8 @@ int launch_wavefront(rtc_context* ctx, const rt_SystemData& sys, uint32_t w, uin
     perBatch = (perBatch + 1) / 2;
   }
   // Material textures (off in every BASELINE configuration, like the reference's GUI default): `cutout` switches to the ordered
-  // any-hit processing, which synchronises with the host between rounds; `tex` selects the texture-aware shade kernels.
+  // any-hit processing, whose rounds repeat on the device without a host synchronisation; `tex` selects the texture-aware
+  // shade kernels.
   const bool cutout = scene->numCutout > 0;
   const bool tex = cutout || scene->albedoTextures;
   if (cutout) { if (int rc = ensure_cutout_buffers(ctx, pixels * perBatch)) return rc; }
@@ -1257,8 +1172,8 @@ int launch_wavefront(rtc_context* ctx, const rt_SystemData& sys, uint32_t w, uin
     WfArgs a;
     a.wf = ctx->wf; a.sys = sys; a.launchWidth = w; a.launchHeight = h; a.raygen = raygen; a.miss = miss;
     a.iterFirst = iterFirst + done; a.iterCount = batch; a.accumFirst = accumFirst + done; a.numPaths = (uint32_t)(pixels * (uint64_t)batch);
-    // schedule tuner: the lane-owned driver on scenes without cutout materials, timed launches only
-    const int tuneSlot = rtc_tuner::begin(ctx, a.numPaths, !countWork && !cutout && ctx->traceDriver == RTC_DRIVER_LANE && !ctx->primaryPackets, preload_capped_kernels);
+    // schedule tuner: scenes without cutout materials, timed launches only
+    const int tuneSlot = rtc_tuner::begin(ctx, a.numPaths, !countWork && !cutout, preload_capped_kernels);
     uint32_t* cnt = ctx->wf.counters;
     RTC_CUDA(cudaMemsetAsync(cnt, 0, 4 * kNumCounters, ctx->stream));
     // Fused primary path (scenes without material textures): no generate pass.  The depth-0 extend computes its rays from the
@@ -1279,29 +1194,11 @@ int launch_wavefront(rtc_context* ctx, const rt_SystemData& sys, uint32_t w, uin
       {
         if (int rc = profile_begin(ctx, RTC_KERNEL_EXTEND)) return rc;
         ExtendPrimary policy = { a };
-        if (ctx->primaryPackets && !countWork)
-        {
-          // the counting pass keeps the per-ray kernel: its counters are the per-ray work the scalar oracle reproduces
-          k_extend_primary_packet<<<ctx->numSMs * RTC_PACKET_BLOCKS, kPrimaryBlock, 0, ctx->stream>>>(scene->desc, policy, a.numPaths, cnt + 128);
-        }
-        else if (ctx->traceDriver == RTC_DRIVER_POOL)
-        {
-          const int gridTrace = ctx->numSMs * RTC_POOL_BLOCKS;
-          uint2* overflow = nullptr;
-          if (int rc = ensure_pool_scratch(ctx, (size_t)gridTrace * (kPrimaryBlock / 32), &overflow)) return rc;
-          RTC_CUDA(cudaFuncSetAttribute(k_extend_primary_pool<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kPrimaryPoolSmem));
-          RTC_CUDA(cudaFuncSetAttribute(k_extend_primary_pool<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kPrimaryPoolSmem));
-          if (countWork) k_extend_primary_pool<true><<<gridTrace, kPrimaryBlock, kPrimaryPoolSmem, ctx->stream>>>(scene->desc, policy, a.numPaths, cnt + 128, ctx->d_launchCounts, overflow);
-          else           k_extend_primary_pool<false><<<gridTrace, kPrimaryBlock, kPrimaryPoolSmem, ctx->stream>>>(scene->desc, policy, a.numPaths, cnt + 128, nullptr, overflow);
-        }
-        else
-        {
-          const int gridTrace = ctx->numSMs * RTC_TRACE_MIN_BLOCKS;
-          if (countWork) k_extend_primary<true><<<gridTrace, kPrimaryBlock, 0, ctx->stream>>>(scene->desc, policy, a.numPaths, cnt + 128, ctx->d_launchCounts);
-          else if (ctx->traceSchedule == RTC_SCHEDULE_ONE_TRI) k_extend_primary<false, 1><<<gridTrace, kPrimaryBlock, 0, ctx->stream>>>(scene->desc, policy, a.numPaths, cnt + 128, nullptr);
-          else if (ctx->traceSchedule == RTC_SCHEDULE_TWO_TRI) k_extend_primary<false, 2><<<gridTrace, kPrimaryBlock, 0, ctx->stream>>>(scene->desc, policy, a.numPaths, cnt + 128, nullptr);
-          else           k_extend_primary<false><<<gridTrace, kPrimaryBlock, 0, ctx->stream>>>(scene->desc, policy, a.numPaths, cnt + 128, nullptr);
-        }
+        const int gridTrace = ctx->numSMs * RTC_TRACE_MIN_BLOCKS;
+        if (countWork) k_extend_primary<true><<<gridTrace, kPrimaryBlock, 0, ctx->stream>>>(scene->desc, policy, a.numPaths, cnt + 128, ctx->d_launchCounts);
+        else if (ctx->traceSchedule == RTC_SCHEDULE_ONE_TRI) k_extend_primary<false, 1><<<gridTrace, kPrimaryBlock, 0, ctx->stream>>>(scene->desc, policy, a.numPaths, cnt + 128, nullptr);
+        else if (ctx->traceSchedule == RTC_SCHEDULE_TWO_TRI) k_extend_primary<false, 2><<<gridTrace, kPrimaryBlock, 0, ctx->stream>>>(scene->desc, policy, a.numPaths, cnt + 128, nullptr);
+        else           k_extend_primary<false><<<gridTrace, kPrimaryBlock, 0, ctx->stream>>>(scene->desc, policy, a.numPaths, cnt + 128, nullptr);
         ctx->kernelLaunches++;
         RTC_CUDA(cudaGetLastError());
         if (int rc = profile_end(ctx)) return rc;

@@ -1,18 +1,10 @@
 // kernels_trace.cu -- the traversal kernels: ray queries (rtc_trace_*), and the wavefront integrator's
 // extend (closest hit of the radiance-ray queue) and connect (any hit of the shadow-ray queue).
-// All of them are persistent-warp kernels, one CTA of 128 threads per resident slot, rays handed out through a
-// device-side cursor, over one of two drivers chosen per launch (rtc_context::traceDriver): trace_stream() (trace.cuh,
-// one ray per lane, the default) or rtpool::trace_pool() (trace_pool.cuh, per-warp ray pool, RTC_TRACE_DRIVER=pool).
+// All of them are persistent-warp kernels over trace_stream() (trace.cuh, one ray per lane): one CTA of 128 threads per
+// resident slot, rays handed out through a device-side cursor.
 // Built for sm_100a with FMA contraction ON: only the box tests may contract; the intersector in
 // trace.cuh pins its own rounding with intrinsics.
-#include "trace_pool.cuh"
-
-#ifndef RTC_TRACE_MIN_BLOCKS
-#define RTC_TRACE_MIN_BLOCKS 8      // one ray per lane: resident CTAs per SM the kernels are compiled for (register budget) and launched with
-#endif
-#ifndef RTC_POOL_BLOCKS
-#define RTC_POOL_BLOCKS 4           // ray pool: resident CTAs (4 warps each) per SM; bounded by shared memory (rtpool::warp_bytes() per warp)
-#endif
+#include "trace.cuh"
 
 namespace {
 
@@ -134,19 +126,6 @@ struct ConnectClosest
 
 // ---- kernels ---------------------------------------------------------------------------------------------------------
 
-// Both drivers are compiled; rtc_context::traceDriver picks one per launch (environment RTC_TRACE_DRIVER=lane|pool, default lane).
-template <bool ANY, bool COUNT, class Policy, bool SKIP = false>
-__global__ void __launch_bounds__(kTraceBlock, RTC_POOL_BLOCKS)
-k_trace_pool(const SceneDesc sc, const Policy policy, uint32_t n, const uint32_t* __restrict__ nPtr, uint32_t* __restrict__ cursor,
-             unsigned long long* __restrict__ counts, uint2* __restrict__ overflow)
-{
-  extern __shared__ uint32_t poolWords[];
-  const uint32_t count = nPtr ? *nPtr : n;      // the wavefront keeps its queue lengths on the device
-  const uint32_t warp = threadIdx.x >> 5;
-  const size_t warpGlobal = (size_t)blockIdx.x * (kTraceBlock / 32) + warp;
-  rtpool::trace_pool<ANY, COUNT, SKIP>(sc, count, cursor, policy, poolWords + warp * rtpool::warp_words(ANY, SKIP), overflow + warpGlobal * rtpool::kOverflowPerWarp, counts);
-}
-
 // TRICAP: the capped schedules of the triangle tests (trace.cuh Traversal::step); 1 and 2 are instantiated for the timed kernels only.
 template <bool ANY, bool COUNT, class Policy, bool SKIP = false, int TRICAP = 0>
 __global__ void __launch_bounds__(kTraceBlock, SKIP ? 4 : RTC_TRACE_MIN_BLOCKS)
@@ -161,17 +140,7 @@ k_trace(const SceneDesc sc, const Policy policy, uint32_t n, const uint32_t* __r
 template <bool ANY, bool COUNT, class Policy, bool SKIP>
 int launch_k_trace(rtc_context* ctx, const SceneDesc* scene, const Policy& p, uint32_t n, const uint32_t* nPtr, uint32_t* cursor, unsigned long long* counts)
 {
-  if (ctx->traceDriver == RTC_DRIVER_POOL)
-  {
-    auto kernel = k_trace_pool<ANY, COUNT, Policy, SKIP>;
-    const int grid = ctx->numSMs * RTC_POOL_BLOCKS;
-    const size_t smem = (size_t)(kTraceBlock / 32) * rtpool::warp_bytes(ANY, SKIP);
-    uint2* overflow = nullptr;
-    if (int rc = ensure_pool_scratch(ctx, (size_t)grid * (kTraceBlock / 32), &overflow)) return rc;
-    RTC_CUDA(cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    kernel<<<grid, kTraceBlock, smem, ctx->stream>>>(*scene, p, n, nPtr, cursor, counts, overflow);
-  }
-  else if (!COUNT && !SKIP && ctx->traceSchedule == RTC_SCHEDULE_ONE_TRI)
+  if (!COUNT && !SKIP && ctx->traceSchedule == RTC_SCHEDULE_ONE_TRI)
   {
     // the counting kernels and the ordered any-hit re-traces keep the one schedule: their per-ray results do not depend on it
     k_trace<ANY, false, Policy, false, 1><<<ctx->numSMs * RTC_TRACE_MIN_BLOCKS, kTraceBlock, 0, ctx->stream>>>(*scene, p, n, nPtr, cursor, counts);
@@ -190,20 +159,6 @@ int launch_k_trace(rtc_context* ctx, const SceneDesc* scene, const Policy& p, ui
 }
 
 } // namespace
-
-// Global scratch of the ray pool: the part of every slot's traversal stack that does not fit in shared memory.
-int ensure_pool_scratch(rtc_context* ctx, size_t warps, uint2** out)
-{
-  const size_t need = warps * rtpool::kOverflowPerWarp * sizeof(uint2);
-  if (ctx->poolScratchBytes < need)
-  {
-    if (ctx->d_poolScratch) { RTC_CUDA(cudaStreamSynchronize(ctx->stream)); RTC_CUDA(cudaFree(ctx->d_poolScratch)); ctx->d_poolScratch = nullptr; ctx->poolScratchBytes = 0; }
-    RTC_CUDA(cudaMalloc(&ctx->d_poolScratch, need));
-    ctx->poolScratchBytes = need;
-  }
-  *out = static_cast<uint2*>(ctx->d_poolScratch);
-  return 0;
-}
 
 // With lazy module loading a kernel is loaded at its first launch; the schedule tuner must not time that.
 void preload_capped_trace_kernels()

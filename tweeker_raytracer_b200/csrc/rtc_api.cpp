@@ -96,10 +96,6 @@ static int context_init(rtc_context* ctx, int deviceOrdinal)
   cudaDeviceProp prop;
   RTC_CUDA(cudaGetDeviceProperties(&prop, deviceOrdinal));
   ctx->numSMs = prop.multiProcessorCount;
-  // traversal driver: one ray per lane (default) or the per-warp ray pool; both are compiled, RTC_TRACE_DRIVER=lane|pool picks
-  ctx->traceDriver = RTC_DRIVER_LANE;
-  if (const char* e = getenv("RTC_PRIMARY_PACKETS")) ctx->primaryPackets = atoi(e) != 0;
-  if (const char* e = getenv("RTC_TRACE_DRIVER")) ctx->traceDriver = (e[0] == 'p' || e[0] == '1') ? RTC_DRIVER_POOL : RTC_DRIVER_LANE;
   // schedule of the lane-owned driver's triangle tests: measured per context (auto) unless RTC_TRACE_SCHEDULE=group|onetri|twotri fixes it
   if (const char* e = getenv("RTC_TRACE_SCHEDULE"))
   {
@@ -166,7 +162,6 @@ int rtc_context_destroy(rtc_context* ctx)
   cudaFree(ctx->d_stats);
   cudaFree(ctx->d_launchCounts);
   cudaFree(ctx->d_cursor);
-  cudaFree(ctx->d_poolScratch);
   for (rtc_context::ProfileSpan& sp : ctx->spans) { cudaEventDestroy(sp.a); cudaEventDestroy(sp.b); }
   for (cudaEvent_t e : ctx->eventPool) cudaEventDestroy(e);
   for (cudaEvent_t e : { ctx->evA, ctx->evB, ctx->evTimerA, ctx->evTimerB }) if (e) cudaEventDestroy(e);
@@ -636,18 +631,6 @@ int rtc_launch_counts_get(rtc_context* ctx, rtc_trace_counts out[2])
     const unsigned long long* c = h + kTraceCountWords * k;
     out[k].nodes = c[0]; out[k].tris = c[1]; out[k].instances = c[2]; out[k].rays = c[3];
   }
-  return 0;
-}
-
-int rtc_launch_pass_stats_get(rtc_context* ctx, rtc_pass_stats out[2])
-{
-  if (!out) RTC_FAIL("out is null");
-  RTC_CUDA(cudaSetDevice(ctx->device));
-  unsigned long long h[2 * kTraceCountWords];
-  RTC_CUDA(cudaMemcpyAsync(h, ctx->d_launchCounts, sizeof(h), cudaMemcpyDeviceToHost, ctx->stream));
-  RTC_CUDA(cudaStreamSynchronize(ctx->stream));
-  for (int k = 0; k < 2; ++k)
-    for (int j = 0; j < 4; ++j) { out[k].passes[j] = h[kTraceCountWords * k + 4 + j]; out[k].lanes[j] = h[kTraceCountWords * k + 8 + j]; }
   return 0;
 }
 

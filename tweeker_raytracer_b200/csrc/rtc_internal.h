@@ -182,19 +182,13 @@ struct rtc_context
   cudaEvent_t  shadeFork = nullptr, shadeJoin[6] = {};
   unsigned long long* d_launchCounts = nullptr;   // 3 x kTraceCountWords: extend, connect, rtc_trace_count
   uint32_t* d_cursor = nullptr;                   // ray cursor of the query kernels (rtc_trace_*)
-  bool   primaryPackets = false;                  // primary rays by packet traversal (trace_packet.cuh): measured slower, RTC_PRIMARY_PACKETS=1 turns it on
-  int    traceDriver = 0;                         // RTC_DRIVER_LANE or RTC_DRIVER_POOL: which traversal driver the launches use
   int    traceSchedule = 0;                       // RTC_SCHEDULE_*: how the lane-owned driver times its triangle tests (what the NEXT launch uses)
   ScheduleTuner tuner;                            // picks traceSchedule by timing one batch with each (kernels_shade.cu, "schedule tuner")
   void*  cutoutGraph = nullptr;                   // CutoutGraph (kernels_shade.cu): the device-side loop of the ordered any-hit rounds
-  void*  d_poolScratch = nullptr;                 // global part of the ray pool's traversal stacks (trace_pool.cuh), grown on demand
-  size_t poolScratchBytes = 0;
 };
 
-enum { RTC_DRIVER_LANE = 0, RTC_DRIVER_POOL = 1 };     // trace.cuh trace_stream / trace_pool.cuh trace_pool
-
-// work counters of one traversal kernel: {nodes, tris, insts, rays}, then the ray pool's passes and occupied lanes per phase (N, T, I, F)
-constexpr int kTraceCountWords = 12;
+// work counters of one traversal kernel: {nodes, tris, insts, rays}
+constexpr int kTraceCountWords = 4;
 
 // RAII-less helpers used by the launchers: bracket one kernel launch with an event pair when profiling is on
 int profile_begin(rtc_context* ctx, int cls);
@@ -233,7 +227,6 @@ int launch_composite(rtc_context* ctx, const rt_CompositorData& args);
 int launch_tonemap(rtc_context* ctx, const rt_TonemapperParams& p, const float4* rgba, uint8_t* rgb, uint64_t n);
 int launch_probe_math(rtc_context* ctx, int fn, const float* x, const float* y, float* out, uint32_t n);   // device pointers
 int ensure_wavefront(rtc_context* ctx, uint64_t capacity, bool* outOfMemory = nullptr);
-int ensure_pool_scratch(rtc_context* ctx, size_t warps, uint2** out);
 void release_cutout_graph(rtc_context* ctx);
 int read_stack_overflows(rtc_context* ctx, uint64_t* out);
 // schedule tuner (kernels_shade.cu); tuner_finish blocks for the last timed batch when a decision is pending

@@ -30,6 +30,9 @@
 #ifndef RTC_FETCH_THRESHOLD
 #define RTC_FETCH_THRESHOLD 12    // refill a warp when at least this many lanes have finished their ray (8: -1.3 %, 16: same; re-swept in round 2)
 #endif
+#ifndef RTC_TRACE_MIN_BLOCKS
+#define RTC_TRACE_MIN_BLOCKS 8    // resident CTAs per SM the persistent traversal kernels are compiled for (register budget) and launched with
+#endif
 
 struct TraceHit
 {
@@ -496,7 +499,7 @@ struct Traversal
 
 // Persistent-warp driver: every lane owns one ray at a time; lanes whose ray has finished take the next ray index from a
 // global cursor (one atomicAdd per warp and refill), so short rays do not leave their lanes idle while the longest ray of
-// the warp finishes.  Policy (stateless, shared with trace_pool.cuh) supplies load(i, org, dir, tag) -> bool (false: skip this
+// the warp finishes.  Policy (stateless) supplies load(i, org, dir, tag) -> bool (false: skip this
 // index; tag = the policy's per-ray word, e.g. the path id), store(tag, hit) and, for SKIP kernels, skip_key(tag, t, inst, prim).
 template <bool ANY, bool COUNT, int BLOCK, bool SKIP, int TRICAP = RTC_ONE_TRI_PER_STEP, class Policy>
 __device__ __forceinline__ void trace_stream(const SceneDesc& sc, uint32_t n, uint32_t* __restrict__ cursor, Policy& policy, uint2* smem,
