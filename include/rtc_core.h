@@ -125,6 +125,24 @@ int rtc_gas_build(rtc_context* ctx, uint64_t attributes, uint32_t strideBytes, u
                   uint64_t indices, uint32_t numTris, uint32_t buildFlags, uint32_t* gas);
 /* Builds the instance level, the per-instance tables and returns SystemData::topObject. */
 int rtc_ias_build(rtc_context* ctx, const rtc_instance_desc* instances, uint32_t numInstances, uint64_t* topObject);
+/*
+ * In-place updates (optixAccelBuild with OPTIX_BUILD_OPERATION_UPDATE).  Both are asynchronous on the context stream and do not
+ * synchronise the host, except for a one-time allocation of refit scratch on a structure's first refit: work enqueued before
+ * sees the old structure, work enqueued after sees the new one.  Topology is never changed -- vertex and triangle counts,
+ * indices, instance count, the GAS of an instance and materials stay as built; changing them is a rebuild.  Node topology and
+ * leaf order stay as built, so traversal cost grows with the size of the deformation (DESIGN.md section 3, "Refit").
+ *
+ * rtc_gas_refit: refit a GAS after its vertex POSITIONS changed; numVerts, numTris, indices and stride must be the build's.
+ *   attributes: the new vertex records (same stride as the build), or 0 = the build's buffer, updated in place by the caller.
+ *   Only boxes and triangle records are rewritten.  Every scene that instances this GAS must then be brought up to date with
+ *   rtc_ias_update before it is traced: until then rtc_launch, rtc_launch_ex and rtc_trace_* on such a scene fail.
+ * rtc_ias_update: transforms of instances first .. first+count-1 are replaced (count x 12 floats, object->world, row-major; may
+ *   be null when count == 0), world->object matrices and shading tables follow, the bounds of every instance whose transform
+ *   changed or whose GAS was refitted since the last build / update are recomputed, and the instance level is refitted.
+ *   `transforms` may be reused on return.
+ */
+int rtc_gas_refit(rtc_context* ctx, uint32_t gas, uint64_t attributes);
+int rtc_ias_update(rtc_context* ctx, uint64_t topObject, uint32_t first, uint32_t count, const float* transforms);
 int rtc_scene_info_get(rtc_context* ctx, uint64_t topObject, rtc_scene_info* info);
 /* Frees one scene (the instance level and its tables; GAS stay alive until rtc_gas_destroy / context destroy). */
 int rtc_scene_destroy(rtc_context* ctx, uint64_t topObject);
@@ -180,6 +198,12 @@ typedef struct rtc_host_accel rtc_host_accel;
 int  rtc_host_gas_build(const void* attributes, uint32_t strideBytes, uint32_t numVerts, const uint32_t* indices, uint32_t numTris,
                         rtc_host_accel** out);
 int  rtc_host_ias_build(const float* transforms, const rtc_host_accel* const* geometry, uint32_t numInstances, rtc_host_accel** out);
+/* Host-only twin of rtc_gas_refit / rtc_ias_update, on what rtc_host_gas_build / rtc_host_ias_build returned: the same node
+ * routine (csrc/bvh_rules.h), visiting the nodes in descending index order (children always sit above their parent).
+ * rtc_host_gas_refit: attributes = the new vertex records, strideBytes = the build's.
+ * rtc_host_ias_refit: every instance's transform and geometry (numInstances = the build's; geometry[i] may have been refitted). */
+int  rtc_host_gas_refit(rtc_host_accel* accel, const void* attributes, uint32_t strideBytes);
+int  rtc_host_ias_refit(rtc_host_accel* accel, const float* transforms, const rtc_host_accel* const* geometry, uint32_t numInstances);
 int  rtc_host_accel_info(const rtc_host_accel* accel, uint64_t* numNodes, uint64_t* numPrims, float bounds[6]);
 int  rtc_host_accel_export(const rtc_host_accel* accel, void* nodes, uint32_t* primOrder, float* tris, float* worldToObject);
 void rtc_host_accel_destroy(rtc_host_accel* accel);

@@ -1,0 +1,230 @@
+#!/usr/bin/env python
+"""Refit against rebuild on one GPU; prints one JSON line per measurement, the first one naming the card and its power limit.
+
+  python tools/refit_bench.py [--sizes 1M,10M,100M] [--rays 8M] [--repeats 5]
+
+  * device-LBVH soups of bench.py's config 3 (centres uniform in the unit cube, edge n^(-1/3)): rtc_gas_build ms against
+    rtc_gas_refit ms, and incoherent closest-hit Mrays/s after a smooth per-vertex displacement of 0, 0.5 and 2 mean edge lengths,
+    refitted against rebuilt (the hits of the two are checked to be equal in the same run);
+  * the 10 001-instance scene (tools/make_instances_scene.py): rtc_ias_build ms against rtc_ias_update ms with every instance and
+    with 1 % of them moved, and incoherent closest-hit Mrays/s through the scene after 1, 10 and 100 animation steps of small
+    rotations, refitted against rebuilt.
+Builds are timed on the host clock (they end in a synchronisation); refits, updates and traces between CUDA events on the
+context stream, each the median of `repeats` runs after one warm-up.
+"""
+import argparse
+import json
+import os
+import subprocess
+import sys
+import tempfile
+import time
+
+import numpy as np
+
+ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
+sys.path.insert(0, ROOT)
+sys.path.insert(0, os.path.join(ROOT, "tools"))
+import bench  # noqa: E402
+import helpers as H  # noqa: E402
+import make_instances_scene  # noqa: E402
+from tweeker_raytracer_b200 import core, host  # noqa: E402
+
+
+def emit(**kw):
+    print(json.dumps(kw), flush=True)
+
+
+def card():
+    try:
+        out = subprocess.run(["nvidia-smi", "-i", "0", "--query-gpu=name,power.limit,clocks.max.sm", "--format=csv,noheader"],
+                             capture_output=True, text=True, timeout=60).stdout.strip()
+    except (OSError, subprocess.SubprocessError) as e:
+        out = "nvidia-smi unavailable: %s" % e
+    return out
+
+
+def timed(ctx, fn, repeats):
+    fn()
+    ms = []
+    for _ in range(repeats):
+        ctx.timer_start()
+        fn()
+        ms.append(ctx.timer_stop())
+    return float(np.median(ms))
+
+
+def wall(ctx, fn, repeats):
+    ms = []
+    for _ in range(repeats):
+        ctx.synchronize()
+        t0 = time.perf_counter()
+        fn()
+        ctx.synchronize()
+        ms.append((time.perf_counter() - t0) * 1e3)
+    return float(np.median(ms))
+
+
+def displace(verts, amount, edge, seed=7):
+    """Smooth per-vertex displacement of `amount` mean edge lengths (a sine field over the position), float32, in chunks."""
+    rng = np.random.default_rng(seed)
+    k = rng.normal(size=(3, 3)).astype(np.float32) * np.float32(6.0)
+    phase = rng.uniform(0, 2 * np.pi, size=3).astype(np.float32)
+    out = np.empty_like(verts)
+    chunk = 1 << 24
+    for a in range(0, len(verts), chunk):
+        v = verts[a:a + chunk]
+        out[a:a + chunk] = v + np.float32(amount * edge) * np.sin(v @ k + phase)
+    return out
+
+
+def mrays(ctx, top, d_rays, nrays, d_hits, repeats):
+    ms = timed(ctx, lambda: ctx.trace_closest(top, d_rays, nrays, d_hits), repeats)
+    return nrays / ms / 1e3
+
+
+def soup_runs(ctx, n, nrays, repeats):
+    verts = bench.soup_numpy(n)
+    edge = float(n) ** (-1.0 / 3.0)
+    idx = np.arange(3 * n, dtype=np.uint32)
+    d_v, d_i = ctx.malloc(verts.nbytes), ctx.malloc(idx.nbytes)
+    ctx.upload(d_v, verts)
+    ctx.upload(d_i, idx)
+    del idx
+    inst = np.zeros(1, dtype=core.INSTANCE_DTYPE)
+    inst[0]["transform"] = [1, 0, 0, 0, 0, 1, 0, 0, 0, 0, 1, 0]
+    def build():
+        return ctx.gas_build(d_v, 12, 3 * n, d_i, n, core.BUILD_GPU_LBVH)
+
+    build_ms = wall(ctx, lambda: ctx.gas_destroy(build()), repeats + 1)
+    gas = build()
+    inst[0]["gas"] = gas
+    top = ctx.ias_build(inst)
+    refit_ms = timed(ctx, lambda: ctx.gas_refit(gas), repeats)
+    update_ms = timed(ctx, lambda: ctx.ias_update(top, np.zeros((0, 12), dtype=np.float32)), repeats)
+    emit(what="gas_build_vs_refit", triangles=n, builder="gpu_lbvh", build_ms=build_ms, refit_ms=refit_ms, ias_update_after_refit_ms=update_ms,
+         speedup=build_ms / refit_ms)
+    rays = bench.rays_numpy(nrays, "incoh", "closest")
+    d_rays, d_hits, d_hits2 = ctx.malloc(rays.nbytes), ctx.malloc(20 * nrays), ctx.malloc(20 * nrays)
+    ctx.upload(d_rays, rays)
+    del rays
+    for amount in (0.0, 0.5, 2.0):
+        ctx.upload(d_v, displace(verts, amount, edge) if amount else verts)
+        ctx.gas_refit(gas)
+        ctx.ias_update(top, np.zeros((0, 12), dtype=np.float32))
+        refit_rate = mrays(ctx, top, d_rays, nrays, d_hits, repeats)
+        fresh = build()
+        inst[0]["gas"] = fresh
+        fresh_top = ctx.ias_build(inst)
+        rebuilt_rate = mrays(ctx, fresh_top, d_rays, nrays, d_hits2, repeats)
+        a = ctx.download(d_hits, np.uint8, 20 * nrays)
+        b = ctx.download(d_hits2, np.uint8, 20 * nrays)
+        emit(what="soup_trace_after_displacement", triangles=n, displacement_edges=amount, rays=nrays, refitted_mrays=refit_rate,
+             rebuilt_mrays=rebuilt_rate, refitted_over_rebuilt=refit_rate / rebuilt_rate, hits_equal=bool(np.array_equal(a, b)))
+        ctx.scene_destroy(fresh_top)
+        ctx.gas_destroy(fresh)
+    ctx.scene_destroy(top)
+    ctx.gas_destroy(gas)
+    for p in (d_v, d_i, d_rays, d_hits, d_hits2):
+        ctx.free(p)
+
+
+def rotation(angle, axis):
+    c, s = np.cos(angle), np.sin(angle)
+    r = np.eye(3)
+    i, j = [(1, 2), (0, 2), (0, 1)][axis]
+    r[i, i], r[i, j], r[j, i], r[j, j] = c, -s, s, c
+    return r
+
+
+def instance_runs(ctx, nrays, repeats):
+    with tempfile.TemporaryDirectory() as tmp:
+        scene = os.path.join(tmp, "instances.txt")
+        make_instances_scene.write_scene(scene, count=10000)
+        app = host.App(H.write_system(tmp, "rtigo3_instances", resolution="64 64", samplesSqrt=1), scene, host_only=True)
+        try:
+            geos = [app.geometry(g) for g in range(app.info.numGeometries)]
+            insts = [app.instance(i)[:2] for i in range(app.info.numInstances)]
+        finally:
+            app.close()
+    keep, handles = [], []
+    for a, ix in geos:
+        d_a, d_i = ctx.to_device(a), ctx.to_device(ix)
+        keep += [d_a, d_i]
+        handles.append(ctx.gas_build(d_a, a.dtype.itemsize, len(a), d_i, len(ix), core.BUILD_HOST_SAH))
+    xf0 = np.asarray([t for t, _ in insts], dtype=np.float32).reshape(-1, 12)
+    n = len(insts)
+
+    def descs(xf):
+        out = np.zeros(n, dtype=core.INSTANCE_DTYPE)
+        out["transform"] = xf
+        out["instanceId"] = np.arange(n)
+        out["gas"] = [handles[g] for _, g in insts]
+        out["lightIndex"] = -1
+        return out
+
+    tops = []
+    build_ms = wall(ctx, lambda: tops.append(ctx.ias_build(descs(xf0))), repeats)
+    for t in tops[1:]:
+        ctx.scene_destroy(t)
+    top = tops[0]
+
+    def step(xf, k):
+        """one animation step: every instance turns by a small angle about its own centre"""
+        out = xf.reshape(n, 3, 4).astype(np.float64)
+        out[:, :, :3] = out[:, :, :3] @ rotation(0.02 * (1 + k % 3), k % 3)
+        return out.astype(np.float32).reshape(n, 12)
+
+    moved = step(xf0, 0)
+    all_ms = timed(ctx, lambda: ctx.ias_update(top, moved), repeats)
+    few = max(1, n // 100)
+    few_ms = timed(ctx, lambda: ctx.ias_update(top, moved[:few]), repeats)
+    emit(what="ias_build_vs_update", instances=n, build_ms=build_ms, update_all_ms=all_ms, update_1pct_ms=few_ms,
+         speedup_all=build_ms / all_ms, speedup_1pct=build_ms / few_ms)
+
+    lo, hi = xf0[:, [3, 7, 11]].min(axis=0) - 1.0, xf0[:, [3, 7, 11]].max(axis=0) + 1.0
+    rays = bench.rays_numpy(nrays, "incoh", "closest")
+    for c, k in zip("xyz", range(3)):
+        rays["o" + c] = lo[k] + rays["o" + c] * (hi[k] - lo[k])
+    d_rays, d_hits, d_hits2 = ctx.to_device(rays), ctx.malloc(20 * nrays), ctx.malloc(20 * nrays)
+    xf = xf0.copy()
+    ctx.ias_update(top, xf)
+    done = 0
+    for steps in (1, 10, 100):
+        while done < steps:
+            xf = step(xf, done)
+            ctx.ias_update(top, xf)
+            done += 1
+        refit_rate = mrays(ctx, top, d_rays, nrays, d_hits, repeats)
+        fresh = ctx.ias_build(descs(xf))
+        rebuilt_rate = mrays(ctx, fresh, d_rays, nrays, d_hits2, repeats)
+        a = ctx.download(d_hits, np.uint8, 20 * nrays)
+        b = ctx.download(d_hits2, np.uint8, 20 * nrays)
+        emit(what="instances_trace_after_steps", instances=n, steps=steps, rays=nrays, refitted_mrays=refit_rate, rebuilt_mrays=rebuilt_rate,
+             refitted_over_rebuilt=refit_rate / rebuilt_rate, hits_equal=bool(np.array_equal(a, b)))
+        ctx.scene_destroy(fresh)
+    for p in keep + [d_rays, d_hits, d_hits2]:
+        ctx.free(p)
+
+
+def main():
+    ap = argparse.ArgumentParser(description=__doc__.split("\n")[0])
+    ap.add_argument("--sizes", default="1M,10M,100M")
+    ap.add_argument("--rays", default="8M")
+    ap.add_argument("--repeats", type=int, default=5)
+    ap.add_argument("--no-instances", action="store_true")
+    args = ap.parse_args()
+    scale = {"K": 10 ** 3, "M": 10 ** 6}
+    count = lambda s: int(float(s[:-1]) * scale[s[-1]]) if s[-1] in scale else int(s)    # noqa: E731
+    if core.device_count() < 1:
+        raise SystemExit("refit_bench needs a CUDA device: " + core.lib().rtc_last_error().decode())
+    emit(what="card", nvidia_smi=card(), rtc_version=core.lib().rtc_version())
+    with core.Context(0) as ctx:
+        for s in args.sizes.split(","):
+            soup_runs(ctx, count(s), count(args.rays), args.repeats)
+        if not args.no_instances:
+            instance_runs(ctx, count(args.rays), args.repeats)
+
+
+if __name__ == "__main__":
+    main()

@@ -33,6 +33,7 @@ SYMBOLS = [
     "rtc_probe_math",
     "rtc_host_gas_build", "rtc_host_ias_build", "rtc_host_accel_info", "rtc_host_accel_export", "rtc_host_accel_destroy",
     "rtc_trace_schedule_get", "rtc_trace_schedule_set",
+    "rtc_gas_refit", "rtc_ias_update", "rtc_host_gas_refit", "rtc_host_ias_refit",
 ]
 
 MATH_FUNCTIONS = ["sin", "cos", "atan", "atan2", "acos", "exp", "log", "pow", "div", "sqrt", "muladd"]     # enum rtc_math_fn
@@ -99,6 +100,8 @@ def lib():
         L.rtc_gas_build.argtypes = [C.c_void_p, C.c_uint64, C.c_uint32, C.c_uint32, C.c_uint64, C.c_uint32, C.c_uint32, C.POINTER(C.c_uint32)]
         L.rtc_gas_destroy.argtypes = [C.c_void_p, C.c_uint32]
         L.rtc_ias_build.argtypes = [C.c_void_p, C.c_void_p, C.c_uint32, C.POINTER(C.c_uint64)]
+        L.rtc_gas_refit.argtypes = [C.c_void_p, C.c_uint32, C.c_uint64]
+        L.rtc_ias_update.argtypes = [C.c_void_p, C.c_uint64, C.c_uint32, C.c_uint32, C.c_void_p]
         L.rtc_scene_info_get.argtypes = [C.c_void_p, C.c_uint64, C.POINTER(SceneInfo)]
         L.rtc_scene_destroy.argtypes = [C.c_void_p, C.c_uint64]
         L.rtc_scene_set_instance_flags.argtypes = [C.c_void_p, C.c_uint64, C.c_uint32, C.c_uint32, C.c_void_p]
@@ -131,6 +134,8 @@ def lib():
         L.rtc_trace_schedule_set.argtypes = [C.c_void_p, C.c_int]
         L.rtc_host_gas_build.argtypes = [C.c_void_p, C.c_uint32, C.c_uint32, C.c_void_p, C.c_uint32, C.POINTER(C.c_void_p)]
         L.rtc_host_ias_build.argtypes = [C.c_void_p, C.c_void_p, C.c_uint32, C.POINTER(C.c_void_p)]
+        L.rtc_host_gas_refit.argtypes = [C.c_void_p, C.c_void_p, C.c_uint32]
+        L.rtc_host_ias_refit.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p, C.c_uint32]
         L.rtc_host_accel_info.argtypes = [C.c_void_p, C.POINTER(C.c_uint64), C.POINTER(C.c_uint64), C.c_void_p]
         L.rtc_host_accel_export.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]
         L.rtc_host_accel_destroy.argtypes = [C.c_void_p]
@@ -144,46 +149,93 @@ def _check(rc):
         raise RtcError(lib().rtc_last_error().decode("utf-8", "replace"))
 
 
+def _vertex_records(attrs):
+    attrs = np.ascontiguousarray(attrs)
+    return attrs, attrs.dtype.itemsize * int(np.prod(attrs.shape[1:], dtype=np.int64))      # records, bytes per vertex record
+
+
+def _transforms(instances):
+    n = len(instances)
+    transforms = np.ascontiguousarray([np.asarray(t, dtype=np.float32).reshape(12) for t, _ in instances], dtype=np.float32).reshape(n, 12)
+    return transforms, np.ascontiguousarray([g for _, g in instances], dtype=np.uint32)
+
+
+def _host_export(L, accels, top, inst_gas, info):
+    """Context.scene_export's layout of host-twin accels (accels[g] = geometry g, top = the instance level)."""
+    gas = {}
+    info["gas_nodes"], info["gas_tris"] = [], []
+    for g, h in enumerate(accels):
+        nn, npr = C.c_uint64(0), C.c_uint64(0)
+        _check(L.rtc_host_accel_info(h, C.byref(nn), C.byref(npr), None))
+        nodes = np.zeros((nn.value, 80), dtype=np.uint8)
+        tris = np.zeros((max(npr.value, 1), 12), dtype=np.float32)
+        _check(L.rtc_host_accel_export(h, nodes.ctypes.data_as(C.c_void_p), None, tris.ctypes.data_as(C.c_void_p), None))
+        gas[g] = (nodes, tris[:npr.value])
+        info["gas_nodes"].append(int(nn.value)); info["gas_tris"].append(int(npr.value))
+    n = len(inst_gas)
+    nn, npr = C.c_uint64(0), C.c_uint64(0)
+    _check(L.rtc_host_accel_info(top, C.byref(nn), C.byref(npr), None))
+    nodes = np.zeros((nn.value, 80), dtype=np.uint8)
+    leaves = np.zeros(max(npr.value, 1), dtype=np.uint32)
+    w2o = np.zeros((n, 12), dtype=np.float32)
+    _check(L.rtc_host_accel_export(top, nodes.ctypes.data_as(C.c_void_p), leaves.ctypes.data_as(C.c_void_p), None, w2o.ctypes.data_as(C.c_void_p)))
+    info["tlas_nodes"] = int(nn.value)
+    return {"tlas_nodes": nodes, "tlas_leaves": leaves[:npr.value], "world_to_object": w2o, "instance_gas": inst_gas, "gas": gas}
+
+
+def _host_build(L, geometries, instances, accels):
+    for attrs, idx in geometries:
+        attrs, stride = _vertex_records(attrs)
+        idx = np.ascontiguousarray(idx, dtype=np.uint32).reshape(-1, 3)
+        h = C.c_void_p()
+        _check(L.rtc_host_gas_build(attrs.ctypes.data_as(C.c_void_p), stride, len(attrs), idx.ctypes.data_as(C.c_void_p), len(idx), C.byref(h)))
+        accels.append(h)
+    transforms, inst_gas = _transforms(instances)
+    n = len(inst_gas)
+    handles = (C.c_void_p * max(n, 1))(*[accels[int(g)] for g in inst_gas])
+    top = C.c_void_p()
+    _check(L.rtc_host_ias_build(transforms.ctypes.data_as(C.c_void_p), C.cast(handles, C.c_void_p), n, C.byref(top)))
+    return top, inst_gas
+
+
 def host_scene_export(geometries, instances):
     """The acceleration structure rtc_gas_build(BUILD_HOST_SAH) + rtc_ias_build would upload for this scene, built WITHOUT a GPU
     (rtc_host_gas_build / rtc_host_ias_build: the same builder code fed from host arrays), in the layout of Context.scene_export.
     geometries: [(attributes structured array or [n, k] float32 with the position first, indices [m, 3] uint32)];
     instances: [(transform 12 floats, geometry index)].  Also returns the build statistics per level."""
     L = lib()
-    accels, gas, info = [], {}, {"gas_nodes": [], "gas_tris": []}
+    accels, info = [], {}
     try:
-        for g, (attrs, idx) in enumerate(geometries):
-            attrs = np.ascontiguousarray(attrs)
-            idx = np.ascontiguousarray(idx, dtype=np.uint32).reshape(-1, 3)
-            h = C.c_void_p()
-            stride = attrs.dtype.itemsize * int(np.prod(attrs.shape[1:], dtype=np.int64))      # bytes per vertex record
-            _check(L.rtc_host_gas_build(attrs.ctypes.data_as(C.c_void_p), stride, len(attrs), idx.ctypes.data_as(C.c_void_p), len(idx), C.byref(h)))
-            accels.append(h)
-            nn, npr = C.c_uint64(0), C.c_uint64(0)
-            _check(L.rtc_host_accel_info(h, C.byref(nn), C.byref(npr), None))
-            nodes = np.zeros((nn.value, 80), dtype=np.uint8)
-            tris = np.zeros((max(npr.value, 1), 12), dtype=np.float32)
-            _check(L.rtc_host_accel_export(h, nodes.ctypes.data_as(C.c_void_p), None, tris.ctypes.data_as(C.c_void_p), None))
-            gas[g] = (nodes, tris[:npr.value])
-            info["gas_nodes"].append(int(nn.value)); info["gas_tris"].append(int(npr.value))
-        n = len(instances)
-        transforms = np.ascontiguousarray([np.asarray(t, dtype=np.float32).reshape(12) for t, _ in instances], dtype=np.float32).reshape(n, 12)
-        inst_gas = np.ascontiguousarray([g for _, g in instances], dtype=np.uint32)
-        handles = (C.c_void_p * max(n, 1))(*[accels[int(g)] for g in inst_gas])
-        top = C.c_void_p()
-        _check(L.rtc_host_ias_build(transforms.ctypes.data_as(C.c_void_p), C.cast(handles, C.c_void_p), n, C.byref(top)))
+        top, inst_gas = _host_build(L, geometries, instances, accels)
         accels.append(top)
-        nn, npr = C.c_uint64(0), C.c_uint64(0)
-        _check(L.rtc_host_accel_info(top, C.byref(nn), C.byref(npr), None))
-        nodes = np.zeros((nn.value, 80), dtype=np.uint8)
-        leaves = np.zeros(max(npr.value, 1), dtype=np.uint32)
-        w2o = np.zeros((n, 12), dtype=np.float32)
-        _check(L.rtc_host_accel_export(top, nodes.ctypes.data_as(C.c_void_p), leaves.ctypes.data_as(C.c_void_p), None, w2o.ctypes.data_as(C.c_void_p)))
-        info["tlas_nodes"] = int(nn.value)
+        export = _host_export(L, accels[:-1], top, inst_gas, info)
     finally:
         for h in accels:
             L.rtc_host_accel_destroy(h)
-    return {"tlas_nodes": nodes, "tlas_leaves": leaves[:npr.value], "world_to_object": w2o, "instance_gas": inst_gas, "gas": gas}, info
+    return export, info
+
+
+def host_scene_refit_export(geometries, instances, new_attributes, new_transforms):
+    """host_scene_export of the scene built from (geometries, instances), then refitted WITHOUT a GPU (rtc_host_gas_refit /
+    rtc_host_ias_refit, the twin of rtc_gas_refit / rtc_ias_update): new_attributes[g] replaces geometry g's vertex records (None:
+    unchanged, not refitted), new_transforms the 12 floats of every instance.  Topology stays the build's."""
+    L = lib()
+    accels, info = [], {}
+    try:
+        top, inst_gas = _host_build(L, geometries, instances, accels)
+        accels.append(top)
+        for g, attrs in enumerate(new_attributes):
+            if attrs is not None:
+                attrs, stride = _vertex_records(attrs)
+                _check(L.rtc_host_gas_refit(accels[g], attrs.ctypes.data_as(C.c_void_p), stride))
+        transforms = np.ascontiguousarray(new_transforms, dtype=np.float32).reshape(len(inst_gas), 12)
+        handles = (C.c_void_p * max(len(inst_gas), 1))(*[accels[int(g)] for g in inst_gas])
+        _check(L.rtc_host_ias_refit(top, transforms.ctypes.data_as(C.c_void_p), C.cast(handles, C.c_void_p), len(inst_gas)))
+        export = _host_export(L, accels[:-1], top, inst_gas, info)
+    finally:
+        for h in accels:
+            L.rtc_host_accel_destroy(h)
+    return export, info
 
 
 def device_count():
@@ -269,6 +321,17 @@ class Context:
         g = C.c_uint32(0)
         _check(self.L.rtc_gas_build(self.h, int(d_attributes), stride, num_verts, int(d_indices), num_tris, flags, C.byref(g)))
         return g.value
+
+    def gas_refit(self, gas, d_attributes=0):
+        """rtc_gas_refit: the GAS's vertex positions changed (in place, or d_attributes = new records of the build's stride).
+        Every scene instancing it must then get ias_update before it is traced."""
+        _check(self.L.rtc_gas_refit(self.h, gas, int(d_attributes)))
+
+    def ias_update(self, top, transforms, first=0):
+        """rtc_ias_update: transforms [count, 12] (object -> world) of instances first .. first + count - 1 (count may be 0: only
+        bring the scene up to date with refitted GAS)."""
+        t = np.ascontiguousarray(transforms, dtype=np.float32).reshape(-1, 12)
+        _check(self.L.rtc_ias_update(self.h, int(top), first, len(t), t.ctypes.data_as(C.c_void_p) if len(t) else None))
 
     def gas_destroy(self, gas):
         _check(self.L.rtc_gas_destroy(self.h, gas))

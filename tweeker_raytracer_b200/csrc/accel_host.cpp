@@ -6,6 +6,7 @@
 // be handed -- wide nodes, leaf-ordered triangles, instance-level leaves, world->object matrices -- and the scalar oracle
 // traverses them in the kernels' order of operations (oracle/wide_bvh.inc).  Nothing here renders or intersects anything.
 #include "rtc_internal.h"
+#include "bvh_rules.h"
 
 #include <cmath>
 #include <cstdlib>
@@ -91,45 +92,6 @@ void instance_bounds_host(const float transform[12], const uint8_t* verts, uint3
   for (int r = 0; r < 3; ++r) { out.lo[r] = lo[r]; out.hi[r] = hi[r]; }
 }
 
-// The box the instance level is built over.  tight: b holds the exact bounds of the transformed vertices on entry and is padded
-// -- the object-space ray is a ROUNDED transform of the world ray, so a hit found in object space may lie a few ulps outside
-// the exact world-space box.  Otherwise b becomes the padded bounds of the eight transformed corners of the GAS box (the
-// round-1 bounds, looser for rotated instances).  Instances of an empty GAS get a point box at the origin.
-void instance_box_finish(const float transform[12], const float gasLo[3], const float gasHi[3], bool tight, bool emptyGas, PrimBox& b)
-{
-  const double ext = std::fabs((double)gasHi[0] - gasLo[0]) + std::fabs((double)gasHi[1] - gasLo[1]) + std::fabs((double)gasHi[2] - gasLo[2]);
-  if (tight)
-  {
-    for (int r = 0; r < 3; ++r)
-    {
-      const float* m = &transform[4 * r];
-      const double scale = std::fabs((double)m[0]) + std::fabs((double)m[1]) + std::fabs((double)m[2]);
-      const double padLo = (std::fabs((double)b.lo[r]) + ext * scale) * 1.0e-5, padHi = (std::fabs((double)b.hi[r]) + ext * scale) * 1.0e-5;
-      b.lo[r] = std::nextafterf((float)((double)b.lo[r] - padLo), -std::numeric_limits<float>::infinity());
-      b.hi[r] = std::nextafterf((float)((double)b.hi[r] + padHi), std::numeric_limits<float>::infinity());
-    }
-  }
-  else
-  {
-    for (int k = 0; k < 3; ++k) { b.lo[k] = std::numeric_limits<float>::infinity(); b.hi[k] = -b.lo[k]; }
-    for (int corner = 0; corner < 8; ++corner)
-    {
-      const double x = (corner & 1) ? gasHi[0] : gasLo[0], y = (corner & 2) ? gasHi[1] : gasLo[1], z = (corner & 4) ? gasHi[2] : gasLo[2];
-      for (int r = 0; r < 3; ++r)
-      {
-        const float* m = &transform[4 * r];
-        const double wv = m[0] * x + m[1] * y + m[2] * z + m[3];
-        const double scale = std::fabs((double)m[0]) + std::fabs((double)m[1]) + std::fabs((double)m[2]);
-        const double pad = (std::fabs(wv) + ext * scale) * 1.0e-5;
-        const float lo = std::nextafterf((float)(wv - pad), -std::numeric_limits<float>::infinity());
-        const float hi = std::nextafterf((float)(wv + pad), std::numeric_limits<float>::infinity());
-        b.lo[r] = std::fmin(b.lo[r], lo); b.hi[r] = std::fmax(b.hi[r], hi);
-      }
-    }
-  }
-  if (emptyGas) { for (int k = 0; k < 3; ++k) { b.lo[k] = 0.0f; b.hi[k] = 0.0f; } }
-}
-
 bool instance_bounds_tight()
 {
   const char* e = getenv("RTC_INSTANCE_BOUNDS");
@@ -144,15 +106,53 @@ void tlas_build_host(const PrimBox* boxes, uint32_t numInstances, WideBvh& bvh)
 // ------------------------------------------------------------------------------------------------
 // Host-only twin of rtc_gas_build(RTC_BUILD_HOST_SAH) + rtc_ias_build (include/rtc_core.h)
 // ------------------------------------------------------------------------------------------------
+struct rtc_host_accel;
+
+namespace {
+
+// The node refit of bvh_refit.cu on host arrays: descending node index is bottom-up, because both builders place every child
+// above its parent.  The root's box becomes the bounds of the structure.
+template <class LeafBox>
+void refit_host(WideBvh& bvh, const LeafBox& leafBox)
+{
+  std::vector<float> box(bvh.nodes.size() * 6u);
+  for (size_t i = bvh.nodes.size(); i-- > 0;)
+    refit_node(bvh.nodes[i], leafBox, [&](uint32_t child, float lo[3], float hi[3]) {
+      for (int k = 0; k < 3; ++k) { lo[k] = box[6u * child + k]; hi[k] = box[6u * child + 3 + k]; }
+    }, &box[6u * i], &box[6u * i + 3]);
+  for (int k = 0; k < 3; ++k) { bvh.lo[k] = box[k]; bvh.hi[k] = box[3 + k]; }
+}
+
+} // namespace
+
 struct rtc_host_accel
 {
   bool isInstanceLevel = false;
   WideBvh bvh;
   std::vector<float4> tris;             // geometry level
   std::vector<uint8_t> positions;       // geometry level: vertex positions, 12 B apart (for the instance bounds)
-  uint32_t numVerts = 0, numTris = 0;
+  std::vector<uint32_t> indices;        // geometry level: the build's index triplets (for the refit)
+  uint32_t numVerts = 0, numTris = 0, strideBytes = 0;
   std::vector<float> inverses;          // instance level: 12 floats per instance
 };
+
+// world->object matrices and padded world boxes of every instance, as rtc_ias_build computes them; false on a bad geometry handle
+static bool instance_boxes_host(const float* transforms, const rtc_host_accel* const* geometry, uint32_t numInstances,
+                                std::vector<float>& inverses, std::vector<PrimBox>& boxes)
+{
+  for (uint32_t i = 0; i < numInstances; ++i) if (!geometry[i] || geometry[i]->isInstanceLevel) return false;
+  boxes.assign(numInstances, PrimBox());
+  const bool tight = instance_bounds_tight();
+  for (uint32_t i = 0; i < numInstances; ++i)
+  {
+    const rtc_host_accel* g = geometry[i];
+    const float* m = transforms + 12u * (size_t)i;
+    invert_3x4(m, &inverses[(size_t)i * 12u]);
+    if (tight) instance_bounds_host(m, g->positions.data(), 12u, g->numTris ? g->numVerts : 0u, boxes[i]);
+    instance_box_finish(m, g->bvh.lo, g->bvh.hi, tight, g->numTris == 0, boxes[i]);
+  }
+  return true;
+}
 
 extern "C" {
 
@@ -163,7 +163,7 @@ int rtc_host_gas_build(const void* attributes, uint32_t strideBytes, uint32_t nu
   if (strideBytes < 12 || (strideBytes & 3u)) RTC_FAIL("vertex stride must be a multiple of 4 and at least 12");
   if ((numVerts && !attributes) || (numTris && !indices)) RTC_FAIL("null input array");
   rtc_host_accel* a = new rtc_host_accel();
-  a->numVerts = numVerts; a->numTris = numTris;
+  a->numVerts = numVerts; a->numTris = numTris; a->strideBytes = strideBytes;
   if (!gas_assemble_host(static_cast<const uint8_t*>(attributes), strideBytes, numVerts, indices, numTris, a->bvh, a->tris))
   {
     delete a;
@@ -171,6 +171,7 @@ int rtc_host_gas_build(const void* attributes, uint32_t strideBytes, uint32_t nu
   }
   a->positions.resize((size_t)numVerts * 12u);
   for (uint32_t v = 0; v < numVerts; ++v) std::memcpy(&a->positions[(size_t)v * 12u], static_cast<const uint8_t*>(attributes) + (size_t)v * strideBytes, 12);
+  a->indices.assign(indices, indices + 3u * (size_t)numTris);
   *out = a;
   return 0;
 }
@@ -182,19 +183,62 @@ int rtc_host_ias_build(const float* transforms, const rtc_host_accel* const* geo
   rtc_host_accel* a = new rtc_host_accel();
   a->isInstanceLevel = true;
   a->inverses.resize((size_t)numInstances * 12u);
-  std::vector<PrimBox> boxes(numInstances);
-  const bool tight = instance_bounds_tight();
-  for (uint32_t i = 0; i < numInstances; ++i)
-  {
-    const rtc_host_accel* g = geometry[i];
-    if (!g || g->isInstanceLevel) { delete a; RTC_FAIL("bad geometry handle in instance"); }
-    const float* m = transforms + 12u * (size_t)i;
-    invert_3x4(m, &a->inverses[(size_t)i * 12u]);
-    if (tight) instance_bounds_host(m, g->positions.data(), 12u, g->numTris ? g->numVerts : 0u, boxes[i]);
-    instance_box_finish(m, g->bvh.lo, g->bvh.hi, tight, g->numTris == 0, boxes[i]);
-  }
+  std::vector<PrimBox> boxes;
+  if (!instance_boxes_host(transforms, geometry, numInstances, a->inverses, boxes)) { delete a; RTC_FAIL("bad geometry handle in instance"); }
   tlas_build_host(boxes.data(), numInstances, a->bvh);
   *out = a;
+  return 0;
+}
+
+int rtc_host_gas_refit(rtc_host_accel* accel, const void* attributes, uint32_t strideBytes)
+{
+  if (!accel || accel->isInstanceLevel) RTC_FAIL("not a geometry-level accel");
+  if (strideBytes != accel->strideBytes) RTC_FAIL("vertex stride differs from the build's");
+  if (accel->numVerts && !attributes) RTC_FAIL("null input array");
+  const uint8_t* verts = static_cast<const uint8_t*>(attributes);
+  for (uint32_t v = 0; v < accel->numVerts; ++v) std::memcpy(&accel->positions[(size_t)v * 12u], verts + (size_t)v * strideBytes, 12);
+  for (uint32_t s = 0; s < accel->numTris; ++s)
+  {
+    const uint32_t prim = accel->bvh.primOrder[s];
+    for (int c = 0; c < 3; ++c)
+    {
+      const float* p = reinterpret_cast<const float*>(verts + (size_t)accel->indices[3u * prim + c] * strideBytes);
+      float4& r = accel->tris[3u * (size_t)s + c];
+      r.x = p[0]; r.y = p[1]; r.z = p[2];
+    }
+  }
+  if (accel->numTris == 0) return 0;
+  const std::vector<float4>& tris = accel->tris;
+  refit_host(accel->bvh, [&](uint32_t first, uint32_t count, float lo[3], float hi[3]) {
+    for (int k = 0; k < 3; ++k) { lo[k] = INFINITY; hi[k] = -INFINITY; }
+    for (uint32_t t = first; t < first + count; ++t)
+      for (int c = 0; c < 3; ++c)
+      {
+        const float4& v = tris[3u * (size_t)t + c];
+        const float x[3] = { v.x, v.y, v.z };
+        for (int k = 0; k < 3; ++k) { lo[k] = x[k] < lo[k] ? x[k] : lo[k]; hi[k] = hi[k] < x[k] ? x[k] : hi[k]; }
+      }
+  });
+  return 0;
+}
+
+int rtc_host_ias_refit(rtc_host_accel* accel, const float* transforms, const rtc_host_accel* const* geometry, uint32_t numInstances)
+{
+  if (!accel || !accel->isInstanceLevel) RTC_FAIL("not an instance-level accel");
+  if ((size_t)numInstances * 12u != accel->inverses.size()) RTC_FAIL("instance count differs from the build's");
+  if (numInstances && (!transforms || !geometry)) RTC_FAIL("null input array");
+  std::vector<PrimBox> boxes;
+  if (!instance_boxes_host(transforms, geometry, numInstances, accel->inverses, boxes)) RTC_FAIL("bad geometry handle in instance");
+  if (numInstances == 0) return 0;
+  const std::vector<uint32_t>& leaves = accel->bvh.primOrder;
+  refit_host(accel->bvh, [&](uint32_t first, uint32_t count, float lo[3], float hi[3]) {
+    for (int k = 0; k < 3; ++k) { lo[k] = INFINITY; hi[k] = -INFINITY; }
+    for (uint32_t t = first; t < first + count; ++t)
+    {
+      const PrimBox& b = boxes[leaves[t]];
+      for (int k = 0; k < 3; ++k) { lo[k] = b.lo[k] < lo[k] ? b.lo[k] : lo[k]; hi[k] = hi[k] < b.hi[k] ? b.hi[k] : hi[k]; }
+    }
+  });
   return 0;
 }
 

@@ -6,6 +6,7 @@
 // builder (bvh_build_gpu.cu) takes over for large inputs and emits the same node format through
 // emit_wide_from_binary().
 #include "rtc_internal.h"
+#include "bvh_rules.h"
 
 #include <algorithm>
 #include <cmath>
@@ -119,8 +120,6 @@ struct Builder
     return idx;
   }
 };
-
-inline float pow2f(int e) { uint32_t u = (uint32_t)(e + 127) << 23; float f; std::memcpy(&f, &u, 4); return f; }
 
 // SAH-optimal collapse of the binary tree into 8-wide nodes (after Ylitie, Karras, Laine, HPG 2017, section 4.1).  The
 // leaves are given, so the cost that is left to minimise is the summed surface area of the wide nodes.  For every binary node
@@ -252,29 +251,15 @@ struct Emitter
     int kidAt[8]; for (int s = 0; s < 8; ++s) kidAt[s] = -1;
     for (int i = 0; i < n; ++i) kidAt[slotOf[i]] = kids[i];
 
-    // 3. quantisation frame.  Per axis: grid step 2^e with (hi - p) <= 254 steps, origin p a sixteenth of a
-    //    step below the box, so every child plane keeps slack on the grid (see DESIGN.md "conservative boxes").
-    float maxExt = 0.0f; for (int k = 0; k < 3; ++k) maxExt = std::max(maxExt, box.hi[k] - box.lo[k]);
-    int   e[3]; float p[3], step[3];
-    for (int k = 0; k < 3; ++k)
-    {
-      float ext = std::max(box.hi[k] - box.lo[k], std::max(maxExt * 0x1p-20f, 1.0e-30f));
-      int ek; std::frexp(ext / 253.0f, &ek);            // 2^ek > ext/253
-      ek = std::min(std::max(ek, -120), 120);
-      for (;;)
-      {
-        step[k] = pow2f(ek);
-        p[k] = box.lo[k] - step[k] * 0.0625f;
-        if (!(p[k] < box.lo[k])) p[k] = std::nextafterf(box.lo[k], -std::numeric_limits<float>::infinity());
-        if (std::fmaf(254.0f, step[k], p[k]) >= box.hi[k] || ek >= 120) break;
-        ++ek;
-      }
-      e[k] = ek;
-    }
-
+    // 3. quantisation frame and conservative child planes (bvh_rules.h)
     Node8 node; std::memset(&node, 0, sizeof(node));
-    node.px = p[0]; node.py = p[1]; node.pz = p[2];
-    node.ex = (uint8_t)(e[0] + 127); node.ey = (uint8_t)(e[1] + 127); node.ez = (uint8_t)(e[2] + 127);
+    uint32_t occupied = 0;
+    for (int s = 0; s < 8; ++s) if (kidAt[s] >= 0) occupied |= 1u << s;
+    float nodeLo[3], nodeHi[3];
+    quantise_node(occupied, [&](int s, float lo[3], float hi[3]) {
+      const Box& cb = bn[kidAt[s]].box;
+      for (int k = 0; k < 3; ++k) { lo[k] = cb.lo[k]; hi[k] = cb.hi[k]; }
+    }, node, nodeLo, nodeHi);
 
     // 4. children: inner ones get one contiguous block of wide nodes, leaf primitives one contiguous run
     uint32_t numInner = 0;
@@ -283,22 +268,10 @@ struct Emitter
     out.nodes.resize(out.nodes.size() + numInner);
     node.triBase = (uint32_t)out.primOrder.size();
     uint32_t triOffset = 0;
-    uint8_t* qlo[3] = { node.qlox, node.qloy, node.qloz };
-    uint8_t* qhi[3] = { node.qhix, node.qhiy, node.qhiz };
     for (int s = 0; s < 8; ++s)
     {
-      if (kidAt[s] < 0) { for (int k = 0; k < 3; ++k) { qlo[k][s] = 255; qhi[k][s] = 0; } continue; }
+      if (kidAt[s] < 0) continue;
       const BinNode& c = bn[kidAt[s]];
-      for (int k = 0; k < 3; ++k)
-      {
-        int ql = (int)std::floor(((double)c.box.lo[k] - (double)p[k]) / (double)step[k]);
-        int qh = (int)std::ceil(((double)c.box.hi[k] - (double)p[k]) / (double)step[k]);
-        ql = std::min(std::max(ql, 0), 255); qh = std::min(std::max(qh, 0), 255);
-        // keep at least 1/64 step of slack, evaluated with the arithmetic the kernels use (q * step + p)
-        while (ql > 0 && !(std::fmaf((float)ql, step[k], p[k]) <= c.box.lo[k] - step[k] * 0.015625f)) --ql;
-        while (qh < 255 && !(std::fmaf((float)qh, step[k], p[k]) >= c.box.hi[k] + step[k] * 0.015625f)) ++qh;
-        qlo[k][s] = (uint8_t)ql; qhi[k][s] = (uint8_t)qh;
-      }
       if (c.left < 0)
       {
         node.meta[s] = (uint8_t)((c.count << 5) | triOffset);

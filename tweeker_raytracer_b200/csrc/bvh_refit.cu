@@ -1,0 +1,305 @@
+// bvh_refit.cu -- in-place update of built acceleration structures (the counterpart of optixAccelBuild with
+// OPTIX_BUILD_OPERATION_UPDATE), and the tight instance bounds the instance level is built and updated over.
+//
+//   GAS refit (rtc_gas_refit)        k_refit_tris   one pass over the leaf-ordered triangle records: new positions, id bits kept
+//                                    k_refit_nodes  bottom-up over the wide nodes (Karras-style arrival counters: the last child
+//                                                   to arrive processes the parent), re-quantised through bvh_rules.h
+//   instance update (rtc_ias_update) k_instance_bounds, k_instance_finish, k_refit_nodes over the instance level
+// Node topology (imask, childBase, triBase, meta) and leaf order stay as built; only the frame, the quantised planes and the
+// triangle positions are rewritten.  Min / max are order-independent, so the result does not depend on the arrival order and
+// equals the host twin (accel_host.cpp), which visits the nodes in descending index order.
+//
+// Compiled with -fmad=false: instance_box_finish (bvh_rules.h) must round like the host, which compiles it with -ffp-contract=off.
+#include "rtc_internal.h"
+#include "bvh_rules.h"
+
+#include <cfloat>
+
+namespace {
+
+constexpr int kB = 256;
+
+union NodeWords
+{
+  uint4 v[5];
+  Node8 n;
+};
+
+__global__ void __launch_bounds__(kB)
+k_refit_parents(const uint4* __restrict__ nodes, uint32_t numNodes, uint32_t* __restrict__ parent)
+{
+  const uint32_t i = blockIdx.x * blockDim.x + threadIdx.x;
+  if (i >= numNodes) return;
+  const uint32_t imask = nodes[5u * (size_t)i].w >> 24;
+  const uint32_t childBase = nodes[5u * (size_t)i + 1].x;
+  for (uint32_t r = 0; r < (uint32_t)__popc(imask); ++r) parent[childBase + r] = i;
+}
+
+__global__ void __launch_bounds__(kB)
+k_refit_tris(float4* __restrict__ tris, uint32_t numTris, const uint8_t* __restrict__ verts, uint32_t stride, uint32_t numVerts,
+             const uint32_t* __restrict__ idx)
+{
+  const uint32_t t = blockIdx.x * blockDim.x + threadIdx.x;
+  if (t >= numTris) return;
+  float4* rec = tris + 3u * (size_t)t;
+  const uint32_t prim = __float_as_uint(rec[0].w);
+  for (int c = 0; c < 3; ++c)
+  {
+    const uint32_t vi = __ldg(idx + 3u * (size_t)prim + c);
+    if (vi >= numVerts) continue;                       // indices are the build's, which checked them
+    const float* p = reinterpret_cast<const float*>(verts + (size_t)vi * stride);
+    rec[c] = make_float4(__ldg(p), __ldg(p + 1), __ldg(p + 2), c == 0 ? __uint_as_float(prim) : 0.0f);
+  }
+}
+
+struct RefitParams
+{
+  uint4* nodes; uint32_t numNodes;
+  const float4* tris;                                   // geometry level: leaf-ordered triangle records
+  const uint32_t* leaves; const PrimBox* primBoxes;     // instance level: leaf slot -> instance, instance boxes
+  const uint32_t* parent; uint32_t* arrivals; float* box;
+};
+
+__device__ void refit_one(const RefitParams& P, uint32_t idx)
+{
+  NodeWords w;
+  for (int j = 0; j < 5; ++j) w.v[j] = P.nodes[5u * (size_t)idx + j];
+  auto leafBox = [&](uint32_t first, uint32_t count, float lo[3], float hi[3]) {
+    for (int k = 0; k < 3; ++k) { lo[k] = INFINITY; hi[k] = -INFINITY; }
+    for (uint32_t t = first; t < first + count; ++t)
+    {
+      if (P.tris)
+      {
+        for (int c = 0; c < 3; ++c)
+        {
+          const float4 v = P.tris[3u * (size_t)t + c];
+          const float x[3] = { v.x, v.y, v.z };
+          for (int k = 0; k < 3; ++k) { lo[k] = x[k] < lo[k] ? x[k] : lo[k]; hi[k] = hi[k] < x[k] ? x[k] : hi[k]; }
+        }
+      }
+      else
+      {
+        const PrimBox b = P.primBoxes[P.leaves[t]];
+        for (int k = 0; k < 3; ++k) { lo[k] = b.lo[k] < lo[k] ? b.lo[k] : lo[k]; hi[k] = hi[k] < b.hi[k] ? b.hi[k] : hi[k]; }
+      }
+    }
+  };
+  // boxes of inner children were written by other threads: read them from L2, behind the fence of the arrival protocol
+  auto innerBox = [&](uint32_t child, float lo[3], float hi[3]) {
+    for (int k = 0; k < 3; ++k) { lo[k] = __ldcg(P.box + 6u * (size_t)child + k); hi[k] = __ldcg(P.box + 6u * (size_t)child + 3 + k); }
+  };
+  float lo[3], hi[3];
+  refit_node(w.n, leafBox, innerBox, lo, hi);
+  for (int j = 0; j < 5; ++j) P.nodes[5u * (size_t)idx + j] = w.v[j];
+  for (int k = 0; k < 3; ++k) { __stcg(P.box + 6u * (size_t)idx + k, lo[k]); __stcg(P.box + 6u * (size_t)idx + 3 + k, hi[k]); }
+}
+
+// One thread per node without inner children; after each node it climbs to the parent, which the LAST child to arrive refits.
+// The arrival counter is reset by that thread, so the next refit starts from zero without a memset.
+__global__ void __launch_bounds__(kB)
+k_refit_nodes(const RefitParams P)
+{
+  const uint32_t i = blockIdx.x * blockDim.x + threadIdx.x;
+  if (i >= P.numNodes) return;
+  if (P.nodes[5u * (size_t)i].w >> 24) return;          // imask != 0: reached from below
+  uint32_t node = i;
+  for (;;)
+  {
+    refit_one(P, node);
+    if (node == 0) return;
+    __threadfence();
+    const uint32_t parent = P.parent[node];
+    const uint32_t expected = (uint32_t)__popc(P.nodes[5u * (size_t)parent].w >> 24);
+    if (atomicAdd(P.arrivals + parent, 1u) != expected - 1u) return;
+    P.arrivals[parent] = 0u;
+    __threadfence();
+    node = parent;
+  }
+}
+
+// ---- instance level: tight world bounds of every instance from its transformed vertices -------------------------
+// The reference hands OptiX the instance transform and lets the driver bound the instance (Device.cpp:1427-1443,
+// optixAccelBuild over OPTIX_BUILD_INPUT_TYPE_INSTANCES :1471-1482).  The first version here bounded the eight transformed
+// corners of the GAS box, which is loose for rotated instances (a torus rotated by 45 degrees: +40 % per axis) and made
+// rays enter instances they cannot hit; an instance entry costs about three node visits.  One CTA per instance now
+// transforms every vertex of the instance's GAS and reduces min/max.
+struct InstanceBoundsIn
+{
+  float transform[12];
+  const uint8_t* verts; uint32_t stride, numVerts;
+  uint32_t pad;
+};
+
+__global__ void __launch_bounds__(kB)
+k_instance_bounds(const InstanceBoundsIn* __restrict__ in, PrimBox* __restrict__ out)
+{
+  const InstanceBoundsIn& I = in[blockIdx.x];
+  float lo[3] = { FLT_MAX, FLT_MAX, FLT_MAX }, hi[3] = { -FLT_MAX, -FLT_MAX, -FLT_MAX };
+  for (uint32_t v = threadIdx.x; v < I.numVerts; v += blockDim.x)
+  {
+    const float* p = reinterpret_cast<const float*>(I.verts + (size_t)v * I.stride);
+    const float x = p[0], y = p[1], z = p[2];
+#pragma unroll
+    for (int r = 0; r < 3; ++r)
+    {
+      const float* m = I.transform + 4 * r;
+      const float w = fmaf(m[0], x, fmaf(m[1], y, fmaf(m[2], z, m[3])));
+      lo[r] = fminf(lo[r], w); hi[r] = fmaxf(hi[r], w);
+    }
+  }
+  __shared__ float sLo[3][kB / 32], sHi[3][kB / 32];
+#pragma unroll
+  for (int r = 0; r < 3; ++r)
+  {
+    for (int off = 16; off; off >>= 1)
+    {
+      lo[r] = fminf(lo[r], __shfl_down_sync(0xffffffffu, lo[r], off));
+      hi[r] = fmaxf(hi[r], __shfl_down_sync(0xffffffffu, hi[r], off));
+    }
+    if ((threadIdx.x & 31) == 0) { sLo[r][threadIdx.x >> 5] = lo[r]; sHi[r][threadIdx.x >> 5] = hi[r]; }
+  }
+  __syncthreads();
+  if (threadIdx.x < 3)
+  {
+    float a = sLo[threadIdx.x][0], b = sHi[threadIdx.x][0];
+    for (int w = 1; w < kB / 32; ++w) { a = fminf(a, sLo[threadIdx.x][w]); b = fmaxf(b, sHi[threadIdx.x][w]); }
+    out[blockIdx.x].lo[threadIdx.x] = a; out[blockIdx.x].hi[threadIdx.x] = b;
+  }
+}
+
+// One thread per updated instance: the padded box (the device twin of what rtc_ias_build does on the host), the instance's
+// rows of the traversal table (world->object) and of the shading tables (object->world, vertex attributes).
+__global__ void __launch_bounds__(128)
+k_instance_finish(const InstanceUpdate* __restrict__ up, uint32_t count, const PrimBox* __restrict__ exact, int tight,
+                  PrimBox* __restrict__ instBoxes, float4* __restrict__ instances, float4* __restrict__ o2w, rt_GeometryInstanceData* __restrict__ gi)
+{
+  const uint32_t i = blockIdx.x * blockDim.x + threadIdx.x;
+  if (i >= count) return;
+  const InstanceUpdate& u = up[i];
+  float gas[6];
+  for (int k = 0; k < 6; ++k) gas[k] = u.gasBox ? u.gasBox[k] : u.gasLoHi[k];
+  PrimBox b = {};
+  if (tight) b = exact[i];
+  instance_box_finish(u.transform, gas, gas + 3, tight != 0, u.emptyGas != 0, b);
+  const uint32_t inst = u.instance;
+  instBoxes[inst] = b;
+  for (int r = 0; r < 3; ++r)
+  {
+    instances[4u * inst + r] = make_float4(u.inverse[4 * r], u.inverse[4 * r + 1], u.inverse[4 * r + 2], u.inverse[4 * r + 3]);
+    o2w[3u * inst + r] = make_float4(u.transform[4 * r], u.transform[4 * r + 1], u.transform[4 * r + 2], u.transform[4 * r + 3]);
+  }
+  gi[inst].attributes = u.attributes;
+}
+
+int alloc_refit_scratch(rtc_context* ctx, RefitScratch& r, const uint4* nodes, uint32_t numNodes)
+{
+  if (r.base) return 0;
+  const size_t n = numNodes;
+  RTC_CUDA(cudaMalloc(&r.base, n * (2 * sizeof(uint32_t) + 6 * sizeof(float))));
+  r.box = static_cast<float*>(r.base);
+  r.parent = reinterpret_cast<uint32_t*>(r.box + 6 * n);
+  r.arrivals = r.parent + n;
+  RTC_CUDA(cudaMemsetAsync(r.arrivals, 0, n * sizeof(uint32_t), ctx->stream));
+  k_refit_parents<<<(numNodes + kB - 1) / kB, kB, 0, ctx->stream>>>(nodes, numNodes, r.parent);
+  ctx->kernelLaunches++;
+  RTC_CUDA(cudaGetLastError());
+  return 0;
+}
+
+int launch_refit_nodes(rtc_context* ctx, const RefitScratch& r, uint4* nodes, uint32_t numNodes, const float4* tris,
+                       const uint32_t* leaves, const PrimBox* primBoxes)
+{
+  RefitParams P;
+  P.nodes = nodes; P.numNodes = numNodes; P.tris = tris; P.leaves = leaves; P.primBoxes = primBoxes;
+  P.parent = r.parent; P.arrivals = r.arrivals; P.box = r.box;
+  k_refit_nodes<<<(numNodes + kB - 1) / kB, kB, 0, ctx->stream>>>(P);
+  ctx->kernelLaunches++;
+  RTC_CUDA(cudaGetLastError());
+  return 0;
+}
+
+} // namespace
+
+void free_refit_scratch(RefitScratch& r)
+{
+  cudaFree(r.base);
+  r = RefitScratch();
+}
+
+int refit_gas_gpu(rtc_context* ctx, GasRecord& rec)
+{
+  if (rec.numTris == 0) return 0;                       // one empty node: nothing to refit, the bounds stay (0, 0)
+  uint4* nodes = static_cast<uint4*>(rec.d_nodes);
+  if (int rc = alloc_refit_scratch(ctx, rec.refit, nodes, rec.numNodes)) return rc;
+  k_refit_tris<<<(rec.numTris + kB - 1) / kB, kB, 0, ctx->stream>>>(static_cast<float4*>(rec.d_tris), rec.numTris,
+                                                                    (const uint8_t*)(uintptr_t)rec.attributes, rec.strideBytes, rec.numVerts,
+                                                                    (const uint32_t*)(uintptr_t)rec.indices);
+  ctx->kernelLaunches++;
+  RTC_CUDA(cudaGetLastError());
+  if (int rc = launch_refit_nodes(ctx, rec.refit, nodes, rec.numNodes, static_cast<const float4*>(rec.d_tris), nullptr, nullptr)) return rc;
+  rec.boundsOnDevice = true;
+  return 0;
+}
+
+int refit_instances_gpu(rtc_context* ctx, SceneRecord& s, const std::vector<InstanceUpdate>& updates, bool tight)
+{
+  const uint32_t m = (uint32_t)updates.size();
+  if (m == 0) return 0;
+  uint4* tlas = static_cast<uint4*>(s.d_tlasNodes);
+  if (int rc = alloc_refit_scratch(ctx, s.refit, tlas, s.desc.numTlasNodes)) return rc;
+  // inputs of this update: staged from pageable memory by the copy itself, and freed stream-ordered behind the kernels
+  std::vector<InstanceBoundsIn> in(tight ? m : 0);
+  for (uint32_t i = 0; i < (uint32_t)in.size(); ++i)
+  {
+    for (int k = 0; k < 12; ++k) in[i].transform[k] = updates[i].transform[k];
+    in[i].verts = updates[i].verts; in[i].stride = updates[i].stride; in[i].numVerts = updates[i].numVerts; in[i].pad = 0u;
+  }
+  const size_t upBytes = m * sizeof(InstanceUpdate), inBytes = in.size() * sizeof(InstanceBoundsIn);
+  uint8_t* d = nullptr;
+  RTC_CUDA(cudaMallocAsync((void**)&d, upBytes + inBytes + m * sizeof(PrimBox), ctx->stream));
+  InstanceUpdate* d_up = reinterpret_cast<InstanceUpdate*>(d);
+  InstanceBoundsIn* d_in = reinterpret_cast<InstanceBoundsIn*>(d + upBytes);
+  PrimBox* d_exact = reinterpret_cast<PrimBox*>(d + upBytes + inBytes);
+  cudaError_t e = cudaMemcpyAsync(d_up, updates.data(), upBytes, cudaMemcpyHostToDevice, ctx->stream);
+  if (e == cudaSuccess && tight) e = cudaMemcpyAsync(d_in, in.data(), inBytes, cudaMemcpyHostToDevice, ctx->stream);
+  if (e == cudaSuccess && tight) { k_instance_bounds<<<m, kB, 0, ctx->stream>>>(d_in, d_exact); ctx->kernelLaunches++; e = cudaGetLastError(); }
+  if (e == cudaSuccess)
+  {
+    k_instance_finish<<<(m + 127) / 128, 128, 0, ctx->stream>>>(d_up, m, d_exact, tight ? 1 : 0, s.d_instBoxes, static_cast<float4*>(s.d_instances),
+                                                                static_cast<float4*>(s.d_o2w), static_cast<rt_GeometryInstanceData*>(s.d_geomInst));
+    ctx->kernelLaunches++;
+    e = cudaGetLastError();
+  }
+  cudaFreeAsync(d, ctx->stream);
+  if (e != cudaSuccess) return rtc_set_error(__FILE__, __LINE__, "refit_instances_gpu", (int)e, cudaGetErrorString(e));
+  return launch_refit_nodes(ctx, s.refit, tlas, s.desc.numTlasNodes, nullptr, static_cast<const uint32_t*>(s.d_tlasLeaves), s.d_instBoxes);
+}
+
+// boxes[i] = exact (unpadded) world bounds of the vertices of instance i; instances of an empty GAS get an inverted box
+int instance_bounds_gpu(rtc_context* ctx, const rtc_instance_desc* instances, uint32_t numInstances, PrimBox* boxes)
+{
+  if (numInstances == 0) return 0;
+  std::vector<InstanceBoundsIn> in(numInstances);
+  for (uint32_t i = 0; i < numInstances; ++i)
+  {
+    const GasRecord& g = ctx->gas[instances[i].gas];
+    for (int k = 0; k < 12; ++k) in[i].transform[k] = instances[i].transform[k];
+    in[i].verts = reinterpret_cast<const uint8_t*>((uintptr_t)g.attributes); in[i].stride = g.strideBytes;
+    in[i].numVerts = g.numTris ? g.numVerts : 0u; in[i].pad = 0u;
+  }
+  InstanceBoundsIn* d_in = nullptr; PrimBox* d_out = nullptr;
+  RTC_CUDA(cudaMalloc(&d_in, sizeof(InstanceBoundsIn) * numInstances));
+  if (cudaMalloc(&d_out, sizeof(PrimBox) * numInstances) != cudaSuccess) { cudaFree(d_in); RTC_FAIL("cudaMalloc failed"); }
+  cudaError_t e = cudaMemcpyAsync(d_in, in.data(), sizeof(InstanceBoundsIn) * numInstances, cudaMemcpyHostToDevice, ctx->stream);
+  if (e == cudaSuccess)
+  {
+    k_instance_bounds<<<numInstances, kB, 0, ctx->stream>>>(d_in, d_out);
+    ctx->kernelLaunches++;
+    e = cudaGetLastError();
+  }
+  if (e == cudaSuccess) e = cudaMemcpyAsync(boxes, d_out, sizeof(PrimBox) * numInstances, cudaMemcpyDeviceToHost, ctx->stream);
+  if (e == cudaSuccess) e = cudaStreamSynchronize(ctx->stream);
+  cudaFree(d_in); cudaFree(d_out);
+  if (e != cudaSuccess) return rtc_set_error(__FILE__, __LINE__, "instance_bounds_gpu", (int)e, cudaGetErrorString(e));
+  return 0;
+}

@@ -3,6 +3,7 @@
 // at the top of rtc_core.h); there is no CPU rendering path here: every entry point that produces
 // rays, hits or pixels ends in a kernel launch on the context's stream.
 #include "rtc_internal.h"
+#include "bvh_rules.h"
 
 #include <chrono>
 #include <cmath>
@@ -31,7 +32,30 @@ SceneRecord* find_scene(rtc_context* ctx, uint64_t topObject)
 void free_scene(SceneRecord* s)
 {
   cudaFree(s->d_desc); cudaFree(s->d_tlasNodes); cudaFree(s->d_instances); cudaFree(s->d_tlasLeaves); cudaFree(s->d_o2w); cudaFree(s->d_geomInst); cudaFree(s->d_instFlags);
+  cudaFree(s->d_instBoxes); free_refit_scratch(s->refit);
   delete s;
+}
+
+// A scene is stale when one of its GAS was refitted after the scene was built or last updated: its instance boxes and instance
+// level no longer bound the triangles, and its shading table may point at a vertex buffer the caller has since freed.
+bool scene_stale(const rtc_context* ctx, const SceneRecord* s)
+{
+  for (const std::pair<uint32_t, uint64_t>& g : s->gasGeneration) if (ctx->gas[g.first].generation != g.second) return true;
+  return false;
+}
+
+constexpr const char* kStaleScene = "a GAS of this scene was refitted after the scene was built or updated: call rtc_ias_update on the scene first";
+
+// the host copy of a GAS's bounds after a refit left them on the device (synchronises the stream; build paths only)
+int fetch_gas_bounds(rtc_context* ctx, GasRecord& g)
+{
+  if (!g.boundsOnDevice) return 0;
+  float box[6];
+  RTC_CUDA(cudaMemcpyAsync(box, g.refit.box, sizeof(box), cudaMemcpyDeviceToHost, ctx->stream));
+  RTC_CUDA(cudaStreamSynchronize(ctx->stream));
+  for (int k = 0; k < 3; ++k) { g.lo[k] = box[k]; g.hi[k] = box[3 + k]; }
+  g.boundsOnDevice = false;
+  return 0;
 }
 
 } // namespace
@@ -84,7 +108,7 @@ int profile_end(rtc_context* ctx)
 
 extern "C" {
 
-int rtc_version(void) { return 100; }
+int rtc_version(void) { return 101; }
 
 const char* rtc_last_error(void) { return g_lastError.c_str(); }
 
@@ -155,7 +179,7 @@ int rtc_context_destroy(rtc_context* ctx)
   release_cutout_graph(ctx);
   tuner_release(ctx);
   for (SceneRecord* s : ctx->scenes) free_scene(s);
-  for (GasRecord& g : ctx->gas) { cudaFree(g.d_nodes); cudaFree(g.d_tris); }
+  for (GasRecord& g : ctx->gas) { cudaFree(g.d_nodes); cudaFree(g.d_tris); free_refit_scratch(g.refit); }
   if (ctx->wf.base) cudaFree(ctx->wf.base);
   if (ctx->wf.cutBase) cudaFree(ctx->wf.cutBase);
   for (void* t : ctx->textures) cudaFree(t);
@@ -354,9 +378,19 @@ int rtc_gas_destroy(rtc_context* ctx, uint32_t gas)
   RTC_CUDA(cudaSetDevice(ctx->device));
   RTC_CUDA(cudaStreamSynchronize(ctx->stream));
   GasRecord& g = ctx->gas[gas];
-  cudaFree(g.d_nodes); cudaFree(g.d_tris);
-  g.d_nodes = nullptr; g.d_tris = nullptr; g.numNodes = 0; g.numTris = 0;
+  cudaFree(g.d_nodes); cudaFree(g.d_tris); free_refit_scratch(g.refit);
+  g.d_nodes = nullptr; g.d_tris = nullptr; g.numNodes = 0; g.numTris = 0; g.boundsOnDevice = false;
   return 0;
+}
+
+int rtc_gas_refit(rtc_context* ctx, uint32_t gas, uint64_t attributes)
+{
+  if (gas >= ctx->gas.size() || ctx->gas[gas].d_nodes == nullptr) RTC_FAIL("bad gas handle");
+  RTC_CUDA(cudaSetDevice(ctx->device));
+  GasRecord& g = ctx->gas[gas];
+  if (attributes) g.attributes = attributes;
+  g.generation++;
+  return refit_gas_gpu(ctx, g);
 }
 
 // ------------------------------------------------------------------------------------------------
@@ -373,6 +407,7 @@ int rtc_ias_build(rtc_context* ctx, const rtc_instance_desc* instances, uint32_t
   std::vector<rt_GeometryInstanceData> gi(numInstances);
   SceneRecord* rec = new SceneRecord();
   rec->inverses.resize((size_t)numInstances * 12u);
+  rec->transforms.resize((size_t)numInstances * 12u);
   rec->instGas.resize(numInstances);
   std::set<uint32_t> distinct;
   for (uint32_t i = 0; i < numInstances; ++i)
@@ -380,9 +415,11 @@ int rtc_ias_build(rtc_context* ctx, const rtc_instance_desc* instances, uint32_t
     const rtc_instance_desc& d = instances[i];
     if (d.instanceId != i) { delete rec; RTC_FAIL("instanceId must equal the array position"); }
     if (d.gas >= ctx->gas.size() || ctx->gas[d.gas].d_nodes == nullptr) { delete rec; RTC_FAIL("bad gas handle in instance"); }
+    if (int rc = fetch_gas_bounds(ctx, ctx->gas[d.gas])) { delete rec; return rc; }
     const GasRecord& g = ctx->gas[d.gas];
     distinct.insert(d.gas);
     rec->instGas[i] = d.gas;
+    std::memcpy(&rec->transforms[(size_t)i * 12u], d.transform, 48);
     float* inv = &rec->inverses[(size_t)i * 12u];
     invert_3x4(d.transform, inv);
     for (int r = 0; r < 3; ++r)
@@ -421,6 +458,7 @@ int rtc_ias_build(rtc_context* ctx, const rtc_instance_desc* instances, uint32_t
   if (e == cudaSuccess) e = upload(&rec->d_geomInst, gi.data(), gi.size() * sizeof(rt_GeometryInstanceData));
   rec->instFlags.assign(numInstances, 0u);
   if (e == cudaSuccess) e = upload(&rec->d_instFlags, rec->instFlags.data(), rec->instFlags.size() * 4u);
+  if (e == cudaSuccess) e = upload((void**)&rec->d_instBoxes, boxes.data(), boxes.size() * sizeof(PrimBox));
   rec->desc.instFlags = (const uint32_t*)rec->d_instFlags;
   rec->desc.tlasNodes = (const uint4*)rec->d_tlasNodes;
   rec->desc.tlasLeaves = (const uint32_t*)rec->d_tlasLeaves;
@@ -433,10 +471,55 @@ int rtc_ias_build(rtc_context* ctx, const rtc_instance_desc* instances, uint32_t
   if (e == cudaSuccess) e = upload((void**)&rec->d_desc, &rec->desc, sizeof(SceneDesc));
   if (e != cudaSuccess) { free_scene(rec); return rtc_set_error(__FILE__, __LINE__, "rtc_ias_build upload", (int)e, cudaGetErrorString(e)); }
   rec->totalNodes = bvh.nodes.size(); rec->totalTris = 0; rec->gasBuildMs = 0.0; rec->numGas = (uint32_t)distinct.size();
-  for (uint32_t g : distinct) { rec->totalNodes += ctx->gas[g].numNodes; rec->totalTris += ctx->gas[g].numTris; rec->gasBuildMs += ctx->gas[g].buildMs; }
+  for (uint32_t g : distinct)
+  {
+    rec->totalNodes += ctx->gas[g].numNodes; rec->totalTris += ctx->gas[g].numTris; rec->gasBuildMs += ctx->gas[g].buildMs;
+    rec->gasGeneration.emplace_back(g, ctx->gas[g].generation);
+  }
   rec->iasBuildMs = now_ms() - t0;
   ctx->scenes.push_back(rec);
   *topObject = (uint64_t)(uintptr_t)rec->d_desc;
+  return 0;
+}
+
+int rtc_ias_update(rtc_context* ctx, uint64_t topObject, uint32_t first, uint32_t count, const float* transforms)
+{
+  SceneRecord* s = find_scene(ctx, topObject);
+  if (!s) RTC_FAIL("unknown topObject");
+  const uint32_t n = s->desc.numInstances;
+  if ((uint64_t)first + count > n) RTC_FAIL("instance range out of bounds");
+  if (count && !transforms) RTC_FAIL("transforms is null");
+  for (const std::pair<uint32_t, uint64_t>& g : s->gasGeneration)
+    if (ctx->gas[g.first].d_nodes == nullptr) RTC_FAIL("a GAS of this scene was destroyed");
+  RTC_CUDA(cudaSetDevice(ctx->device));
+  for (uint32_t i = first; i < first + count; ++i)
+  {
+    std::memcpy(&s->transforms[(size_t)i * 12u], transforms + (size_t)(i - first) * 12u, 48);
+    invert_3x4(&s->transforms[(size_t)i * 12u], &s->inverses[(size_t)i * 12u]);
+  }
+  // instances to recompute: the moved ones and every instance of a GAS refitted since the last build / update
+  std::vector<uint8_t> refitted(ctx->gas.size(), 0u);
+  bool anyRefitted = false;
+  for (const std::pair<uint32_t, uint64_t>& g : s->gasGeneration)
+    if (ctx->gas[g.first].generation != g.second) { refitted[g.first] = 1u; anyRefitted = true; }
+  std::vector<InstanceUpdate> updates;
+  updates.reserve(anyRefitted ? n : count);
+  for (uint32_t i = anyRefitted ? 0u : first; i < (anyRefitted ? n : first + count); ++i)
+  {
+    if (!(first <= i && i < first + count) && !refitted[s->instGas[i]]) continue;
+    const GasRecord& g = ctx->gas[s->instGas[i]];
+    InstanceUpdate u;
+    std::memcpy(u.transform, &s->transforms[(size_t)i * 12u], 48);
+    std::memcpy(u.inverse, &s->inverses[(size_t)i * 12u], 48);
+    u.verts = reinterpret_cast<const uint8_t*>((uintptr_t)g.attributes); u.stride = g.strideBytes; u.numVerts = g.numTris ? g.numVerts : 0u;
+    u.gasBox = g.boundsOnDevice ? g.refit.box : nullptr;
+    for (int k = 0; k < 3; ++k) { u.gasLoHi[k] = g.lo[k]; u.gasLoHi[3 + k] = g.hi[k]; }
+    u.attributes = g.attributes;
+    u.instance = i; u.emptyGas = g.numTris == 0 ? 1u : 0u;
+    updates.push_back(u);
+  }
+  if (int rc = refit_instances_gpu(ctx, *s, updates, instance_bounds_tight())) return rc;
+  for (std::pair<uint32_t, uint64_t>& g : s->gasGeneration) g.second = ctx->gas[g.first].generation;
   return 0;
 }
 
@@ -572,6 +655,7 @@ int rtc_launch(rtc_context* ctx, const rt_SystemData* sys, uint32_t launchWidth,
   if (raygen != RTC_RAYGEN_FULL_FRAME && raygen != RTC_RAYGEN_LOCAL_COPY) RTC_FAIL("bad raygen selector");
   if (miss < RT_MISS_NULL || miss > RT_MISS_SPHERE) RTC_FAIL("bad miss selector");
   if (miss == RT_MISS_SPHERE && (sys->envTexture == 0 || sys->envCDF_U == 0 || sys->envCDF_V == 0)) RTC_FAIL("miss 2 needs envTexture/envCDF_U/envCDF_V");
+  if (const SceneRecord* s = find_scene(ctx, sys->topObject)) { if (scene_stale(ctx, s)) RTC_FAIL(kStaleScene); }
   RTC_CUDA(cudaSetDevice(ctx->device));
   return launch_wavefront(ctx, *sys, launchWidth, launchHeight, raygen, miss, iterationFirst, iterationCount, iterationFirst, false);
 }
@@ -584,6 +668,7 @@ int rtc_launch_ex(rtc_context* ctx, const rt_SystemData* sys, uint32_t launchWid
   if (miss < RT_MISS_NULL || miss > RT_MISS_SPHERE) RTC_FAIL("bad miss selector");
   if (miss == RT_MISS_SPHERE && (sys->envTexture == 0 || sys->envCDF_U == 0 || sys->envCDF_V == 0)) RTC_FAIL("miss 2 needs envTexture/envCDF_U/envCDF_V");
   if (accumulationFirst < 0) RTC_FAIL("accumulationFirst < 0");
+  if (const SceneRecord* s = find_scene(ctx, sys->topObject)) { if (scene_stale(ctx, s)) RTC_FAIL(kStaleScene); }
   RTC_CUDA(cudaSetDevice(ctx->device));
   return launch_wavefront(ctx, *sys, launchWidth, launchHeight, raygen, miss, iterationFirst, iterationCount, accumulationFirst, countWork != 0);
 }
@@ -695,6 +780,7 @@ int rtc_trace_closest(rtc_context* ctx, uint64_t topObject, uint64_t rays, uint6
 {
   SceneRecord* s = find_scene(ctx, topObject);
   if (!s) RTC_FAIL("unknown topObject");
+  if (scene_stale(ctx, s)) RTC_FAIL(kStaleScene);
   RTC_CUDA(cudaSetDevice(ctx->device));
   RTC_CUDA(cudaEventRecord(ctx->evA, ctx->stream));
   if (int rc = launch_trace_closest(ctx, &s->desc, (const rtc_ray*)(uintptr_t)rays, numRays, (rtc_hit*)(uintptr_t)hits)) return rc;
@@ -707,6 +793,7 @@ int rtc_trace_any(rtc_context* ctx, uint64_t topObject, uint64_t rays, uint64_t 
 {
   SceneRecord* s = find_scene(ctx, topObject);
   if (!s) RTC_FAIL("unknown topObject");
+  if (scene_stale(ctx, s)) RTC_FAIL(kStaleScene);
   RTC_CUDA(cudaSetDevice(ctx->device));
   RTC_CUDA(cudaEventRecord(ctx->evA, ctx->stream));
   if (int rc = launch_trace_any(ctx, &s->desc, (const rtc_ray*)(uintptr_t)rays, numRays, (uint32_t*)(uintptr_t)occluded)) return rc;
@@ -720,6 +807,7 @@ int rtc_trace_count(rtc_context* ctx, uint64_t topObject, uint64_t rays, uint64_
   SceneRecord* s = find_scene(ctx, topObject);
   if (!s) RTC_FAIL("unknown topObject");
   if (!out) RTC_FAIL("out is null");
+  if (scene_stale(ctx, s)) RTC_FAIL(kStaleScene);
   RTC_CUDA(cudaSetDevice(ctx->device));
   unsigned long long* d = ctx->d_launchCounts + 2 * kTraceCountWords;
   RTC_CUDA(cudaMemsetAsync(d, 0, kTraceCountWords * sizeof(uint64_t), ctx->stream));

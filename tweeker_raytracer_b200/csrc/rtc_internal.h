@@ -14,6 +14,7 @@
 
 #include <cstdint>
 #include <string>
+#include <utility>
 #include <vector>
 
 #include <cuda_runtime.h>
@@ -78,9 +79,18 @@ void invert_3x4(const float m[12], float out[12]);
 bool gas_assemble_host(const uint8_t* verts, uint32_t strideBytes, uint32_t numVerts, const uint32_t* idx, uint32_t numTris,
                        WideBvh& bvh, std::vector<float4>& tris);
 void instance_bounds_host(const float transform[12], const uint8_t* verts, uint32_t strideBytes, uint32_t numVerts, PrimBox& out);
-void instance_box_finish(const float transform[12], const float gasLo[3], const float gasHi[3], bool tight, bool emptyGas, PrimBox& b);
 bool instance_bounds_tight();      // false with RTC_INSTANCE_BOUNDS=box
 void tlas_build_host(const PrimBox* boxes, uint32_t numInstances, WideBvh& bvh);
+
+// Refit scratch of one wide BVH (bvh_refit.cu): the parent and an arrival counter per node, and the float box each node computed
+// for itself (6 floats; node 0's box bounds the whole structure).  One allocation, made on the structure's first refit.
+struct RefitScratch
+{
+  void*     base = nullptr;
+  uint32_t* parent = nullptr;
+  uint32_t* arrivals = nullptr;
+  float*    box = nullptr;
+};
 
 struct GasRecord
 {
@@ -92,6 +102,9 @@ struct GasRecord
   uint32_t strideBytes = 0, numVerts = 0;
   double   buildMs = 0.0;
   int      builder = 0;                    // RTC_BUILD_HOST_SAH or RTC_BUILD_GPU_LBVH
+  uint64_t generation = 0;                 // rtc_gas_refit count: scenes built / updated at an older generation are stale
+  RefitScratch refit;
+  bool     boundsOnDevice = false;         // lo / hi are stale: the refitted bounds are refit.box[0..5] on the device
 };
 
 struct SceneRecord
@@ -104,6 +117,10 @@ struct SceneRecord
   bool     albedoTextures = false;         // MaterialDefinition.textureAlbedo may be non-zero: selects the textured shade kernels
   std::vector<float> inverses;             // 12 floats per instance (host copy of the world->object matrices)
   std::vector<uint32_t> instGas;           // GAS handle per instance
+  std::vector<float> transforms;           // 12 floats per instance (host copy of the object->world matrices)
+  std::vector<std::pair<uint32_t, uint64_t>> gasGeneration;   // each distinct GAS and its generation at the last build / update
+  PrimBox* d_instBoxes = nullptr;          // the padded world box of every instance (leaf boxes of the instance level)
+  RefitScratch refit;
   uint64_t totalNodes = 0, totalTris = 0;  // unique GAS nodes / triangles referenced + instance level
   uint32_t numGas = 0;
   double   gasBuildMs = 0.0, iasBuildMs = 0.0;
@@ -199,8 +216,27 @@ constexpr uint32_t kGpuBuildThreshold = 1u << 20;
 // bvh_build_gpu.cu: Morton LBVH on the device, straight into rec.d_nodes / rec.d_tris; fills numNodes, lo, hi
 int build_gas_gpu(rtc_context* ctx, GasRecord& rec);
 
-// bvh_build_gpu.cu: exact world bounds of every instance's transformed vertices (one CTA per instance)
+// bvh_refit.cu: exact world bounds of every instance's transformed vertices (one CTA per instance)
 int instance_bounds_gpu(rtc_context* ctx, const rtc_instance_desc* instances, uint32_t numInstances, PrimBox* boxes);
+
+// bvh_refit.cu: refits, all enqueued on ctx->stream without a host synchronisation (except the one-time scratch allocation).
+// refit_gas_gpu rewrites the triangle records from rec.attributes and re-quantises every node bottom-up.
+int refit_gas_gpu(rtc_context* ctx, GasRecord& rec);
+// One instance whose box must be recomputed by rtc_ias_update.
+struct InstanceUpdate
+{
+  float    transform[12];          // object -> world
+  float    inverse[12];            // world -> object (invert_3x4)
+  const uint8_t* verts;            // the GAS's vertex records (tight bounds)
+  uint32_t stride, numVerts;       // numVerts = 0 for an empty GAS
+  const float* gasBox;             // device lo[3], hi[3] of a refitted GAS, or null: gasLoHi
+  float    gasLoHi[6];
+  uint64_t attributes;             // rt_GeometryInstanceData::attributes
+  uint32_t instance, emptyGas;
+};
+// Writes the matrices, shading-table attributes and padded boxes of the listed instances and refits the instance level.
+int refit_instances_gpu(rtc_context* ctx, SceneRecord& s, const std::vector<InstanceUpdate>& updates, bool tight);
+void free_refit_scratch(RefitScratch& r);
 
 // error plumbing (rtc_api.cpp)
 int rtc_set_error(const char* file, int line, const char* call, int code, const char* text);

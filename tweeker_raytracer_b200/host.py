@@ -58,7 +58,8 @@ SYMBOLS = ["rth_last_error", "rth_app_create", "rth_app_destroy", "rth_app_info"
            "rth_app_materials", "rth_app_lights", "rth_app_camera", "rth_app_system_data", "rth_app_tonemapper",
            "rth_app_environment", "rth_app_render", "rth_app_render_calls", "rth_app_set_coalesce", "rth_app_synchronize", "rth_app_frame", "rth_app_local_frame", "rth_app_restart",
            "rth_app_set_composite", "rth_app_save_system", "rth_app_set_camera", "rth_app_update_material", "rth_app_update_light_emission", "rth_app_benchmark", "rth_app_screenshot", "rth_app_tonemap", "rth_app_context", "rth_app_stats",
-           "rth_app_update_material_textures", "rth_app_picture", "rth_process_group_id", "rth_app_join_group", "rth_app_group_reduce_mean", "rth_sample_range"]
+           "rth_app_update_material_textures", "rth_app_picture", "rth_process_group_id", "rth_app_join_group", "rth_app_group_reduce_mean", "rth_sample_range",
+           "rth_app_update_instance_transform"]
 
 _lib = None
 
@@ -99,6 +100,7 @@ def lib():
         L.rth_app_update_material_textures.argtypes = [C.c_void_p, C.c_int, C.c_int, C.c_int]
         L.rth_app_picture.argtypes = [C.c_void_p, C.c_char_p, C.POINTER(C.c_uint), C.POINTER(C.c_uint), C.POINTER(C.c_void_p)]
         L.rth_app_update_light_emission.argtypes = [C.c_void_p, C.c_int, C.c_void_p]
+        L.rth_app_update_instance_transform.argtypes = [C.c_void_p, C.c_int, C.c_void_p]
         L.rth_app_render.argtypes = [C.c_void_p, C.c_uint]
         L.rth_app_render.restype = C.c_uint
         L.rth_app_render_calls.argtypes = [C.c_void_p, C.c_uint]
@@ -262,6 +264,14 @@ class App:
         e = np.asarray(emission, dtype=np.float32)
         if self.L.rth_app_update_light_emission(self.h, index, e.ctypes.data_as(C.c_void_p)) != 0:
             raise core.RtcError("updateLight(%d) failed" % index)
+
+    def update_instance_transform(self, i, m):
+        """Moves instance i (the numbering of instance(i)) to the object -> world matrix m (12 floats, row-major 3x4): the instance
+        level is refitted on every device and the accumulation restarts.  Frames already requested are rendered at the old place."""
+        t = np.ascontiguousarray(m, dtype=np.float32).reshape(12)
+        rc = self.L.rth_app_update_instance_transform(self.h, i, t.ctypes.data_as(C.c_void_p))
+        if rc != 0:
+            raise core.RtcError("updateInstanceTransform(%d) failed: %s" % (i, self.L.rth_last_error().decode() if rc == -2 else "index out of range"))
 
     # ---- device side
     def render(self, count=1):

@@ -332,6 +332,14 @@ bool Application::updateLightEmission(int index, const float emission[3])
   return true;
 }
 
+bool Application::updateInstanceTransform(int index, const float matrix[12])
+{
+  if (index < 0 || (size_t)index >= m_flatInstances.size()) return false;
+  std::memcpy(m_flatInstances[index].transform, matrix, sizeof(float) * 12);
+  if (m_raytracer) m_raytracer->updateInstanceTransforms((unsigned int)index, 1u, matrix);
+  return true;
+}
+
 void Application::restartAccumulation() { if (m_raytracer) m_raytracer->updateState(m_state); }
 
 unsigned int Application::render(const unsigned int count)

@@ -39,6 +39,8 @@ public:
   void setCamera(float phi, float theta, float fov, float distance, const float center[3]);
   bool updateMaterial(int index, MaterialGUI const& material);
   bool updateLightEmission(int index, const float emission[3]);
+  // object->world matrix (row-major 3x4) of flattened instance `index` (getFlatInstances); restarts the accumulation
+  bool updateInstanceTransform(int index, const float matrix[12]);
 
   // accessors
   Raytracer* getRaytracer() { return m_raytracer.get(); }

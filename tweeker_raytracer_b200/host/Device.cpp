@@ -310,6 +310,14 @@ void Device::updateMaterial(const int idMaterial, MaterialGUI const& materialGUI
   if (hadCutout != (material.textureCutout != 0) || hadAlbedo != (material.textureAlbedo != 0)) updateHitRecords();   // "changeShader", Device.cpp:1111
 }
 
+void Device::updateInstanceTransforms(const unsigned int first, const unsigned int count, const float* matrices)
+{
+  activateContext();
+  MY_ASSERT((size_t)first + count <= m_instances.size());
+  for (unsigned int i = 0; i < count; ++i) std::memcpy(m_instances[first + i].transform, matrices + 12u * i, sizeof(float) * 12);
+  RTC_CHECK(rtc_ias_update(m_context, m_systemData.topObject, first, count, matrices));
+}
+
 void Device::setState(DeviceState const& state)
 {
   activateContext();

@@ -40,6 +40,9 @@ public:
   virtual void updateCamera(const int idCamera, CameraDefinition const& camera);
   virtual void updateLight(const int idLight, LightDefinition const& light);
   virtual void updateMaterial(const int idMaterial, MaterialGUI const& materialGUI);
+  // B200 extension: object->world matrices (12 floats each) of instances first .. first + count - 1 (the traversal order of
+  // initScene); refits the instance level on the device (rtc_ias_update), stream-ordered behind the launches already enqueued
+  virtual void updateInstanceTransforms(const unsigned int first, const unsigned int count, const float* matrices);
 
   virtual void setState(DeviceState const& state);
   virtual void compositor(Device* other);

@@ -208,6 +208,12 @@ void Raytracer::initState(DeviceState const& state)
 void Raytracer::updateCamera(const int idCamera, CameraDefinition const& camera) { flush(); for (Device* d : m_activeDevices) d->updateCamera(idCamera, camera); m_iterationIndex = 0; }
 void Raytracer::updateLight(const int idLight, LightDefinition const& light) { flush(); for (Device* d : m_activeDevices) d->updateLight(idLight, light); m_iterationIndex = 0; }
 void Raytracer::updateMaterial(const int idMaterial, MaterialGUI const& src) { flush(); for (Device* d : m_activeDevices) d->updateMaterial(idMaterial, src); m_iterationIndex = 0; }
+void Raytracer::updateInstanceTransforms(const unsigned int first, const unsigned int count, const float* matrices)
+{
+  flush();
+  for (Device* d : m_activeDevices) d->updateInstanceTransforms(first, count, matrices);
+  m_iterationIndex = 0;
+}
 void Raytracer::updateState(DeviceState const& state)
 {
   // a new resolution makes the owner free and reallocate the shared frame: no device may still be writing to the old one

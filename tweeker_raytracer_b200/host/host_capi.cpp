@@ -146,6 +146,12 @@ int rth_app_update_light_emission(void* h, int index, const float emission[3])
   try { return static_cast<Application*>(h)->updateLightEmission(index, emission) ? 0 : -1; } catch (std::exception const& e) { g_error = e.what(); return -2; }
 }
 
+// instance `index` in the numbering of rth_app_instance; matrix: object -> world, row-major 3x4
+int rth_app_update_instance_transform(void* h, int index, const float matrix[12])
+{
+  try { return static_cast<Application*>(h)->updateInstanceTransform(index, matrix) ? 0 : -1; } catch (std::exception const& e) { g_error = e.what(); return -2; }
+}
+
 // --- device side (needs a GPU) ---
 unsigned int rth_app_render(void* h, unsigned int count) { return static_cast<Application*>(h)->render(count); }
 // the reference's calling pattern: `calls` times the unchanged `unsigned int Raytracer::render()` (one iteration per call)
