@@ -64,6 +64,7 @@ typedef struct {
   uint64_t kernelLaunches;   /* kernels of this library launched */
   double   lastTraceMs;      /* device time of the last rtc_trace_* call (CUDA events on the context stream) */
   uint64_t stackOverflows;   /* rays whose traversal stack overflowed since the library was loaded; must be 0 */
+  uint64_t cutoutGraphBuilds; /* CUDA graphs of the cutout any-hit rounds captured since the last reset (one per pair) */
 } rtc_stats;
 
 /* BVH statistics of a built scene. */
@@ -146,6 +147,7 @@ int rtc_ias_update(rtc_context* ctx, uint64_t topObject, uint32_t first, uint32_
 int rtc_scene_info_get(rtc_context* ctx, uint64_t topObject, rtc_scene_info* info);
 /* Frees one scene (the instance level and its tables; GAS stay alive until rtc_gas_destroy / context destroy). */
 int rtc_scene_destroy(rtc_context* ctx, uint64_t topObject);
+/* A scene that instances a destroyed GAS can only be destroyed: launches, rtc_trace_* and rtc_ias_update on it fail. */
 int rtc_gas_destroy(rtc_context* ctx, uint32_t gas);
 /*
  * Which hit records an instance uses.  The reference writes the cutout program group (__anyhit__radiance_cutout,

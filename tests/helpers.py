@@ -43,14 +43,16 @@ def scene_path(name):
     return os.path.join(SCENES, "scene_%s.txt" % name)
 
 
-def oracle_scene(app, variant="pinned"):
-    """Feeds the scene an App loaded (geometries, flattened instances, materials, lights, camera, environment) to the oracle."""
+def oracle_scene(app, variant="pinned", instances=None):
+    """Feeds the scene an App loaded (geometries, flattened instances, materials, lights, camera, environment) to the oracle.
+    instances: [(transform, geometry, material, light)] replaces the App's instance list."""
     s = orc.Scene(variant)
     for g in range(app.info.numGeometries):
         attrs, idx = app.geometry(g)
         s.add_geometry(attrs, idx)
-    for i in range(app.info.numInstances):
-        t, g, m, l = app.instance(i)
+    if instances is None:
+        instances = [app.instance(i) for i in range(app.info.numInstances)]
+    for t, g, m, l in instances:
         s.add_instance(t, g, m, l)
     s.set_materials(app.materials())
     s.set_lights(app.lights())

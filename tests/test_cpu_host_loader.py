@@ -33,7 +33,24 @@ def test_libraries_export_every_declared_symbol(built):
     assert declared <= set(core.SYMBOLS), declared - set(core.SYMBOLS)
     Hh = host.lib()
     assert not [s for s in host.SYMBOLS if not hasattr(Hh, s)]
-    assert L.rtc_version() >= 100
+    assert L.rtc_version() == 102
+
+
+def test_stats_layout_matches_the_header(tmp_path):
+    """core.Stats is read through rtc_stats_get, which writes sizeof(rtc_stats) bytes: the binding must have the C compiler's
+    layout of include/rtc_core.h, field for field."""
+    import subprocess
+    names = [name for name, _ in core.Stats._fields_]
+    src = os.path.join(str(tmp_path), "layout.c")
+    with open(src, "w") as f:
+        f.write('#include <stdio.h>\n#include "rtc_core.h"\nint main(void) {\n  printf("%zu\\n", sizeof(rtc_stats));\n')
+        f.writelines('  printf("%%zu\\n", offsetof(rtc_stats, %s));\n' % n for n in names)
+        f.write("  return 0;\n}\n")
+    exe = os.path.join(str(tmp_path), "layout")
+    subprocess.check_call(["gcc", "-std=c99", "-Wall", "-Werror", "-I" + os.path.join(H.ROOT, "include"), "-o", exe, src])
+    got = [int(v) for v in subprocess.check_output([exe]).split()]
+    assert got == [C.sizeof(core.Stats)] + [getattr(core.Stats, n).offset for n in names]
+    assert names[-1] == "cutoutGraphBuilds" and C.sizeof(core.Stats) == 56
 
 
 def test_struct_layouts_match_the_reference_contract(built):

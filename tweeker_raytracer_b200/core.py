@@ -41,7 +41,8 @@ MATH_FUNCTIONS = ["sin", "cos", "atan", "atan2", "acos", "exp", "log", "pow", "d
 
 class Stats(C.Structure):
     _fields_ = [("radianceRays", C.c_uint64), ("shadowRays", C.c_uint64), ("pathSamples", C.c_uint64),
-                ("kernelLaunches", C.c_uint64), ("lastTraceMs", C.c_double), ("stackOverflows", C.c_uint64)]
+                ("kernelLaunches", C.c_uint64), ("lastTraceMs", C.c_double), ("stackOverflows", C.c_uint64),
+                ("cutoutGraphBuilds", C.c_uint64)]
 
 
 class SceneInfo(C.Structure):

@@ -851,7 +851,16 @@ int ensure_wavefront(rtc_context* ctx, uint64_t capacity, bool* outOfMemory)
   WavefrontBuffers& wf = ctx->wf;
   if (outOfMemory) *outOfMemory = false;
   if (wf.capacity >= capacity) return 0;
-  if (wf.base) { RTC_CUDA(cudaStreamSynchronize(ctx->stream)); RTC_CUDA(cudaFree(wf.base)); wf = WavefrontBuffers(); }
+  if (wf.base)
+  {
+    // The any-hit graph holds pointers into both allocations.  The reset below also forgets the any-hit scratch queues, so they
+    // are freed here rather than leaked; they grow with the batch anyway.
+    RTC_CUDA(cudaStreamSynchronize(ctx->stream));
+    release_cutout_graph(ctx);
+    RTC_CUDA(cudaFree(wf.base));
+    if (wf.cutBase) RTC_CUDA(cudaFree(wf.cutBase));
+    wf = WavefrontBuffers();
+  }
   // one allocation, carved into 256-byte aligned SoA arrays
   auto align = [](uint64_t v) { return (v + 255u) & ~(uint64_t)255u; };
   const uint64_t n = capacity;
@@ -959,7 +968,12 @@ int ensure_cutout_buffers(rtc_context* ctx, uint64_t capacity)
 {
   WavefrontBuffers& wf = ctx->wf;
   if (wf.cutCapacity >= capacity) return 0;
-  if (wf.cutBase) { RTC_CUDA(cudaStreamSynchronize(ctx->stream)); RTC_CUDA(cudaFree(wf.cutBase)); wf.cutBase = nullptr; wf.cutCapacity = 0; }
+  if (wf.cutBase)
+  {
+    RTC_CUDA(cudaStreamSynchronize(ctx->stream));
+    release_cutout_graph(ctx);         // it captured pointers into this allocation
+    RTC_CUDA(cudaFree(wf.cutBase)); wf.cutBase = nullptr; wf.cutCapacity = 0;
+  }
   const uint64_t q = (4 * capacity + 255u) & ~(uint64_t)255u;
   void* base = nullptr;
   RTC_CUDA(cudaMalloc(&base, 2 * q + 256));
@@ -977,21 +991,22 @@ inline CutoutNext* cutout_next(const WavefrontBuffers& wf) { return reinterpret_
 // conditional WHILE node whose body holds two rounds (the ping-pong of the two scratch queues makes every kernel argument
 // static) and whose condition is set on the device from the ignored-candidate counter (cudaGraphSetConditional).  No host
 // synchronisation: a launch of a scene with cutout materials is as asynchronous as any other.  One graph pair per wavefront
-// allocation / scene / SystemData, rebuilt when one of them changes.
+// allocation / scene / SystemData (without iterationIndex, which no captured kernel reads), captured again when one of them
+// changes.  The graph is released wherever what it points at is freed (wavefront or scratch regrowth, rtc_scene_destroy), so a
+// new allocation or scene that happens to get the old address is never served by a stale capture.
 struct CutoutGraph
 {
   cudaGraphExec_t radiance = nullptr, shadow = nullptr;
   cudaGraph_t radianceGraph = nullptr, shadowGraph = nullptr;
   const void* wfBase = nullptr; const void* cutBase = nullptr; const void* scene = nullptr;
-  rt_SystemData sys{};
+  rt_SystemData sys{};       // iterationIndex zeroed
   int grid = 0;
 };
 
-int build_cutout_loop(rtc_context* ctx, const SceneRecord* scene, const WfArgs& a, int grid, bool shadow, cudaGraph_t* outGraph, cudaGraphExec_t* outExec)
+// Adds the WHILE loop of the any-hit rounds to `graph`; the caller owns the graph (and destroys it when this fails).
+int fill_cutout_loop(rtc_context* ctx, const SceneRecord* scene, const WfArgs& a, int grid, bool shadow, cudaGraph_t graph)
 {
   const WavefrontBuffers& wf = ctx->wf;
-  cudaGraph_t graph = nullptr;
-  RTC_CUDA(cudaGraphCreate(&graph, 0));
   cudaGraphConditionalHandle handle;
   RTC_CUDA(cudaGraphConditionalHandleCreate(&handle, graph, 0, cudaGraphCondAssignDefault));
   // root: the condition from round 1's counter
@@ -1012,7 +1027,12 @@ int build_cutout_loop(rtc_context* ctx, const SceneRecord* scene, const WfArgs& 
   // body: two rounds, captured from the ordinary launch code
   const bool wasProfiling = ctx->profiling;
   ctx->profiling = false;                       // event pairs cannot be timed from inside a graph; the caller brackets the whole loop
-  RTC_CUDA(cudaStreamBeginCaptureToGraph(ctx->stream, body, nullptr, nullptr, 0, cudaStreamCaptureModeRelaxed));
+  const cudaError_t eb = cudaStreamBeginCaptureToGraph(ctx->stream, body, nullptr, nullptr, 0, cudaStreamCaptureModeRelaxed);
+  if (eb != cudaSuccess)
+  {
+    ctx->profiling = wasProfiling;
+    return rtc_set_error(__FILE__, __LINE__, "cudaStreamBeginCaptureToGraph(any-hit rounds)", (int)eb, cudaGetErrorString(eb));
+  }
   int rc = 0;
   for (int o = 0; o < 2 && rc == 0; ++o)
   {
@@ -1033,14 +1053,25 @@ int build_cutout_loop(rtc_context* ctx, const SceneRecord* scene, const WfArgs& 
   ctx->profiling = wasProfiling;
   if (rc != 0 || e != cudaSuccess)
   {
-    cudaGraphDestroy(graph);
     cudaGetLastError();
     if (rc != 0) return rc;
     return rtc_set_error(__FILE__, __LINE__, "cudaStreamEndCapture(any-hit rounds)", (int)e, cudaGetErrorString(e));
   }
+  return 0;
+}
+
+int build_cutout_loop(rtc_context* ctx, const SceneRecord* scene, const WfArgs& a, int grid, bool shadow, cudaGraph_t* outGraph, cudaGraphExec_t* outExec)
+{
+  cudaGraph_t graph = nullptr;
+  RTC_CUDA(cudaGraphCreate(&graph, 0));
+  int rc = fill_cutout_loop(ctx, scene, a, grid, shadow, graph);
   cudaGraphExec_t exec = nullptr;
-  const cudaError_t ei = cudaGraphInstantiate(&exec, graph, 0);
-  if (ei != cudaSuccess) { cudaGraphDestroy(graph); return rtc_set_error(__FILE__, __LINE__, "cudaGraphInstantiate(any-hit rounds)", (int)ei, cudaGetErrorString(ei)); }
+  if (rc == 0)
+  {
+    const cudaError_t ei = cudaGraphInstantiate(&exec, graph, 0);
+    if (ei != cudaSuccess) rc = rtc_set_error(__FILE__, __LINE__, "cudaGraphInstantiate(any-hit rounds)", (int)ei, cudaGetErrorString(ei));
+  }
+  if (rc != 0) { cudaGraphDestroy(graph); return rc; }
   *outGraph = graph; *outExec = exec;
   return 0;
 }
@@ -1060,13 +1091,16 @@ int ensure_cutout_graph(rtc_context* ctx, const SceneRecord* scene, const WfArgs
   CutoutGraph* g = static_cast<CutoutGraph*>(ctx->cutoutGraph);
   if (!g) { g = new CutoutGraph(); ctx->cutoutGraph = g; }
   const WavefrontBuffers& wf = ctx->wf;
-  if (g->radiance && g->wfBase == wf.base && g->cutBase == wf.cutBase && g->scene == scene && g->grid == grid && std::memcmp(&g->sys, &a.sys, sizeof(rt_SystemData)) == 0)
+  rt_SystemData sys = a.sys;
+  sys.iterationIndex = 0;                             // Device::launch writes a new one before every launch
+  if (g->radiance && g->wfBase == wf.base && g->cutBase == wf.cutBase && g->scene == scene && g->grid == grid && std::memcmp(&g->sys, &sys, sizeof(rt_SystemData)) == 0)
     return 0;
   RTC_CUDA(cudaStreamSynchronize(ctx->stream));      // an old graph may still be running
   destroy_cutout_graph(g);
   if (int rc = build_cutout_loop(ctx, scene, a, grid, false, &g->radianceGraph, &g->radiance)) { destroy_cutout_graph(g); return rc; }
   if (int rc = build_cutout_loop(ctx, scene, a, grid, true, &g->shadowGraph, &g->shadow)) { destroy_cutout_graph(g); return rc; }
-  g->wfBase = wf.base; g->cutBase = wf.cutBase; g->scene = scene; g->grid = grid; g->sys = a.sys;
+  g->wfBase = wf.base; g->cutBase = wf.cutBase; g->scene = scene; g->grid = grid; g->sys = sys;
+  ctx->cutoutGraphBuilds++;
   return 0;
 }
 

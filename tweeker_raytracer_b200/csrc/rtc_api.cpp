@@ -36,15 +36,23 @@ void free_scene(SceneRecord* s)
   delete s;
 }
 
-// A scene is stale when one of its GAS was refitted after the scene was built or last updated: its instance boxes and instance
-// level no longer bound the triangles, and its shading table may point at a vertex buffer the caller has since freed.
-bool scene_stale(const rtc_context* ctx, const SceneRecord* s)
-{
-  for (const std::pair<uint32_t, uint64_t>& g : s->gasGeneration) if (ctx->gas[g.first].generation != g.second) return true;
-  return false;
-}
-
+constexpr const char* kDestroyedGas = "a GAS of this scene was destroyed";
 constexpr const char* kStaleScene = "a GAS of this scene was refitted after the scene was built or updated: call rtc_ias_update on the scene first";
+
+// Why the scene cannot be traced, or nullptr.  A GAS it instances was destroyed: its nodes and triangles are freed, and the
+// scene's instance records still point at them.  Or (unless `refitAllowed`, for rtc_ias_update, which cures it) the scene is
+// stale: a GAS was refitted after the scene was built or last updated, so its instance boxes and instance level no longer
+// bound the triangles, and its shading table may point at a vertex buffer the caller has since freed.
+const char* scene_unusable(const rtc_context* ctx, const SceneRecord* s, bool refitAllowed = false)
+{
+  bool stale = false;
+  for (const std::pair<uint32_t, uint64_t>& g : s->gasGeneration)
+  {
+    if (ctx->gas[g.first].d_nodes == nullptr) return kDestroyedGas;
+    stale = stale || ctx->gas[g.first].generation != g.second;
+  }
+  return (stale && !refitAllowed) ? kStaleScene : nullptr;
+}
 
 // the host copy of a GAS's bounds after a refit left them on the device (synchronises the stream; build paths only)
 int fetch_gas_bounds(rtc_context* ctx, GasRecord& g)
@@ -108,7 +116,7 @@ int profile_end(rtc_context* ctx)
 
 extern "C" {
 
-int rtc_version(void) { return 101; }
+int rtc_version(void) { return 102; }
 
 const char* rtc_last_error(void) { return g_lastError.c_str(); }
 
@@ -489,8 +497,7 @@ int rtc_ias_update(rtc_context* ctx, uint64_t topObject, uint32_t first, uint32_
   const uint32_t n = s->desc.numInstances;
   if ((uint64_t)first + count > n) RTC_FAIL("instance range out of bounds");
   if (count && !transforms) RTC_FAIL("transforms is null");
-  for (const std::pair<uint32_t, uint64_t>& g : s->gasGeneration)
-    if (ctx->gas[g.first].d_nodes == nullptr) RTC_FAIL("a GAS of this scene was destroyed");
+  if (const char* why = scene_unusable(ctx, s, true)) RTC_FAIL(why);
   RTC_CUDA(cudaSetDevice(ctx->device));
   for (uint32_t i = first; i < first + count; ++i)
   {
@@ -540,6 +547,7 @@ int rtc_scene_destroy(rtc_context* ctx, uint64_t topObject)
     if ((uint64_t)(uintptr_t)ctx->scenes[i]->d_desc == topObject)
     {
       RTC_CUDA(cudaStreamSynchronize(ctx->stream));
+      release_cutout_graph(ctx);          // it may have captured this scene's tables; a later scene can get the same addresses
       free_scene(ctx->scenes[i]);
       ctx->scenes.erase(ctx->scenes.begin() + (long)i);
       return 0;
@@ -655,7 +663,7 @@ int rtc_launch(rtc_context* ctx, const rt_SystemData* sys, uint32_t launchWidth,
   if (raygen != RTC_RAYGEN_FULL_FRAME && raygen != RTC_RAYGEN_LOCAL_COPY) RTC_FAIL("bad raygen selector");
   if (miss < RT_MISS_NULL || miss > RT_MISS_SPHERE) RTC_FAIL("bad miss selector");
   if (miss == RT_MISS_SPHERE && (sys->envTexture == 0 || sys->envCDF_U == 0 || sys->envCDF_V == 0)) RTC_FAIL("miss 2 needs envTexture/envCDF_U/envCDF_V");
-  if (const SceneRecord* s = find_scene(ctx, sys->topObject)) { if (scene_stale(ctx, s)) RTC_FAIL(kStaleScene); }
+  if (const SceneRecord* s = find_scene(ctx, sys->topObject)) { if (const char* why = scene_unusable(ctx, s)) RTC_FAIL(why); }
   RTC_CUDA(cudaSetDevice(ctx->device));
   return launch_wavefront(ctx, *sys, launchWidth, launchHeight, raygen, miss, iterationFirst, iterationCount, iterationFirst, false);
 }
@@ -668,7 +676,7 @@ int rtc_launch_ex(rtc_context* ctx, const rt_SystemData* sys, uint32_t launchWid
   if (miss < RT_MISS_NULL || miss > RT_MISS_SPHERE) RTC_FAIL("bad miss selector");
   if (miss == RT_MISS_SPHERE && (sys->envTexture == 0 || sys->envCDF_U == 0 || sys->envCDF_V == 0)) RTC_FAIL("miss 2 needs envTexture/envCDF_U/envCDF_V");
   if (accumulationFirst < 0) RTC_FAIL("accumulationFirst < 0");
-  if (const SceneRecord* s = find_scene(ctx, sys->topObject)) { if (scene_stale(ctx, s)) RTC_FAIL(kStaleScene); }
+  if (const SceneRecord* s = find_scene(ctx, sys->topObject)) { if (const char* why = scene_unusable(ctx, s)) RTC_FAIL(why); }
   RTC_CUDA(cudaSetDevice(ctx->device));
   return launch_wavefront(ctx, *sys, launchWidth, launchHeight, raygen, miss, iterationFirst, iterationCount, accumulationFirst, countWork != 0);
 }
@@ -780,7 +788,7 @@ int rtc_trace_closest(rtc_context* ctx, uint64_t topObject, uint64_t rays, uint6
 {
   SceneRecord* s = find_scene(ctx, topObject);
   if (!s) RTC_FAIL("unknown topObject");
-  if (scene_stale(ctx, s)) RTC_FAIL(kStaleScene);
+  if (const char* why = scene_unusable(ctx, s)) RTC_FAIL(why);
   RTC_CUDA(cudaSetDevice(ctx->device));
   RTC_CUDA(cudaEventRecord(ctx->evA, ctx->stream));
   if (int rc = launch_trace_closest(ctx, &s->desc, (const rtc_ray*)(uintptr_t)rays, numRays, (rtc_hit*)(uintptr_t)hits)) return rc;
@@ -793,7 +801,7 @@ int rtc_trace_any(rtc_context* ctx, uint64_t topObject, uint64_t rays, uint64_t 
 {
   SceneRecord* s = find_scene(ctx, topObject);
   if (!s) RTC_FAIL("unknown topObject");
-  if (scene_stale(ctx, s)) RTC_FAIL(kStaleScene);
+  if (const char* why = scene_unusable(ctx, s)) RTC_FAIL(why);
   RTC_CUDA(cudaSetDevice(ctx->device));
   RTC_CUDA(cudaEventRecord(ctx->evA, ctx->stream));
   if (int rc = launch_trace_any(ctx, &s->desc, (const rtc_ray*)(uintptr_t)rays, numRays, (uint32_t*)(uintptr_t)occluded)) return rc;
@@ -807,7 +815,7 @@ int rtc_trace_count(rtc_context* ctx, uint64_t topObject, uint64_t rays, uint64_
   SceneRecord* s = find_scene(ctx, topObject);
   if (!s) RTC_FAIL("unknown topObject");
   if (!out) RTC_FAIL("out is null");
-  if (scene_stale(ctx, s)) RTC_FAIL(kStaleScene);
+  if (const char* why = scene_unusable(ctx, s)) RTC_FAIL(why);
   RTC_CUDA(cudaSetDevice(ctx->device));
   unsigned long long* d = ctx->d_launchCounts + 2 * kTraceCountWords;
   RTC_CUDA(cudaMemsetAsync(d, 0, kTraceCountWords * sizeof(uint64_t), ctx->stream));
@@ -873,7 +881,7 @@ int rtc_stats_get(rtc_context* ctx, rtc_stats* out)
     ctx->lastTraceMs = ms;
   }
   out->radianceRays = h[0]; out->shadowRays = h[1]; out->pathSamples = h[2];
-  out->kernelLaunches = ctx->kernelLaunches; out->lastTraceMs = ctx->lastTraceMs;
+  out->kernelLaunches = ctx->kernelLaunches; out->lastTraceMs = ctx->lastTraceMs; out->cutoutGraphBuilds = ctx->cutoutGraphBuilds;
   return read_stack_overflows(ctx, &out->stackOverflows);
 }
 
@@ -882,6 +890,7 @@ int rtc_stats_reset(rtc_context* ctx)
   RTC_CUDA(cudaSetDevice(ctx->device));
   RTC_CUDA(cudaMemsetAsync(ctx->d_stats, 0, 4 * sizeof(uint64_t), ctx->stream));
   ctx->kernelLaunches = 0;
+  ctx->cutoutGraphBuilds = 0;
   return 0;
 }
 

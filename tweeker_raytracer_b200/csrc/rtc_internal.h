@@ -202,6 +202,7 @@ struct rtc_context
   int    traceSchedule = 0;                       // RTC_SCHEDULE_*: how the lane-owned driver times its triangle tests (what the NEXT launch uses)
   ScheduleTuner tuner;                            // picks traceSchedule by timing one batch with each (kernels_shade.cu, "schedule tuner")
   void*  cutoutGraph = nullptr;                   // CutoutGraph (kernels_shade.cu): the device-side loop of the ordered any-hit rounds
+  uint64_t cutoutGraphBuilds = 0;                 // graph pairs captured since the last rtc_stats_reset (rtc_stats)
 };
 
 // work counters of one traversal kernel: {nodes, tris, insts, rays}

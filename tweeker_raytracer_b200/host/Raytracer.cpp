@@ -280,6 +280,7 @@ void Raytracer::getStats(rtc_stats& total)
     rtc_stats s; device->getStats(s);
     total.radianceRays += s.radianceRays; total.shadowRays += s.shadowRays; total.pathSamples += s.pathSamples;
     total.kernelLaunches += s.kernelLaunches; total.lastTraceMs = s.lastTraceMs; total.stackOverflows += s.stackOverflows;
+    total.cutoutGraphBuilds += s.cutoutGraphBuilds;
   }
 }
 
