@@ -144,6 +144,19 @@ int rtc_ias_build(rtc_context* ctx, const rtc_instance_desc* instances, uint32_t
  */
 int rtc_gas_refit(rtc_context* ctx, uint32_t gas, uint64_t attributes);
 int rtc_ias_update(rtc_context* ctx, uint64_t topObject, uint32_t first, uint32_t count, const float* transforms);
+/*
+ * rtc_ias_rebuild: a new TOPOLOGY for the scene's instance level, built on the device (LBVH, one instance per leaf slot) over the
+ *   instance boxes of the last rtc_ias_build / rtc_ias_update, written in place: topObject, the tables, instance flags and every
+ *   SystemData that holds topObject stay valid, and hits are bit-identical (closest hit does not depend on the node order, any
+ *   hit is a boolean); only the nodes, the leaf order and the traversal cost change.  Use it after large motion, which a refit
+ *   handles badly (DESIGN.md section 3): animate with rtc_ias_update, then rtc_ias_rebuild.  Asynchronous on the context stream,
+ *   like the refits; the first rebuild of a scene allocates its build arrays and a node array of the worst-case size and
+ *   synchronises once.  Two rebuilds of the same boxes give the same bytes (rtc_host_ias_rebuild reproduces them).  Refused, as
+ *   launches are, for a scene with a GAS refitted since its last update and for a scene that instances a destroyed GAS.
+ *   After a rebuild the instance level's node count lives on the device: rtc_scene_info_get and rtc_scene_export read it back
+ *   and therefore synchronise the stream.
+ */
+int rtc_ias_rebuild(rtc_context* ctx, uint64_t topObject);
 int rtc_scene_info_get(rtc_context* ctx, uint64_t topObject, rtc_scene_info* info);
 /* Frees one scene (the instance level and its tables; GAS stay alive until rtc_gas_destroy / context destroy). */
 int rtc_scene_destroy(rtc_context* ctx, uint64_t topObject);
@@ -206,6 +219,9 @@ int  rtc_host_ias_build(const float* transforms, const rtc_host_accel* const* ge
  * rtc_host_ias_refit: every instance's transform and geometry (numInstances = the build's; geometry[i] may have been refitted). */
 int  rtc_host_gas_refit(rtc_host_accel* accel, const void* attributes, uint32_t strideBytes);
 int  rtc_host_ias_refit(rtc_host_accel* accel, const float* transforms, const rtc_host_accel* const* geometry, uint32_t numInstances);
+/* Host-only twin of rtc_ias_rebuild, on an instance-level accel (after rtc_host_ias_build or rtc_host_ias_refit): the same LBVH
+ * over the same boxes in the same float arithmetic, so nodes and leaves equal the device rebuild's byte for byte. */
+int  rtc_host_ias_rebuild(rtc_host_accel* accel);
 int  rtc_host_accel_info(const rtc_host_accel* accel, uint64_t* numNodes, uint64_t* numPrims, float bounds[6]);
 int  rtc_host_accel_export(const rtc_host_accel* accel, void* nodes, uint32_t* primOrder, float* tris, float* worldToObject);
 void rtc_host_accel_destroy(rtc_host_accel* accel);

@@ -7,8 +7,12 @@
     rtc_gas_refit ms, and incoherent closest-hit Mrays/s after a smooth per-vertex displacement of 0, 0.5 and 2 mean edge lengths,
     refitted against rebuilt (the hits of the two are checked to be equal in the same run);
   * the 10 001-instance scene (tools/make_instances_scene.py): rtc_ias_build ms against rtc_ias_update ms with every instance and
-    with 1 % of them moved, and incoherent closest-hit Mrays/s through the scene after 1, 10 and 100 animation steps of small
-    rotations, refitted against rebuilt.
+    with 1 % of them moved and against rtc_ias_rebuild ms, and incoherent closest-hit Mrays/s through the scene after 1, 10 and 100
+    animation steps of small rotations and after a random permutation of the tori's transforms (same boxes, no spatial coherence
+    left in the built topology): refitted, rebuilt on the device (rtc_ias_rebuild) and rebuilt by rtc_ias_build, whose hits are
+    checked to be equal in the same run;
+  * about a million small instances (a 12-triangle box on a jittered lattice): rtc_ias_build ms (one run) against
+    rtc_ias_update ms of every instance and rtc_ias_rebuild ms.
 Builds are timed on the host clock (they end in a synchronisation); refits, updates and traces between CUDA events on the
 context stream, each the median of `repeats` runs after one warm-up.
 """
@@ -179,14 +183,36 @@ def instance_runs(ctx, nrays, repeats):
     all_ms = timed(ctx, lambda: ctx.ias_update(top, moved), repeats)
     few = max(1, n // 100)
     few_ms = timed(ctx, lambda: ctx.ias_update(top, moved[:few]), repeats)
-    emit(what="ias_build_vs_update", instances=n, build_ms=build_ms, update_all_ms=all_ms, update_1pct_ms=few_ms,
-         speedup_all=build_ms / all_ms, speedup_1pct=build_ms / few_ms)
+    spare = ctx.ias_build(descs(xf0))
+    rebuild_ms = timed(ctx, lambda: ctx.ias_rebuild(spare), repeats)             # the warm-up is the scene's first rebuild
+    ctx.scene_destroy(spare)
+    emit(what="ias_build_vs_update", instances=n, build_ms=build_ms, update_all_ms=all_ms, update_1pct_ms=few_ms, rebuild_ms=rebuild_ms,
+         speedup_all=build_ms / all_ms, speedup_1pct=build_ms / few_ms, build_over_rebuild=build_ms / rebuild_ms)
 
     lo, hi = xf0[:, [3, 7, 11]].min(axis=0) - 1.0, xf0[:, [3, 7, 11]].max(axis=0) + 1.0
     rays = bench.rays_numpy(nrays, "incoh", "closest")
     for c, k in zip("xyz", range(3)):
         rays["o" + c] = lo[k] + rays["o" + c] * (hi[k] - lo[k])
     d_rays, d_hits, d_hits2 = ctx.to_device(rays), ctx.malloc(20 * nrays), ctx.malloc(20 * nrays)
+    d_hits3 = ctx.malloc(20 * nrays)
+
+    def three_ways(refitted, xf, **row):
+        """Mrays/s of the refitted scene, of a scene rebuilt on the device over the same boxes and of one rtc_ias_build built"""
+        refit_rate = mrays(ctx, refitted, d_rays, nrays, d_hits, repeats)
+        device = ctx.ias_build(descs(xf))
+        ctx.ias_rebuild(device)
+        device_rate = mrays(ctx, device, d_rays, nrays, d_hits3, repeats)
+        fresh = ctx.ias_build(descs(xf))
+        rebuilt_rate = mrays(ctx, fresh, d_rays, nrays, d_hits2, repeats)
+        a = ctx.download(d_hits, np.uint8, 20 * nrays)
+        b = ctx.download(d_hits2, np.uint8, 20 * nrays)
+        c = ctx.download(d_hits3, np.uint8, 20 * nrays)
+        emit(instances=n, rays=nrays, refitted_mrays=refit_rate, device_rebuilt_mrays=device_rate, rebuilt_mrays=rebuilt_rate,
+             refitted_over_rebuilt=refit_rate / rebuilt_rate, device_rebuilt_over_rebuilt=device_rate / rebuilt_rate,
+             hits_equal=bool(np.array_equal(a, b) and np.array_equal(a, c)), **row)
+        ctx.scene_destroy(device)
+        ctx.scene_destroy(fresh)
+
     xf = xf0.copy()
     ctx.ias_update(top, xf)
     done = 0
@@ -195,16 +221,52 @@ def instance_runs(ctx, nrays, repeats):
             xf = step(xf, done)
             ctx.ias_update(top, xf)
             done += 1
-        refit_rate = mrays(ctx, top, d_rays, nrays, d_hits, repeats)
-        fresh = ctx.ias_build(descs(xf))
-        rebuilt_rate = mrays(ctx, fresh, d_rays, nrays, d_hits2, repeats)
-        a = ctx.download(d_hits, np.uint8, 20 * nrays)
-        b = ctx.download(d_hits2, np.uint8, 20 * nrays)
-        emit(what="instances_trace_after_steps", instances=n, steps=steps, rays=nrays, refitted_mrays=refit_rate, rebuilt_mrays=rebuilt_rate,
-             refitted_over_rebuilt=refit_rate / rebuilt_rate, hits_equal=bool(np.array_equal(a, b)))
-        ctx.scene_destroy(fresh)
-    for p in keep + [d_rays, d_hits, d_hits2]:
+        three_ways(top, xf, what="instances_trace_after_steps", steps=steps)
+    # the tori trade places: every box keeps its size, the built topology no longer groups neighbours
+    tori = np.array([i for i, (_, g) in enumerate(insts) if g == insts[-1][1]])
+    permuted = xf0.copy()
+    permuted[tori] = xf0[np.random.default_rng(1).permutation(tori)]
+    ctx.ias_update(top, xf0)
+    ctx.ias_update(top, permuted)
+    three_ways(top, permuted, what="instances_trace_after_permutation")
+    ctx.scene_destroy(top)
+    for p in keep + [d_rays, d_hits, d_hits2, d_hits3]:
         ctx.free(p)
+
+
+def box_mesh(size):
+    v = np.array([[x, y, z] for x in (0, size) for y in (0, size) for z in (0, size)], dtype=np.float32)
+    faces = [(0, 1, 3), (0, 3, 2), (4, 6, 7), (4, 7, 5), (0, 4, 5), (0, 5, 1), (2, 3, 7), (2, 7, 6), (0, 2, 6), (0, 6, 4), (1, 5, 7), (1, 7, 3)]
+    attrs = np.zeros(8, dtype=[("vertex", "f4", 3), ("tangent", "f4", 3), ("normal", "f4", 3), ("texcoord", "f4", 3)])
+    attrs["vertex"] = v
+    return attrs, np.asarray(faces, dtype=np.uint32)
+
+
+def many_instance_runs(ctx, count, repeats):
+    side = int(round(count ** (1.0 / 3.0)))
+    n = side ** 3
+    rng = np.random.default_rng(3)
+    attrs, idx = box_mesh(0.4)
+    d_a, d_i = ctx.to_device(attrs), ctx.to_device(idx)
+    gas = ctx.gas_build(d_a, attrs.dtype.itemsize, len(attrs), d_i, len(idx), core.BUILD_HOST_SAH)
+    g = np.stack(np.meshgrid(*[np.arange(side)] * 3, indexing="ij"), axis=-1).reshape(-1, 3).astype(np.float64)
+    xf = np.zeros((n, 3, 4))
+    xf[:, :, :3] = np.eye(3)
+    xf[:, :, 3] = g + rng.uniform(-0.3, 0.3, size=(n, 3))
+    xf = xf.astype(np.float32).reshape(n, 12)
+    inst = np.zeros(n, dtype=core.INSTANCE_DTYPE)
+    inst["transform"], inst["instanceId"], inst["gas"], inst["lightIndex"] = xf, np.arange(n), gas, -1
+    tops = []
+    build_ms = wall(ctx, lambda: tops.append(ctx.ias_build(inst)), 1)
+    top = tops[0]
+    update_ms = timed(ctx, lambda: ctx.ias_update(top, xf), repeats)
+    rebuild_ms = timed(ctx, lambda: ctx.ias_rebuild(top), repeats)
+    emit(what="many_instances_build_vs_update_vs_rebuild", instances=n, build_ms=build_ms, build_runs=1, update_all_ms=update_ms,
+         rebuild_ms=rebuild_ms, build_over_rebuild=build_ms / rebuild_ms)
+    ctx.scene_destroy(top)
+    ctx.gas_destroy(gas)
+    ctx.free(d_a)
+    ctx.free(d_i)
 
 
 def main():
@@ -213,6 +275,7 @@ def main():
     ap.add_argument("--rays", default="8M")
     ap.add_argument("--repeats", type=int, default=5)
     ap.add_argument("--no-instances", action="store_true")
+    ap.add_argument("--many-instances", default="1M", help="instance count of the small-instance scene (0: skip)")
     args = ap.parse_args()
     scale = {"K": 10 ** 3, "M": 10 ** 6}
     count = lambda s: int(float(s[:-1]) * scale[s[-1]]) if s[-1] in scale else int(s)    # noqa: E731
@@ -224,6 +287,8 @@ def main():
             soup_runs(ctx, count(s), count(args.rays), args.repeats)
         if not args.no_instances:
             instance_runs(ctx, count(args.rays), args.repeats)
+            if count(args.many_instances):
+                many_instance_runs(ctx, count(args.many_instances), args.repeats)
 
 
 if __name__ == "__main__":

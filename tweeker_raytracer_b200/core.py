@@ -34,6 +34,7 @@ SYMBOLS = [
     "rtc_host_gas_build", "rtc_host_ias_build", "rtc_host_accel_info", "rtc_host_accel_export", "rtc_host_accel_destroy",
     "rtc_trace_schedule_get", "rtc_trace_schedule_set",
     "rtc_gas_refit", "rtc_ias_update", "rtc_host_gas_refit", "rtc_host_ias_refit",
+    "rtc_ias_rebuild", "rtc_host_ias_rebuild",
 ]
 
 MATH_FUNCTIONS = ["sin", "cos", "atan", "atan2", "acos", "exp", "log", "pow", "div", "sqrt", "muladd"]     # enum rtc_math_fn
@@ -103,6 +104,7 @@ def lib():
         L.rtc_ias_build.argtypes = [C.c_void_p, C.c_void_p, C.c_uint32, C.POINTER(C.c_uint64)]
         L.rtc_gas_refit.argtypes = [C.c_void_p, C.c_uint32, C.c_uint64]
         L.rtc_ias_update.argtypes = [C.c_void_p, C.c_uint64, C.c_uint32, C.c_uint32, C.c_void_p]
+        L.rtc_ias_rebuild.argtypes = [C.c_void_p, C.c_uint64]
         L.rtc_scene_info_get.argtypes = [C.c_void_p, C.c_uint64, C.POINTER(SceneInfo)]
         L.rtc_scene_destroy.argtypes = [C.c_void_p, C.c_uint64]
         L.rtc_scene_set_instance_flags.argtypes = [C.c_void_p, C.c_uint64, C.c_uint32, C.c_uint32, C.c_void_p]
@@ -137,6 +139,7 @@ def lib():
         L.rtc_host_ias_build.argtypes = [C.c_void_p, C.c_void_p, C.c_uint32, C.POINTER(C.c_void_p)]
         L.rtc_host_gas_refit.argtypes = [C.c_void_p, C.c_void_p, C.c_uint32]
         L.rtc_host_ias_refit.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p, C.c_uint32]
+        L.rtc_host_ias_rebuild.argtypes = [C.c_void_p]
         L.rtc_host_accel_info.argtypes = [C.c_void_p, C.POINTER(C.c_uint64), C.POINTER(C.c_uint64), C.c_void_p]
         L.rtc_host_accel_export.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]
         L.rtc_host_accel_destroy.argtypes = [C.c_void_p]
@@ -239,6 +242,34 @@ def host_scene_refit_export(geometries, instances, new_attributes, new_transform
     return export, info
 
 
+def host_scene_rebuild_export(geometries, instances, steps):
+    """host_scene_export of the scene built from (geometries, instances), then taken WITHOUT a GPU through `steps`, in order:
+    "rebuild" (rtc_host_ias_rebuild, the twin of rtc_ias_rebuild) or (new_attributes, new_transforms), a refit as in
+    host_scene_refit_export (rtc_gas_refit of the geometries given, then rtc_ias_update of every instance)."""
+    L = lib()
+    accels, info = [], {}
+    try:
+        top, inst_gas = _host_build(L, geometries, instances, accels)
+        accels.append(top)
+        handles = (C.c_void_p * max(len(inst_gas), 1))(*[accels[int(g)] for g in inst_gas])
+        for step in steps:
+            if isinstance(step, str) and step == "rebuild":
+                _check(L.rtc_host_ias_rebuild(top))
+                continue
+            new_attributes, new_transforms = step
+            for g, attrs in enumerate(new_attributes):
+                if attrs is not None:
+                    attrs, stride = _vertex_records(attrs)
+                    _check(L.rtc_host_gas_refit(accels[g], attrs.ctypes.data_as(C.c_void_p), stride))
+            transforms = np.ascontiguousarray(new_transforms, dtype=np.float32).reshape(len(inst_gas), 12)
+            _check(L.rtc_host_ias_refit(top, transforms.ctypes.data_as(C.c_void_p), C.cast(handles, C.c_void_p), len(inst_gas)))
+        export = _host_export(L, accels[:-1], top, inst_gas, info)
+    finally:
+        for h in accels:
+            L.rtc_host_accel_destroy(h)
+    return export, info
+
+
 def device_count():
     n = C.c_int(0)
     rc = lib().rtc_device_count(C.byref(n))
@@ -333,6 +364,11 @@ class Context:
         bring the scene up to date with refitted GAS)."""
         t = np.ascontiguousarray(transforms, dtype=np.float32).reshape(-1, 12)
         _check(self.L.rtc_ias_update(self.h, int(top), first, len(t), t.ctypes.data_as(C.c_void_p) if len(t) else None))
+
+    def ias_rebuild(self, top):
+        """rtc_ias_rebuild: a new instance-level topology over the instance boxes of the last build / update, on the device and
+        in place (`top` stays valid, hits do not change).  Asynchronous, except for the first rebuild of a scene."""
+        _check(self.L.rtc_ias_rebuild(self.h, int(top)))
 
     def gas_destroy(self, gas):
         _check(self.L.rtc_gas_destroy(self.h, gas))

@@ -8,6 +8,8 @@
 #include "rtc_internal.h"
 #include "bvh_rules.h"
 
+#include <algorithm>
+#include <cfloat>
 #include <cmath>
 #include <cstdlib>
 #include <cstring>
@@ -134,6 +136,7 @@ struct rtc_host_accel
   std::vector<uint32_t> indices;        // geometry level: the build's index triplets (for the refit)
   uint32_t numVerts = 0, numTris = 0, strideBytes = 0;
   std::vector<float> inverses;          // instance level: 12 floats per instance
+  std::vector<PrimBox> boxes;           // instance level: the padded instance boxes of the last build / refit (for the rebuild)
 };
 
 // world->object matrices and padded world boxes of every instance, as rtc_ias_build computes them; false on a bad geometry handle
@@ -186,6 +189,7 @@ int rtc_host_ias_build(const float* transforms, const rtc_host_accel* const* geo
   std::vector<PrimBox> boxes;
   if (!instance_boxes_host(transforms, geometry, numInstances, a->inverses, boxes)) { delete a; RTC_FAIL("bad geometry handle in instance"); }
   tlas_build_host(boxes.data(), numInstances, a->bvh);
+  a->boxes = std::move(boxes);
   *out = a;
   return 0;
 }
@@ -229,6 +233,7 @@ int rtc_host_ias_refit(rtc_host_accel* accel, const float* transforms, const rtc
   if (numInstances && (!transforms || !geometry)) RTC_FAIL("null input array");
   std::vector<PrimBox> boxes;
   if (!instance_boxes_host(transforms, geometry, numInstances, accel->inverses, boxes)) RTC_FAIL("bad geometry handle in instance");
+  accel->boxes = boxes;
   if (numInstances == 0) return 0;
   const std::vector<uint32_t>& leaves = accel->bvh.primOrder;
   refit_host(accel->bvh, [&](uint32_t first, uint32_t count, float lo[3], float hi[3]) {
@@ -239,6 +244,85 @@ int rtc_host_ias_refit(rtc_host_accel* accel, const float* transforms, const rtc
       for (int k = 0; k < 3; ++k) { lo[k] = b.lo[k] < lo[k] ? b.lo[k] : lo[k]; hi[k] = hi[k] < b.hi[k] ? b.hi[k] : hi[k]; }
     }
   });
+  return 0;
+}
+
+// The steps of bvh_build_ias_gpu.cu on host arrays: centre bounds, Morton codes, a stable sort, the radix tree, the fit (min / max,
+// exact in any order) and the breadth-first collapse, whose running counters are the device's per-level exclusive scans.
+int rtc_host_ias_rebuild(rtc_host_accel* accel)
+{
+  if (!accel || !accel->isInstanceLevel) RTC_FAIL("not an instance-level accel");
+  const std::vector<PrimBox>& boxes = accel->boxes;
+  const int n = (int)boxes.size();
+  if (n == 0) return 0;
+  std::vector<float4> lo(n), hi(n);
+  float centreBox[6] = { FLT_MAX, FLT_MAX, FLT_MAX, -FLT_MAX, -FLT_MAX, -FLT_MAX };
+  for (int i = 0; i < n; ++i)
+  {
+    const PrimBox& b = boxes[i];
+    lo[i] = make_float4(b.lo[0], b.lo[1], b.lo[2], 0.0f);
+    hi[i] = make_float4(b.hi[0], b.hi[1], b.hi[2], 0.0f);
+    for (int k = 0; k < 3; ++k)
+    {
+      const float c = 0.5f * (b.lo[k] + b.hi[k]);
+      centreBox[k] = std::fmin(centreBox[k], c); centreBox[3 + k] = std::fmax(centreBox[3 + k], c);
+    }
+  }
+  std::vector<unsigned long long> code(n);
+  std::vector<uint32_t> order(n);
+  for (int i = 0; i < n; ++i) { code[i] = lbvh_morton(lo[i], hi[i], centreBox); order[i] = (uint32_t)i; }
+  std::stable_sort(order.begin(), order.end(), [&](uint32_t a, uint32_t b) { return code[a] < code[b]; });
+  std::vector<unsigned long long> keys(n);
+  for (int p = 0; p < n; ++p) keys[p] = code[order[p]];
+
+  // binary tree: ids 0..n-2 internal, n-1..2n-2 leaves; the fit climbs from every leaf, the second child to arrive carries on
+  std::vector<int2> child(n > 1 ? n - 1 : 1), range(n > 1 ? n - 1 : 1);
+  std::vector<int> parent(2 * (size_t)n, -1);
+  for (int i = 0; i < n - 1; ++i) lbvh_radix_node(keys.data(), n, i, child.data(), parent.data(), range.data());
+  std::vector<PrimBox> box(2 * (size_t)n);
+  std::vector<uint8_t> arrived(n, 0);
+  for (int p = 0; p < n; ++p)
+  {
+    box[n - 1 + p] = boxes[order[p]];
+    if (n == 1) break;
+    for (int node = parent[n - 1 + p]; node >= 0; node = parent[node])
+    {
+      if (!arrived[node]++) break;
+      const PrimBox &a = box[child[node].x], &b = box[child[node].y];
+      for (int k = 0; k < 3; ++k) { box[node].lo[k] = std::fmin(a.lo[k], b.lo[k]); box[node].hi[k] = std::fmax(a.hi[k], b.hi[k]); }
+    }
+  }
+
+  WideBvh& out = accel->bvh;
+  out.nodes.assign(1, Node8());
+  out.primOrder.assign(n, 0u);
+  std::vector<int2> work(1, make_int2(0, 0)), next;
+  uint32_t numNodes = 1, numLeaves = 0;
+  while (!work.empty())
+  {
+    next.clear();
+    for (const int2& item : work)
+    {
+      int kidAt[8];
+      Node8 node;
+      uint32_t numInner, nodeLeaves;
+      lbvh_instance_node(item.x, n,
+                         [&](int id, float l[3], float h[3]) { for (int k = 0; k < 3; ++k) { l[k] = box[id].lo[k]; h[k] = box[id].hi[k]; } },
+                         [&](int id) { return child[id]; }, kidAt, node, numInner, nodeLeaves);
+      if (numInner) node.childBase = numNodes;
+      if (nodeLeaves) node.triBase = numLeaves;
+      for (int s = 0; s < 8; ++s)
+      {
+        if (kidAt[s] < 0) continue;
+        if (kidAt[s] >= n - 1) out.primOrder[numLeaves++] = order[kidAt[s] - (n - 1)];
+        else next.push_back(make_int2(kidAt[s], (int)numNodes++));
+      }
+      out.nodes[item.y] = node;
+    }
+    out.nodes.resize(numNodes);
+    work.swap(next);
+  }
+  for (int k = 0; k < 3; ++k) { out.lo[k] = box[0].lo[k]; out.hi[k] = box[0].hi[k]; }
   return 0;
 }
 

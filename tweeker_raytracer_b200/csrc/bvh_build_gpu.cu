@@ -13,6 +13,7 @@
 // The node format is that of bvh_build_host.cpp; both builders quantise through bvh_rules.h.
 #include "rtc_internal.h"
 #include "bvh_rules.h"
+#include "lbvh.cuh"
 
 #include <cub/device/device_radix_sort.cuh>
 
@@ -26,18 +27,6 @@ namespace {
 
 constexpr int kB = 256;
 constexpr uint32_t kLeafMax = 3;      // a wide leaf child holds 1..3 triangles
-
-// ---- float atomics through the order-preserving integer image -------------------------------------------------
-__device__ __forceinline__ void atomicMinF(float* addr, float v)
-{
-  if (v >= 0.0f) atomicMin(reinterpret_cast<int*>(addr), __float_as_int(v));
-  else           atomicMax(reinterpret_cast<unsigned int*>(addr), __float_as_uint(v));
-}
-__device__ __forceinline__ void atomicMaxF(float* addr, float v)
-{
-  if (v >= 0.0f) atomicMax(reinterpret_cast<int*>(addr), __float_as_int(v));
-  else           atomicMin(reinterpret_cast<unsigned int*>(addr), __float_as_uint(v));
-}
 
 struct BuildArrays
 {
@@ -86,104 +75,6 @@ k_tri_bounds(const uint8_t* __restrict__ verts, uint32_t stride, const uint32_t*
     float a = FLT_MAX, b = -FLT_MAX;
     for (int w = 0; w < kB / 32; ++w) { a = fminf(a, sLo[threadIdx.x][w]); b = fmaxf(b, sHi[threadIdx.x][w]); }
     if (a <= b) { atomicMinF(sceneBox + threadIdx.x, a); atomicMaxF(sceneBox + 3 + threadIdx.x, b); }
-  }
-}
-
-__device__ __forceinline__ unsigned long long spread21(uint32_t v)
-{
-  unsigned long long x = v & 0x1fffffull;
-  x = (x | (x << 32)) & 0x1f00000000ffffull;
-  x = (x | (x << 16)) & 0x1f0000ff0000ffull;
-  x = (x | (x << 8))  & 0x100f00f00f00f00full;
-  x = (x | (x << 4))  & 0x10c30c30c30c30c3ull;
-  x = (x | (x << 2))  & 0x1249249249249249ull;
-  return x;
-}
-
-__global__ void __launch_bounds__(kB)
-k_morton(const float4* __restrict__ triLo, const float4* __restrict__ triHi, uint32_t n, const float* __restrict__ sceneBox,
-         unsigned long long* __restrict__ keys, uint32_t* __restrict__ order)
-{
-  const uint32_t t = blockIdx.x * blockDim.x + threadIdx.x;
-  if (t >= n) return;
-  const float4 lo = triLo[t], hi = triHi[t];
-  const float c[3] = { 0.5f * (lo.x + hi.x), 0.5f * (lo.y + hi.y), 0.5f * (lo.z + hi.z) };
-  uint32_t q[3];
-  for (int k = 0; k < 3; ++k)
-  {
-    const float ext = sceneBox[3 + k] - sceneBox[k];
-    float u = ext > 0.0f ? (c[k] - sceneBox[k]) / ext : 0.5f;
-    u = fminf(fmaxf(u, 0.0f), 1.0f);
-    q[k] = (uint32_t)fminf(u * 2097152.0f, 2097151.0f);
-  }
-  keys[t] = (spread21(q[0]) << 2) | (spread21(q[1]) << 1) | spread21(q[2]);
-  order[t] = t;
-}
-
-// common prefix length of sorted keys i and j, index bits break ties between equal codes
-__device__ __forceinline__ int delta(const unsigned long long* __restrict__ keys, int n, int i, int j)
-{
-  if (j < 0 || j >= n) return -1;
-  const unsigned long long a = keys[i], b = keys[j];
-  if (a != b) return __clzll((long long)(a ^ b));
-  return 64 + __clz(i ^ j);
-}
-
-__global__ void __launch_bounds__(kB)
-k_radix_tree(const unsigned long long* __restrict__ keys, int n, int2* __restrict__ child, int* __restrict__ parent, int2* __restrict__ range)
-{
-  const int i = blockIdx.x * blockDim.x + threadIdx.x;
-  if (i >= n - 1) return;
-  const int d = (delta(keys, n, i, i + 1) - delta(keys, n, i, i - 1)) >= 0 ? 1 : -1;
-  const int dmin = delta(keys, n, i, i - d);
-  int lmax = 2;
-  while (delta(keys, n, i, i + lmax * d) > dmin) lmax <<= 1;
-  int l = 0;
-  for (int t = lmax >> 1; t >= 1; t >>= 1) if (delta(keys, n, i, i + (l + t) * d) > dmin) l += t;
-  const int j = i + l * d;
-  const int dnode = delta(keys, n, i, j);
-  int s = 0;
-  for (int t = (l + 1) >> 1; ; t = (t + 1) >> 1)
-  {
-    if (delta(keys, n, i, i + (s + t) * d) > dnode) s += t;
-    if (t == 1) break;
-  }
-  const int gamma = i + s * d + min(d, 0);
-  const int first = min(i, j), last = max(i, j);
-  const int left = (first == gamma) ? (n - 1 + gamma) : gamma;
-  const int right = (last == gamma + 1) ? (n - 1 + gamma + 1) : (gamma + 1);
-  child[i] = make_int2(left, right);
-  range[i] = make_int2(first, last);
-  parent[left] = i;
-  parent[right] = i;
-  if (i == 0) parent[0] = -1;
-}
-
-__global__ void __launch_bounds__(kB)
-k_fit_boxes(int n, const uint32_t* __restrict__ order, const float4* __restrict__ triLo, const float4* __restrict__ triHi,
-            const int2* __restrict__ child, const int* __restrict__ parent, float4* __restrict__ boxLo, float4* __restrict__ boxHi,
-            uint32_t* __restrict__ flags)
-{
-  const int p = blockIdx.x * blockDim.x + threadIdx.x;
-  if (p >= n) return;
-  const uint32_t t = order[p];
-  float4 lo = triLo[t], hi = triHi[t];
-  int node = n - 1 + p;
-  boxLo[node] = lo; boxHi[node] = hi;
-  if (n == 1) return;
-  __threadfence();
-  node = parent[node];
-  while (node >= 0)
-  {
-    if (atomicAdd(flags + node, 1u) == 0u) return;      // the second child to arrive carries on
-    __threadfence();
-    const int2 c = child[node];
-    const volatile float4* vLo = boxLo; const volatile float4* vHi = boxHi;
-    const float lx = fminf(vLo[c.x].x, vLo[c.y].x), ly = fminf(vLo[c.x].y, vLo[c.y].y), lz = fminf(vLo[c.x].z, vLo[c.y].z);
-    const float hx = fmaxf(vHi[c.x].x, vHi[c.y].x), hy = fmaxf(vHi[c.x].y, vHi[c.y].y), hz = fmaxf(vHi[c.x].z, vHi[c.y].z);
-    boxLo[node] = make_float4(lx, ly, lz, 0.0f); boxHi[node] = make_float4(hx, hy, hz, 0.0f);
-    __threadfence();
-    node = parent[node];
   }
 }
 

@@ -96,11 +96,8 @@ __device__ void refit_one(const RefitParams& P, uint32_t idx)
 
 // One thread per node without inner children; after each node it climbs to the parent, which the LAST child to arrive refits.
 // The arrival counter is reset by that thread, so the next refit starts from zero without a memset.
-__global__ void __launch_bounds__(kB)
-k_refit_nodes(const RefitParams P)
+__device__ __forceinline__ void refit_from(const RefitParams& P, uint32_t i)
 {
-  const uint32_t i = blockIdx.x * blockDim.x + threadIdx.x;
-  if (i >= P.numNodes) return;
   if (P.nodes[5u * (size_t)i].w >> 24) return;          // imask != 0: reached from below
   uint32_t node = i;
   for (;;)
@@ -115,6 +112,23 @@ k_refit_nodes(const RefitParams P)
     __threadfence();
     node = parent;
   }
+}
+
+__global__ void __launch_bounds__(kB)
+k_refit_nodes(const RefitParams P)
+{
+  const uint32_t i = blockIdx.x * blockDim.x + threadIdx.x;
+  if (i >= P.numNodes) return;
+  refit_from(P, i);
+}
+
+// An instance level rtc_ias_rebuild wrote: its node count is on the device, and the nodes above it are not part of the structure.
+__global__ void __launch_bounds__(kB)
+k_refit_nodes_live(const RefitParams P, const uint32_t* __restrict__ numNodes)
+{
+  const uint32_t i = blockIdx.x * blockDim.x + threadIdx.x;
+  if (i >= *numNodes) return;
+  refit_from(P, i);
 }
 
 // ---- instance level: tight world bounds of every instance from its transformed vertices -------------------------
@@ -206,13 +220,15 @@ int alloc_refit_scratch(rtc_context* ctx, RefitScratch& r, const uint4* nodes, u
   return 0;
 }
 
+// liveCount: the device word that holds the node count (numNodes is then the capacity), or null
 int launch_refit_nodes(rtc_context* ctx, const RefitScratch& r, uint4* nodes, uint32_t numNodes, const float4* tris,
-                       const uint32_t* leaves, const PrimBox* primBoxes)
+                       const uint32_t* leaves, const PrimBox* primBoxes, const uint32_t* liveCount = nullptr)
 {
   RefitParams P;
   P.nodes = nodes; P.numNodes = numNodes; P.tris = tris; P.leaves = leaves; P.primBoxes = primBoxes;
   P.parent = r.parent; P.arrivals = r.arrivals; P.box = r.box;
-  k_refit_nodes<<<(numNodes + kB - 1) / kB, kB, 0, ctx->stream>>>(P);
+  if (liveCount) k_refit_nodes_live<<<(numNodes + kB - 1) / kB, kB, 0, ctx->stream>>>(P, liveCount);
+  else           k_refit_nodes<<<(numNodes + kB - 1) / kB, kB, 0, ctx->stream>>>(P);
   ctx->kernelLaunches++;
   RTC_CUDA(cudaGetLastError());
   return 0;
@@ -246,6 +262,7 @@ int refit_instances_gpu(rtc_context* ctx, SceneRecord& s, const std::vector<Inst
   const uint32_t m = (uint32_t)updates.size();
   if (m == 0) return 0;
   uint4* tlas = static_cast<uint4*>(s.d_tlasNodes);
+  // after a rebuild the scratch exists (bvh_build_ias_gpu.cu sized it for the node capacity and keeps its parents up to date)
   if (int rc = alloc_refit_scratch(ctx, s.refit, tlas, s.desc.numTlasNodes)) return rc;
   // inputs of this update: staged from pageable memory by the copy itself, and freed stream-ordered behind the kernels
   std::vector<InstanceBoundsIn> in(tight ? m : 0);
@@ -272,6 +289,9 @@ int refit_instances_gpu(rtc_context* ctx, SceneRecord& s, const std::vector<Inst
   }
   cudaFreeAsync(d, ctx->stream);
   if (e != cudaSuccess) return rtc_set_error(__FILE__, __LINE__, "refit_instances_gpu", (int)e, cudaGetErrorString(e));
+  if (s.rebuild)
+    return launch_refit_nodes(ctx, s.refit, tlas, ias_rebuild_capacity(s.desc.numInstances), nullptr, static_cast<const uint32_t*>(s.d_tlasLeaves), s.d_instBoxes,
+                              s.d_numTlasNodes);
   return launch_refit_nodes(ctx, s.refit, tlas, s.desc.numTlasNodes, nullptr, static_cast<const uint32_t*>(s.d_tlasLeaves), s.d_instBoxes);
 }
 

@@ -1,6 +1,7 @@
-// bvh_rules.h -- arithmetic that the host builder (bvh_build_host.cpp), the device builder (bvh_build_gpu.cu), the device refit
-// (bvh_refit.cu) and the host-only refit twin (accel_host.cpp) must apply bit for bit: the quantisation of one wide node and the
-// padding of an instance's world box.  One definition, compiled for the host and for sm_100a.
+// bvh_rules.h -- arithmetic that the host builder (bvh_build_host.cpp), the device builders (bvh_build_gpu.cu,
+// bvh_build_ias_gpu.cu), the device refit (bvh_refit.cu) and the host-only twins (accel_host.cpp) must apply bit for bit: the
+// quantisation of one wide node, the padding of an instance's world box, and the Morton codes, radix tree and wide nodes of the
+// LBVH.  One definition, compiled for the host and for sm_100a.
 //
 // FMA contraction: every product in quantise_node is by a power of two (step * 2^-4, step * 2^-6 with step >= 2^-120, which
 // stays a normal float) and is therefore exact, so a contracted multiply-add rounds exactly like the separate operations.
@@ -8,6 +9,7 @@
 // -ffp-contract=off and bvh_refit.cu with -fmad=false.
 #pragma once
 
+#include <algorithm>
 #include <cmath>
 #include <cstdint>
 #include <cstring>
@@ -140,4 +142,150 @@ RTC_HD void instance_box_finish(const float transform[12], const float gasLo[3],
     }
   }
   if (emptyGas) { for (int k = 0; k < 3; ++k) { b.lo[k] = 0.0f; b.hi[k] = 0.0f; } }
+}
+
+// ---- LBVH (Karras 2012) ---------------------------------------------------------------------------------------------------------
+RTC_HD unsigned long long lbvh_spread21(uint32_t v)
+{
+  unsigned long long x = v & 0x1fffffull;
+  x = (x | (x << 32)) & 0x1f00000000ffffull;
+  x = (x | (x << 16)) & 0x1f0000ff0000ffull;
+  x = (x | (x << 8))  & 0x100f00f00f00f00full;
+  x = (x | (x << 4))  & 0x10c30c30c30c30c3ull;
+  x = (x | (x << 2))  & 0x1249249249249249ull;
+  return x;
+}
+
+// 63-bit Morton code of the centre of the box (lo, hi) in the frame sceneBox = {lo[3], hi[3]}
+RTC_HD unsigned long long lbvh_morton(const float4 lo, const float4 hi, const float* sceneBox)
+{
+  const float c[3] = { 0.5f * (lo.x + hi.x), 0.5f * (lo.y + hi.y), 0.5f * (lo.z + hi.z) };
+  uint32_t q[3];
+  for (int k = 0; k < 3; ++k)
+  {
+    const float ext = sceneBox[3 + k] - sceneBox[k];
+    float u = ext > 0.0f ? (c[k] - sceneBox[k]) / ext : 0.5f;
+    u = fminf(fmaxf(u, 0.0f), 1.0f);
+    q[k] = (uint32_t)fminf(u * 2097152.0f, 2097151.0f);
+  }
+  return (lbvh_spread21(q[0]) << 2) | (lbvh_spread21(q[1]) << 1) | lbvh_spread21(q[2]);
+}
+
+// common prefix length of sorted keys i and j, index bits break ties between equal codes
+RTC_HD int lbvh_delta(const unsigned long long* __restrict__ keys, int n, int i, int j)
+{
+  if (j < 0 || j >= n) return -1;
+  const unsigned long long a = keys[i], b = keys[j];
+#if defined(__CUDA_ARCH__)
+  if (a != b) return __clzll((long long)(a ^ b));
+  return 64 + __clz(i ^ j);
+#else
+  if (a != b) return __builtin_clzll(a ^ b);
+  return 64 + __builtin_clz((unsigned)(i ^ j));
+#endif
+}
+
+// Internal node i (0 <= i < n - 1) of the binary radix tree over n sorted keys: node ids 0..n-2 are internal (0 = root),
+// n-1..2n-2 the leaves (sorted position p -> n-1+p).
+RTC_HD void lbvh_radix_node(const unsigned long long* __restrict__ keys, int n, int i, int2* __restrict__ child, int* __restrict__ parent,
+                            int2* __restrict__ range)
+{
+  const int d = (lbvh_delta(keys, n, i, i + 1) - lbvh_delta(keys, n, i, i - 1)) >= 0 ? 1 : -1;
+  const int dmin = lbvh_delta(keys, n, i, i - d);
+  int lmax = 2;
+  while (lbvh_delta(keys, n, i, i + lmax * d) > dmin) lmax <<= 1;
+  int l = 0;
+  for (int t = lmax >> 1; t >= 1; t >>= 1) if (lbvh_delta(keys, n, i, i + (l + t) * d) > dmin) l += t;
+  const int j = i + l * d;
+  const int dnode = lbvh_delta(keys, n, i, j);
+  int s = 0;
+  for (int t = (l + 1) >> 1; ; t = (t + 1) >> 1)
+  {
+    if (lbvh_delta(keys, n, i, i + (s + t) * d) > dnode) s += t;
+    if (t == 1) break;
+  }
+#if defined(__CUDA_ARCH__)
+  const int gamma = i + s * d + min(d, 0);
+  const int first = min(i, j), last = max(i, j);
+#else
+  const int gamma = i + s * d + std::min(d, 0);
+  const int first = std::min(i, j), last = std::max(i, j);
+#endif
+  const int left = (first == gamma) ? (n - 1 + gamma) : gamma;
+  const int right = (last == gamma + 1) ? (n - 1 + gamma + 1) : (gamma + 1);
+  child[i] = make_int2(left, right);
+  range[i] = make_int2(first, last);
+  parent[left] = i;
+  parent[right] = i;
+  if (i == 0) parent[0] = -1;
+}
+
+// One wide node of the instance-level LBVH (one instance per leaf slot) over binary node src of the radix tree: the greedy
+// collapse of the geometry builder's k_collapse_level (open the child with the largest surface area until eight remain, octant
+// slots, bvh_rules quantisation).  box(id, lo, hi) yields a binary node's box, child(id) its children.  kidAt[s] = the binary
+// node in slot s or -1; the node gets imask and meta (leaf offsets in slot order), childBase = triBase = 0.
+template <class Box, class Child>
+RTC_HD void lbvh_instance_node(int src, int n, const Box& box, const Child& child, int kidAt[8], Node8& node, uint32_t& numInner,
+                               uint32_t& numLeaves)
+{
+  auto is_leaf = [&](int id) { return id >= n - 1; };
+  auto half_area = [](const float lo[3], const float hi[3]) {
+    const float dx = hi[0] - lo[0], dy = hi[1] - lo[1], dz = hi[2] - lo[2];
+    return dx * dy + dy * dz + dz * dx;
+  };
+  int kids[8]; int nk = 0;
+  float kLo[8][3], kHi[8][3];
+  if (is_leaf(src)) kids[nk++] = src;
+  else { const int2 c = child(src); kids[nk++] = c.x; kids[nk++] = c.y; }
+  for (int i = 0; i < nk; ++i) box(kids[i], kLo[i], kHi[i]);
+  while (nk < 8)
+  {
+    int best = -1; float bestArea = -1.0f;
+    for (int i = 0; i < nk; ++i)
+      if (!is_leaf(kids[i])) { const float a = half_area(kLo[i], kHi[i]); if (a > bestArea) { bestArea = a; best = i; } }
+    if (best < 0) break;
+    const int2 c = child(kids[best]);
+    kids[best] = c.x; kids[nk] = c.y;
+    box(c.x, kLo[best], kHi[best]); box(c.y, kLo[nk], kHi[nk]);
+    ++nk;
+  }
+  float sLo[3], sHi[3];
+  box(src, sLo, sHi);
+  int slotKid[8]; for (int s = 0; s < 8; ++s) slotKid[s] = -1;
+  {
+    float centre[3]; for (int k = 0; k < 3; ++k) centre[k] = 0.5f * (sLo[k] + sHi[k]);
+    uint32_t slotUsed = 0, kidDone = 0;
+    for (int round = 0; round < nk; ++round)
+    {
+      int bi = -1, bs = -1; float bc = -3.402823466e38f;
+      for (int i = 0; i < nk; ++i)
+      {
+        if (kidDone & (1u << i)) continue;
+        const float d0 = 0.5f * (kLo[i][0] + kHi[i][0]) - centre[0], d1 = 0.5f * (kLo[i][1] + kHi[i][1]) - centre[1], d2 = 0.5f * (kLo[i][2] + kHi[i][2]) - centre[2];
+        for (int s = 0; s < 8; ++s)
+        {
+          if (slotUsed & (1u << s)) continue;
+          const float c = ((s & 4) ? d0 : -d0) + ((s & 2) ? d1 : -d1) + ((s & 1) ? d2 : -d2);
+          if (c > bc || bi < 0) { bc = c; bi = i; bs = s; }
+        }
+      }
+      slotKid[bs] = bi; slotUsed |= 1u << bs; kidDone |= 1u << bi;
+    }
+  }
+  uint32_t occupied = 0;
+  for (int s = 0; s < 8; ++s) if (slotKid[s] >= 0) occupied |= 1u << s;
+  float nodeLo[3], nodeHi[3];
+  quantise_node(occupied, [&](int s, float lo[3], float hi[3]) {
+    for (int k = 0; k < 3; ++k) { lo[k] = kLo[slotKid[s]][k]; hi[k] = kHi[slotKid[s]][k]; }
+  }, node, nodeLo, nodeHi);
+  node.imask = 0; node.childBase = 0; node.triBase = 0;
+  numInner = 0; numLeaves = 0;
+  for (int s = 0; s < 8; ++s)
+  {
+    node.meta[s] = 0;
+    kidAt[s] = slotKid[s] >= 0 ? kids[slotKid[s]] : -1;
+    if (kidAt[s] < 0) continue;
+    if (is_leaf(kidAt[s])) { node.meta[s] = (uint8_t)((1u << 5) | numLeaves); ++numLeaves; }
+    else { node.imask |= (uint8_t)(1u << s); ++numInner; }
+  }
 }

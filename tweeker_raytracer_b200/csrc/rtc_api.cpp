@@ -32,7 +32,7 @@ SceneRecord* find_scene(rtc_context* ctx, uint64_t topObject)
 void free_scene(SceneRecord* s)
 {
   cudaFree(s->d_desc); cudaFree(s->d_tlasNodes); cudaFree(s->d_instances); cudaFree(s->d_tlasLeaves); cudaFree(s->d_o2w); cudaFree(s->d_geomInst); cudaFree(s->d_instFlags);
-  cudaFree(s->d_instBoxes); free_refit_scratch(s->refit);
+  cudaFree(s->d_instBoxes); free_refit_scratch(s->refit); free_ias_rebuild(s->rebuild);
   delete s;
 }
 
@@ -63,6 +63,19 @@ int fetch_gas_bounds(rtc_context* ctx, GasRecord& g)
   RTC_CUDA(cudaStreamSynchronize(ctx->stream));
   for (int k = 0; k < 3; ++k) { g.lo[k] = box[k]; g.hi[k] = box[3 + k]; }
   g.boundsOnDevice = false;
+  return 0;
+}
+
+// After rtc_ias_rebuild the instance level's node count is only on the device: bring the host copy (desc.numTlasNodes and the
+// scene's node total) up to date.  Synchronises the stream.
+int sync_tlas_node_count(rtc_context* ctx, SceneRecord* s)
+{
+  if (!s->d_numTlasNodes) return 0;
+  uint32_t count = 0;
+  RTC_CUDA(cudaMemcpyAsync(&count, s->d_numTlasNodes, sizeof(count), cudaMemcpyDeviceToHost, ctx->stream));
+  RTC_CUDA(cudaStreamSynchronize(ctx->stream));
+  s->totalNodes = s->totalNodes - s->desc.numTlasNodes + count;
+  s->desc.numTlasNodes = count;
   return 0;
 }
 
@@ -530,10 +543,21 @@ int rtc_ias_update(rtc_context* ctx, uint64_t topObject, uint32_t first, uint32_
   return 0;
 }
 
+int rtc_ias_rebuild(rtc_context* ctx, uint64_t topObject)
+{
+  SceneRecord* s = find_scene(ctx, topObject);
+  if (!s) RTC_FAIL("unknown topObject");
+  if (const char* why = scene_unusable(ctx, s)) RTC_FAIL(why);
+  RTC_CUDA(cudaSetDevice(ctx->device));
+  return rebuild_instances_gpu(ctx, *s);
+}
+
 int rtc_scene_info_get(rtc_context* ctx, uint64_t topObject, rtc_scene_info* info)
 {
   SceneRecord* s = find_scene(ctx, topObject);
   if (!s) RTC_FAIL("unknown topObject");
+  RTC_CUDA(cudaSetDevice(ctx->device));
+  if (int rc = sync_tlas_node_count(ctx, s)) return rc;
   std::memset(info, 0, sizeof(*info));
   info->numNodes = s->totalNodes; info->numTris = s->totalTris; info->numInstances = s->desc.numInstances;
   info->numTlasNodes = s->desc.numTlasNodes; info->numTlasLeaves = s->desc.numTlasLeaves; info->numGas = s->numGas; info->gasBuildMs = s->gasBuildMs; info->iasBuildMs = s->iasBuildMs;
@@ -618,6 +642,7 @@ int rtc_scene_export(rtc_context* ctx, uint64_t topObject, void* tlasNodes, uint
   if (!s) RTC_FAIL("unknown topObject");
   RTC_CUDA(cudaSetDevice(ctx->device));
   RTC_CUDA(cudaStreamSynchronize(ctx->stream));
+  if (int rc = sync_tlas_node_count(ctx, s)) return rc;
   if (tlasNodes) RTC_CUDA(cudaMemcpy(tlasNodes, s->d_tlasNodes, (size_t)s->desc.numTlasNodes * sizeof(Node8), cudaMemcpyDeviceToHost));
   if (tlasLeaves && s->desc.numTlasLeaves) RTC_CUDA(cudaMemcpy(tlasLeaves, s->d_tlasLeaves, (size_t)s->desc.numTlasLeaves * 4u, cudaMemcpyDeviceToHost));
   if (worldToObject) std::memcpy(worldToObject, s->inverses.data(), s->inverses.size() * sizeof(float));

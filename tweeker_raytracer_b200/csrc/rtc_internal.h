@@ -107,6 +107,8 @@ struct GasRecord
   bool     boundsOnDevice = false;         // lo / hi are stale: the refitted bounds are refit.box[0..5] on the device
 };
 
+struct IasRebuild;
+
 struct SceneRecord
 {
   SceneDesc desc{};          // host copy
@@ -121,6 +123,10 @@ struct SceneRecord
   std::vector<std::pair<uint32_t, uint64_t>> gasGeneration;   // each distinct GAS and its generation at the last build / update
   PrimBox* d_instBoxes = nullptr;          // the padded world box of every instance (leaf boxes of the instance level)
   RefitScratch refit;
+  // rtc_ias_rebuild (bvh_build_ias_gpu.cu): its arrays, made by the first rebuild, and from then on the instance level's node count
+  // on the device -- desc.numTlasNodes is then only brought up to date by sync_tlas_node_count (rtc_api.cpp)
+  IasRebuild* rebuild = nullptr;
+  const uint32_t* d_numTlasNodes = nullptr;
   uint64_t totalNodes = 0, totalTris = 0;  // unique GAS nodes / triangles referenced + instance level
   uint32_t numGas = 0;
   double   gasBuildMs = 0.0, iasBuildMs = 0.0;
@@ -238,6 +244,13 @@ struct InstanceUpdate
 // Writes the matrices, shading-table attributes and padded boxes of the listed instances and refits the instance level.
 int refit_instances_gpu(rtc_context* ctx, SceneRecord& s, const std::vector<InstanceUpdate>& updates, bool tight);
 void free_refit_scratch(RefitScratch& r);
+
+// bvh_build_ias_gpu.cu: a new LBVH topology of the instance level over s.d_instBoxes, in place and stream-ordered; the first call
+// on a scene allocates (and synchronises once), later calls never block the host
+int rebuild_instances_gpu(rtc_context* ctx, SceneRecord& s);
+// the wide nodes its node array holds: every wide node but the root has a sibling-group parent, so one-instance leaves give < n + 16
+inline uint32_t ias_rebuild_capacity(uint32_t numInstances) { return numInstances + 16u; }
+void free_ias_rebuild(IasRebuild* r);
 
 // error plumbing (rtc_api.cpp)
 int rtc_set_error(const char* file, int line, const char* call, int code, const char* text);

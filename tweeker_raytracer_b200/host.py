@@ -59,7 +59,7 @@ SYMBOLS = ["rth_last_error", "rth_app_create", "rth_app_destroy", "rth_app_info"
            "rth_app_environment", "rth_app_render", "rth_app_render_calls", "rth_app_set_coalesce", "rth_app_synchronize", "rth_app_frame", "rth_app_local_frame", "rth_app_restart",
            "rth_app_set_composite", "rth_app_save_system", "rth_app_set_camera", "rth_app_update_material", "rth_app_update_light_emission", "rth_app_benchmark", "rth_app_screenshot", "rth_app_tonemap", "rth_app_context", "rth_app_stats",
            "rth_app_update_material_textures", "rth_app_picture", "rth_process_group_id", "rth_app_join_group", "rth_app_group_reduce_mean", "rth_sample_range",
-           "rth_app_update_instance_transform"]
+           "rth_app_update_instance_transform", "rth_app_rebuild_instance_level"]
 
 _lib = None
 
@@ -101,6 +101,7 @@ def lib():
         L.rth_app_picture.argtypes = [C.c_void_p, C.c_char_p, C.POINTER(C.c_uint), C.POINTER(C.c_uint), C.POINTER(C.c_void_p)]
         L.rth_app_update_light_emission.argtypes = [C.c_void_p, C.c_int, C.c_void_p]
         L.rth_app_update_instance_transform.argtypes = [C.c_void_p, C.c_int, C.c_void_p]
+        L.rth_app_rebuild_instance_level.argtypes = [C.c_void_p]
         L.rth_app_render.argtypes = [C.c_void_p, C.c_uint]
         L.rth_app_render.restype = C.c_uint
         L.rth_app_render_calls.argtypes = [C.c_void_p, C.c_uint]
@@ -272,6 +273,13 @@ class App:
         rc = self.L.rth_app_update_instance_transform(self.h, i, t.ctypes.data_as(C.c_void_p))
         if rc != 0:
             raise core.RtcError("updateInstanceTransform(%d) failed: %s" % (i, self.L.rth_last_error().decode() if rc == -2 else "index out of range"))
+
+    def rebuild_instance_level(self):
+        """Rebuilds the instance level's topology on every device, over the instance boxes of the last update (after large motion,
+        which the refit of update_instance_transform handles badly).  Hits do not change, so the accumulation goes on; iterations
+        already requested are rendered first."""
+        if self.L.rth_app_rebuild_instance_level(self.h) != 0:
+            raise core.RtcError("rebuildInstanceLevel failed: %s" % self.L.rth_last_error().decode())
 
     # ---- device side
     def render(self, count=1):

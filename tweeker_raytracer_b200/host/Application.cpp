@@ -340,6 +340,8 @@ bool Application::updateInstanceTransform(int index, const float matrix[12])
   return true;
 }
 
+void Application::rebuildInstanceLevel() { if (m_raytracer) m_raytracer->rebuildInstanceLevel(); }
+
 void Application::restartAccumulation() { if (m_raytracer) m_raytracer->updateState(m_state); }
 
 unsigned int Application::render(const unsigned int count)

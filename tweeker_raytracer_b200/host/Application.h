@@ -41,6 +41,7 @@ public:
   bool updateLightEmission(int index, const float emission[3]);
   // object->world matrix (row-major 3x4) of flattened instance `index` (getFlatInstances); restarts the accumulation
   bool updateInstanceTransform(int index, const float matrix[12]);
+  void rebuildInstanceLevel();
 
   // accessors
   Raytracer* getRaytracer() { return m_raytracer.get(); }

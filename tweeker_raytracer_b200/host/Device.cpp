@@ -318,6 +318,12 @@ void Device::updateInstanceTransforms(const unsigned int first, const unsigned i
   RTC_CHECK(rtc_ias_update(m_context, m_systemData.topObject, first, count, matrices));
 }
 
+void Device::rebuildInstanceLevel()
+{
+  activateContext();
+  RTC_CHECK(rtc_ias_rebuild(m_context, m_systemData.topObject));
+}
+
 void Device::setState(DeviceState const& state)
 {
   activateContext();

@@ -43,6 +43,7 @@ public:
   // B200 extension: object->world matrices (12 floats each) of instances first .. first + count - 1 (the traversal order of
   // initScene); refits the instance level on the device (rtc_ias_update), stream-ordered behind the launches already enqueued
   virtual void updateInstanceTransforms(const unsigned int first, const unsigned int count, const float* matrices);
+  virtual void rebuildInstanceLevel();
 
   virtual void setState(DeviceState const& state);
   virtual void compositor(Device* other);

@@ -214,6 +214,12 @@ void Raytracer::updateInstanceTransforms(const unsigned int first, const unsigne
   for (Device* d : m_activeDevices) d->updateInstanceTransforms(first, count, matrices);
   m_iterationIndex = 0;
 }
+// A new topology over the same instance boxes: hits, and so frames, do not change, and the accumulation goes on.
+void Raytracer::rebuildInstanceLevel()
+{
+  flush();
+  for (Device* d : m_activeDevices) d->rebuildInstanceLevel();
+}
 void Raytracer::updateState(DeviceState const& state)
 {
   // a new resolution makes the owner free and reallocate the shared frame: no device may still be writing to the old one

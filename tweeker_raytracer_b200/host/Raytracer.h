@@ -41,6 +41,7 @@ public:
   virtual void updateMaterial(const int idMaterial, MaterialGUI const& src);
   // B200 extension (the reference rebuilt nothing after initScene): moves instances first .. first + count - 1
   virtual void updateInstanceTransforms(const unsigned int first, const unsigned int count, const float* matrices);
+  virtual void rebuildInstanceLevel();
   virtual void updateState(DeviceState const& state);
 
   virtual unsigned int render() = 0;                 // one iteration; returns the iterations done so far

@@ -152,6 +152,12 @@ int rth_app_update_instance_transform(void* h, int index, const float matrix[12]
   try { return static_cast<Application*>(h)->updateInstanceTransform(index, matrix) ? 0 : -1; } catch (std::exception const& e) { g_error = e.what(); return -2; }
 }
 
+// a new instance-level topology on every device (after large motion); frames do not change
+int rth_app_rebuild_instance_level(void* h)
+{
+  try { static_cast<Application*>(h)->rebuildInstanceLevel(); return 0; } catch (std::exception const& e) { g_error = e.what(); return -2; }
+}
+
 // --- device side (needs a GPU) ---
 unsigned int rth_app_render(void* h, unsigned int count) { return static_cast<Application*>(h)->render(count); }
 // the reference's calling pattern: `calls` times the unchanged `unsigned int Raytracer::render()` (one iteration per call)
