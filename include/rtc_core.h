@@ -127,8 +127,8 @@ int rtc_gas_build(rtc_context* ctx, uint64_t attributes, uint32_t strideBytes, u
 /* Builds the instance level, the per-instance tables and returns SystemData::topObject. */
 int rtc_ias_build(rtc_context* ctx, const rtc_instance_desc* instances, uint32_t numInstances, uint64_t* topObject);
 /*
- * In-place updates (optixAccelBuild with OPTIX_BUILD_OPERATION_UPDATE).  Both are asynchronous on the context stream and do not
- * synchronise the host, except for a one-time allocation of refit scratch on a structure's first refit: work enqueued before
+ * In-place updates (optixAccelBuild with OPTIX_BUILD_OPERATION_UPDATE).  All are asynchronous on the context stream and do not
+ * synchronise the host, except for a one-time allocation of refit scratch on a GAS's first refit: work enqueued before
  * sees the old structure, work enqueued after sees the new one.  Topology is never changed -- vertex and triangle counts,
  * indices, instance count, the GAS of an instance and materials stay as built; changing them is a rebuild.  Node topology and
  * leaf order stay as built, so traversal cost grows with the size of the deformation (DESIGN.md section 3, "Refit").
@@ -140,10 +140,22 @@ int rtc_ias_build(rtc_context* ctx, const rtc_instance_desc* instances, uint32_t
  * rtc_ias_update: transforms of instances first .. first+count-1 are replaced (count x 12 floats, object->world, row-major; may
  *   be null when count == 0), world->object matrices and shading tables follow, the bounds of every instance whose transform
  *   changed or whose GAS was refitted since the last build / update are recomputed, and the instance level is refitted.
- *   `transforms` may be reused on return.
+ *   `transforms` is host memory, pageable or page-locked (rtc_host_alloc, registered or managed memory), and may be reused on
+ *   return: the call has read it by then.  Device memory is refused: that is rtc_ias_update_device.
+ * rtc_ias_update_device: rtc_ias_update with the matrices in memory the context's GPU can read (its device memory, or mapped
+ *   host memory) -- the counterpart of optixAccelBuild reading OptixInstance records from device memory.  The matrix of instance
+ *   first + i is the 12 floats (object->world, row-major 3x4) at transforms + i * strideBytes; strideBytes is a multiple of 4
+ *   and at least 48: 48 for a dense [count, 12] float array, 80 for an OptixInstance array (its transform[12] is at offset 0,
+ *   the other bytes are ignored).  `transforms` must be 4-byte aligned; it may be 0 when count == 0.
+ *   The buffer is read ON THE CONTEXT STREAM, when the stream reaches the update, not during the call -- the opposite of
+ *   rtc_ias_update.  The caller must have finished writing it by then and must not overwrite it until the update has run: write
+ *   it on the same stream (rtc_context_stream) or order the writer and later writers with events.
+ *   The results are those of rtc_ias_update with the same matrices, byte for byte; everything else is as there (refitted GAS,
+ *   count == 0, refusals).  Never synchronises the host and allocates only from the stream-ordered pool.
  */
 int rtc_gas_refit(rtc_context* ctx, uint32_t gas, uint64_t attributes);
 int rtc_ias_update(rtc_context* ctx, uint64_t topObject, uint32_t first, uint32_t count, const float* transforms);
+int rtc_ias_update_device(rtc_context* ctx, uint64_t topObject, uint32_t first, uint32_t count, uint64_t transforms, uint32_t strideBytes);
 /*
  * rtc_ias_rebuild: a new TOPOLOGY for the scene's instance level, built on the device (LBVH, one instance per leaf slot) over the
  *   instance boxes of the last rtc_ias_build / rtc_ias_update, written in place: topObject, the tables, instance flags and every
@@ -196,7 +208,8 @@ int rtc_texture_destroy(rtc_context* ctx, uint64_t handle);
 int rtc_scene_export(rtc_context* ctx, uint64_t topObject, void* tlasNodes, uint32_t* tlasLeaves, float* worldToObject, uint32_t* instanceGas);
 int rtc_gas_info(rtc_context* ctx, uint32_t gas, uint64_t* numNodes, uint64_t* numTris);
 int rtc_gas_export(rtc_context* ctx, uint32_t gas, void* nodes, float* tris);
-/* Copies out the 3x4 world->object matrix of one instance. */
+/* Copies out the 3x4 world->object matrix of one instance.  The matrices live on the device (the updates compute them there), so
+ * this reads one row set back and synchronises the context stream. */
 int rtc_instance_inverse(rtc_context* ctx, uint64_t topObject, uint32_t instance, float out[12]);
 
 /*

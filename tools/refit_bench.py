@@ -7,12 +7,13 @@
     rtc_gas_refit ms, and incoherent closest-hit Mrays/s after a smooth per-vertex displacement of 0, 0.5 and 2 mean edge lengths,
     refitted against rebuilt (the hits of the two are checked to be equal in the same run);
   * the 10 001-instance scene (tools/make_instances_scene.py): rtc_ias_build ms against rtc_ias_update ms with every instance and
-    with 1 % of them moved and against rtc_ias_rebuild ms, and incoherent closest-hit Mrays/s through the scene after 1, 10 and 100
+    with 1 % of them moved, rtc_ias_update_device ms with every instance moved (matrices uploaded once, outside the timed call)
+    and rtc_ias_rebuild ms, and incoherent closest-hit Mrays/s through the scene after 1, 10 and 100
     animation steps of small rotations and after a random permutation of the tori's transforms (same boxes, no spatial coherence
     left in the built topology): refitted, rebuilt on the device (rtc_ias_rebuild) and rebuilt by rtc_ias_build, whose hits are
     checked to be equal in the same run;
   * about a million small instances (a 12-triangle box on a jittered lattice): rtc_ias_build ms (one run) against
-    rtc_ias_update ms of every instance and rtc_ias_rebuild ms.
+    rtc_ias_update ms and rtc_ias_update_device ms of every instance, and rtc_ias_rebuild ms.
 Builds are timed on the host clock (they end in a synchronisation); refits, updates and traces between CUDA events on the
 context stream, each the median of `repeats` runs after one warm-up.
 """
@@ -183,10 +184,14 @@ def instance_runs(ctx, nrays, repeats):
     all_ms = timed(ctx, lambda: ctx.ias_update(top, moved), repeats)
     few = max(1, n // 100)
     few_ms = timed(ctx, lambda: ctx.ias_update(top, moved[:few]), repeats)
+    d_moved = ctx.to_device(moved)
+    all_device_ms = timed(ctx, lambda: ctx.ias_update_device(top, d_moved, n), repeats)
+    ctx.free(d_moved)
     spare = ctx.ias_build(descs(xf0))
     rebuild_ms = timed(ctx, lambda: ctx.ias_rebuild(spare), repeats)             # the warm-up is the scene's first rebuild
     ctx.scene_destroy(spare)
-    emit(what="ias_build_vs_update", instances=n, build_ms=build_ms, update_all_ms=all_ms, update_1pct_ms=few_ms, rebuild_ms=rebuild_ms,
+    emit(what="ias_build_vs_update", instances=n, build_ms=build_ms, update_all_ms=all_ms, update_1pct_ms=few_ms,
+         update_all_device_ms=all_device_ms, rebuild_ms=rebuild_ms,
          speedup_all=build_ms / all_ms, speedup_1pct=build_ms / few_ms, build_over_rebuild=build_ms / rebuild_ms)
 
     lo, hi = xf0[:, [3, 7, 11]].min(axis=0) - 1.0, xf0[:, [3, 7, 11]].max(axis=0) + 1.0
@@ -260,9 +265,12 @@ def many_instance_runs(ctx, count, repeats):
     build_ms = wall(ctx, lambda: tops.append(ctx.ias_build(inst)), 1)
     top = tops[0]
     update_ms = timed(ctx, lambda: ctx.ias_update(top, xf), repeats)
+    d_xf = ctx.to_device(xf)
+    update_device_ms = timed(ctx, lambda: ctx.ias_update_device(top, d_xf, n), repeats)
+    ctx.free(d_xf)
     rebuild_ms = timed(ctx, lambda: ctx.ias_rebuild(top), repeats)
     emit(what="many_instances_build_vs_update_vs_rebuild", instances=n, build_ms=build_ms, build_runs=1, update_all_ms=update_ms,
-         rebuild_ms=rebuild_ms, build_over_rebuild=build_ms / rebuild_ms)
+         update_all_device_ms=update_device_ms, rebuild_ms=rebuild_ms, build_over_rebuild=build_ms / rebuild_ms)
     ctx.scene_destroy(top)
     ctx.gas_destroy(gas)
     ctx.free(d_a)

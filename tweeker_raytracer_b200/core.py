@@ -34,7 +34,7 @@ SYMBOLS = [
     "rtc_host_gas_build", "rtc_host_ias_build", "rtc_host_accel_info", "rtc_host_accel_export", "rtc_host_accel_destroy",
     "rtc_trace_schedule_get", "rtc_trace_schedule_set",
     "rtc_gas_refit", "rtc_ias_update", "rtc_host_gas_refit", "rtc_host_ias_refit",
-    "rtc_ias_rebuild", "rtc_host_ias_rebuild",
+    "rtc_ias_rebuild", "rtc_host_ias_rebuild", "rtc_ias_update_device",
 ]
 
 MATH_FUNCTIONS = ["sin", "cos", "atan", "atan2", "acos", "exp", "log", "pow", "div", "sqrt", "muladd"]     # enum rtc_math_fn
@@ -104,6 +104,7 @@ def lib():
         L.rtc_ias_build.argtypes = [C.c_void_p, C.c_void_p, C.c_uint32, C.POINTER(C.c_uint64)]
         L.rtc_gas_refit.argtypes = [C.c_void_p, C.c_uint32, C.c_uint64]
         L.rtc_ias_update.argtypes = [C.c_void_p, C.c_uint64, C.c_uint32, C.c_uint32, C.c_void_p]
+        L.rtc_ias_update_device.argtypes = [C.c_void_p, C.c_uint64, C.c_uint32, C.c_uint32, C.c_uint64, C.c_uint32]
         L.rtc_ias_rebuild.argtypes = [C.c_void_p, C.c_uint64]
         L.rtc_scene_info_get.argtypes = [C.c_void_p, C.c_uint64, C.POINTER(SceneInfo)]
         L.rtc_scene_destroy.argtypes = [C.c_void_p, C.c_uint64]
@@ -364,6 +365,13 @@ class Context:
         bring the scene up to date with refitted GAS)."""
         t = np.ascontiguousarray(transforms, dtype=np.float32).reshape(-1, 12)
         _check(self.L.rtc_ias_update(self.h, int(top), first, len(t), t.ctypes.data_as(C.c_void_p) if len(t) else None))
+
+    def ias_update_device(self, top, d_transforms, count, first=0, stride=48):
+        """rtc_ias_update_device: the object -> world matrices of instances first .. first + count - 1 are the 12 floats at the
+        device address d_transforms + i * stride (an int, e.g. tensor.data_ptr() of a CUDA tensor; stride 48: dense [count, 12],
+        80: OptixInstance records).  The buffer is read on the context stream when the update runs, not during the call: write
+        it on `self.stream` (or order the writer with events) and keep it unchanged until the update has run."""
+        _check(self.L.rtc_ias_update_device(self.h, int(top), first, count, int(d_transforms), stride))
 
     def ias_rebuild(self, top):
         """rtc_ias_rebuild: a new instance-level topology over the instance boxes of the last build / update, on the device and

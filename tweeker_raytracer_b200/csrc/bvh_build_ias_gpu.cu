@@ -305,7 +305,7 @@ int setup_rebuild(rtc_context* ctx, SceneRecord& s, IasRebuild& R)
   // switch the scene to the new arrays; the cutout graph captured its SceneDesc, and with it the node array freed here
   release_cutout_graph(ctx);
   cudaFree(s.d_tlasNodes);
-  free_refit_scratch(s.refit);
+  free_refit_scratch(s.refit, ctx->stream);
   s.d_tlasNodes = R.nodes; R.nodes = nullptr;
   s.refit = R.refit; R.refit = RefitScratch();
   s.desc.tlasNodes = static_cast<const uint4*>(s.d_tlasNodes);
@@ -321,7 +321,7 @@ void free_ias_rebuild(IasRebuild* r)
   if (!r) return;
   if (r->exec) cudaGraphExecDestroy(r->exec);
   if (r->graph) cudaGraphDestroy(r->graph);
-  cudaFree(r->base); cudaFree(r->nodes); free_refit_scratch(r->refit);
+  cudaFree(r->base); cudaFree(r->nodes); free_refit_scratch(r->refit, nullptr);      // allocated with cudaMalloc by setup_rebuild
   delete r;
 }
 

@@ -4,12 +4,16 @@
 //   GAS refit (rtc_gas_refit)        k_refit_tris   one pass over the leaf-ordered triangle records: new positions, id bits kept
 //                                    k_refit_nodes  bottom-up over the wide nodes (Karras-style arrival counters: the last child
 //                                                   to arrive processes the parent), re-quantised through bvh_rules.h
-//   instance update (rtc_ias_update) k_instance_bounds, k_instance_finish, k_refit_nodes over the instance level
+//   instance update                  k_instance_gather  one record per recomputed instance: its matrix (device memory: the
+//   (rtc_ias_update,                                    caller's for rtc_ias_update_device, staged by rtc_ias_update), the
+//    rtc_ias_update_device)                             inverse, its GAS's inputs
+//                                    k_instance_bounds, k_instance_finish, k_refit_nodes over the instance level
 // Node topology (imask, childBase, triBase, meta) and leaf order stay as built; only the frame, the quantised planes and the
 // triangle positions are rewritten.  Min / max are order-independent, so the result does not depend on the arrival order and
 // equals the host twin (accel_host.cpp), which visits the nodes in descending index order.
 //
-// Compiled with -fmad=false: instance_box_finish (bvh_rules.h) must round like the host, which compiles it with -ffp-contract=off.
+// Compiled with -fmad=false: invert_3x4 and instance_box_finish (bvh_rules.h) must round like the host, which compiles them with
+// -ffp-contract=off.
 #include "rtc_internal.h"
 #include "bvh_rules.h"
 
@@ -181,6 +185,69 @@ k_instance_bounds(const InstanceBoundsIn* __restrict__ in, PrimBox* __restrict__
   }
 }
 
+// One instance an update recomputes, as k_instance_gather assembles it.
+struct InstanceUpdate
+{
+  float    transform[12];          // object -> world
+  float    inverse[12];            // world -> object (invert_3x4)
+  const uint8_t* verts;            // the GAS's vertex records (tight bounds)
+  uint32_t stride, numVerts;       // numVerts = 0 for an empty GAS
+  const float* gasBox;             // device lo[3], hi[3] of a refitted GAS, or null: gasLoHi
+  float    gasLoHi[6];
+  uint64_t attributes;             // rt_GeometryInstanceData::attributes
+  uint32_t instance, emptyGas;
+};
+
+struct GatherParams
+{
+  const uint32_t* candidates;      // candidate -> instance, or null: candidate j is instance first + j
+  uint32_t numCandidates, first, count, stride;
+  const uint8_t* transforms;       // the caller's object->world matrices of instances first .. first + count - 1, `stride` bytes apart
+  const float4* o2w;               // the scene's current object->world rows (3 per instance)
+  const uint32_t* gasSlot;         // instance -> its entry of `gas`
+  const GasUpdateInput* gas;
+  InstanceUpdate* up; InstanceBoundsIn* in;   // in: null unless the bounds are tight
+};
+
+// One thread per candidate: its matrix (new from the caller's buffer, or the current one), the inverse (bvh_rules.h, the bits of
+// the host's invert_3x4: this file is compiled with -fmad=false) and its GAS's inputs, as the records the two kernels below read.
+__global__ void __launch_bounds__(128)
+k_instance_gather(const GatherParams P)
+{
+  const uint32_t j = blockIdx.x * blockDim.x + threadIdx.x;
+  if (j >= P.numCandidates) return;
+  const uint32_t i = P.candidates ? P.candidates[j] : P.first + j;
+  InstanceUpdate u;
+  if (i - P.first < P.count)                            // unsigned: first <= i < first + count
+  {
+    const float* t = reinterpret_cast<const float*>(P.transforms + (size_t)(i - P.first) * P.stride);
+    for (int k = 0; k < 12; ++k) u.transform[k] = t[k];
+  }
+  else
+  {
+    for (int r = 0; r < 3; ++r)
+    {
+      const float4 v = P.o2w[3u * (size_t)i + r];
+      u.transform[4 * r] = v.x; u.transform[4 * r + 1] = v.y; u.transform[4 * r + 2] = v.z; u.transform[4 * r + 3] = v.w;
+    }
+  }
+  invert_3x4(u.transform, u.inverse);
+  const GasUpdateInput& g = P.gas[P.gasSlot[i]];
+  u.verts = g.verts; u.stride = g.stride; u.numVerts = g.numVerts;
+  u.gasBox = g.gasBox;
+  for (int k = 0; k < 6; ++k) u.gasLoHi[k] = g.gasLoHi[k];
+  u.attributes = g.attributes;
+  u.instance = i; u.emptyGas = g.emptyGas;
+  P.up[j] = u;
+  if (P.in)
+  {
+    InstanceBoundsIn b;
+    for (int k = 0; k < 12; ++k) b.transform[k] = u.transform[k];
+    b.verts = g.verts; b.stride = g.stride; b.numVerts = g.numVerts; b.pad = 0u;
+    P.in[j] = b;
+  }
+}
+
 // One thread per updated instance: the padded box (the device twin of what rtc_ias_build does on the host), the instance's
 // rows of the traversal table (world->object) and of the shading tables (object->world, vertex attributes).
 __global__ void __launch_bounds__(128)
@@ -205,11 +272,14 @@ k_instance_finish(const InstanceUpdate* __restrict__ up, uint32_t count, const P
   gi[inst].attributes = u.attributes;
 }
 
-int alloc_refit_scratch(rtc_context* ctx, RefitScratch& r, const uint4* nodes, uint32_t numNodes)
+// pooled: from the stream-ordered pool (the instance level: its updates never allocate with a call that may block)
+int alloc_refit_scratch(rtc_context* ctx, RefitScratch& r, const uint4* nodes, uint32_t numNodes, bool pooled = false)
 {
   if (r.base) return 0;
   const size_t n = numNodes;
-  RTC_CUDA(cudaMalloc(&r.base, n * (2 * sizeof(uint32_t) + 6 * sizeof(float))));
+  if (pooled) RTC_CUDA(cudaMallocAsync(&r.base, n * (2 * sizeof(uint32_t) + 6 * sizeof(float)), ctx->stream));
+  else        RTC_CUDA(cudaMalloc(&r.base, n * (2 * sizeof(uint32_t) + 6 * sizeof(float))));
+  r.pooled = pooled;
   r.box = static_cast<float*>(r.base);
   r.parent = reinterpret_cast<uint32_t*>(r.box + 6 * n);
   r.arrivals = r.parent + n;
@@ -236,9 +306,10 @@ int launch_refit_nodes(rtc_context* ctx, const RefitScratch& r, uint4* nodes, ui
 
 } // namespace
 
-void free_refit_scratch(RefitScratch& r)
+void free_refit_scratch(RefitScratch& r, cudaStream_t stream)
 {
-  cudaFree(r.base);
+  if (r.pooled) cudaFreeAsync(r.base, stream);
+  else cudaFree(r.base);
   r = RefitScratch();
 }
 
@@ -257,42 +328,62 @@ int refit_gas_gpu(rtc_context* ctx, GasRecord& rec)
   return 0;
 }
 
-int refit_instances_gpu(rtc_context* ctx, SceneRecord& s, const std::vector<InstanceUpdate>& updates, bool tight)
+// The tail of every instance update, over m gathered records: exact bounds (tight), the padded boxes and table rows, then the
+// instance level's nodes -- the built array, or the one rtc_ias_build rebuilt, whose live node count is on the device.
+static int finish_instance_update(rtc_context* ctx, SceneRecord& s, const InstanceUpdate* d_up, const InstanceBoundsIn* d_in, PrimBox* d_exact,
+                                  uint32_t m, bool tight)
 {
-  const uint32_t m = (uint32_t)updates.size();
-  if (m == 0) return 0;
-  uint4* tlas = static_cast<uint4*>(s.d_tlasNodes);
-  // after a rebuild the scratch exists (bvh_build_ias_gpu.cu sized it for the node capacity and keeps its parents up to date)
-  if (int rc = alloc_refit_scratch(ctx, s.refit, tlas, s.desc.numTlasNodes)) return rc;
-  // inputs of this update: staged from pageable memory by the copy itself, and freed stream-ordered behind the kernels
-  std::vector<InstanceBoundsIn> in(tight ? m : 0);
-  for (uint32_t i = 0; i < (uint32_t)in.size(); ++i)
+  if (tight)
   {
-    for (int k = 0; k < 12; ++k) in[i].transform[k] = updates[i].transform[k];
-    in[i].verts = updates[i].verts; in[i].stride = updates[i].stride; in[i].numVerts = updates[i].numVerts; in[i].pad = 0u;
+    k_instance_bounds<<<m, kB, 0, ctx->stream>>>(d_in, d_exact);
+    ctx->kernelLaunches++;
+    RTC_CUDA(cudaGetLastError());
   }
-  const size_t upBytes = m * sizeof(InstanceUpdate), inBytes = in.size() * sizeof(InstanceBoundsIn);
+  k_instance_finish<<<(m + 127) / 128, 128, 0, ctx->stream>>>(d_up, m, d_exact, tight ? 1 : 0, s.d_instBoxes, static_cast<float4*>(s.d_instances),
+                                                              static_cast<float4*>(s.d_o2w), static_cast<rt_GeometryInstanceData*>(s.d_geomInst));
+  ctx->kernelLaunches++;
+  RTC_CUDA(cudaGetLastError());
+  uint4* tlas = static_cast<uint4*>(s.d_tlasNodes);
+  const uint32_t* leaves = static_cast<const uint32_t*>(s.d_tlasLeaves);
+  if (s.rebuild)
+    return launch_refit_nodes(ctx, s.refit, tlas, ias_rebuild_capacity(s.desc.numInstances), nullptr, leaves, s.d_instBoxes, s.d_numTlasNodes);
+  return launch_refit_nodes(ctx, s.refit, tlas, s.desc.numTlasNodes, nullptr, leaves, s.d_instBoxes);
+}
+
+int refit_instances_gpu(rtc_context* ctx, SceneRecord& s, const uint8_t* transforms, uint32_t strideBytes, uint32_t first, uint32_t count,
+                        const std::vector<uint32_t>& candidates, const std::vector<GasUpdateInput>& gas, bool tight)
+{
+  const uint32_t m = candidates.empty() ? count : (uint32_t)candidates.size();
+  if (m == 0) return 0;
+  // after a rebuild the scratch exists (bvh_build_ias_gpu.cu sized it for the node capacity and keeps its parents up to date)
+  if (int rc = alloc_refit_scratch(ctx, s.refit, static_cast<const uint4*>(s.d_tlasNodes), s.desc.numTlasNodes, true)) return rc;
+  // this update's records, per-GAS table and candidate list, one stream-ordered allocation freed behind the kernels; the two
+  // host arrays are small (nothing per instance unless a GAS was refitted) and staged by the copies themselves
+  const size_t upBytes = m * sizeof(InstanceUpdate), inBytes = tight ? m * sizeof(InstanceBoundsIn) : 0, exactBytes = m * sizeof(PrimBox);
+  const size_t gasBytes = gas.size() * sizeof(GasUpdateInput), listBytes = candidates.size() * sizeof(uint32_t);
   uint8_t* d = nullptr;
-  RTC_CUDA(cudaMallocAsync((void**)&d, upBytes + inBytes + m * sizeof(PrimBox), ctx->stream));
-  InstanceUpdate* d_up = reinterpret_cast<InstanceUpdate*>(d);
-  InstanceBoundsIn* d_in = reinterpret_cast<InstanceBoundsIn*>(d + upBytes);
+  RTC_CUDA(cudaMallocAsync((void**)&d, upBytes + inBytes + exactBytes + gasBytes + listBytes, ctx->stream));
+  GatherParams P;
+  P.up = reinterpret_cast<InstanceUpdate*>(d);
+  P.in = tight ? reinterpret_cast<InstanceBoundsIn*>(d + upBytes) : nullptr;
   PrimBox* d_exact = reinterpret_cast<PrimBox*>(d + upBytes + inBytes);
-  cudaError_t e = cudaMemcpyAsync(d_up, updates.data(), upBytes, cudaMemcpyHostToDevice, ctx->stream);
-  if (e == cudaSuccess && tight) e = cudaMemcpyAsync(d_in, in.data(), inBytes, cudaMemcpyHostToDevice, ctx->stream);
-  if (e == cudaSuccess && tight) { k_instance_bounds<<<m, kB, 0, ctx->stream>>>(d_in, d_exact); ctx->kernelLaunches++; e = cudaGetLastError(); }
+  GasUpdateInput* d_gas = reinterpret_cast<GasUpdateInput*>(d + upBytes + inBytes + exactBytes);
+  uint32_t* d_list = reinterpret_cast<uint32_t*>(d + upBytes + inBytes + exactBytes + gasBytes);
+  P.candidates = candidates.empty() ? nullptr : d_list;
+  P.numCandidates = m; P.first = first; P.count = count; P.stride = strideBytes; P.transforms = transforms;
+  P.o2w = static_cast<const float4*>(s.d_o2w); P.gasSlot = s.d_instGasSlot; P.gas = d_gas;
+  cudaError_t e = cudaMemcpyAsync(d_gas, gas.data(), gasBytes, cudaMemcpyHostToDevice, ctx->stream);
+  if (e == cudaSuccess && listBytes) e = cudaMemcpyAsync(d_list, candidates.data(), listBytes, cudaMemcpyHostToDevice, ctx->stream);
   if (e == cudaSuccess)
   {
-    k_instance_finish<<<(m + 127) / 128, 128, 0, ctx->stream>>>(d_up, m, d_exact, tight ? 1 : 0, s.d_instBoxes, static_cast<float4*>(s.d_instances),
-                                                                static_cast<float4*>(s.d_o2w), static_cast<rt_GeometryInstanceData*>(s.d_geomInst));
+    k_instance_gather<<<(m + 127) / 128, 128, 0, ctx->stream>>>(P);
     ctx->kernelLaunches++;
     e = cudaGetLastError();
   }
+  const int rc = e == cudaSuccess ? finish_instance_update(ctx, s, P.up, P.in, d_exact, m, tight)
+                                  : rtc_set_error(__FILE__, __LINE__, "refit_instances_gpu", (int)e, cudaGetErrorString(e));
   cudaFreeAsync(d, ctx->stream);
-  if (e != cudaSuccess) return rtc_set_error(__FILE__, __LINE__, "refit_instances_gpu", (int)e, cudaGetErrorString(e));
-  if (s.rebuild)
-    return launch_refit_nodes(ctx, s.refit, tlas, ias_rebuild_capacity(s.desc.numInstances), nullptr, static_cast<const uint32_t*>(s.d_tlasLeaves), s.d_instBoxes,
-                              s.d_numTlasNodes);
-  return launch_refit_nodes(ctx, s.refit, tlas, s.desc.numTlasNodes, nullptr, static_cast<const uint32_t*>(s.d_tlasLeaves), s.d_instBoxes);
+  return rc;
 }
 
 // boxes[i] = exact (unpadded) world bounds of the vertices of instance i; instances of an empty GAS get an inverted box

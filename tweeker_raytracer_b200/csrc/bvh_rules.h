@@ -1,11 +1,11 @@
 // bvh_rules.h -- arithmetic that the host builder (bvh_build_host.cpp), the device builders (bvh_build_gpu.cu,
 // bvh_build_ias_gpu.cu), the device refit (bvh_refit.cu) and the host-only twins (accel_host.cpp) must apply bit for bit: the
-// quantisation of one wide node, the padding of an instance's world box, and the Morton codes, radix tree and wide nodes of the
-// LBVH.  One definition, compiled for the host and for sm_100a.
+// world->object matrix of an instance, the quantisation of one wide node, the padding of an instance's world box, and the Morton
+// codes, radix tree and wide nodes of the LBVH.  One definition, compiled for the host and for sm_100a.
 //
 // FMA contraction: every product in quantise_node is by a power of two (step * 2^-4, step * 2^-6 with step >= 2^-120, which
 // stays a normal float) and is therefore exact, so a contracted multiply-add rounds exactly like the separate operations.
-// instance_box_finish multiplies in double by values that are not powers of two: the host compiles it with
+// invert_3x4 and instance_box_finish multiply in double by values that are not powers of two: the host compiles them with
 // -ffp-contract=off and bvh_refit.cu with -fmad=false.
 #pragma once
 
@@ -28,6 +28,29 @@ RTC_HD float rules_pow2f(int e)
   float f;
   memcpy(&f, &u, 4);
   return f;
+}
+
+// World->object matrix of an instance.  DEFINED here (OptiX computed it inside optixAccelBuild,
+// Device.cpp:1478, read back by closesthit.cu:49-52): adjugate / determinant of the upper 3x3 in double,
+// rounded once to float; translation -(Minv * t) in double.  The oracle states the same definition.
+// rtc_ias_build (accel_host.cpp's host twin too) computes it on the host, rtc_ias_update / rtc_ias_update_device on the device
+// (bvh_refit.cu k_instance_gather); IEEE double division and no contraction give the same bits on both.
+RTC_HD void invert_3x4(const float m[12], float out[12])
+{
+  const double a = m[0], b = m[1], c = m[2],  tx = m[3];
+  const double d = m[4], e = m[5], f = m[6],  ty = m[7];
+  const double g = m[8], h = m[9], i = m[10], tz = m[11];
+  const double c00 = e * i - f * h, c01 = c * h - b * i, c02 = b * f - c * e;
+  const double c10 = f * g - d * i, c11 = a * i - c * g, c12 = c * d - a * f;
+  const double c20 = d * h - e * g, c21 = b * g - a * h, c22 = a * e - b * d;
+  const double det = a * c00 + b * c10 + c * c20;
+  const double r = 1.0 / det;
+  const double i00 = c00 * r, i01 = c01 * r, i02 = c02 * r;
+  const double i10 = c10 * r, i11 = c11 * r, i12 = c12 * r;
+  const double i20 = c20 * r, i21 = c21 * r, i22 = c22 * r;
+  out[0] = (float)i00; out[1] = (float)i01; out[2]  = (float)i02; out[3]  = (float)(-(i00 * tx + i01 * ty + i02 * tz));
+  out[4] = (float)i10; out[5] = (float)i11; out[6]  = (float)i12; out[7]  = (float)(-(i10 * tx + i11 * ty + i12 * tz));
+  out[8] = (float)i20; out[9] = (float)i21; out[10] = (float)i22; out[11] = (float)(-(i20 * tx + i21 * ty + i22 * tz));
 }
 
 // Quantisation frame and conservative planes of one wide node.  child(s, lo, hi) yields the float box of the child in slot s for

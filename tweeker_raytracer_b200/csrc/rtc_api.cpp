@@ -10,6 +10,7 @@
 #include <cstdio>
 #include <cstdlib>
 #include <cstring>
+#include <iterator>
 #include <limits>
 #include <set>
 
@@ -29,10 +30,10 @@ SceneRecord* find_scene(rtc_context* ctx, uint64_t topObject)
   return nullptr;
 }
 
-void free_scene(SceneRecord* s)
+void free_scene(SceneRecord* s, cudaStream_t stream)
 {
   cudaFree(s->d_desc); cudaFree(s->d_tlasNodes); cudaFree(s->d_instances); cudaFree(s->d_tlasLeaves); cudaFree(s->d_o2w); cudaFree(s->d_geomInst); cudaFree(s->d_instFlags);
-  cudaFree(s->d_instBoxes); free_refit_scratch(s->refit); free_ias_rebuild(s->rebuild);
+  cudaFree(s->d_instBoxes); cudaFree(s->d_instGasSlot); free_refit_scratch(s->refit, stream); free_ias_rebuild(s->rebuild);
   delete s;
 }
 
@@ -40,7 +41,7 @@ constexpr const char* kDestroyedGas = "a GAS of this scene was destroyed";
 constexpr const char* kStaleScene = "a GAS of this scene was refitted after the scene was built or updated: call rtc_ias_update on the scene first";
 
 // Why the scene cannot be traced, or nullptr.  A GAS it instances was destroyed: its nodes and triangles are freed, and the
-// scene's instance records still point at them.  Or (unless `refitAllowed`, for rtc_ias_update, which cures it) the scene is
+// scene's instance records still point at them.  Or (unless `refitAllowed`, for the instance updates, which cure it) the scene is
 // stale: a GAS was refitted after the scene was built or last updated, so its instance boxes and instance level no longer
 // bound the triangles, and its shading table may point at a vertex buffer the caller has since freed.
 const char* scene_unusable(const rtc_context* ctx, const SceneRecord* s, bool refitAllowed = false)
@@ -76,6 +77,34 @@ int sync_tlas_node_count(rtc_context* ctx, SceneRecord* s)
   RTC_CUDA(cudaStreamSynchronize(ctx->stream));
   s->totalNodes = s->totalNodes - s->desc.numTlasNodes + count;
   s->desc.numTlasNodes = count;
+  return 0;
+}
+
+// rtc_ias_update and rtc_ias_update_device (arguments checked): instance first + i takes the matrix at transforms + i * strideBytes
+// (device-readable).  Recomputes exactly the instances of the range and those of every GAS refitted since the last build / update
+// -- no other: the vertex buffer of a GAS that was not refitted may already hold positions its boxes do not bound yet.
+int update_instances(rtc_context* ctx, SceneRecord* s, uint32_t first, uint32_t count, const uint8_t* transforms, uint32_t strideBytes)
+{
+  std::vector<GasUpdateInput> gas(s->gasGeneration.size());
+  std::vector<uint8_t> refitted(ctx->gas.size(), 0u);
+  bool anyRefitted = false;
+  for (size_t k = 0; k < gas.size(); ++k)
+  {
+    const GasRecord& g = ctx->gas[s->gasGeneration[k].first];
+    GasUpdateInput& u = gas[k];
+    u.verts = reinterpret_cast<const uint8_t*>((uintptr_t)g.attributes); u.stride = g.strideBytes; u.numVerts = g.numTris ? g.numVerts : 0u;
+    u.gasBox = g.boundsOnDevice ? g.refit.box : nullptr;
+    for (int c = 0; c < 3; ++c) { u.gasLoHi[c] = g.lo[c]; u.gasLoHi[3 + c] = g.hi[c]; }
+    u.attributes = g.attributes;
+    u.emptyGas = g.numTris == 0 ? 1u : 0u; u.pad = 0u;
+    if (g.generation != s->gasGeneration[k].second) { refitted[s->gasGeneration[k].first] = 1u; anyRefitted = true; }
+  }
+  std::vector<uint32_t> candidates;           // empty: the range
+  if (anyRefitted)
+    for (uint32_t i = 0; i < s->desc.numInstances; ++i)
+      if ((first <= i && i < first + count) || refitted[s->instGas[i]]) candidates.push_back(i);
+  if (int rc = refit_instances_gpu(ctx, *s, transforms, strideBytes, first, count, candidates, gas, instance_bounds_tight())) return rc;
+  for (std::pair<uint32_t, uint64_t>& g : s->gasGeneration) g.second = ctx->gas[g.first].generation;
   return 0;
 }
 
@@ -199,8 +228,8 @@ int rtc_context_destroy(rtc_context* ctx)
   if (ctx->stream) cudaStreamSynchronize(ctx->stream);
   release_cutout_graph(ctx);
   tuner_release(ctx);
-  for (SceneRecord* s : ctx->scenes) free_scene(s);
-  for (GasRecord& g : ctx->gas) { cudaFree(g.d_nodes); cudaFree(g.d_tris); free_refit_scratch(g.refit); }
+  for (SceneRecord* s : ctx->scenes) free_scene(s, ctx->stream);
+  for (GasRecord& g : ctx->gas) { cudaFree(g.d_nodes); cudaFree(g.d_tris); free_refit_scratch(g.refit, ctx->stream); }
   if (ctx->wf.base) cudaFree(ctx->wf.base);
   if (ctx->wf.cutBase) cudaFree(ctx->wf.cutBase);
   for (void* t : ctx->textures) cudaFree(t);
@@ -399,7 +428,7 @@ int rtc_gas_destroy(rtc_context* ctx, uint32_t gas)
   RTC_CUDA(cudaSetDevice(ctx->device));
   RTC_CUDA(cudaStreamSynchronize(ctx->stream));
   GasRecord& g = ctx->gas[gas];
-  cudaFree(g.d_nodes); cudaFree(g.d_tris); free_refit_scratch(g.refit);
+  cudaFree(g.d_nodes); cudaFree(g.d_tris); free_refit_scratch(g.refit, ctx->stream);
   g.d_nodes = nullptr; g.d_tris = nullptr; g.numNodes = 0; g.numTris = 0; g.boundsOnDevice = false;
   return 0;
 }
@@ -427,8 +456,6 @@ int rtc_ias_build(rtc_context* ctx, const rtc_instance_desc* instances, uint32_t
   std::vector<float4> inst((size_t)numInstances * 4u), o2w((size_t)numInstances * 3u);
   std::vector<rt_GeometryInstanceData> gi(numInstances);
   SceneRecord* rec = new SceneRecord();
-  rec->inverses.resize((size_t)numInstances * 12u);
-  rec->transforms.resize((size_t)numInstances * 12u);
   rec->instGas.resize(numInstances);
   std::set<uint32_t> distinct;
   for (uint32_t i = 0; i < numInstances; ++i)
@@ -440,8 +467,7 @@ int rtc_ias_build(rtc_context* ctx, const rtc_instance_desc* instances, uint32_t
     const GasRecord& g = ctx->gas[d.gas];
     distinct.insert(d.gas);
     rec->instGas[i] = d.gas;
-    std::memcpy(&rec->transforms[(size_t)i * 12u], d.transform, 48);
-    float* inv = &rec->inverses[(size_t)i * 12u];
+    float inv[12];
     invert_3x4(d.transform, inv);
     for (int r = 0; r < 3; ++r)
     {
@@ -480,6 +506,12 @@ int rtc_ias_build(rtc_context* ctx, const rtc_instance_desc* instances, uint32_t
   rec->instFlags.assign(numInstances, 0u);
   if (e == cudaSuccess) e = upload(&rec->d_instFlags, rec->instFlags.data(), rec->instFlags.size() * 4u);
   if (e == cudaSuccess) e = upload((void**)&rec->d_instBoxes, boxes.data(), boxes.size() * sizeof(PrimBox));
+  {
+    // the updates' instance -> GAS table entry (the position of the GAS in gasGeneration below, which follows `distinct`)
+    std::vector<uint32_t> slot(numInstances);
+    for (uint32_t i = 0; i < numInstances; ++i) slot[i] = (uint32_t)std::distance(distinct.begin(), distinct.find(rec->instGas[i]));
+    if (e == cudaSuccess) e = upload((void**)&rec->d_instGasSlot, slot.data(), slot.size() * 4u);
+  }
   rec->desc.instFlags = (const uint32_t*)rec->d_instFlags;
   rec->desc.tlasNodes = (const uint4*)rec->d_tlasNodes;
   rec->desc.tlasLeaves = (const uint32_t*)rec->d_tlasLeaves;
@@ -490,7 +522,7 @@ int rtc_ias_build(rtc_context* ctx, const rtc_instance_desc* instances, uint32_t
   rec->desc.numTlasNodes = (uint32_t)bvh.nodes.size();
   rec->desc.numTlasLeaves = (uint32_t)bvh.primOrder.size();
   if (e == cudaSuccess) e = upload((void**)&rec->d_desc, &rec->desc, sizeof(SceneDesc));
-  if (e != cudaSuccess) { free_scene(rec); return rtc_set_error(__FILE__, __LINE__, "rtc_ias_build upload", (int)e, cudaGetErrorString(e)); }
+  if (e != cudaSuccess) { free_scene(rec, ctx->stream); return rtc_set_error(__FILE__, __LINE__, "rtc_ias_build upload", (int)e, cudaGetErrorString(e)); }
   rec->totalNodes = bvh.nodes.size(); rec->totalTris = 0; rec->gasBuildMs = 0.0; rec->numGas = (uint32_t)distinct.size();
   for (uint32_t g : distinct)
   {
@@ -512,35 +544,42 @@ int rtc_ias_update(rtc_context* ctx, uint64_t topObject, uint32_t first, uint32_
   if (count && !transforms) RTC_FAIL("transforms is null");
   if (const char* why = scene_unusable(ctx, s, true)) RTC_FAIL(why);
   RTC_CUDA(cudaSetDevice(ctx->device));
-  for (uint32_t i = first; i < first + count; ++i)
+  // The device path on a stream-ordered device copy of the matrices, freed behind the update.  `transforms` may be reused on
+  // return, so the call must have read it by then.  A copy from pageable memory is staged before cudaMemcpyAsync returns; one
+  // from page-locked memory (rtc_host_alloc, cudaHostRegister, pinned tensors) or managed memory reads it only when the stream
+  // gets there, so such a source is first copied into pageable memory of the library's.
+  const float* src = transforms;
+  std::vector<float> pageable;
+  if (count)
   {
-    std::memcpy(&s->transforms[(size_t)i * 12u], transforms + (size_t)(i - first) * 12u, 48);
-    invert_3x4(&s->transforms[(size_t)i * 12u], &s->inverses[(size_t)i * 12u]);
+    cudaPointerAttributes attr{};
+    if (cudaPointerGetAttributes(&attr, transforms) != cudaSuccess) { cudaGetLastError(); attr.type = cudaMemoryTypeUnregistered; }
+    if (attr.type == cudaMemoryTypeDevice) RTC_FAIL("transforms is device memory: use rtc_ias_update_device");
+    if (attr.type != cudaMemoryTypeUnregistered) { pageable.assign(transforms, transforms + (size_t)count * 12u); src = pageable.data(); }
   }
-  // instances to recompute: the moved ones and every instance of a GAS refitted since the last build / update
-  std::vector<uint8_t> refitted(ctx->gas.size(), 0u);
-  bool anyRefitted = false;
-  for (const std::pair<uint32_t, uint64_t>& g : s->gasGeneration)
-    if (ctx->gas[g.first].generation != g.second) { refitted[g.first] = 1u; anyRefitted = true; }
-  std::vector<InstanceUpdate> updates;
-  updates.reserve(anyRefitted ? n : count);
-  for (uint32_t i = anyRefitted ? 0u : first; i < (anyRefitted ? n : first + count); ++i)
+  uint8_t* staged = nullptr;
+  if (count)
   {
-    if (!(first <= i && i < first + count) && !refitted[s->instGas[i]]) continue;
-    const GasRecord& g = ctx->gas[s->instGas[i]];
-    InstanceUpdate u;
-    std::memcpy(u.transform, &s->transforms[(size_t)i * 12u], 48);
-    std::memcpy(u.inverse, &s->inverses[(size_t)i * 12u], 48);
-    u.verts = reinterpret_cast<const uint8_t*>((uintptr_t)g.attributes); u.stride = g.strideBytes; u.numVerts = g.numTris ? g.numVerts : 0u;
-    u.gasBox = g.boundsOnDevice ? g.refit.box : nullptr;
-    for (int k = 0; k < 3; ++k) { u.gasLoHi[k] = g.lo[k]; u.gasLoHi[3 + k] = g.hi[k]; }
-    u.attributes = g.attributes;
-    u.instance = i; u.emptyGas = g.numTris == 0 ? 1u : 0u;
-    updates.push_back(u);
+    RTC_CUDA(cudaMallocAsync((void**)&staged, (size_t)count * 48u, ctx->stream));
+    const cudaError_t e = cudaMemcpyAsync(staged, src, (size_t)count * 48u, cudaMemcpyHostToDevice, ctx->stream);
+    if (e != cudaSuccess) { cudaFreeAsync(staged, ctx->stream); return rtc_set_error(__FILE__, __LINE__, "rtc_ias_update upload", (int)e, cudaGetErrorString(e)); }
   }
-  if (int rc = refit_instances_gpu(ctx, *s, updates, instance_bounds_tight())) return rc;
-  for (std::pair<uint32_t, uint64_t>& g : s->gasGeneration) g.second = ctx->gas[g.first].generation;
-  return 0;
+  const int rc = update_instances(ctx, s, first, count, staged, 48u);
+  if (staged) cudaFreeAsync(staged, ctx->stream);
+  return rc;
+}
+
+int rtc_ias_update_device(rtc_context* ctx, uint64_t topObject, uint32_t first, uint32_t count, uint64_t transforms, uint32_t strideBytes)
+{
+  SceneRecord* s = find_scene(ctx, topObject);
+  if (!s) RTC_FAIL("unknown topObject");
+  if ((uint64_t)first + count > s->desc.numInstances) RTC_FAIL("instance range out of bounds");
+  if (count && !transforms) RTC_FAIL("transforms is null");
+  if (count && (transforms & 3u)) RTC_FAIL("transforms is not 4-byte aligned");
+  if (strideBytes < 48 || (strideBytes & 3u)) RTC_FAIL("strideBytes must be a multiple of 4 and at least 48");
+  if (const char* why = scene_unusable(ctx, s, true)) RTC_FAIL(why);
+  RTC_CUDA(cudaSetDevice(ctx->device));
+  return update_instances(ctx, s, first, count, reinterpret_cast<const uint8_t*>((uintptr_t)transforms), strideBytes);
 }
 
 int rtc_ias_rebuild(rtc_context* ctx, uint64_t topObject)
@@ -572,7 +611,7 @@ int rtc_scene_destroy(rtc_context* ctx, uint64_t topObject)
     {
       RTC_CUDA(cudaStreamSynchronize(ctx->stream));
       release_cutout_graph(ctx);          // it may have captured this scene's tables; a later scene can get the same addresses
-      free_scene(ctx->scenes[i]);
+      free_scene(ctx->scenes[i], ctx->stream);
       ctx->scenes.erase(ctx->scenes.begin() + (long)i);
       return 0;
     }
@@ -645,7 +684,9 @@ int rtc_scene_export(rtc_context* ctx, uint64_t topObject, void* tlasNodes, uint
   if (int rc = sync_tlas_node_count(ctx, s)) return rc;
   if (tlasNodes) RTC_CUDA(cudaMemcpy(tlasNodes, s->d_tlasNodes, (size_t)s->desc.numTlasNodes * sizeof(Node8), cudaMemcpyDeviceToHost));
   if (tlasLeaves && s->desc.numTlasLeaves) RTC_CUDA(cudaMemcpy(tlasLeaves, s->d_tlasLeaves, (size_t)s->desc.numTlasLeaves * 4u, cudaMemcpyDeviceToHost));
-  if (worldToObject) std::memcpy(worldToObject, s->inverses.data(), s->inverses.size() * sizeof(float));
+  // world->object rows 0..2 of each 64-byte instance record, where the updates computed them
+  if (worldToObject && s->desc.numInstances)
+    RTC_CUDA(cudaMemcpy2D(worldToObject, 48, s->d_instances, 64, 48, s->desc.numInstances, cudaMemcpyDeviceToHost));
   if (instanceGas) std::memcpy(instanceGas, s->instGas.data(), s->instGas.size() * sizeof(uint32_t));
   return 0;
 }
@@ -674,7 +715,9 @@ int rtc_instance_inverse(rtc_context* ctx, uint64_t topObject, uint32_t instance
   SceneRecord* s = find_scene(ctx, topObject);
   if (!s) RTC_FAIL("unknown topObject");
   if (instance >= s->desc.numInstances) RTC_FAIL("instance out of range");
-  std::memcpy(out, &s->inverses[(size_t)instance * 12u], 48);
+  RTC_CUDA(cudaSetDevice(ctx->device));
+  RTC_CUDA(cudaMemcpyAsync(out, static_cast<const float4*>(s->d_instances) + 4u * (size_t)instance, 48, cudaMemcpyDeviceToHost, ctx->stream));
+  RTC_CUDA(cudaStreamSynchronize(ctx->stream));
   return 0;
 }
 
