@@ -30,10 +30,10 @@ $(LIB)/bvh_build_gpu.o: $(CSRC)/bvh_build_gpu.cu $(CSRC)/lbvh.cuh $(CSRC)/bvh_ru
 # instance-level rebuild: FMA contraction off, so the collapse (bvh_rules.h) rounds like its host twin
 $(LIB)/bvh_build_ias_gpu.o: $(CSRC)/bvh_build_ias_gpu.cu $(CSRC)/lbvh.cuh $(CSRC)/bvh_rules.h $(CSRC)/rtc_internal.h include/rtc_core.h
 	$(NVCC) $(NVFLAGS) -fmad=false -c $< -o $@
-# refit and instance bounds: FMA contraction off, so instance_box_finish (bvh_rules.h) rounds like the host build
+# refit and instance records: FMA contraction off, so invert_3x4 and instance_box_finish (bvh_rules.h) round like the host twin
 $(LIB)/bvh_refit.o: $(CSRC)/bvh_refit.cu $(CSRC)/bvh_rules.h $(CSRC)/rtc_internal.h include/rtc_core.h include/rtigo3_abi.h
 	$(NVCC) $(NVFLAGS) -fmad=false -c $< -o $@
-$(LIB)/rtc_api.o: $(CSRC)/rtc_api.cpp $(CSRC)/bvh_rules.h $(CSRC)/rtc_internal.h include/rtc_core.h
+$(LIB)/rtc_api.o: $(CSRC)/rtc_api.cpp $(CSRC)/rtc_internal.h include/rtc_core.h
 	g++ $(CXXFLAGS) -c $< -o $@
 $(LIB)/bvh_build_host.o: $(CSRC)/bvh_build_host.cpp $(CSRC)/bvh_rules.h $(CSRC)/rtc_internal.h
 	g++ $(CXXFLAGS) -c $< -o $@

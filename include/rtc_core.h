@@ -208,7 +208,7 @@ int rtc_texture_destroy(rtc_context* ctx, uint64_t handle);
 int rtc_scene_export(rtc_context* ctx, uint64_t topObject, void* tlasNodes, uint32_t* tlasLeaves, float* worldToObject, uint32_t* instanceGas);
 int rtc_gas_info(rtc_context* ctx, uint32_t gas, uint64_t* numNodes, uint64_t* numTris);
 int rtc_gas_export(rtc_context* ctx, uint32_t gas, void* nodes, float* tris);
-/* Copies out the 3x4 world->object matrix of one instance.  The matrices live on the device (the updates compute them there), so
+/* Copies out the 3x4 world->object matrix of one instance.  The matrices live on the device (the builds and updates compute them there), so
  * this reads one row set back and synchronises the context stream. */
 int rtc_instance_inverse(rtc_context* ctx, uint64_t topObject, uint32_t instance, float out[12]);
 

@@ -68,8 +68,11 @@ def test_equals_the_host_update_and_the_twin(cuda_device, n):
         for i in sorted(set(np.linspace(0, n - 1, min(n, 64)).astype(int))):
             inv = ctx.instance_inverse(by_device, int(i))
             assert inv.tobytes() == ctx.instance_inverse(by_host, int(i)).tobytes() == twin["world_to_object"][i].tobytes()
+        # a build from the same matrices writes its instance records with the update kernels: the host twin's build, byte for byte
+        fresh = s.build(x)
+        built, _ = core.host_scene_export(geos, [(x[i], g) for i, (_, g) in enumerate(insts)])
+        assert same_export(ctx.scene_export(fresh), built)
         if n <= 10001:
-            fresh = s.build(x)
             check_hits(ctx, by_device, fresh, rays_for(n, 20000, seed=3), got)
         ctx.free(d_x)
 
@@ -132,6 +135,7 @@ def test_interleavings(cuda_device, monkeypatch, bounds):
     with core.Context(0) as ctx:
         s = Scene(ctx, geos, insts)
         top = s.build()
+        assert same_export(ctx.scene_export(top), core.host_scene_export(geos, insts)[0])
         d_xs = [ctx.to_device(x) for x in xs]
         steps, current = [], xf0.copy()
 
@@ -149,6 +153,9 @@ def test_interleavings(cuda_device, monkeypatch, bounds):
         # a GAS refit, then a device update of a sub-range: instances of the refitted GAS outside it keep their matrices
         ctx.upload(s.keep[0], new0)
         ctx.gas_refit(s.gas[0])
+        on_refitted = s.build()                                           # reads GAS 0's refitted bounds on the device
+        assert same_export(ctx.scene_export(on_refitted), core.host_scene_export([(new0, geo0[1]), geo1], insts)[0])
+        ctx.scene_destroy(on_refitted)
         ctx.ias_update_device(top, d_xs[0] + 48 * 100, 100, first=100)
         current[100:200] = xs[0][100:200]
         check(([new0, None], current.copy()))

@@ -54,7 +54,7 @@ bool gas_assemble_host(const uint8_t* verts, uint32_t strideBytes, uint32_t numV
   return true;
 }
 
-// Exact world bounds of the transformed vertices of one instance, in the arithmetic of k_instance_bounds (bvh_build_gpu.cu):
+// Exact world bounds of the transformed vertices of one instance, in the arithmetic of k_instance_bounds (bvh_refit.cu):
 // one fmaf chain per row, min / max are order-independent, so the device reduction and this loop agree bit for bit.
 void instance_bounds_host(const float transform[12], const uint8_t* verts, uint32_t strideBytes, uint32_t numVerts, PrimBox& out)
 {

@@ -1,19 +1,22 @@
 // bvh_refit.cu -- in-place update of built acceleration structures (the counterpart of optixAccelBuild with
-// OPTIX_BUILD_OPERATION_UPDATE), and the tight instance bounds the instance level is built and updated over.
+// OPTIX_BUILD_OPERATION_UPDATE), and the instance records the instance level is built and updated over.
 //
 //   GAS refit (rtc_gas_refit)        k_refit_tris   one pass over the leaf-ordered triangle records: new positions, id bits kept
 //                                    k_refit_nodes  bottom-up over the wide nodes (Karras-style arrival counters: the last child
 //                                                   to arrive processes the parent), re-quantised through bvh_rules.h
-//   instance update                  k_instance_gather  one record per recomputed instance: its matrix (device memory: the
-//   (rtc_ias_update,                                    caller's for rtc_ias_update_device, staged by rtc_ias_update), the
-//    rtc_ias_update_device)                             inverse, its GAS's inputs
-//                                    k_instance_bounds, k_instance_finish, k_refit_nodes over the instance level
+//   instance records                 k_instance_gather  one record per written instance: its matrix (device memory: the
+//   (rtc_ias_build,                                     caller's for rtc_ias_update_device, staged by rtc_ias_update, the
+//    rtc_ias_update,                                    scene's own object->world rows for rtc_ias_build), the inverse, its
+//    rtc_ias_update_device)                             GAS's entry of the per-GAS table
+//                                    k_instance_bounds, k_instance_finish: the padded world box, the traversal and shading rows
+//   instance-level refit             k_refit_nodes over the instance level (rtc_ias_build builds its nodes on the host instead,
+//   (the updates)                                   over the boxes the records hold)
 // Node topology (imask, childBase, triBase, meta) and leaf order stay as built; only the frame, the quantised planes and the
 // triangle positions are rewritten.  Min / max are order-independent, so the result does not depend on the arrival order and
 // equals the host twin (accel_host.cpp), which visits the nodes in descending index order.
 //
-// Compiled with -fmad=false: invert_3x4 and instance_box_finish (bvh_rules.h) must round like the host, which compiles them with
-// -ffp-contract=off.
+// Compiled with -fmad=false: invert_3x4 and instance_box_finish (bvh_rules.h) must round like the host twin, which compiles them
+// with -ffp-contract=off.
 #include "rtc_internal.h"
 #include "bvh_rules.h"
 
@@ -135,27 +138,30 @@ k_refit_nodes_live(const RefitParams P, const uint32_t* __restrict__ numNodes)
   refit_from(P, i);
 }
 
+// One instance whose records are written, as k_instance_gather assembles it.
+struct InstanceUpdate
+{
+  float    transform[12];          // object -> world
+  float    inverse[12];            // world -> object (invert_3x4)
+  GasUpdateInput gas;              // its GAS's entry of the per-GAS table
+  uint32_t instance, pad;
+};
+
 // ---- instance level: tight world bounds of every instance from its transformed vertices -------------------------
 // The reference hands OptiX the instance transform and lets the driver bound the instance (Device.cpp:1427-1443,
 // optixAccelBuild over OPTIX_BUILD_INPUT_TYPE_INSTANCES :1471-1482).  The first version here bounded the eight transformed
 // corners of the GAS box, which is loose for rotated instances (a torus rotated by 45 degrees: +40 % per axis) and made
 // rays enter instances they cannot hit; an instance entry costs about three node visits.  One CTA per instance now
 // transforms every vertex of the instance's GAS and reduces min/max.
-struct InstanceBoundsIn
-{
-  float transform[12];
-  const uint8_t* verts; uint32_t stride, numVerts;
-  uint32_t pad;
-};
-
 __global__ void __launch_bounds__(kB)
-k_instance_bounds(const InstanceBoundsIn* __restrict__ in, PrimBox* __restrict__ out)
+k_instance_bounds(const InstanceUpdate* __restrict__ up, PrimBox* __restrict__ out)
 {
-  const InstanceBoundsIn& I = in[blockIdx.x];
+  const InstanceUpdate& I = up[blockIdx.x];
+  const GasUpdateInput& g = I.gas;
   float lo[3] = { FLT_MAX, FLT_MAX, FLT_MAX }, hi[3] = { -FLT_MAX, -FLT_MAX, -FLT_MAX };
-  for (uint32_t v = threadIdx.x; v < I.numVerts; v += blockDim.x)
+  for (uint32_t v = threadIdx.x; v < g.numVerts; v += blockDim.x)
   {
-    const float* p = reinterpret_cast<const float*>(I.verts + (size_t)v * I.stride);
+    const float* p = reinterpret_cast<const float*>(g.verts + (size_t)v * g.stride);
     const float x = p[0], y = p[1], z = p[2];
 #pragma unroll
     for (int r = 0; r < 3; ++r)
@@ -185,32 +191,19 @@ k_instance_bounds(const InstanceBoundsIn* __restrict__ in, PrimBox* __restrict__
   }
 }
 
-// One instance an update recomputes, as k_instance_gather assembles it.
-struct InstanceUpdate
-{
-  float    transform[12];          // object -> world
-  float    inverse[12];            // world -> object (invert_3x4)
-  const uint8_t* verts;            // the GAS's vertex records (tight bounds)
-  uint32_t stride, numVerts;       // numVerts = 0 for an empty GAS
-  const float* gasBox;             // device lo[3], hi[3] of a refitted GAS, or null: gasLoHi
-  float    gasLoHi[6];
-  uint64_t attributes;             // rt_GeometryInstanceData::attributes
-  uint32_t instance, emptyGas;
-};
-
 struct GatherParams
 {
   const uint32_t* candidates;      // candidate -> instance, or null: candidate j is instance first + j
   uint32_t numCandidates, first, count, stride;
-  const uint8_t* transforms;       // the caller's object->world matrices of instances first .. first + count - 1, `stride` bytes apart
+  const uint8_t* transforms;       // the object->world matrices of instances first .. first + count - 1, `stride` bytes apart
   const float4* o2w;               // the scene's current object->world rows (3 per instance)
   const uint32_t* gasSlot;         // instance -> its entry of `gas`
   const GasUpdateInput* gas;
-  InstanceUpdate* up; InstanceBoundsIn* in;   // in: null unless the bounds are tight
+  InstanceUpdate* up;
 };
 
-// One thread per candidate: its matrix (new from the caller's buffer, or the current one), the inverse (bvh_rules.h, the bits of
-// the host's invert_3x4: this file is compiled with -fmad=false) and its GAS's inputs, as the records the two kernels below read.
+// One thread per candidate: its matrix (new from `transforms`, or the current one), the inverse (bvh_rules.h, the bits of the
+// host's invert_3x4: this file is compiled with -fmad=false) and its GAS's table entry, as the records the two kernels below read.
 __global__ void __launch_bounds__(128)
 k_instance_gather(const GatherParams P)
 {
@@ -232,24 +225,14 @@ k_instance_gather(const GatherParams P)
     }
   }
   invert_3x4(u.transform, u.inverse);
-  const GasUpdateInput& g = P.gas[P.gasSlot[i]];
-  u.verts = g.verts; u.stride = g.stride; u.numVerts = g.numVerts;
-  u.gasBox = g.gasBox;
-  for (int k = 0; k < 6; ++k) u.gasLoHi[k] = g.gasLoHi[k];
-  u.attributes = g.attributes;
-  u.instance = i; u.emptyGas = g.emptyGas;
+  u.gas = P.gas[P.gasSlot[i]];
+  u.instance = i; u.pad = 0u;
   P.up[j] = u;
-  if (P.in)
-  {
-    InstanceBoundsIn b;
-    for (int k = 0; k < 12; ++k) b.transform[k] = u.transform[k];
-    b.verts = g.verts; b.stride = g.stride; b.numVerts = g.numVerts; b.pad = 0u;
-    P.in[j] = b;
-  }
 }
 
-// One thread per updated instance: the padded box (the device twin of what rtc_ias_build does on the host), the instance's
-// rows of the traversal table (world->object) and of the shading tables (object->world, vertex attributes).
+// One thread per written instance: the padded box (instance_box_finish, bvh_rules.h), the instance's 64 B traversal record
+// (world->object rows 0..2, row 3 = {GAS nodes, GAS triangles}) and its rows of the shading tables (object->world, vertex
+// attributes).
 __global__ void __launch_bounds__(128)
 k_instance_finish(const InstanceUpdate* __restrict__ up, uint32_t count, const PrimBox* __restrict__ exact, int tight,
                   PrimBox* __restrict__ instBoxes, float4* __restrict__ instances, float4* __restrict__ o2w, rt_GeometryInstanceData* __restrict__ gi)
@@ -257,11 +240,12 @@ k_instance_finish(const InstanceUpdate* __restrict__ up, uint32_t count, const P
   const uint32_t i = blockIdx.x * blockDim.x + threadIdx.x;
   if (i >= count) return;
   const InstanceUpdate& u = up[i];
+  const GasUpdateInput& g = u.gas;
   float gas[6];
-  for (int k = 0; k < 6; ++k) gas[k] = u.gasBox ? u.gasBox[k] : u.gasLoHi[k];
+  for (int k = 0; k < 6; ++k) gas[k] = g.gasBox ? g.gasBox[k] : g.gasLoHi[k];
   PrimBox b = {};
   if (tight) b = exact[i];
-  instance_box_finish(u.transform, gas, gas + 3, tight != 0, u.emptyGas != 0, b);
+  instance_box_finish(u.transform, gas, gas + 3, tight != 0, g.emptyGas != 0, b);
   const uint32_t inst = u.instance;
   instBoxes[inst] = b;
   for (int r = 0; r < 3; ++r)
@@ -269,7 +253,8 @@ k_instance_finish(const InstanceUpdate* __restrict__ up, uint32_t count, const P
     instances[4u * inst + r] = make_float4(u.inverse[4 * r], u.inverse[4 * r + 1], u.inverse[4 * r + 2], u.inverse[4 * r + 3]);
     o2w[3u * inst + r] = make_float4(u.transform[4 * r], u.transform[4 * r + 1], u.transform[4 * r + 2], u.transform[4 * r + 3]);
   }
-  gi[inst].attributes = u.attributes;
+  *reinterpret_cast<ulonglong2*>(instances + 4u * inst + 3) = make_ulonglong2((uintptr_t)g.nodes, (uintptr_t)g.tris);
+  gi[inst].attributes = g.attributes;
 }
 
 // pooled: from the stream-ordered pool (the instance level: its updates never allocate with a call that may block)
@@ -328,47 +313,22 @@ int refit_gas_gpu(rtc_context* ctx, GasRecord& rec)
   return 0;
 }
 
-// The tail of every instance update, over m gathered records: exact bounds (tight), the padded boxes and table rows, then the
-// instance level's nodes -- the built array, or the one rtc_ias_build rebuilt, whose live node count is on the device.
-static int finish_instance_update(rtc_context* ctx, SceneRecord& s, const InstanceUpdate* d_up, const InstanceBoundsIn* d_in, PrimBox* d_exact,
-                                  uint32_t m, bool tight)
-{
-  if (tight)
-  {
-    k_instance_bounds<<<m, kB, 0, ctx->stream>>>(d_in, d_exact);
-    ctx->kernelLaunches++;
-    RTC_CUDA(cudaGetLastError());
-  }
-  k_instance_finish<<<(m + 127) / 128, 128, 0, ctx->stream>>>(d_up, m, d_exact, tight ? 1 : 0, s.d_instBoxes, static_cast<float4*>(s.d_instances),
-                                                              static_cast<float4*>(s.d_o2w), static_cast<rt_GeometryInstanceData*>(s.d_geomInst));
-  ctx->kernelLaunches++;
-  RTC_CUDA(cudaGetLastError());
-  uint4* tlas = static_cast<uint4*>(s.d_tlasNodes);
-  const uint32_t* leaves = static_cast<const uint32_t*>(s.d_tlasLeaves);
-  if (s.rebuild)
-    return launch_refit_nodes(ctx, s.refit, tlas, ias_rebuild_capacity(s.desc.numInstances), nullptr, leaves, s.d_instBoxes, s.d_numTlasNodes);
-  return launch_refit_nodes(ctx, s.refit, tlas, s.desc.numTlasNodes, nullptr, leaves, s.d_instBoxes);
-}
-
-int refit_instances_gpu(rtc_context* ctx, SceneRecord& s, const uint8_t* transforms, uint32_t strideBytes, uint32_t first, uint32_t count,
-                        const std::vector<uint32_t>& candidates, const std::vector<GasUpdateInput>& gas, bool tight)
+int write_instance_records_gpu(rtc_context* ctx, SceneRecord& s, const uint8_t* transforms, uint32_t strideBytes, uint32_t first,
+                               uint32_t count, const std::vector<uint32_t>& candidates, const std::vector<GasUpdateInput>& gas, bool tight)
 {
   const uint32_t m = candidates.empty() ? count : (uint32_t)candidates.size();
   if (m == 0) return 0;
-  // after a rebuild the scratch exists (bvh_build_ias_gpu.cu sized it for the node capacity and keeps its parents up to date)
-  if (int rc = alloc_refit_scratch(ctx, s.refit, static_cast<const uint4*>(s.d_tlasNodes), s.desc.numTlasNodes, true)) return rc;
-  // this update's records, per-GAS table and candidate list, one stream-ordered allocation freed behind the kernels; the two
+  // the records, exact bounds, per-GAS table and candidate list, one stream-ordered allocation freed behind the kernels; the two
   // host arrays are small (nothing per instance unless a GAS was refitted) and staged by the copies themselves
-  const size_t upBytes = m * sizeof(InstanceUpdate), inBytes = tight ? m * sizeof(InstanceBoundsIn) : 0, exactBytes = m * sizeof(PrimBox);
+  const size_t upBytes = m * sizeof(InstanceUpdate), exactBytes = m * sizeof(PrimBox);
   const size_t gasBytes = gas.size() * sizeof(GasUpdateInput), listBytes = candidates.size() * sizeof(uint32_t);
   uint8_t* d = nullptr;
-  RTC_CUDA(cudaMallocAsync((void**)&d, upBytes + inBytes + exactBytes + gasBytes + listBytes, ctx->stream));
+  RTC_CUDA(cudaMallocAsync((void**)&d, upBytes + exactBytes + gasBytes + listBytes, ctx->stream));
   GatherParams P;
   P.up = reinterpret_cast<InstanceUpdate*>(d);
-  P.in = tight ? reinterpret_cast<InstanceBoundsIn*>(d + upBytes) : nullptr;
-  PrimBox* d_exact = reinterpret_cast<PrimBox*>(d + upBytes + inBytes);
-  GasUpdateInput* d_gas = reinterpret_cast<GasUpdateInput*>(d + upBytes + inBytes + exactBytes);
-  uint32_t* d_list = reinterpret_cast<uint32_t*>(d + upBytes + inBytes + exactBytes + gasBytes);
+  PrimBox* d_exact = reinterpret_cast<PrimBox*>(d + upBytes);
+  GasUpdateInput* d_gas = reinterpret_cast<GasUpdateInput*>(d + upBytes + exactBytes);
+  uint32_t* d_list = reinterpret_cast<uint32_t*>(d + upBytes + exactBytes + gasBytes);
   P.candidates = candidates.empty() ? nullptr : d_list;
   P.numCandidates = m; P.first = first; P.count = count; P.stride = strideBytes; P.transforms = transforms;
   P.o2w = static_cast<const float4*>(s.d_o2w); P.gasSlot = s.d_instGasSlot; P.gas = d_gas;
@@ -380,37 +340,32 @@ int refit_instances_gpu(rtc_context* ctx, SceneRecord& s, const uint8_t* transfo
     ctx->kernelLaunches++;
     e = cudaGetLastError();
   }
-  const int rc = e == cudaSuccess ? finish_instance_update(ctx, s, P.up, P.in, d_exact, m, tight)
-                                  : rtc_set_error(__FILE__, __LINE__, "refit_instances_gpu", (int)e, cudaGetErrorString(e));
-  cudaFreeAsync(d, ctx->stream);
-  return rc;
-}
-
-// boxes[i] = exact (unpadded) world bounds of the vertices of instance i; instances of an empty GAS get an inverted box
-int instance_bounds_gpu(rtc_context* ctx, const rtc_instance_desc* instances, uint32_t numInstances, PrimBox* boxes)
-{
-  if (numInstances == 0) return 0;
-  std::vector<InstanceBoundsIn> in(numInstances);
-  for (uint32_t i = 0; i < numInstances; ++i)
+  if (e == cudaSuccess && tight)
   {
-    const GasRecord& g = ctx->gas[instances[i].gas];
-    for (int k = 0; k < 12; ++k) in[i].transform[k] = instances[i].transform[k];
-    in[i].verts = reinterpret_cast<const uint8_t*>((uintptr_t)g.attributes); in[i].stride = g.strideBytes;
-    in[i].numVerts = g.numTris ? g.numVerts : 0u; in[i].pad = 0u;
-  }
-  InstanceBoundsIn* d_in = nullptr; PrimBox* d_out = nullptr;
-  RTC_CUDA(cudaMalloc(&d_in, sizeof(InstanceBoundsIn) * numInstances));
-  if (cudaMalloc(&d_out, sizeof(PrimBox) * numInstances) != cudaSuccess) { cudaFree(d_in); RTC_FAIL("cudaMalloc failed"); }
-  cudaError_t e = cudaMemcpyAsync(d_in, in.data(), sizeof(InstanceBoundsIn) * numInstances, cudaMemcpyHostToDevice, ctx->stream);
-  if (e == cudaSuccess)
-  {
-    k_instance_bounds<<<numInstances, kB, 0, ctx->stream>>>(d_in, d_out);
+    k_instance_bounds<<<m, kB, 0, ctx->stream>>>(P.up, d_exact);
     ctx->kernelLaunches++;
     e = cudaGetLastError();
   }
-  if (e == cudaSuccess) e = cudaMemcpyAsync(boxes, d_out, sizeof(PrimBox) * numInstances, cudaMemcpyDeviceToHost, ctx->stream);
-  if (e == cudaSuccess) e = cudaStreamSynchronize(ctx->stream);
-  cudaFree(d_in); cudaFree(d_out);
-  if (e != cudaSuccess) return rtc_set_error(__FILE__, __LINE__, "instance_bounds_gpu", (int)e, cudaGetErrorString(e));
+  if (e == cudaSuccess)
+  {
+    k_instance_finish<<<(m + 127) / 128, 128, 0, ctx->stream>>>(P.up, m, d_exact, tight ? 1 : 0, s.d_instBoxes, static_cast<float4*>(s.d_instances),
+                                                                static_cast<float4*>(s.d_o2w), static_cast<rt_GeometryInstanceData*>(s.d_geomInst));
+    ctx->kernelLaunches++;
+    e = cudaGetLastError();
+  }
+  cudaFreeAsync(d, ctx->stream);
+  if (e != cudaSuccess) return rtc_set_error(__FILE__, __LINE__, "write_instance_records_gpu", (int)e, cudaGetErrorString(e));
   return 0;
+}
+
+// The built node array, or the one rtc_ias_rebuild rebuilt, whose live node count is on the device.
+int refit_instance_level_gpu(rtc_context* ctx, SceneRecord& s)
+{
+  uint4* tlas = static_cast<uint4*>(s.d_tlasNodes);
+  // after a rebuild the scratch exists (bvh_build_ias_gpu.cu sized it for the node capacity and keeps its parents up to date)
+  if (int rc = alloc_refit_scratch(ctx, s.refit, tlas, s.desc.numTlasNodes, true)) return rc;
+  const uint32_t* leaves = static_cast<const uint32_t*>(s.d_tlasLeaves);
+  if (s.rebuild)
+    return launch_refit_nodes(ctx, s.refit, tlas, ias_rebuild_capacity(s.desc.numInstances), nullptr, leaves, s.d_instBoxes, s.d_numTlasNodes);
+  return launch_refit_nodes(ctx, s.refit, tlas, s.desc.numTlasNodes, nullptr, leaves, s.d_instBoxes);
 }

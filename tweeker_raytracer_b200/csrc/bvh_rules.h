@@ -1,11 +1,11 @@
 // bvh_rules.h -- arithmetic that the host builder (bvh_build_host.cpp), the device builders (bvh_build_gpu.cu,
-// bvh_build_ias_gpu.cu), the device refit (bvh_refit.cu) and the host-only twins (accel_host.cpp) must apply bit for bit: the
-// world->object matrix of an instance, the quantisation of one wide node, the padding of an instance's world box, and the Morton
-// codes, radix tree and wide nodes of the LBVH.  One definition, compiled for the host and for sm_100a.
+// bvh_build_ias_gpu.cu), the device instance records and refit (bvh_refit.cu) and the host-only twins (accel_host.cpp) must apply
+// bit for bit: the world->object matrix of an instance, the quantisation of one wide node, the padding of an instance's world box,
+// and the Morton codes, radix tree and wide nodes of the LBVH.  One definition, compiled for the host and for sm_100a.
 //
 // FMA contraction: every product in quantise_node is by a power of two (step * 2^-4, step * 2^-6 with step >= 2^-120, which
 // stays a normal float) and is therefore exact, so a contracted multiply-add rounds exactly like the separate operations.
-// invert_3x4 and instance_box_finish multiply in double by values that are not powers of two: the host compiles them with
+// invert_3x4 and instance_box_finish multiply in double by values that are not powers of two: the host twin compiles them with
 // -ffp-contract=off and bvh_refit.cu with -fmad=false.
 #pragma once
 
@@ -33,8 +33,8 @@ RTC_HD float rules_pow2f(int e)
 // World->object matrix of an instance.  DEFINED here (OptiX computed it inside optixAccelBuild,
 // Device.cpp:1478, read back by closesthit.cu:49-52): adjugate / determinant of the upper 3x3 in double,
 // rounded once to float; translation -(Minv * t) in double.  The oracle states the same definition.
-// rtc_ias_build (accel_host.cpp's host twin too) computes it on the host, rtc_ias_update / rtc_ias_update_device on the device
-// (bvh_refit.cu k_instance_gather); IEEE double division and no contraction give the same bits on both.
+// rtc_ias_build, rtc_ias_update and rtc_ias_update_device compute it on the device (bvh_refit.cu k_instance_gather), the host twin
+// (accel_host.cpp) on the host; IEEE double division and no contraction give the same bits on both.
 RTC_HD void invert_3x4(const float m[12], float out[12])
 {
   const double a = m[0], b = m[1], c = m[2],  tx = m[3];

@@ -3,7 +3,6 @@
 // at the top of rtc_core.h); there is no CPU rendering path here: every entry point that produces
 // rays, hits or pixels ends in a kernel launch on the context's stream.
 #include "rtc_internal.h"
-#include "bvh_rules.h"
 
 #include <chrono>
 #include <cmath>
@@ -55,18 +54,6 @@ const char* scene_unusable(const rtc_context* ctx, const SceneRecord* s, bool re
   return (stale && !refitAllowed) ? kStaleScene : nullptr;
 }
 
-// the host copy of a GAS's bounds after a refit left them on the device (synchronises the stream; build paths only)
-int fetch_gas_bounds(rtc_context* ctx, GasRecord& g)
-{
-  if (!g.boundsOnDevice) return 0;
-  float box[6];
-  RTC_CUDA(cudaMemcpyAsync(box, g.refit.box, sizeof(box), cudaMemcpyDeviceToHost, ctx->stream));
-  RTC_CUDA(cudaStreamSynchronize(ctx->stream));
-  for (int k = 0; k < 3; ++k) { g.lo[k] = box[k]; g.hi[k] = box[3 + k]; }
-  g.boundsOnDevice = false;
-  return 0;
-}
-
 // After rtc_ias_rebuild the instance level's node count is only on the device: bring the host copy (desc.numTlasNodes and the
 // scene's node total) up to date.  Synchronises the stream.
 int sync_tlas_node_count(rtc_context* ctx, SceneRecord* s)
@@ -80,30 +67,43 @@ int sync_tlas_node_count(rtc_context* ctx, SceneRecord* s)
   return 0;
 }
 
-// rtc_ias_update and rtc_ias_update_device (arguments checked): instance first + i takes the matrix at transforms + i * strideBytes
-// (device-readable).  Recomputes exactly the instances of the range and those of every GAS refitted since the last build / update
-// -- no other: the vertex buffer of a GAS that was not refitted may already hold positions its boxes do not bound yet.
-int update_instances(rtc_context* ctx, SceneRecord* s, uint32_t first, uint32_t count, const uint8_t* transforms, uint32_t strideBytes)
+// The per-GAS table of the scene's instance records, in gasGeneration order.  A refitted GAS's bounds are read on the device.
+std::vector<GasUpdateInput> gas_update_inputs(const rtc_context* ctx, const SceneRecord* s)
 {
   std::vector<GasUpdateInput> gas(s->gasGeneration.size());
-  std::vector<uint8_t> refitted(ctx->gas.size(), 0u);
-  bool anyRefitted = false;
   for (size_t k = 0; k < gas.size(); ++k)
   {
     const GasRecord& g = ctx->gas[s->gasGeneration[k].first];
     GasUpdateInput& u = gas[k];
+    u.nodes = g.d_nodes; u.tris = g.d_tris;
     u.verts = reinterpret_cast<const uint8_t*>((uintptr_t)g.attributes); u.stride = g.strideBytes; u.numVerts = g.numTris ? g.numVerts : 0u;
     u.gasBox = g.boundsOnDevice ? g.refit.box : nullptr;
     for (int c = 0; c < 3; ++c) { u.gasLoHi[c] = g.lo[c]; u.gasLoHi[3 + c] = g.hi[c]; }
     u.attributes = g.attributes;
     u.emptyGas = g.numTris == 0 ? 1u : 0u; u.pad = 0u;
-    if (g.generation != s->gasGeneration[k].second) { refitted[s->gasGeneration[k].first] = 1u; anyRefitted = true; }
   }
+  return gas;
+}
+
+// rtc_ias_update and rtc_ias_update_device (arguments checked): instance first + i takes the matrix at transforms + i * strideBytes
+// (device-readable).  Recomputes exactly the instances of the range and those of every GAS refitted since the last build / update
+// -- no other: the vertex buffer of a GAS that was not refitted may already hold positions its boxes do not bound yet.
+int update_instances(rtc_context* ctx, SceneRecord* s, uint32_t first, uint32_t count, const uint8_t* transforms, uint32_t strideBytes)
+{
+  std::vector<uint8_t> refitted(ctx->gas.size(), 0u);
+  bool anyRefitted = false;
+  for (const std::pair<uint32_t, uint64_t>& g : s->gasGeneration)
+    if (ctx->gas[g.first].generation != g.second) { refitted[g.first] = 1u; anyRefitted = true; }
   std::vector<uint32_t> candidates;           // empty: the range
   if (anyRefitted)
     for (uint32_t i = 0; i < s->desc.numInstances; ++i)
       if ((first <= i && i < first + count) || refitted[s->instGas[i]]) candidates.push_back(i);
-  if (int rc = refit_instances_gpu(ctx, *s, transforms, strideBytes, first, count, candidates, gas, instance_bounds_tight())) return rc;
+  if (count || !candidates.empty())
+  {
+    if (int rc = write_instance_records_gpu(ctx, *s, transforms, strideBytes, first, count, candidates, gas_update_inputs(ctx, s),
+                                            instance_bounds_tight())) return rc;
+    if (int rc = refit_instance_level_gpu(ctx, *s)) return rc;
+  }
   for (std::pair<uint32_t, uint64_t>& g : s->gasGeneration) g.second = ctx->gas[g.first].generation;
   return 0;
 }
@@ -452,8 +452,7 @@ int rtc_ias_build(rtc_context* ctx, const rtc_instance_desc* instances, uint32_t
   if (!topObject) RTC_FAIL("topObject is null");
   RTC_CUDA(cudaSetDevice(ctx->device));
   const double t0 = now_ms();
-  std::vector<PrimBox> boxes(numInstances);
-  std::vector<float4> inst((size_t)numInstances * 4u), o2w((size_t)numInstances * 3u);
+  std::vector<float4> o2w((size_t)numInstances * 3u);
   std::vector<rt_GeometryInstanceData> gi(numInstances);
   SceneRecord* rec = new SceneRecord();
   rec->instGas.resize(numInstances);
@@ -463,55 +462,58 @@ int rtc_ias_build(rtc_context* ctx, const rtc_instance_desc* instances, uint32_t
     const rtc_instance_desc& d = instances[i];
     if (d.instanceId != i) { delete rec; RTC_FAIL("instanceId must equal the array position"); }
     if (d.gas >= ctx->gas.size() || ctx->gas[d.gas].d_nodes == nullptr) { delete rec; RTC_FAIL("bad gas handle in instance"); }
-    if (int rc = fetch_gas_bounds(ctx, ctx->gas[d.gas])) { delete rec; return rc; }
-    const GasRecord& g = ctx->gas[d.gas];
     distinct.insert(d.gas);
     rec->instGas[i] = d.gas;
-    float inv[12];
-    invert_3x4(d.transform, inv);
     for (int r = 0; r < 3; ++r)
-    {
-      inst[4u * i + r] = make_float4(inv[4 * r], inv[4 * r + 1], inv[4 * r + 2], inv[4 * r + 3]);
       o2w[3u * i + r] = make_float4(d.transform[4 * r], d.transform[4 * r + 1], d.transform[4 * r + 2], d.transform[4 * r + 3]);
-    }
-    const uint64_t np = (uint64_t)(uintptr_t)g.d_nodes, tp = (uint64_t)(uintptr_t)g.d_tris;
-    const uint32_t w[4] = { (uint32_t)np, (uint32_t)(np >> 32), (uint32_t)tp, (uint32_t)(tp >> 32) };
-    std::memcpy(&inst[4u * i + 3], w, 16);
-    gi[i].attributes = g.attributes; gi[i].indices = g.indices; gi[i].materialIndex = d.materialIndex; gi[i].lightIndex = d.lightIndex;
-
+    gi[i].indices = ctx->gas[d.gas].indices; gi[i].materialIndex = d.materialIndex; gi[i].lightIndex = d.lightIndex;
   }
-  // World bounds per instance: exact bounds of the transformed vertices (device kernel), padded by instance_box_finish
-  // (accel_host.cpp).  RTC_INSTANCE_BOUNDS=box falls back to the eight transformed corners of the GAS box.
-  const bool tight = instance_bounds_tight();
-  if (tight) { if (int rc = instance_bounds_gpu(ctx, instances, numInstances, boxes.data())) { delete rec; return rc; } }
-  for (uint32_t i = 0; i < numInstances; ++i)
+  rec->numGas = (uint32_t)distinct.size();
+  for (uint32_t g : distinct)
   {
-    const GasRecord& g = ctx->gas[instances[i].gas];
-    instance_box_finish(instances[i].transform, g.lo, g.hi, tight, g.numTris == 0, boxes[i]);
+    rec->totalNodes += ctx->gas[g].numNodes; rec->totalTris += ctx->gas[g].numTris; rec->gasBuildMs += ctx->gas[g].buildMs;
+    rec->gasGeneration.emplace_back(g, ctx->gas[g].generation);
+  }
+  // the instance -> GAS table entry of the instance records (the position of the GAS in gasGeneration, which follows `distinct`)
+  std::vector<uint32_t> slot(numInstances);
+  for (uint32_t i = 0; i < numInstances; ++i) slot[i] = (uint32_t)std::distance(distinct.begin(), distinct.find(rec->instGas[i]));
+  rec->instFlags.assign(numInstances, 0u);
+
+  auto alloc = [](void** dst, size_t bytes) { return cudaMalloc(dst, bytes ? bytes : 16); };
+  // stream-ordered: the kernels that write the instance records read what is staged here
+  auto upload = [&](void** dst, const void* src, size_t bytes) -> cudaError_t {
+    cudaError_t e = alloc(dst, bytes);
+    if (e != cudaSuccess) return e;
+    return bytes ? cudaMemcpyAsync(*dst, src, bytes, cudaMemcpyHostToDevice, ctx->stream) : cudaSuccess;
+  };
+  cudaError_t e = cudaSuccess;
+  if (e == cudaSuccess) e = alloc(&rec->d_instances, (size_t)numInstances * 4u * sizeof(float4));
+  if (e == cudaSuccess) e = upload(&rec->d_o2w, o2w.data(), o2w.size() * sizeof(float4));
+  if (e == cudaSuccess) e = upload(&rec->d_geomInst, gi.data(), gi.size() * sizeof(rt_GeometryInstanceData));
+  if (e == cudaSuccess) e = upload(&rec->d_instFlags, rec->instFlags.data(), rec->instFlags.size() * 4u);
+  if (e == cudaSuccess) e = alloc((void**)&rec->d_instBoxes, (size_t)numInstances * sizeof(PrimBox));
+  if (e == cudaSuccess) e = upload((void**)&rec->d_instGasSlot, slot.data(), slot.size() * 4u);
+  if (e != cudaSuccess) { free_scene(rec, ctx->stream); return rtc_set_error(__FILE__, __LINE__, "rtc_ias_build upload", (int)e, cudaGetErrorString(e)); }
+  // Every instance's records from the object->world rows staged above; the instance level is built on the host over the boxes
+  // they hold.  RTC_INSTANCE_BOUNDS=box bounds the eight transformed corners of the GAS box instead of the transformed vertices.
+  std::vector<PrimBox> boxes(numInstances);
+  if (numInstances)
+  {
+    if (int rc = write_instance_records_gpu(ctx, *rec, static_cast<const uint8_t*>(rec->d_o2w), 48u, 0u, numInstances, {},
+                                            gas_update_inputs(ctx, rec), instance_bounds_tight()))
+    {
+      free_scene(rec, ctx->stream);
+      return rc;
+    }
+    e = cudaMemcpyAsync(boxes.data(), rec->d_instBoxes, boxes.size() * sizeof(PrimBox), cudaMemcpyDeviceToHost, ctx->stream);
+    if (e == cudaSuccess) e = cudaStreamSynchronize(ctx->stream);
+    if (e != cudaSuccess) { free_scene(rec, ctx->stream); return rtc_set_error(__FILE__, __LINE__, "rtc_ias_build instance boxes", (int)e, cudaGetErrorString(e)); }
   }
   WideBvh bvh;
   tlas_build_host(boxes.data(), numInstances, bvh);
 
-  auto upload = [&](void** dst, const void* src, size_t bytes) -> cudaError_t {
-    cudaError_t e = cudaMalloc(dst, bytes ? bytes : 16);
-    if (e != cudaSuccess) return e;
-    return bytes ? cudaMemcpy(*dst, src, bytes, cudaMemcpyHostToDevice) : cudaSuccess;
-  };
-  cudaError_t e = cudaSuccess;
   if (e == cudaSuccess) e = upload(&rec->d_tlasNodes, bvh.nodes.data(), bvh.nodes.size() * sizeof(Node8));
   if (e == cudaSuccess) e = upload(&rec->d_tlasLeaves, bvh.primOrder.data(), bvh.primOrder.size() * 4u);
-  if (e == cudaSuccess) e = upload(&rec->d_instances, inst.data(), inst.size() * sizeof(float4));
-  if (e == cudaSuccess) e = upload(&rec->d_o2w, o2w.data(), o2w.size() * sizeof(float4));
-  if (e == cudaSuccess) e = upload(&rec->d_geomInst, gi.data(), gi.size() * sizeof(rt_GeometryInstanceData));
-  rec->instFlags.assign(numInstances, 0u);
-  if (e == cudaSuccess) e = upload(&rec->d_instFlags, rec->instFlags.data(), rec->instFlags.size() * 4u);
-  if (e == cudaSuccess) e = upload((void**)&rec->d_instBoxes, boxes.data(), boxes.size() * sizeof(PrimBox));
-  {
-    // the updates' instance -> GAS table entry (the position of the GAS in gasGeneration below, which follows `distinct`)
-    std::vector<uint32_t> slot(numInstances);
-    for (uint32_t i = 0; i < numInstances; ++i) slot[i] = (uint32_t)std::distance(distinct.begin(), distinct.find(rec->instGas[i]));
-    if (e == cudaSuccess) e = upload((void**)&rec->d_instGasSlot, slot.data(), slot.size() * 4u);
-  }
   rec->desc.instFlags = (const uint32_t*)rec->d_instFlags;
   rec->desc.tlasNodes = (const uint4*)rec->d_tlasNodes;
   rec->desc.tlasLeaves = (const uint32_t*)rec->d_tlasLeaves;
@@ -523,12 +525,7 @@ int rtc_ias_build(rtc_context* ctx, const rtc_instance_desc* instances, uint32_t
   rec->desc.numTlasLeaves = (uint32_t)bvh.primOrder.size();
   if (e == cudaSuccess) e = upload((void**)&rec->d_desc, &rec->desc, sizeof(SceneDesc));
   if (e != cudaSuccess) { free_scene(rec, ctx->stream); return rtc_set_error(__FILE__, __LINE__, "rtc_ias_build upload", (int)e, cudaGetErrorString(e)); }
-  rec->totalNodes = bvh.nodes.size(); rec->totalTris = 0; rec->gasBuildMs = 0.0; rec->numGas = (uint32_t)distinct.size();
-  for (uint32_t g : distinct)
-  {
-    rec->totalNodes += ctx->gas[g].numNodes; rec->totalTris += ctx->gas[g].numTris; rec->gasBuildMs += ctx->gas[g].buildMs;
-    rec->gasGeneration.emplace_back(g, ctx->gas[g].generation);
-  }
+  rec->totalNodes += bvh.nodes.size();
   rec->iasBuildMs = now_ms() - t0;
   ctx->scenes.push_back(rec);
   *topObject = (uint64_t)(uintptr_t)rec->d_desc;

@@ -73,9 +73,10 @@ struct PrimBox { float lo[3], hi[3]; };
 // (geometry scene: 1.30 -> 1.06 instance entries per ray, +7.5 % samples/s).
 void build_wide_bvh_host(const PrimBox* prims, uint32_t numPrims, WideBvh& out, uint32_t leafMax = 3, bool instanceLevel = false);
 
-// accel_host.cpp: the host halves of rtc_gas_build (host SAH builder) and rtc_ias_build -- no CUDA call in any of them -- shared
-// with the host-only twin of the two builds (rtc_host_gas_build / rtc_host_ias_build, include/rtc_core.h).  The world->object
-// matrix of an instance is invert_3x4 (bvh_rules.h), compiled for the host and the device.
+// accel_host.cpp: the host halves of rtc_gas_build (host SAH builder) and rtc_ias_build (the instance level's SAH build) -- no
+// CUDA call in any of them -- shared with the host-only twin of the two builds (rtc_host_gas_build / rtc_host_ias_build,
+// include/rtc_core.h).  The twin's instance boxes and world->object matrices are the reference for the device's instance records
+// (bvh_refit.cu): the same bvh_rules.h arithmetic, compiled for the host and the device.
 bool gas_assemble_host(const uint8_t* verts, uint32_t strideBytes, uint32_t numVerts, const uint32_t* idx, uint32_t numTris,
                        WideBvh& bvh, std::vector<float4>& tris);
 void instance_bounds_host(const float transform[12], const uint8_t* verts, uint32_t strideBytes, uint32_t numVerts, PrimBox& out);
@@ -118,11 +119,11 @@ struct SceneRecord
   std::vector<uint32_t> instFlags;         // host copy of the per-instance flags
   uint32_t numCutout = 0;                  // instances using the cutout hit records: > 0 selects the ordered any-hit path
   bool     albedoTextures = false;         // MaterialDefinition.textureAlbedo may be non-zero: selects the textured shade kernels
-  // The current object->world and world->object matrices live on the device only (d_o2w, d_instances): rtc_ias_update and
-  // rtc_ias_update_device write them there, rtc_scene_export and rtc_instance_inverse read them back.
+  // The current object->world and world->object matrices live on the device only (d_o2w, d_instances): the instance records of
+  // rtc_ias_build, rtc_ias_update and rtc_ias_update_device write them there, rtc_scene_export and rtc_instance_inverse read them back.
   std::vector<uint32_t> instGas;           // GAS handle per instance
   std::vector<std::pair<uint32_t, uint64_t>> gasGeneration;   // each distinct GAS and its generation at the last build / update
-  uint32_t* d_instGasSlot = nullptr;       // per instance: the position of its GAS in gasGeneration (the updates' per-GAS table)
+  uint32_t* d_instGasSlot = nullptr;       // per instance: the position of its GAS in gasGeneration (the instance records' per-GAS table)
   PrimBox* d_instBoxes = nullptr;          // the padded world box of every instance (leaf boxes of the instance level)
   RefitScratch refit;
   // rtc_ias_rebuild (bvh_build_ias_gpu.cu): its arrays, made by the first rebuild, and from then on the instance level's node count
@@ -225,15 +226,15 @@ constexpr uint32_t kGpuBuildThreshold = 1u << 20;
 // bvh_build_gpu.cu: Morton LBVH on the device, straight into rec.d_nodes / rec.d_tris; fills numNodes, lo, hi
 int build_gas_gpu(rtc_context* ctx, GasRecord& rec);
 
-// bvh_refit.cu: exact world bounds of every instance's transformed vertices (one CTA per instance)
-int instance_bounds_gpu(rtc_context* ctx, const rtc_instance_desc* instances, uint32_t numInstances, PrimBox* boxes);
-
-// bvh_refit.cu: refits, all enqueued on ctx->stream without a host synchronisation (except the one-time scratch allocation).
-// refit_gas_gpu rewrites the triangle records from rec.attributes and re-quantises every node bottom-up.
+// bvh_refit.cu: refits and instance records, all enqueued on ctx->stream without a host synchronisation (except the one-time
+// scratch allocation of a GAS refit).  refit_gas_gpu rewrites the triangle records from rec.attributes and re-quantises every
+// node bottom-up.
 int refit_gas_gpu(rtc_context* ctx, GasRecord& rec);
-// One distinct GAS of a scene as an instance update reads it (SceneRecord::gasGeneration order).
+// One distinct GAS of a scene as its instance records read it (SceneRecord::gasGeneration order).
 struct GasUpdateInput
 {
+  const void*    nodes;            // the GAS's node and triangle arrays: row 3 of the traversal record of each of its instances
+  const void*    tris;
   const uint8_t* verts;            // the GAS's vertex records (tight bounds)
   uint32_t stride, numVerts;       // numVerts = 0 for an empty GAS
   const float* gasBox;             // device lo[3], hi[3] of a refitted GAS, or null: gasLoHi
@@ -241,13 +242,17 @@ struct GasUpdateInput
   uint64_t attributes;             // rt_GeometryInstanceData::attributes
   uint32_t emptyGas, pad;
 };
-// The instances an update recomputes (rtc_ias_update, rtc_ias_update_device): candidate j is instance candidates[j], or first + j
-// when `candidates` is empty.  Instance i in [first, first + count) takes the object->world matrix at transforms + (i - first) *
-// strideBytes (device-readable memory, read when the stream gets there), every other candidate keeps its current one (d_o2w).
-// Writes the matrices, shading-table attributes and padded boxes of the candidates and refits the instance level; allocates
-// only from the stream-ordered pool.
-int refit_instances_gpu(rtc_context* ctx, SceneRecord& s, const uint8_t* transforms, uint32_t strideBytes, uint32_t first, uint32_t count,
-                        const std::vector<uint32_t>& candidates, const std::vector<GasUpdateInput>& gas, bool tight);
+// The records of the candidate instances (rtc_ias_build: every instance; rtc_ias_update, rtc_ias_update_device: the recomputed
+// ones): candidate j is instance candidates[j], or first + j when `candidates` is empty.  Instance i in [first, first + count)
+// takes the object->world matrix at transforms + (i - first) * strideBytes (device-readable memory, read when the stream gets
+// there), every other candidate keeps its current one (d_o2w).  Writes the 64 B traversal records (world->object rows, GAS
+// pointers), the object->world rows, shading-table attributes and padded boxes of the candidates; allocates only from the
+// stream-ordered pool.
+int write_instance_records_gpu(rtc_context* ctx, SceneRecord& s, const uint8_t* transforms, uint32_t strideBytes, uint32_t first,
+                               uint32_t count, const std::vector<uint32_t>& candidates, const std::vector<GasUpdateInput>& gas, bool tight);
+// The updates' refit of the instance level's nodes over s.d_instBoxes; a scene's first refit allocates its scratch from the
+// stream-ordered pool.
+int refit_instance_level_gpu(rtc_context* ctx, SceneRecord& s);
 // stream: the one the structure's work runs on (a pooled scratch is freed behind it)
 void free_refit_scratch(RefitScratch& r, cudaStream_t stream);
 
