@@ -12,7 +12,7 @@ CXXFLAGS  := -O2 -std=c++17 -fPIC -ffp-contract=off $(INC) -I/usr/local/cuda/inc
 
 # e.g. make TRACE_DEFS='-DRTC_TRACE_MIN_BLOCKS=5 -DRTC_FETCH_THRESHOLD=16' to explore the traversal kernel's tuning knobs
 TRACE_DEFS ?=
-CORE_OBJS := $(LIB)/kernels_trace.o $(LIB)/kernels_shade.o $(LIB)/probes.o $(LIB)/bvh_build_gpu.o $(LIB)/bvh_build_ias_gpu.o $(LIB)/bvh_refit.o $(LIB)/rtc_api.o $(LIB)/bvh_build_host.o $(LIB)/accel_host.o
+CORE_OBJS := $(LIB)/kernels_trace.o $(LIB)/kernels_shade.o $(LIB)/probes.o $(LIB)/bvh_build_gpu.o $(LIB)/bvh_build_ias_gpu.o $(LIB)/bvh_build_gas_rebuild_gpu.o $(LIB)/bvh_refit.o $(LIB)/rtc_api.o $(LIB)/bvh_build_host.o $(LIB)/accel_host.o
 
 all: core host oracle
 
@@ -27,8 +27,10 @@ $(LIB)/probes.o: $(CSRC)/probes.cu $(CSRC)/rtc_internal.h include/rtc_core.h
 	$(NVCC) $(NVFLAGS) -c $< -o $@
 $(LIB)/bvh_build_gpu.o: $(CSRC)/bvh_build_gpu.cu $(CSRC)/lbvh.cuh $(CSRC)/bvh_rules.h $(CSRC)/rtc_internal.h
 	$(NVCC) $(NVFLAGS) -c $< -o $@
-# instance-level rebuild: FMA contraction off, so the collapse (bvh_rules.h) rounds like its host twin
-$(LIB)/bvh_build_ias_gpu.o: $(CSRC)/bvh_build_ias_gpu.cu $(CSRC)/lbvh.cuh $(CSRC)/bvh_rules.h $(CSRC)/rtc_internal.h include/rtc_core.h
+# instance-level and geometry rebuilds: FMA contraction off, so the collapse (bvh_rules.h) rounds like their host twins
+$(LIB)/bvh_build_ias_gpu.o: $(CSRC)/bvh_build_ias_gpu.cu $(CSRC)/lbvh_collapse.cuh $(CSRC)/lbvh.cuh $(CSRC)/bvh_rules.h $(CSRC)/rtc_internal.h include/rtc_core.h
+	$(NVCC) $(NVFLAGS) -fmad=false -c $< -o $@
+$(LIB)/bvh_build_gas_rebuild_gpu.o: $(CSRC)/bvh_build_gas_rebuild_gpu.cu $(CSRC)/lbvh_collapse.cuh $(CSRC)/lbvh.cuh $(CSRC)/bvh_rules.h $(CSRC)/rtc_internal.h include/rtc_core.h
 	$(NVCC) $(NVFLAGS) -fmad=false -c $< -o $@
 # refit and instance records: FMA contraction off, so invert_3x4 and instance_box_finish (bvh_rules.h) round like the host twin
 $(LIB)/bvh_refit.o: $(CSRC)/bvh_refit.cu $(CSRC)/bvh_rules.h $(CSRC)/rtc_internal.h include/rtc_core.h include/rtigo3_abi.h

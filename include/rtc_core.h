@@ -169,6 +169,20 @@ int rtc_ias_update_device(rtc_context* ctx, uint64_t topObject, uint32_t first, 
  *   and therefore synchronise the stream.
  */
 int rtc_ias_rebuild(rtc_context* ctx, uint64_t topObject);
+/*
+ * rtc_gas_rebuild: a new TOPOLOGY for a GAS, built on the device (LBVH, one triangle per leaf slot) from its current vertex
+ *   positions and written in place: the handle stays valid.  Use it after large deformation, which rtc_gas_refit handles badly
+ *   (DESIGN.md section 3).  attributes: as in rtc_gas_refit (the new vertex records, same stride as the build, which replace the
+ *   GAS's buffer; or 0 = its own buffer, updated in place by the caller); numVerts, numTris, indices and stride stay as built.
+ *   Asynchronous on the context stream: the vertices are read when the stream reaches the rebuild, work enqueued before sees the
+ *   old structure and work enqueued after the new one.  The first rebuild of a GAS allocates its build arrays and a node array of
+ *   the worst-case size and synchronises once; later rebuilds never block the host.  Like a refit it makes every scene that
+ *   instances the GAS stale until rtc_ias_update.  Two rebuilds of the same positions give the same bytes, whichever builder
+ *   made the GAS and whatever refits or rebuilds came before (rtc_host_gas_rebuild reproduces them).  A GAS without triangles
+ *   is left as it is.  After a rebuild the node count lives on the device: rtc_gas_info, rtc_gas_export and rtc_scene_info_get
+ *   read it back and therefore synchronise the stream.  Detect the feature by this export (rtc_version is unchanged).
+ */
+int rtc_gas_rebuild(rtc_context* ctx, uint32_t gas, uint64_t attributes);
 int rtc_scene_info_get(rtc_context* ctx, uint64_t topObject, rtc_scene_info* info);
 /* Frees one scene (the instance level and its tables; GAS stay alive until rtc_gas_destroy / context destroy). */
 int rtc_scene_destroy(rtc_context* ctx, uint64_t topObject);
@@ -235,6 +249,10 @@ int  rtc_host_ias_refit(rtc_host_accel* accel, const float* transforms, const rt
 /* Host-only twin of rtc_ias_rebuild, on an instance-level accel (after rtc_host_ias_build or rtc_host_ias_refit): the same LBVH
  * over the same boxes in the same float arithmetic, so nodes and leaves equal the device rebuild's byte for byte. */
 int  rtc_host_ias_rebuild(rtc_host_accel* accel);
+/* Host-only twin of rtc_gas_rebuild, on a geometry accel from rtc_host_gas_build: the same LBVH over the same triangles in the
+ * same float arithmetic, so nodes and triangle records equal the device rebuild's byte for byte.  attributes: the new vertex
+ * records (strideBytes = the build's), or null to rebuild over the positions of the last build, refit or rebuild. */
+int  rtc_host_gas_rebuild(rtc_host_accel* accel, const void* attributes, uint32_t strideBytes);
 int  rtc_host_accel_info(const rtc_host_accel* accel, uint64_t* numNodes, uint64_t* numPrims, float bounds[6]);
 int  rtc_host_accel_export(const rtc_host_accel* accel, void* nodes, uint32_t* primOrder, float* tris, float* worldToObject);
 void rtc_host_accel_destroy(rtc_host_accel* accel);

@@ -6,6 +6,10 @@
   * device-LBVH soups of bench.py's config 3 (centres uniform in the unit cube, edge n^(-1/3)): rtc_gas_build ms against
     rtc_gas_refit ms, and incoherent closest-hit Mrays/s after a smooth per-vertex displacement of 0, 0.5 and 2 mean edge lengths,
     refitted against rebuilt (the hits of the two are checked to be equal in the same run);
+  * the same soups with their vertex triplets traded among the triangles (a random permutation: the refit's topology is
+    useless): rtc_gas_rebuild ms (the first call, which allocates and synchronises, and the median of later ones), the device
+    memory the first rebuild leaves resident, and incoherent closest-hit Mrays/s refitted (over the first thousandth of the rays),
+    rebuilt on the device (rtc_gas_rebuild) and built anew by rtc_gas_build, whose hits are checked to be equal in the same run;
   * the 10 001-instance scene (tools/make_instances_scene.py): rtc_ias_build ms against rtc_ias_update ms with every instance and
     with 1 % of them moved, rtc_ias_update_device ms with every instance moved (matrices uploaded once, outside the timed call)
     and rtc_ias_rebuild ms, and incoherent closest-hit Mrays/s through the scene after 1, 10 and 100
@@ -83,6 +87,15 @@ def displace(verts, amount, edge, seed=7):
     return out
 
 
+def mem_free():
+    """free bytes of the current device (cudaMemGetInfo of the runtime the library runs on)"""
+    import ctypes as C
+    cudart = C.CDLL("libcudart.so.12")
+    free, total = C.c_size_t(0), C.c_size_t(0)
+    assert cudart.cudaMemGetInfo(C.byref(free), C.byref(total)) == 0
+    return free.value
+
+
 def mrays(ctx, top, d_rays, nrays, d_hits, repeats):
     ms = timed(ctx, lambda: ctx.trace_closest(top, d_rays, nrays, d_hits), repeats)
     return nrays / ms / 1e3
@@ -128,9 +141,36 @@ def soup_runs(ctx, n, nrays, repeats):
              rebuilt_mrays=rebuilt_rate, refitted_over_rebuilt=refit_rate / rebuilt_rate, hits_equal=bool(np.array_equal(a, b)))
         ctx.scene_destroy(fresh_top)
         ctx.gas_destroy(fresh)
+    # the vertex triplets traded among the triangles: refitted, rebuilt on the device, built anew
+    ctx.upload(d_v, verts.reshape(n, 9)[np.random.default_rng(3).permutation(n)].reshape(-1, 3))
+    ctx.gas_refit(gas)
+    ctx.ias_update(top, np.zeros((0, 12), dtype=np.float32))
+    # the refitted GAS traces three orders of magnitude slower: a thousandth of the rays (the first ones, whose hits are compared)
+    nslow = max(1, nrays // 1000)
+    refit_rate = mrays(ctx, top, d_rays, nslow, d_hits, repeats)
+    ctx.synchronize()
+    free0 = mem_free()
+    first_ms = wall(ctx, lambda: ctx.gas_rebuild(gas), 1)
+    resident = free0 - mem_free()
+    rebuild_ms = timed(ctx, lambda: ctx.gas_rebuild(gas), repeats)
+    ctx.ias_update(top, np.zeros((0, 12), dtype=np.float32))
+    rebuilt_rate = mrays(ctx, top, d_rays, nrays, d_hits2, repeats)
+    fresh = build()
+    inst[0]["gas"] = fresh
+    fresh_top = ctx.ias_build(inst)
+    d_hits3 = ctx.malloc(20 * nrays)
+    built_rate = mrays(ctx, fresh_top, d_rays, nrays, d_hits3, repeats)
+    a, b, c = (ctx.download(d, np.uint8, 20 * nrays) for d in (d_hits, d_hits2, d_hits3))
+    a, b_head = a[:20 * nslow], b[:20 * nslow]
+    emit(what="gas_rebuild", triangles=n, build_ms=build_ms, refit_ms=refit_ms, first_rebuild_ms=first_ms, rebuild_ms=rebuild_ms,
+         resident_bytes_after_first_rebuild=resident, resident_bytes_per_triangle=resident / n)
+    emit(what="soup_trace_after_trading_places", triangles=n, rays=nrays, refitted_rays=nslow, refitted_mrays=refit_rate, rebuilt_mrays=rebuilt_rate,
+         built_mrays=built_rate, hits_equal=bool(np.array_equal(a, b_head) and np.array_equal(b, c)))
+    ctx.scene_destroy(fresh_top)
+    ctx.gas_destroy(fresh)
     ctx.scene_destroy(top)
     ctx.gas_destroy(gas)
-    for p in (d_v, d_i, d_rays, d_hits, d_hits2):
+    for p in (d_v, d_i, d_rays, d_hits, d_hits2, d_hits3):
         ctx.free(p)
 
 

@@ -35,6 +35,7 @@ SYMBOLS = [
     "rtc_trace_schedule_get", "rtc_trace_schedule_set",
     "rtc_gas_refit", "rtc_ias_update", "rtc_host_gas_refit", "rtc_host_ias_refit",
     "rtc_ias_rebuild", "rtc_host_ias_rebuild", "rtc_ias_update_device",
+    "rtc_gas_rebuild", "rtc_host_gas_rebuild",
 ]
 
 MATH_FUNCTIONS = ["sin", "cos", "atan", "atan2", "acos", "exp", "log", "pow", "div", "sqrt", "muladd"]     # enum rtc_math_fn
@@ -106,6 +107,7 @@ def lib():
         L.rtc_ias_update.argtypes = [C.c_void_p, C.c_uint64, C.c_uint32, C.c_uint32, C.c_void_p]
         L.rtc_ias_update_device.argtypes = [C.c_void_p, C.c_uint64, C.c_uint32, C.c_uint32, C.c_uint64, C.c_uint32]
         L.rtc_ias_rebuild.argtypes = [C.c_void_p, C.c_uint64]
+        L.rtc_gas_rebuild.argtypes = [C.c_void_p, C.c_uint32, C.c_uint64]
         L.rtc_scene_info_get.argtypes = [C.c_void_p, C.c_uint64, C.POINTER(SceneInfo)]
         L.rtc_scene_destroy.argtypes = [C.c_void_p, C.c_uint64]
         L.rtc_scene_set_instance_flags.argtypes = [C.c_void_p, C.c_uint64, C.c_uint32, C.c_uint32, C.c_void_p]
@@ -141,6 +143,7 @@ def lib():
         L.rtc_host_gas_refit.argtypes = [C.c_void_p, C.c_void_p, C.c_uint32]
         L.rtc_host_ias_refit.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p, C.c_uint32]
         L.rtc_host_ias_rebuild.argtypes = [C.c_void_p]
+        L.rtc_host_gas_rebuild.argtypes = [C.c_void_p, C.c_void_p, C.c_uint32]
         L.rtc_host_accel_info.argtypes = [C.c_void_p, C.POINTER(C.c_uint64), C.POINTER(C.c_uint64), C.c_void_p]
         L.rtc_host_accel_export.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]
         L.rtc_host_accel_destroy.argtypes = [C.c_void_p]
@@ -245,8 +248,11 @@ def host_scene_refit_export(geometries, instances, new_attributes, new_transform
 
 def host_scene_rebuild_export(geometries, instances, steps):
     """host_scene_export of the scene built from (geometries, instances), then taken WITHOUT a GPU through `steps`, in order:
-    "rebuild" (rtc_host_ias_rebuild, the twin of rtc_ias_rebuild) or (new_attributes, new_transforms), a refit as in
-    host_scene_refit_export (rtc_gas_refit of the geometries given, then rtc_ias_update of every instance)."""
+    "rebuild" (rtc_host_ias_rebuild, the twin of rtc_ias_rebuild), ("gas_rebuild", g, attributes) (rtc_host_gas_rebuild, the
+    twin of rtc_gas_rebuild of geometry g: attributes = its new vertex records, or None for its current positions) or
+    (new_attributes, new_transforms), a refit as in host_scene_refit_export (rtc_gas_refit of the geometries given, then
+    rtc_ias_update of every instance).  A device program of rtc_gas_rebuild / rtc_gas_refit calls followed by rtc_ias_update is
+    ("gas_rebuild", ...) steps and then one refit step that refits the other geometries."""
     L = lib()
     accels, info = [], {}
     try:
@@ -256,6 +262,14 @@ def host_scene_rebuild_export(geometries, instances, steps):
         for step in steps:
             if isinstance(step, str) and step == "rebuild":
                 _check(L.rtc_host_ias_rebuild(top))
+                continue
+            if isinstance(step, tuple) and len(step) == 3 and step[0] == "gas_rebuild":
+                _, g, attrs = step
+                if attrs is None:
+                    _check(L.rtc_host_gas_rebuild(accels[g], None, 0))
+                else:
+                    attrs, stride = _vertex_records(attrs)
+                    _check(L.rtc_host_gas_rebuild(accels[g], attrs.ctypes.data_as(C.c_void_p), stride))
                 continue
             new_attributes, new_transforms = step
             for g, attrs in enumerate(new_attributes):
@@ -359,6 +373,12 @@ class Context:
         """rtc_gas_refit: the GAS's vertex positions changed (in place, or d_attributes = new records of the build's stride).
         Every scene instancing it must then get ias_update before it is traced."""
         _check(self.L.rtc_gas_refit(self.h, gas, int(d_attributes)))
+
+    def gas_rebuild(self, gas, d_attributes=0):
+        """rtc_gas_rebuild: a new topology for the GAS from its current vertex positions (its own buffer, updated in place, or
+        d_attributes = new records of the build's stride), on the device and in place (the handle stays valid).  Asynchronous,
+        except for the first rebuild of a GAS.  Every scene instancing it must then get ias_update before it is traced."""
+        _check(self.L.rtc_gas_rebuild(self.h, gas, int(d_attributes)))
 
     def ias_update(self, top, transforms, first=0):
         """rtc_ias_update: transforms [count, 12] (object -> world) of instances first .. first + count - 1 (count may be 0: only

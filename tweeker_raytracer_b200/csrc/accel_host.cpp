@@ -111,7 +111,7 @@ struct rtc_host_accel
   bool isInstanceLevel = false;
   WideBvh bvh;
   std::vector<float4> tris;             // geometry level
-  std::vector<uint8_t> positions;       // geometry level: vertex positions, 12 B apart (for the instance bounds)
+  std::vector<uint8_t> positions;       // geometry level: vertex positions, 12 B apart (for the instance bounds and the rebuild)
   std::vector<uint32_t> indices;        // geometry level: the build's index triplets (for the refit)
   uint32_t numVerts = 0, numTris = 0, strideBytes = 0;
   std::vector<float> inverses;          // instance level: 12 floats per instance
@@ -226,14 +226,14 @@ int rtc_host_ias_refit(rtc_host_accel* accel, const float* transforms, const rtc
   return 0;
 }
 
-// The steps of bvh_build_ias_gpu.cu on host arrays: centre bounds, Morton codes, a stable sort, the radix tree, the fit (min / max,
-// exact in any order) and the breadth-first collapse, whose running counters are the device's per-level exclusive scans.
-int rtc_host_ias_rebuild(rtc_host_accel* accel)
+} // extern "C"
+
+// The steps of the device rebuilds (lbvh_collapse.cuh) on host arrays: centre bounds, Morton codes, a stable sort, the radix tree,
+// the fit (min / max, exact in any order) and the breadth-first collapse, whose running counters are the device's per-level
+// exclusive scans.  out.primOrder: leaf slot -> primitive; out.lo / hi: the fitted box of the root.
+static void lbvh_rebuild_host(const std::vector<PrimBox>& boxes, WideBvh& out)
 {
-  if (!accel || !accel->isInstanceLevel) RTC_FAIL("not an instance-level accel");
-  const std::vector<PrimBox>& boxes = accel->boxes;
   const int n = (int)boxes.size();
-  if (n == 0) return 0;
   std::vector<float4> lo(n), hi(n);
   float centreBox[6] = { FLT_MAX, FLT_MAX, FLT_MAX, -FLT_MAX, -FLT_MAX, -FLT_MAX };
   for (int i = 0; i < n; ++i)
@@ -272,7 +272,6 @@ int rtc_host_ias_rebuild(rtc_host_accel* accel)
     }
   }
 
-  WideBvh& out = accel->bvh;
   out.nodes.assign(1, Node8());
   out.primOrder.assign(n, 0u);
   std::vector<int2> work(1, make_int2(0, 0)), next;
@@ -302,6 +301,55 @@ int rtc_host_ias_rebuild(rtc_host_accel* accel)
     work.swap(next);
   }
   for (int k = 0; k < 3; ++k) { out.lo[k] = box[0].lo[k]; out.hi[k] = box[0].hi[k]; }
+}
+
+extern "C" {
+
+int rtc_host_ias_rebuild(rtc_host_accel* accel)
+{
+  if (!accel || !accel->isInstanceLevel) RTC_FAIL("not an instance-level accel");
+  if (accel->boxes.empty()) return 0;
+  lbvh_rebuild_host(accel->boxes, accel->bvh);
+  return 0;
+}
+
+// rtc_gas_rebuild (bvh_build_gas_rebuild_gpu.cu): triangle boxes as k_gas_boxes computes them, the LBVH over them, the triangle
+// records in leaf order
+int rtc_host_gas_rebuild(rtc_host_accel* accel, const void* attributes, uint32_t strideBytes)
+{
+  if (!accel || accel->isInstanceLevel) RTC_FAIL("not a geometry-level accel");
+  if (attributes)
+  {
+    if (strideBytes != accel->strideBytes) RTC_FAIL("vertex stride differs from the build's");
+    const uint8_t* verts = static_cast<const uint8_t*>(attributes);
+    for (uint32_t v = 0; v < accel->numVerts; ++v) std::memcpy(&accel->positions[(size_t)v * 12u], verts + (size_t)v * strideBytes, 12);
+  }
+  const uint32_t n = accel->numTris;
+  if (n == 0) return 0;
+  auto vertex = [&](uint32_t prim, int c) { return reinterpret_cast<const float*>(&accel->positions[(size_t)accel->indices[3u * prim + c] * 12u]); };
+  std::vector<PrimBox> boxes(n);
+  for (uint32_t t = 0; t < n; ++t)
+  {
+    PrimBox& b = boxes[t];
+    for (int k = 0; k < 3; ++k) { b.lo[k] = FLT_MAX; b.hi[k] = -FLT_MAX; }
+    for (int c = 0; c < 3; ++c)
+    {
+      const float* p = vertex(t, c);
+      for (int k = 0; k < 3; ++k) { b.lo[k] = std::fmin(b.lo[k], p[k]); b.hi[k] = std::fmax(b.hi[k], p[k]); }
+    }
+  }
+  lbvh_rebuild_host(boxes, accel->bvh);
+  for (uint32_t s = 0; s < n; ++s)
+  {
+    const uint32_t prim = accel->bvh.primOrder[s];
+    for (int c = 0; c < 3; ++c)
+    {
+      const float* p = vertex(prim, c);
+      float w = 0.0f;
+      if (c == 0) std::memcpy(&w, &prim, 4);
+      accel->tris[3u * (size_t)s + c] = make_float4(p[0], p[1], p[2], w);
+    }
+  }
   return 0;
 }
 

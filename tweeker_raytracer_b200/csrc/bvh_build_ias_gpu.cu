@@ -2,52 +2,20 @@
 // instance boxes the scene holds (SceneRecord::d_instBoxes) and written in place into its node and leaf arrays.
 //
 //   1. instance boxes -> float4 boxes, exact min / max of their centres          k_ias_boxes
-//   2. 63-bit Morton codes, stable radix sort (key, then index)                   k_morton, cub::DeviceRadixSort
-//   3. binary radix tree (Karras 2012), bottom-up fit                             k_radix_tree, k_fit_boxes (lbvh.cuh)
-//   4. collapse to 8-wide nodes, one instance per leaf slot, level by level       k_ias_pick, k_ias_scan, k_ias_emit
-//   5. instance-level leaves in leaf order, the refit's parent index and zeroed arrival counters (in k_ias_emit)
+//   2. Morton codes, sort, radix tree, fit                                        lbvh_rebuild_tail (lbvh_collapse.cuh)
+//   3. collapse to 8-wide nodes, one instance per leaf slot, level by level       k_ias_pick, k_ias_scan, k_ias_emit
+//   4. instance-level leaves in leaf order, the refit's parent index and zeroed arrival counters (in k_ias_emit)
 //
-// Deterministic bytes: the geometry builder's collapse hands out child blocks with atomicAdd, so its node order depends on the
-// order threads arrive in.  Here every level's child blocks and leaf runs come from an exclusive scan over the level's work
-// items, so the nodes are in breadth-first order, slot by slot: two rebuilds of the same boxes give the same bytes, and the host
-// twin (rtc_host_ias_rebuild, accel_host.cpp) reproduces them.  Children still sit above their parent (the refit relies on it).
-//
-// No host synchronisation after the first call on a scene: the geometry builder reads every level's work count back to the
-// host to size the next launch.  Here the levels are a CUDA graph with a conditional WHILE node (as the cutout any-hit rounds in
-// kernels_shade.cu): the kernels read the level's work count from device memory, and the scan kernel sets the loop condition
-// when the next level is empty.  Everything the graph captures is allocated on the first call, so it stays valid for the scene.
+// The pipeline, its deterministic bytes and its one-time synchronisation are those of lbvh_collapse.cuh, which the geometry
+// rebuild (bvh_build_gas_rebuild_gpu.cu) shares; the leaf slot here holds an instance id.
 //
 // Compiled with -fmad=false: the collapse's surface areas and slot costs (bvh_rules.h) must round like the host twin, which is
 // compiled with -ffp-contract=off.
 #include "rtc_internal.h"
 #include "bvh_rules.h"
-#include "lbvh.cuh"
-
-#include <cub/block/block_scan.cuh>
-#include <cub/device/device_radix_sort.cuh>
-
-#include <cfloat>
+#include "lbvh_collapse.cuh"
 
 namespace {
-
-constexpr int kCollapseBlock = 128;
-constexpr int kScanThreads = 256;
-// words of IasRebuild::counters
-enum { kNodeCount = 0, kLeafCount = 1, kWorkCount = 2 /* two: ping-pong */, kLevelNodeBase = 4, kLevelLeafBase = 5, kNumCounters = 8 };
-
-struct CollapseArgs
-{
-  int n;
-  const int2* child; const float4* boxLo; const float4* boxHi;
-  const uint32_t* order;          // sorted position -> instance
-  uint4* nodes; uint32_t* leaves;
-  uint32_t* parent; uint32_t* arrivals;
-  int* kidAt;                     // 8 per work item: the binary node in each slot, -1 empty
-  uint32_t* local;                // per work item: exclusive prefix in its block, inner count | leaf count << 16
-  uint32_t* blockSums;            // per block: the same packing
-  uint2* blockPrefix;             // per block: exclusive prefix of the level (inner, leaves)
-  uint32_t* counters;
-};
 
 __global__ void __launch_bounds__(kLbvhBlock)
 k_ias_boxes(const PrimBox* __restrict__ boxes, uint32_t n, float4* __restrict__ lo, float4* __restrict__ hi, float* __restrict__ centreBox)
@@ -61,245 +29,47 @@ k_ias_boxes(const PrimBox* __restrict__ boxes, uint32_t n, float4* __restrict__ 
     hi[t] = make_float4(b.hi[0], b.hi[1], b.hi[2], 0.0f);
     for (int k = 0; k < 3; ++k) { cLo[k] = 0.5f * (b.lo[k] + b.hi[k]); cHi[k] = cLo[k]; }
   }
-  __shared__ float sLo[3][kLbvhBlock / 32], sHi[3][kLbvhBlock / 32];
-  for (int k = 0; k < 3; ++k)
-  {
-    float a = cLo[k], b = cHi[k];
-    for (int off = 16; off; off >>= 1) { a = fminf(a, __shfl_down_sync(0xffffffffu, a, off)); b = fmaxf(b, __shfl_down_sync(0xffffffffu, b, off)); }
-    if ((threadIdx.x & 31) == 0) { sLo[k][threadIdx.x >> 5] = a; sHi[k][threadIdx.x >> 5] = b; }
-  }
-  __syncthreads();
-  if (threadIdx.x < 3)
-  {
-    float a = FLT_MAX, b = -FLT_MAX;
-    for (int w = 0; w < kLbvhBlock / 32; ++w) { a = fminf(a, sLo[threadIdx.x][w]); b = fmaxf(b, sHi[threadIdx.x][w]); }
-    if (a <= b) { atomicMinF(centreBox + threadIdx.x, a); atomicMaxF(centreBox + 3 + threadIdx.x, b); }
-  }
+  lbvh_reduce_centre_box(cLo, cHi, centreBox);
 }
 
-// the state of one rebuild: the centre box to reduce into, one wide node (the root, over binary node 0) to collapse
 __global__ void k_ias_begin(float* __restrict__ centreBox, uint32_t* __restrict__ counters, int2* __restrict__ work)
 {
-  for (int k = 0; k < 3; ++k) { centreBox[k] = FLT_MAX; centreBox[3 + k] = -FLT_MAX; }
-  counters[kNodeCount] = 1u; counters[kLeafCount] = 0u;
-  counters[kWorkCount] = 1u; counters[kWorkCount + 1] = 0u;
-  work[0] = make_int2(0, 0);
+  collapse_begin(centreBox, counters, work);
 }
 
-// One thread per work item (binary node, wide node index) of the level: the wide node without its childBase / triBase, its
-// slots' binary nodes, and the exclusive scan of (inner children, leaf slots) within the block.  (Four blocks per SM in the
-// launch bounds: with the bound on threads alone ptxas keeps it at 64 registers and spills.)
+// (Four blocks per SM in the launch bounds: with the bound on threads alone ptxas keeps it at 64 registers and spills.)
 __global__ void __launch_bounds__(kCollapseBlock, 4)
 k_ias_pick(const CollapseArgs A, const int2* __restrict__ work, const uint32_t* __restrict__ workCount)
 {
-  const uint32_t count = *workCount;
-  if (blockIdx.x * kCollapseBlock >= count) return;             // the whole block: no thread reaches the scan
-  const uint32_t w = blockIdx.x * kCollapseBlock + threadIdx.x;
-  uint32_t packed = 0;
-  if (w < count)
-  {
-    const int2 item = work[w];
-    int kidAt[8];
-    union { Node8 n; uint4 v[5]; } node;
-    uint32_t numInner, numLeaves;
-    lbvh_instance_node(item.x, A.n,
-                       [&](int id, float lo[3], float hi[3]) {
-                         const float4 a = A.boxLo[id], b = A.boxHi[id];
-                         lo[0] = a.x; lo[1] = a.y; lo[2] = a.z; hi[0] = b.x; hi[1] = b.y; hi[2] = b.z;
-                       },
-                       [&](int id) { return A.child[id]; }, kidAt, node.n, numInner, numLeaves);
-    for (int j = 0; j < 5; ++j) A.nodes[5u * (size_t)item.y + j] = node.v[j];
-    for (int s = 0; s < 8; ++s) A.kidAt[8u * (size_t)w + s] = kidAt[s];
-    packed = numInner | (numLeaves << 16);
-  }
-  using Scan = cub::BlockScan<uint32_t, kCollapseBlock>;
-  __shared__ typename Scan::TempStorage tmp;
-  uint32_t prefix, total;
-  Scan(tmp).ExclusiveSum(packed, prefix, total);
-  if (w < count) A.local[w] = prefix;
-  if (threadIdx.x == 0) A.blockSums[blockIdx.x] = total;
+  collapse_pick(A, work, workCount);
 }
 
-// One block: the exclusive scan of the level's block sums, the level's bases in the node and leaf arrays, the next level's work
-// count, and (setCondition) the loop condition: run again while the next level has work.
 __global__ void __launch_bounds__(kScanThreads)
 k_ias_scan(const CollapseArgs A, const uint32_t* __restrict__ workCount, uint32_t* __restrict__ nextCount,
            cudaGraphConditionalHandle handle, int setCondition)
 {
-  const uint32_t numBlocks = (*workCount + kCollapseBlock - 1) / kCollapseBlock;
-  const uint32_t per = (numBlocks + kScanThreads - 1) / kScanThreads;
-  const uint32_t first = threadIdx.x * per, last = min(first + per, numBlocks);
-  unsigned long long sum = 0;                                  // inner children in the low word, leaf slots in the high word
-  for (uint32_t b = first; b < last; ++b) { const uint32_t v = A.blockSums[b]; sum += (v & 0xffffu) | ((unsigned long long)(v >> 16) << 32); }
-  using Scan = cub::BlockScan<unsigned long long, kScanThreads>;
-  __shared__ typename Scan::TempStorage tmp;
-  unsigned long long prefix, total;
-  Scan(tmp).ExclusiveSum(sum, prefix, total);
-  for (uint32_t b = first; b < last; ++b)
-  {
-    A.blockPrefix[b] = make_uint2((uint32_t)prefix, (uint32_t)(prefix >> 32));
-    const uint32_t v = A.blockSums[b];
-    prefix += (v & 0xffffu) | ((unsigned long long)(v >> 16) << 32);
-  }
-  if (threadIdx.x == 0)
-  {
-    const uint32_t inner = (uint32_t)total, leaves = (uint32_t)(total >> 32);
-    A.counters[kLevelNodeBase] = A.counters[kNodeCount];
-    A.counters[kLevelLeafBase] = A.counters[kLeafCount];
-    A.counters[kNodeCount] += inner;
-    A.counters[kLeafCount] += leaves;
-    *nextCount = inner;
-    if (setCondition) cudaGraphSetConditional(handle, inner != 0u ? 1u : 0u);
-  }
+  collapse_scan(A, workCount, nextCount, handle, setCondition);
 }
 
-// One thread per work item: childBase / triBase from the scans, the next level's work items, the leaves, the parent of every
-// child and a zero arrival counter for the refit (bvh_refit.cu).
+// the leaf slot holds the instance
 __global__ void __launch_bounds__(kCollapseBlock)
 k_ias_emit(const CollapseArgs A, const int2* __restrict__ work, const uint32_t* __restrict__ workCount, int2* __restrict__ nextWork)
 {
-  const uint32_t w = blockIdx.x * kCollapseBlock + threadIdx.x;
-  if (w >= *workCount) return;
-  const uint32_t dst = (uint32_t)work[w].y;
-  const uint2 bp = A.blockPrefix[blockIdx.x];
-  const uint32_t loc = A.local[w];
-  const uint32_t innerOff = bp.x + (loc & 0xffffu), leafOff = bp.y + (loc >> 16);
-  const uint32_t childBase = A.counters[kLevelNodeBase] + innerOff, triBase = A.counters[kLevelLeafBase] + leafOff;
-  uint32_t inner = 0, leaf = 0;
-  for (int s = 0; s < 8; ++s)
-  {
-    const int kid = A.kidAt[8u * (size_t)w + s];
-    if (kid < 0) continue;
-    if (kid >= A.n - 1) { A.leaves[triBase + leaf] = A.order[kid - (A.n - 1)]; ++leaf; }
-    else
-    {
-      nextWork[innerOff + inner] = make_int2(kid, (int)(childBase + inner));
-      A.parent[childBase + inner] = dst;
-      ++inner;
-    }
-  }
-  uint32_t* words = reinterpret_cast<uint32_t*>(A.nodes + 5u * (size_t)dst);
-  words[4] = inner ? childBase : 0u;
-  words[5] = leaf ? triBase : 0u;
-  A.arrivals[dst] = 0u;
+  collapse_emit(A, work, workCount, nextWork, [&](uint32_t slot, uint32_t p) { A.leaves[slot] = A.order[p]; });
 }
 
-} // namespace
-
-// Everything one scene's rebuilds use, allocated by the first.
-struct IasRebuild
+// First call on a scene: the arrays of lbvh_rebuild_alloc and the collapse graph.  Only then does the scene switch to the new
+// node array: a failure leaves it as it was.
+int setup_rebuild(rtc_context* ctx, SceneRecord& s, LbvhRebuild& R)
 {
-  uint32_t n = 0, capacity = 0;                 // instances, wide nodes the node array holds
-  void* base = nullptr;
-  void* nodes = nullptr; RefitScratch refit;     // the scene's new node array and refit scratch until setup has succeeded
-  float4 *lo = nullptr, *hi = nullptr, *boxLo = nullptr, *boxHi = nullptr;
-  unsigned long long *keys = nullptr, *keysAlt = nullptr;
-  uint32_t *order = nullptr, *orderAlt = nullptr, *flags = nullptr;
-  int2 *child = nullptr, *range = nullptr, *work[2] = { nullptr, nullptr };
-  int* parent = nullptr;
-  float* centreBox = nullptr;
-  void* sortTemp = nullptr; size_t sortBytes = 0;
-  const unsigned long long* sortedKeys = nullptr; const uint32_t* sortedOrder = nullptr;
-  CollapseArgs args{};
-  cudaGraph_t graph = nullptr;
-  cudaGraphExec_t exec = nullptr;
-};
-
-namespace {
-
-// The WHILE loop of the collapse: its body holds two levels (work[0] -> work[1] -> work[0]), so every kernel argument is static.
-int build_collapse_graph(rtc_context* ctx, IasRebuild& R)
-{
-  RTC_CUDA(cudaGraphCreate(&R.graph, 0));
-  cudaGraphConditionalHandle handle;
-  RTC_CUDA(cudaGraphConditionalHandleCreate(&handle, R.graph, 1u, cudaGraphCondAssignDefault));   // the root level always runs
-  cudaGraphNodeParams wp{};
-  wp.type = cudaGraphNodeTypeConditional;
-  wp.conditional.handle = handle; wp.conditional.type = cudaGraphCondTypeWhile; wp.conditional.size = 1;
-  cudaGraphNode_t whileNode = nullptr;
-  RTC_CUDA(cudaGraphAddNode(&whileNode, R.graph, nullptr, 0, &wp));
-  cudaGraph_t body = wp.conditional.phGraph_out[0];
-  RTC_CUDA(cudaStreamBeginCaptureToGraph(ctx->stream, body, nullptr, nullptr, 0, cudaStreamCaptureModeRelaxed));
-  const unsigned grid = (R.capacity + kCollapseBlock - 1) / kCollapseBlock;
-  for (int level = 0; level < 2; ++level)
-  {
-    const uint32_t* count = R.args.counters + kWorkCount + level;
-    uint32_t* nextCount = R.args.counters + kWorkCount + (level ^ 1);
-    k_ias_pick<<<grid, kCollapseBlock, 0, ctx->stream>>>(R.args, R.work[level], count);
-    k_ias_scan<<<1, kScanThreads, 0, ctx->stream>>>(R.args, count, nextCount, handle, level);
-    k_ias_emit<<<grid, kCollapseBlock, 0, ctx->stream>>>(R.args, R.work[level], count, R.work[level ^ 1]);
-  }
-  cudaGraph_t captured = nullptr;
-  const cudaError_t launchError = cudaGetLastError();
-  RTC_CUDA(cudaStreamEndCapture(ctx->stream, &captured));
-  RTC_CUDA(launchError);
-  RTC_CUDA(cudaGraphInstantiate(&R.exec, R.graph, 0));
-  return 0;
-}
-
-// First call on a scene: drains the stream once, allocates a node array of the worst-case size, refit scratch sized for it and
-// the build arrays, and captures the collapse graph.  Only then does the scene switch to the new node array: a failure leaves it
-// as it was.
-int setup_rebuild(rtc_context* ctx, SceneRecord& s, IasRebuild& R)
-{
-  const uint32_t n = s.desc.numInstances;
-  R.n = n;
-  R.capacity = ias_rebuild_capacity(n);
-  const size_t cap = R.capacity, nBin = 2 * (size_t)n;
-  RTC_CUDA(cudaStreamSynchronize(ctx->stream)); // launches in flight may still read the old nodes
-
-  // node array and refit scratch (the layout of alloc_refit_scratch, bvh_refit.cu) of the new capacity
-  RTC_CUDA(cudaMalloc(&R.nodes, cap * sizeof(Node8)));
-  RTC_CUDA(cudaMalloc(&R.refit.base, cap * (2 * sizeof(uint32_t) + 6 * sizeof(float))));
-  R.refit.box = static_cast<float*>(R.refit.base);
-  R.refit.parent = reinterpret_cast<uint32_t*>(R.refit.box + 6 * cap);
-  R.refit.arrivals = R.refit.parent + cap;
-
-  // build arrays, one allocation
-  {
-    cub::DoubleBuffer<unsigned long long> k(nullptr, nullptr);
-    cub::DoubleBuffer<uint32_t> v(nullptr, nullptr);
-    RTC_CUDA(cub::DeviceRadixSort::SortPairs(nullptr, R.sortBytes, k, v, (int)n, 0, 63, ctx->stream));
-  }
-  const size_t numBlocks = (cap + kCollapseBlock - 1) / kCollapseBlock;
-  size_t offset = 0;
-  auto carve = [&](size_t bytes) { const size_t at = offset; offset += (bytes + 255) & ~(size_t)255; return at; };
-  const size_t oLo = carve(n * sizeof(float4)), oHi = carve(n * sizeof(float4));
-  const size_t oBoxLo = carve(nBin * sizeof(float4)), oBoxHi = carve(nBin * sizeof(float4));
-  const size_t oKeys = carve(n * 8u), oKeysAlt = carve(n * 8u), oOrder = carve(n * 4u), oOrderAlt = carve(n * 4u), oFlags = carve(n * 4u);
-  const size_t oChild = carve(n * sizeof(int2)), oRange = carve(n * sizeof(int2)), oParent = carve(nBin * 4u);
-  const size_t oWork0 = carve(cap * sizeof(int2)), oWork1 = carve(cap * sizeof(int2));
-  const size_t oCentre = carve(6 * sizeof(float)), oSort = carve(R.sortBytes);
-  const size_t oKidAt = carve(cap * 8u * sizeof(int)), oLocal = carve(cap * 4u), oBlockSums = carve(numBlocks * 4u);
-  const size_t oBlockPrefix = carve(numBlocks * sizeof(uint2)), oCounters = carve(kNumCounters * 4u);
-  RTC_CUDA(cudaMalloc(&R.base, offset));
-  uint8_t* b = static_cast<uint8_t*>(R.base);
-  R.lo = reinterpret_cast<float4*>(b + oLo); R.hi = reinterpret_cast<float4*>(b + oHi);
-  R.boxLo = reinterpret_cast<float4*>(b + oBoxLo); R.boxHi = reinterpret_cast<float4*>(b + oBoxHi);
-  R.keys = reinterpret_cast<unsigned long long*>(b + oKeys); R.keysAlt = reinterpret_cast<unsigned long long*>(b + oKeysAlt);
-  R.order = reinterpret_cast<uint32_t*>(b + oOrder); R.orderAlt = reinterpret_cast<uint32_t*>(b + oOrderAlt);
-  R.flags = reinterpret_cast<uint32_t*>(b + oFlags);
-  R.child = reinterpret_cast<int2*>(b + oChild); R.range = reinterpret_cast<int2*>(b + oRange);
-  R.parent = reinterpret_cast<int*>(b + oParent);
-  R.work[0] = reinterpret_cast<int2*>(b + oWork0); R.work[1] = reinterpret_cast<int2*>(b + oWork1);
-  R.centreBox = reinterpret_cast<float*>(b + oCentre);
-  R.sortTemp = b + oSort;
-  {
-    // which buffer the sort leaves its result in depends only on n and the key bits: found once (over the still unwritten
-    // arrays), the collapse graph captures it
-    cub::DoubleBuffer<unsigned long long> k(R.keys, R.keysAlt);
-    cub::DoubleBuffer<uint32_t> v(R.order, R.orderAlt);
-    RTC_CUDA(cub::DeviceRadixSort::SortPairs(R.sortTemp, R.sortBytes, k, v, (int)n, 0, 63, ctx->stream));
-    R.sortedKeys = k.Current(); R.sortedOrder = v.Current();
-  }
-  CollapseArgs& A = R.args;
-  A.n = (int)n; A.child = R.child; A.boxLo = R.boxLo; A.boxHi = R.boxHi; A.order = R.sortedOrder;
-  A.nodes = static_cast<uint4*>(R.nodes); A.leaves = static_cast<uint32_t*>(s.d_tlasLeaves);
-  A.parent = R.refit.parent; A.arrivals = R.refit.arrivals;
-  A.kidAt = reinterpret_cast<int*>(b + oKidAt); A.local = reinterpret_cast<uint32_t*>(b + oLocal);
-  A.blockSums = reinterpret_cast<uint32_t*>(b + oBlockSums); A.blockPrefix = reinterpret_cast<uint2*>(b + oBlockPrefix);
-  A.counters = reinterpret_cast<uint32_t*>(b + oCounters);
-  if (int rc = build_collapse_graph(ctx, R)) return rc;
+  if (int rc = lbvh_rebuild_alloc(ctx, R, s.desc.numInstances, static_cast<uint32_t*>(s.d_tlasLeaves))) return rc;
+  const CollapseArgs& A = R.args;
+  if (int rc = build_collapse_graph(ctx, R, [&](int level, unsigned grid, int2* work, const uint32_t* count, uint32_t* nextCount, int2* nextWork,
+                                                cudaGraphConditionalHandle handle) {
+        k_ias_pick<<<grid, kCollapseBlock, 0, ctx->stream>>>(A, work, count);
+        k_ias_scan<<<1, kScanThreads, 0, ctx->stream>>>(A, count, nextCount, handle, level);
+        k_ias_emit<<<grid, kCollapseBlock, 0, ctx->stream>>>(A, work, count, nextWork);
+      })) return rc;
   RTC_CUDA(cudaStreamSynchronize(ctx->stream));
 
   // switch the scene to the new arrays; the cutout graph captured its SceneDesc, and with it the node array freed here
@@ -316,12 +86,12 @@ int setup_rebuild(rtc_context* ctx, SceneRecord& s, IasRebuild& R)
 
 } // namespace
 
-void free_ias_rebuild(IasRebuild* r)
+void free_lbvh_rebuild(LbvhRebuild* r)
 {
   if (!r) return;
   if (r->exec) cudaGraphExecDestroy(r->exec);
   if (r->graph) cudaGraphDestroy(r->graph);
-  cudaFree(r->base); cudaFree(r->nodes); free_refit_scratch(r->refit, nullptr);      // allocated with cudaMalloc by setup_rebuild
+  cudaFree(r->base); cudaFree(r->nodes); free_refit_scratch(r->refit, nullptr);      // allocated with cudaMalloc by lbvh_rebuild_alloc
   delete r;
 }
 
@@ -331,40 +101,22 @@ int rebuild_instances_gpu(rtc_context* ctx, SceneRecord& s)
   if (n == 0) return 0;                          // one empty node: nothing to rebuild
   if (!s.rebuild)
   {
-    IasRebuild* r = new IasRebuild();
+    LbvhRebuild* r = new LbvhRebuild();
     if (int rc = setup_rebuild(ctx, s, *r))
     {
       cudaStreamSynchronize(ctx->stream);
-      free_ias_rebuild(r);
+      free_lbvh_rebuild(r);
       cudaGetLastError();
       return rc;
     }
     s.rebuild = r;
   }
-  IasRebuild& R = *s.rebuild;
+  LbvhRebuild& R = *s.rebuild;
   cudaStream_t st = ctx->stream;
-  const unsigned gridN = (n + kLbvhBlock - 1) / kLbvhBlock;
   k_ias_begin<<<1, 1, 0, st>>>(R.centreBox, R.args.counters, R.work[0]);
   RTC_CUDA(cudaMemsetAsync(R.flags, 0, (size_t)n * sizeof(uint32_t), st));
-  k_ias_boxes<<<gridN, kLbvhBlock, 0, st>>>(s.d_instBoxes, n, R.lo, R.hi, R.centreBox);
-  k_morton<<<gridN, kLbvhBlock, 0, st>>>(R.lo, R.hi, n, R.centreBox, R.keys, R.order);
-  ctx->kernelLaunches += 3;
+  k_ias_boxes<<<(n + kLbvhBlock - 1) / kLbvhBlock, kLbvhBlock, 0, st>>>(s.d_instBoxes, n, R.lo, R.hi, R.centreBox);
+  ctx->kernelLaunches += 2;
   RTC_CUDA(cudaGetLastError());
-  {
-    cub::DoubleBuffer<unsigned long long> k(R.keys, R.keysAlt);
-    cub::DoubleBuffer<uint32_t> v(R.order, R.orderAlt);
-    RTC_CUDA(cub::DeviceRadixSort::SortPairs(R.sortTemp, R.sortBytes, k, v, (int)n, 0, 63, st));
-    if (k.Current() != R.sortedKeys || v.Current() != R.sortedOrder) RTC_FAIL("radix sort changed its output buffer (internal error)");
-  }
-  if (n > 1)
-  {
-    k_radix_tree<<<(n - 1 + kLbvhBlock - 1) / kLbvhBlock, kLbvhBlock, 0, st>>>(R.sortedKeys, (int)n, R.child, R.parent, R.range);
-    ctx->kernelLaunches++;
-  }
-  k_fit_boxes<<<gridN, kLbvhBlock, 0, st>>>((int)n, R.sortedOrder, R.lo, R.hi, R.child, R.parent, R.boxLo, R.boxHi, R.flags);
-  ctx->kernelLaunches++;
-  RTC_CUDA(cudaGetLastError());
-  RTC_CUDA(cudaGraphLaunch(R.exec, st));
-  ctx->kernelLaunches += 6;                      // one body execution; further levels are not counted
-  return 0;
+  return lbvh_rebuild_tail(ctx, R);
 }

@@ -129,7 +129,8 @@ k_refit_nodes(const RefitParams P)
   refit_from(P, i);
 }
 
-// An instance level rtc_ias_rebuild wrote: its node count is on the device, and the nodes above it are not part of the structure.
+// A structure rtc_ias_rebuild or rtc_gas_rebuild wrote: its node count is on the device, and the nodes above it are not part of
+// the structure.
 __global__ void __launch_bounds__(kB)
 k_refit_nodes_live(const RefitParams P, const uint32_t* __restrict__ numNodes)
 {
@@ -308,7 +309,12 @@ int refit_gas_gpu(rtc_context* ctx, GasRecord& rec)
                                                                     (const uint32_t*)(uintptr_t)rec.indices);
   ctx->kernelLaunches++;
   RTC_CUDA(cudaGetLastError());
-  if (int rc = launch_refit_nodes(ctx, rec.refit, nodes, rec.numNodes, static_cast<const float4*>(rec.d_tris), nullptr, nullptr)) return rc;
+  // after rtc_gas_rebuild the scratch is the rebuild's (sized for the node capacity, parents kept up to date by every rebuild) and
+  // the live node count is on the device
+  const int rc = rec.rebuild ? launch_refit_nodes(ctx, rec.refit, nodes, ias_rebuild_capacity(rec.numTris), static_cast<const float4*>(rec.d_tris),
+                                                  nullptr, nullptr, rec.d_numNodes)
+                             : launch_refit_nodes(ctx, rec.refit, nodes, rec.numNodes, static_cast<const float4*>(rec.d_tris), nullptr, nullptr);
+  if (rc) return rc;
   rec.boundsOnDevice = true;
   return 0;
 }

@@ -32,7 +32,7 @@ SceneRecord* find_scene(rtc_context* ctx, uint64_t topObject)
 void free_scene(SceneRecord* s, cudaStream_t stream)
 {
   cudaFree(s->d_desc); cudaFree(s->d_tlasNodes); cudaFree(s->d_instances); cudaFree(s->d_tlasLeaves); cudaFree(s->d_o2w); cudaFree(s->d_geomInst); cudaFree(s->d_instFlags);
-  cudaFree(s->d_instBoxes); cudaFree(s->d_instGasSlot); free_refit_scratch(s->refit, stream); free_ias_rebuild(s->rebuild);
+  cudaFree(s->d_instBoxes); cudaFree(s->d_instGasSlot); free_refit_scratch(s->refit, stream); free_lbvh_rebuild(s->rebuild);
   delete s;
 }
 
@@ -64,6 +64,22 @@ int sync_tlas_node_count(rtc_context* ctx, SceneRecord* s)
   RTC_CUDA(cudaStreamSynchronize(ctx->stream));
   s->totalNodes = s->totalNodes - s->desc.numTlasNodes + count;
   s->desc.numTlasNodes = count;
+  return 0;
+}
+
+// After rtc_gas_rebuild a GAS's node count is only on the device: bring the host copy (numNodes, and the node total of every
+// scene that instances the GAS) up to date.  Synchronises the stream.
+int sync_gas_node_count(rtc_context* ctx, uint32_t gas)
+{
+  GasRecord& g = ctx->gas[gas];
+  if (!g.d_numNodes) return 0;
+  uint32_t count = 0;
+  RTC_CUDA(cudaMemcpyAsync(&count, g.d_numNodes, sizeof(count), cudaMemcpyDeviceToHost, ctx->stream));
+  RTC_CUDA(cudaStreamSynchronize(ctx->stream));
+  for (SceneRecord* s : ctx->scenes)
+    for (const std::pair<uint32_t, uint64_t>& e : s->gasGeneration)
+      if (e.first == gas) s->totalNodes = s->totalNodes - g.numNodes + count;
+  g.numNodes = count;
   return 0;
 }
 
@@ -229,7 +245,7 @@ int rtc_context_destroy(rtc_context* ctx)
   release_cutout_graph(ctx);
   tuner_release(ctx);
   for (SceneRecord* s : ctx->scenes) free_scene(s, ctx->stream);
-  for (GasRecord& g : ctx->gas) { cudaFree(g.d_nodes); cudaFree(g.d_tris); free_refit_scratch(g.refit, ctx->stream); }
+  for (GasRecord& g : ctx->gas) { cudaFree(g.d_nodes); cudaFree(g.d_tris); free_refit_scratch(g.refit, ctx->stream); free_lbvh_rebuild(g.rebuild); }
   if (ctx->wf.base) cudaFree(ctx->wf.base);
   if (ctx->wf.cutBase) cudaFree(ctx->wf.cutBase);
   for (void* t : ctx->textures) cudaFree(t);
@@ -428,8 +444,9 @@ int rtc_gas_destroy(rtc_context* ctx, uint32_t gas)
   RTC_CUDA(cudaSetDevice(ctx->device));
   RTC_CUDA(cudaStreamSynchronize(ctx->stream));
   GasRecord& g = ctx->gas[gas];
-  cudaFree(g.d_nodes); cudaFree(g.d_tris); free_refit_scratch(g.refit, ctx->stream);
+  cudaFree(g.d_nodes); cudaFree(g.d_tris); free_refit_scratch(g.refit, ctx->stream); free_lbvh_rebuild(g.rebuild);
   g.d_nodes = nullptr; g.d_tris = nullptr; g.numNodes = 0; g.numTris = 0; g.boundsOnDevice = false;
+  g.rebuild = nullptr; g.d_numNodes = nullptr;
   return 0;
 }
 
@@ -441,6 +458,16 @@ int rtc_gas_refit(rtc_context* ctx, uint32_t gas, uint64_t attributes)
   if (attributes) g.attributes = attributes;
   g.generation++;
   return refit_gas_gpu(ctx, g);
+}
+
+int rtc_gas_rebuild(rtc_context* ctx, uint32_t gas, uint64_t attributes)
+{
+  if (gas >= ctx->gas.size() || ctx->gas[gas].d_nodes == nullptr) RTC_FAIL("bad gas handle");
+  RTC_CUDA(cudaSetDevice(ctx->device));
+  GasRecord& g = ctx->gas[gas];
+  if (attributes) g.attributes = attributes;
+  g.generation++;
+  return rebuild_gas_gpu(ctx, g);
 }
 
 // ------------------------------------------------------------------------------------------------
@@ -471,6 +498,7 @@ int rtc_ias_build(rtc_context* ctx, const rtc_instance_desc* instances, uint32_t
   rec->numGas = (uint32_t)distinct.size();
   for (uint32_t g : distinct)
   {
+    if (int rc = sync_gas_node_count(ctx, g)) { delete rec; return rc; }
     rec->totalNodes += ctx->gas[g].numNodes; rec->totalTris += ctx->gas[g].numTris; rec->gasBuildMs += ctx->gas[g].buildMs;
     rec->gasGeneration.emplace_back(g, ctx->gas[g].generation);
   }
@@ -594,6 +622,7 @@ int rtc_scene_info_get(rtc_context* ctx, uint64_t topObject, rtc_scene_info* inf
   if (!s) RTC_FAIL("unknown topObject");
   RTC_CUDA(cudaSetDevice(ctx->device));
   if (int rc = sync_tlas_node_count(ctx, s)) return rc;
+  for (const std::pair<uint32_t, uint64_t>& g : s->gasGeneration) if (int rc = sync_gas_node_count(ctx, g.first)) return rc;
   std::memset(info, 0, sizeof(*info));
   info->numNodes = s->totalNodes; info->numTris = s->totalTris; info->numInstances = s->desc.numInstances;
   info->numTlasNodes = s->desc.numTlasNodes; info->numTlasLeaves = s->desc.numTlasLeaves; info->numGas = s->numGas; info->gasBuildMs = s->gasBuildMs; info->iasBuildMs = s->iasBuildMs;
@@ -691,6 +720,11 @@ int rtc_scene_export(rtc_context* ctx, uint64_t topObject, void* tlasNodes, uint
 int rtc_gas_info(rtc_context* ctx, uint32_t gas, uint64_t* numNodes, uint64_t* numTris)
 {
   if (gas >= ctx->gas.size() || ctx->gas[gas].d_nodes == nullptr) RTC_FAIL("bad gas handle");
+  if (ctx->gas[gas].d_numNodes)
+  {
+    RTC_CUDA(cudaSetDevice(ctx->device));
+    if (int rc = sync_gas_node_count(ctx, gas)) return rc;
+  }
   if (numNodes) *numNodes = ctx->gas[gas].numNodes;
   if (numTris) *numTris = ctx->gas[gas].numTris;
   return 0;
@@ -702,6 +736,7 @@ int rtc_gas_export(rtc_context* ctx, uint32_t gas, void* nodes, float* tris)
   const GasRecord& g = ctx->gas[gas];
   RTC_CUDA(cudaSetDevice(ctx->device));
   RTC_CUDA(cudaStreamSynchronize(ctx->stream));
+  if (int rc = sync_gas_node_count(ctx, gas)) return rc;
   if (nodes) RTC_CUDA(cudaMemcpy(nodes, g.d_nodes, (size_t)g.numNodes * sizeof(Node8), cudaMemcpyDeviceToHost));
   if (tris && g.numTris) RTC_CUDA(cudaMemcpy(tris, g.d_tris, (size_t)g.numTris * 12u * sizeof(float), cudaMemcpyDeviceToHost));
   return 0;

@@ -94,6 +94,8 @@ struct RefitScratch
   bool      pooled = false;          // base came from the stream-ordered pool (cudaMallocAsync)
 };
 
+struct LbvhRebuild;
+
 struct GasRecord
 {
   void*    d_nodes = nullptr;              // Node8[numNodes]
@@ -104,12 +106,14 @@ struct GasRecord
   uint32_t strideBytes = 0, numVerts = 0;
   double   buildMs = 0.0;
   int      builder = 0;                    // RTC_BUILD_HOST_SAH or RTC_BUILD_GPU_LBVH
-  uint64_t generation = 0;                 // rtc_gas_refit count: scenes built / updated at an older generation are stale
+  uint64_t generation = 0;                 // rtc_gas_refit / rtc_gas_rebuild count: scenes built / updated at an older generation are stale
   RefitScratch refit;
-  bool     boundsOnDevice = false;         // lo / hi are stale: the refitted bounds are refit.box[0..5] on the device
+  bool     boundsOnDevice = false;         // lo / hi are stale: the refitted or rebuilt bounds are refit.box[0..5] on the device
+  // rtc_gas_rebuild (bvh_build_gas_rebuild_gpu.cu): its arrays, made by the first rebuild, and from then on the node count on the
+  // device -- numNodes is then only brought up to date by sync_gas_node_count (rtc_api.cpp)
+  LbvhRebuild* rebuild = nullptr;
+  const uint32_t* d_numNodes = nullptr;
 };
-
-struct IasRebuild;
 
 struct SceneRecord
 {
@@ -128,7 +132,7 @@ struct SceneRecord
   RefitScratch refit;
   // rtc_ias_rebuild (bvh_build_ias_gpu.cu): its arrays, made by the first rebuild, and from then on the instance level's node count
   // on the device -- desc.numTlasNodes is then only brought up to date by sync_tlas_node_count (rtc_api.cpp)
-  IasRebuild* rebuild = nullptr;
+  LbvhRebuild* rebuild = nullptr;
   const uint32_t* d_numTlasNodes = nullptr;
   uint64_t totalNodes = 0, totalTris = 0;  // unique GAS nodes / triangles referenced + instance level
   uint32_t numGas = 0;
@@ -259,9 +263,13 @@ void free_refit_scratch(RefitScratch& r, cudaStream_t stream);
 // bvh_build_ias_gpu.cu: a new LBVH topology of the instance level over s.d_instBoxes, in place and stream-ordered; the first call
 // on a scene allocates (and synchronises once), later calls never block the host
 int rebuild_instances_gpu(rtc_context* ctx, SceneRecord& s);
-// the wide nodes its node array holds: every wide node but the root has a sibling-group parent, so one-instance leaves give < n + 16
-inline uint32_t ias_rebuild_capacity(uint32_t numInstances) { return numInstances + 16u; }
-void free_ias_rebuild(IasRebuild* r);
+// bvh_build_gas_rebuild_gpu.cu: the same for a geometry, over the triangles of rec.attributes / rec.indices; writes the triangle
+// records in leaf order and the root box into rec.refit.box[0..5]
+int rebuild_gas_gpu(rtc_context* ctx, GasRecord& rec);
+// the wide nodes a rebuilt node array holds: every wide node but the root has a sibling-group parent, so one-primitive leaves give
+// < n + 16 (the same bound as build_gas_gpu's)
+inline uint32_t ias_rebuild_capacity(uint32_t numPrims) { return numPrims + 16u; }
+void free_lbvh_rebuild(LbvhRebuild* r);
 
 // error plumbing (rtc_api.cpp)
 int rtc_set_error(const char* file, int line, const char* call, int code, const char* text);

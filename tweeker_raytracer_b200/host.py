@@ -59,7 +59,7 @@ SYMBOLS = ["rth_last_error", "rth_app_create", "rth_app_destroy", "rth_app_info"
            "rth_app_environment", "rth_app_render", "rth_app_render_calls", "rth_app_set_coalesce", "rth_app_synchronize", "rth_app_frame", "rth_app_local_frame", "rth_app_restart",
            "rth_app_set_composite", "rth_app_save_system", "rth_app_set_camera", "rth_app_update_material", "rth_app_update_light_emission", "rth_app_benchmark", "rth_app_screenshot", "rth_app_tonemap", "rth_app_context", "rth_app_stats",
            "rth_app_update_material_textures", "rth_app_picture", "rth_process_group_id", "rth_app_join_group", "rth_app_group_reduce_mean", "rth_sample_range",
-           "rth_app_update_instance_transform", "rth_app_rebuild_instance_level"]
+           "rth_app_update_instance_transform", "rth_app_rebuild_instance_level", "rth_app_update_geometry"]
 
 _lib = None
 
@@ -102,6 +102,7 @@ def lib():
         L.rth_app_update_light_emission.argtypes = [C.c_void_p, C.c_int, C.c_void_p]
         L.rth_app_update_instance_transform.argtypes = [C.c_void_p, C.c_int, C.c_void_p]
         L.rth_app_rebuild_instance_level.argtypes = [C.c_void_p]
+        L.rth_app_update_geometry.argtypes = [C.c_void_p, C.c_int, C.c_void_p, C.c_uint, C.c_int]
         L.rth_app_render.argtypes = [C.c_void_p, C.c_uint]
         L.rth_app_render.restype = C.c_uint
         L.rth_app_render_calls.argtypes = [C.c_void_p, C.c_uint]
@@ -280,6 +281,16 @@ class App:
         already requested are rendered first."""
         if self.L.rth_app_rebuild_instance_level(self.h) != 0:
             raise core.RtcError("rebuildInstanceLevel failed: %s" % self.L.rth_last_error().decode())
+
+    def update_geometry(self, g, attributes, rebuild=False):
+        """Deforms geometry g (the numbering of geometry(g)): `attributes` are its new vertex records (ATTR_DTYPE, the same count;
+        geometry(g) returns them from then on).  Its GAS is refitted on every device, or rebuilt with rebuild=True (after large
+        deformation, which a refit handles badly), the instances are updated and the accumulation restarts.  Frames already
+        requested are rendered with the old mesh.  A light's definition does not follow a deformed light geometry."""
+        a = np.ascontiguousarray(attributes, dtype=ATTR_DTYPE)
+        rc = self.L.rth_app_update_geometry(self.h, g, a.ctypes.data_as(C.c_void_p), len(a), 1 if rebuild else 0)
+        if rc != 0:
+            raise core.RtcError("updateGeometry(%d) failed: %s" % (g, self.L.rth_last_error().decode() if rc == -2 else "bad index or vertex count"))
 
     # ---- device side
     def render(self, count=1):

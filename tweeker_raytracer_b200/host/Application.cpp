@@ -342,6 +342,16 @@ bool Application::updateInstanceTransform(int index, const float matrix[12])
 
 void Application::rebuildInstanceLevel() { if (m_raytracer) m_raytracer->rebuildInstanceLevel(); }
 
+bool Application::updateGeometry(int index, const TriangleAttributes* attributes, size_t numVerts, bool rebuild)
+{
+  if (index < 0 || (size_t)index >= m_geometries.size()) return false;
+  sg::Triangles& t = *m_geometries[index];
+  if (numVerts != t.getAttributes().size()) return false;
+  t.setAttributes(std::vector<TriangleAttributes>(attributes, attributes + numVerts));
+  if (m_raytracer) m_raytracer->updateGeometry(t.getId(), t.getAttributes().data(), numVerts, rebuild);
+  return true;
+}
+
 void Application::restartAccumulation() { if (m_raytracer) m_raytracer->updateState(m_state); }
 
 unsigned int Application::render(const unsigned int count)

@@ -42,6 +42,8 @@ public:
   // object->world matrix (row-major 3x4) of flattened instance `index` (getFlatInstances); restarts the accumulation
   bool updateInstanceTransform(int index, const float matrix[12]);
   void rebuildInstanceLevel();
+  // new vertex records of geometry `index` (the numbering of getGeometries()); false for a bad index or another vertex count
+  bool updateGeometry(int index, const TriangleAttributes* attributes, size_t numVerts, bool rebuild);
 
   // accessors
   Raytracer* getRaytracer() { return m_raytracer.get(); }

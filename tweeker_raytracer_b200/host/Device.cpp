@@ -324,6 +324,17 @@ void Device::rebuildInstanceLevel()
   RTC_CHECK(rtc_ias_rebuild(m_context, m_systemData.topObject));
 }
 
+void Device::updateGeometry(const unsigned int id, const TriangleAttributes* attributes, const size_t numAttributes, const bool rebuild)
+{
+  activateContext();
+  MY_ASSERT(id < m_geometryData.size() && m_geometryData[id].built && m_geometryData[id].numAttributes == numAttributes);
+  GeometryData& g = m_geometryData[id];
+  RTC_CHECK(rtc_upload(m_context, g.d_attributes, attributes, sizeof(TriangleAttributes) * numAttributes));
+  if (rebuild) RTC_CHECK(rtc_gas_rebuild(m_context, g.gas, 0));
+  else         RTC_CHECK(rtc_gas_refit(m_context, g.gas, 0));
+  RTC_CHECK(rtc_ias_update(m_context, m_systemData.topObject, 0, 0, nullptr));
+}
+
 void Device::setState(DeviceState const& state)
 {
   activateContext();

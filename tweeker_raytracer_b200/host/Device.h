@@ -44,6 +44,10 @@ public:
   // initScene); refits the instance level on the device (rtc_ias_update), stream-ordered behind the launches already enqueued
   virtual void updateInstanceTransforms(const unsigned int first, const unsigned int count, const float* matrices);
   virtual void rebuildInstanceLevel();
+  // new vertex records (48 B TriangleAttributes, the build's count) of geometry `id` (sg::Triangles id): uploaded into this
+  // device's buffer, the GAS refitted (rtc_gas_refit) or rebuilt (rtc_gas_rebuild), the instances updated (rtc_ias_update);
+  // all stream-ordered behind the launches already enqueued
+  virtual void updateGeometry(const unsigned int id, const TriangleAttributes* attributes, const size_t numAttributes, const bool rebuild);
 
   virtual void setState(DeviceState const& state);
   virtual void compositor(Device* other);

@@ -220,6 +220,13 @@ void Raytracer::rebuildInstanceLevel()
   flush();
   for (Device* d : m_activeDevices) d->rebuildInstanceLevel();
 }
+// A deformed mesh (an extension of the reference's Raytracer surface): refitted, or rebuilt after large deformation.
+void Raytracer::updateGeometry(const unsigned int id, const TriangleAttributes* attributes, const size_t numAttributes, const bool rebuild)
+{
+  flush();
+  for (Device* d : m_activeDevices) d->updateGeometry(id, attributes, numAttributes, rebuild);
+  m_iterationIndex = 0;
+}
 void Raytracer::updateState(DeviceState const& state)
 {
   // a new resolution makes the owner free and reallocate the shared frame: no device may still be writing to the old one

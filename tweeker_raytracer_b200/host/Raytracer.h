@@ -42,6 +42,7 @@ public:
   // B200 extension (the reference rebuilt nothing after initScene): moves instances first .. first + count - 1
   virtual void updateInstanceTransforms(const unsigned int first, const unsigned int count, const float* matrices);
   virtual void rebuildInstanceLevel();
+  virtual void updateGeometry(const unsigned int id, const TriangleAttributes* attributes, const size_t numAttributes, const bool rebuild);
   virtual void updateState(DeviceState const& state);
 
   virtual unsigned int render() = 0;                 // one iteration; returns the iterations done so far

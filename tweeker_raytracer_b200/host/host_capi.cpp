@@ -158,6 +158,17 @@ int rth_app_rebuild_instance_level(void* h)
   try { static_cast<Application*>(h)->rebuildInstanceLevel(); return 0; } catch (std::exception const& e) { g_error = e.what(); return -2; }
 }
 
+// new vertex records (48 B each, numVerts = the geometry's) of geometry `g` in the numbering of rth_app_geometry; rebuild != 0: a
+// new GAS topology (after large deformation) instead of a refit
+int rth_app_update_geometry(void* h, int g, const rt_TriangleAttributes* attributes, unsigned int numVerts, int rebuild)
+{
+  try
+  {
+    return static_cast<Application*>(h)->updateGeometry(g, reinterpret_cast<const TriangleAttributes*>(attributes), numVerts, rebuild != 0) ? 0 : -1;
+  }
+  catch (std::exception const& e) { g_error = e.what(); return -2; }
+}
+
 // --- device side (needs a GPU) ---
 unsigned int rth_app_render(void* h, unsigned int count) { return static_cast<Application*>(h)->render(count); }
 // the reference's calling pattern: `calls` times the unchanged `unsigned int Raytracer::render()` (one iteration per call)
