@@ -183,6 +183,45 @@ int rtc_ias_rebuild(rtc_context* ctx, uint64_t topObject);
  *   read it back and therefore synchronise the stream.  Detect the feature by this export (rtc_version is unchanged).
  */
 int rtc_gas_rebuild(rtc_context* ctx, uint32_t gas, uint64_t attributes);
+/*
+ * Scenes whose instance set lives on the device (optixAccelBuild over OPTIX_BUILD_INPUT_TYPE_INSTANCES, called every frame into
+ * the same buffers): spawn and despawn objects, swap an instance's GAS (level of detail, a broken variant) or reassign its
+ * material without a host stall and without a new topObject.
+ *
+ * rtc_ias_create: an empty scene with room for `capacity` instances (0 instances: every ray misses).  Allocates everything its
+ *   builds will use -- tables, boxes, a node array for the capacity, the LBVH arrays and the collapse graph -- and synchronises
+ *   once.  topObject stays valid until rtc_scene_destroy.
+ * rtc_ias_build_device: replaces the scene's whole instance set with numInstances <= capacity rtc_instance_desc records at
+ *   instances + i * strideBytes (device memory or mapped host memory; strideBytes >= 64 and a multiple of 4; 4-byte aligned;
+ *   `instances` and strideBytes may be 0 when numInstances == 0), and builds a new LBVH instance level over them in place.
+ *   - Stream order: the records are read ON THE CONTEXT STREAM, as rtc_ias_update_device reads its matrices: written before the
+ *     stream reaches the call and left unchanged until it has run.  Never synchronises the host; allocates only from the
+ *     stream-ordered pool.  Work enqueued before sees the old instance set, work enqueued after sees the new one.
+ *   - What stays valid: topObject, the SceneDesc it points at, instance flags (they belong to positions and persist across
+ *     builds) and every SystemData that holds the scene.  The cutout any-hit graph is not captured again.
+ *   - Per record: transform, gas, materialIndex and lightIndex come from device memory; the shading table's indices and
+ *     attributes come from the GAS.
+ *   - Rejected records: a record whose gas is out of range or destroyed, or whose instanceId differs from its position, becomes
+ *     an empty instance -- the box and root node of a GAS without triangles, so nothing of it is ever hit or shaded -- and is
+ *     counted for rtc_scene_rejected_instances.  No record can make the traversal read freed or foreign memory.
+ *   - Result bytes: nodes, leaves and world->object matrices equal rtc_host_ias_build + rtc_host_ias_rebuild (and rtc_ias_build
+ *     + rtc_ias_rebuild) of the same records; hits and frames equal those of rtc_ias_build of the same records, bit for bit.
+ *   - Refused (synchronously, nothing enqueued): an unknown topObject, a scene of rtc_ias_build, numInstances > capacity, a bad
+ *     stride or alignment, null records with numInstances > 0.
+ *   rtc_ias_update, rtc_ias_update_device, rtc_ias_rebuild, rtc_scene_set_instance_flags (range checked against the capacity),
+ *   rtc_scene_info_get, rtc_scene_export and rtc_instance_inverse accept created scenes, over the current instance count.
+ *   rtc_scene_info_get and rtc_scene_export read the device's instance -> GAS map (rejected records: 0xffffffff) and node count
+ *   back, and so synchronise.
+ *   Staleness: the host does not know which GAS a created scene references, so it is stale after a refit or rebuild of ANY GAS of
+ *   the context until rtc_ias_update (count 0 is enough) or rtc_ias_build_device runs on it -- conservative: the update then
+ *   recomputes exactly the instances whose GAS changed, selected on the device.  rtc_gas_destroy of a GAS the last build
+ *   references makes the scene unusable ("a GAS of this scene was destroyed") until the next rtc_ias_build_device.
+ * rtc_scene_rejected_instances: the records the last rtc_ias_build_device of the scene rejected.  Synchronises.
+ * Detect the feature by these exports (rtc_version is unchanged).
+ */
+int rtc_ias_create(rtc_context* ctx, uint32_t capacity, uint64_t* topObject);
+int rtc_ias_build_device(rtc_context* ctx, uint64_t topObject, uint64_t instances, uint32_t strideBytes, uint32_t numInstances);
+int rtc_scene_rejected_instances(rtc_context* ctx, uint64_t topObject, uint32_t* count);
 int rtc_scene_info_get(rtc_context* ctx, uint64_t topObject, rtc_scene_info* info);
 /* Frees one scene (the instance level and its tables; GAS stay alive until rtc_gas_destroy / context destroy). */
 int rtc_scene_destroy(rtc_context* ctx, uint64_t topObject);

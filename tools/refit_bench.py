@@ -17,7 +17,13 @@
     left in the built topology): refitted, rebuilt on the device (rtc_ias_rebuild) and rebuilt by rtc_ias_build, whose hits are
     checked to be equal in the same run;
   * about a million small instances (a 12-triangle box on a jittered lattice): rtc_ias_build ms (one run) against
-    rtc_ias_update ms and rtc_ias_update_device ms of every instance, and rtc_ias_rebuild ms.
+    rtc_ias_update ms and rtc_ias_update_device ms of every instance, and rtc_ias_rebuild ms;
+  * an instance set that changes every step, on 10 001 and 1 M of those boxes (two meshes: a box and a smaller one, its level
+    of detail): the whole set, a tenth of it despawned, and a tenth of the instances swapped to the other mesh with new
+    materials.  Each is built into one scene of rtc_ias_create by rtc_ias_build_device from records already in device memory
+    (device ms between events, and host ms of the call and its synchronisation), against rtc_ias_build of the same records and,
+    for the counts a scene of rtc_ias_build can hold, rtc_ias_update_device + rtc_ias_rebuild; incoherent closest-hit Mrays/s of
+    the created and the built scene after each, whose hits are checked to be equal in the same run.
 Builds are timed on the host clock (they end in a synchronisation); refits, updates and traces between CUDA events on the
 context stream, each the median of `repeats` runs after one warm-up.
 """
@@ -317,6 +323,67 @@ def many_instance_runs(ctx, count, repeats):
     ctx.free(d_i)
 
 
+def changing_instance_runs(ctx, count, nrays, repeats):
+    side = int(np.ceil(count ** (1.0 / 3.0)))
+    n = count
+    rng = np.random.default_rng(5)
+    keep, gas = [], []
+    for size in (0.4, 0.25):
+        attrs, idx = box_mesh(size)
+        d_a, d_i = ctx.to_device(attrs), ctx.to_device(idx)
+        keep += [d_a, d_i]
+        gas.append(ctx.gas_build(d_a, attrs.dtype.itemsize, len(attrs), d_i, len(idx), core.BUILD_HOST_SAH))
+    g = np.stack(np.meshgrid(*[np.arange(side)] * 3, indexing="ij"), axis=-1).reshape(-1, 3)[:n].astype(np.float64)
+    xf = np.zeros((n, 3, 4))
+    xf[:, :, :3] = np.eye(3)
+    xf[:, :, 3] = g + rng.uniform(-0.3, 0.3, size=(n, 3))
+    xf = xf.astype(np.float32).reshape(n, 12)
+    full = np.zeros(n, dtype=core.INSTANCE_DTYPE)
+    full["transform"], full["instanceId"], full["gas"], full["lightIndex"] = xf, np.arange(n), gas[0], -1
+    swapped = full.copy()
+    pick = rng.choice(n, n // 10, replace=False)
+    swapped["gas"][pick] = gas[1]
+    swapped["materialIndex"][pick] = 1
+    variants = [("full", full), ("despawned", full[:n - n // 10].copy()), ("swapped", swapped)]
+    rays = bench.rays_numpy(nrays, "incoh", "closest")
+    for c, k in zip("xyz", range(3)):
+        rays["o" + c] = -1.0 + rays["o" + c] * (side + 1.0)
+    d_rays, d_hits, d_hits2 = ctx.to_device(rays), ctx.malloc(20 * nrays), ctx.malloc(20 * nrays)
+    top = ctx.ias_create(n)
+    for what, records in variants:
+        d_rec = ctx.to_device(records)
+        m = len(records)
+        device_ms = timed(ctx, lambda: ctx.ias_build_device(top, d_rec, m), repeats)
+        device_wall_ms = wall(ctx, lambda: ctx.ias_build_device(top, d_rec, m), repeats)
+        tops = []
+        build_ms = wall(ctx, lambda: tops.append(ctx.ias_build(records)), 1 if n > 100000 else repeats)
+        for t in tops[1:]:
+            ctx.scene_destroy(t)
+        built = tops[0]
+        d_xf = ctx.to_device(np.ascontiguousarray(records["transform"]))
+        ctx.ias_rebuild(built)                                            # the scene's first rebuild allocates
+        update_rebuild_ms = timed(ctx, lambda: (ctx.ias_update_device(built, d_xf, m), ctx.ias_rebuild(built)), repeats)
+        ctx.free(d_xf)
+        ctx.ias_build_device(top, d_rec, m)
+        created_rate = mrays(ctx, top, d_rays, nrays, d_hits, repeats)
+        built_fresh = ctx.ias_build(records)
+        built_rate = mrays(ctx, built_fresh, d_rays, nrays, d_hits2, repeats)
+        a = ctx.download(d_hits, np.uint8, 20 * nrays)
+        b = ctx.download(d_hits2, np.uint8, 20 * nrays)
+        emit(what="changing_instances_" + what, capacity=n, instances=m, build_device_ms=device_ms, build_device_wall_ms=device_wall_ms,
+             ias_build_ms=build_ms, update_device_plus_rebuild_ms=update_rebuild_ms, ias_build_over_build_device=build_ms / device_ms,
+             rays=nrays, created_mrays=created_rate, built_mrays=built_rate, hits_equal=bool(np.array_equal(a, b)),
+             rejected=ctx.scene_rejected_instances(top))
+        ctx.scene_destroy(built)
+        ctx.scene_destroy(built_fresh)
+        ctx.free(d_rec)
+    ctx.scene_destroy(top)
+    for h in gas:
+        ctx.gas_destroy(h)
+    for p in keep + [d_rays, d_hits, d_hits2]:
+        ctx.free(p)
+
+
 def main():
     ap = argparse.ArgumentParser(description=__doc__.split("\n")[0])
     ap.add_argument("--sizes", default="1M,10M,100M")
@@ -324,6 +391,7 @@ def main():
     ap.add_argument("--repeats", type=int, default=5)
     ap.add_argument("--no-instances", action="store_true")
     ap.add_argument("--many-instances", default="1M", help="instance count of the small-instance scene (0: skip)")
+    ap.add_argument("--changing-instances", default="10001,1M", help="capacities of the changing instance sets (0: skip)")
     args = ap.parse_args()
     scale = {"K": 10 ** 3, "M": 10 ** 6}
     count = lambda s: int(float(s[:-1]) * scale[s[-1]]) if s[-1] in scale else int(s)    # noqa: E731
@@ -331,12 +399,15 @@ def main():
         raise SystemExit("refit_bench needs a CUDA device: " + core.lib().rtc_last_error().decode())
     emit(what="card", nvidia_smi=card(), rtc_version=core.lib().rtc_version())
     with core.Context(0) as ctx:
-        for s in args.sizes.split(","):
+        for s in filter(None, args.sizes.split(",")):
             soup_runs(ctx, count(s), count(args.rays), args.repeats)
         if not args.no_instances:
             instance_runs(ctx, count(args.rays), args.repeats)
             if count(args.many_instances):
                 many_instance_runs(ctx, count(args.many_instances), args.repeats)
+            for c in args.changing_instances.split(","):
+                if count(c):
+                    changing_instance_runs(ctx, count(c), count(args.rays), args.repeats)
 
 
 if __name__ == "__main__":

@@ -18,6 +18,7 @@ assert RAY_DTYPE.itemsize == 32 and HIT_DTYPE.itemsize == 20 and INSTANCE_DTYPE.
 
 RAYGEN_FULL_FRAME, RAYGEN_LOCAL_COPY = 0, 1
 BUILD_DEFAULT, BUILD_HOST_SAH, BUILD_GPU_LBVH = 0, 1, 2
+REJECTED_INSTANCE = 0xFFFFFFFF      # instance_gas of a record rtc_ias_build_device rejected
 
 # every symbol include/rtc_core.h declares (tests check that the built library exports all of them)
 SYMBOLS = [
@@ -36,6 +37,7 @@ SYMBOLS = [
     "rtc_gas_refit", "rtc_ias_update", "rtc_host_gas_refit", "rtc_host_ias_refit",
     "rtc_ias_rebuild", "rtc_host_ias_rebuild", "rtc_ias_update_device",
     "rtc_gas_rebuild", "rtc_host_gas_rebuild",
+    "rtc_ias_create", "rtc_ias_build_device", "rtc_scene_rejected_instances",
 ]
 
 MATH_FUNCTIONS = ["sin", "cos", "atan", "atan2", "acos", "exp", "log", "pow", "div", "sqrt", "muladd"]     # enum rtc_math_fn
@@ -108,6 +110,9 @@ def lib():
         L.rtc_ias_update_device.argtypes = [C.c_void_p, C.c_uint64, C.c_uint32, C.c_uint32, C.c_uint64, C.c_uint32]
         L.rtc_ias_rebuild.argtypes = [C.c_void_p, C.c_uint64]
         L.rtc_gas_rebuild.argtypes = [C.c_void_p, C.c_uint32, C.c_uint64]
+        L.rtc_ias_create.argtypes = [C.c_void_p, C.c_uint32, C.POINTER(C.c_uint64)]
+        L.rtc_ias_build_device.argtypes = [C.c_void_p, C.c_uint64, C.c_uint64, C.c_uint32, C.c_uint32]
+        L.rtc_scene_rejected_instances.argtypes = [C.c_void_p, C.c_uint64, C.POINTER(C.c_uint32)]
         L.rtc_scene_info_get.argtypes = [C.c_void_p, C.c_uint64, C.POINTER(SceneInfo)]
         L.rtc_scene_destroy.argtypes = [C.c_void_p, C.c_uint64]
         L.rtc_scene_set_instance_flags.argtypes = [C.c_void_p, C.c_uint64, C.c_uint32, C.c_uint32, C.c_void_p]
@@ -407,6 +412,25 @@ class Context:
         _check(self.L.rtc_ias_build(self.h, inst.ctypes.data_as(C.c_void_p), len(inst), C.byref(top)))
         return top.value
 
+    def ias_create(self, capacity):
+        """rtc_ias_create: an empty scene (every ray misses) with room for `capacity` instances, whose instance set
+        ias_build_device replaces in place.  Synchronises once."""
+        top = C.c_uint64(0)
+        _check(self.L.rtc_ias_create(self.h, int(capacity), C.byref(top)))
+        return top.value
+
+    def ias_build_device(self, top, d_records, count, stride=64):
+        """rtc_ias_build_device: the scene's instances become the `count` INSTANCE_DTYPE records at the device address
+        d_records + i * stride (an int, e.g. tensor.data_ptr() of a CUDA uint8 tensor), and its instance level is rebuilt in place.
+        The records are read on the context stream when the build runs, as in ias_update_device.  Never blocks the host."""
+        _check(self.L.rtc_ias_build_device(self.h, int(top), int(d_records), int(stride), int(count)))
+
+    def scene_rejected_instances(self, top):
+        """rtc_scene_rejected_instances: records the last ias_build_device rejected (synchronises)."""
+        n = C.c_uint32(0)
+        _check(self.L.rtc_scene_rejected_instances(self.h, int(top), C.byref(n)))
+        return n.value
+
     def scene_info(self, top):
         info = SceneInfo()
         _check(self.L.rtc_scene_info_get(self.h, int(top), C.byref(info)))
@@ -461,7 +485,7 @@ class Context:
         _check(self.L.rtc_scene_export(self.h, int(top), nodes.ctypes.data_as(C.c_void_p), leaves.ctypes.data_as(C.c_void_p),
                                        w2o.ctypes.data_as(C.c_void_p), inst_gas.ctypes.data_as(C.c_void_p)))
         gas = {}
-        for g in sorted(set(int(v) for v in inst_gas[:info.numInstances])):
+        for g in sorted(set(int(v) for v in inst_gas[:info.numInstances]) - {REJECTED_INSTANCE}):
             nn, nt = C.c_uint64(0), C.c_uint64(0)
             _check(self.L.rtc_gas_info(self.h, g, C.byref(nn), C.byref(nt)))
             gn = np.zeros((nn.value, 80), dtype=np.uint8)

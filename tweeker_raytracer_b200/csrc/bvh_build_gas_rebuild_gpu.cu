@@ -72,7 +72,7 @@ __global__ void k_gas_bounds(const float4* __restrict__ boxLo, const float4* __r
 __global__ void __launch_bounds__(kCollapseBlock, 4)
 k_gas_pick(const CollapseArgs A, const int2* __restrict__ work, const uint32_t* __restrict__ workCount)
 {
-  collapse_pick(A, work, workCount);
+  collapse_pick(A, A.n, work, workCount);
 }
 
 __global__ void __launch_bounds__(kScanThreads)
@@ -87,7 +87,7 @@ __global__ void __launch_bounds__(kCollapseBlock)
 k_gas_emit(const CollapseArgs A, const TriangleLeaves L, const int2* __restrict__ work, const uint32_t* __restrict__ workCount,
            int2* __restrict__ nextWork)
 {
-  collapse_emit(A, work, workCount, nextWork, [&](uint32_t slot, uint32_t p) {
+  collapse_emit(A, A.n, work, workCount, nextWork, [&](uint32_t slot, uint32_t p) {
     const uint8_t* verts = rebuild_verts(A);
     const uint32_t prim = A.order[p];
     float4* out = L.tris + 3u * (size_t)slot;
@@ -160,7 +160,7 @@ int rebuild_gas_gpu(rtc_context* ctx, GasRecord& rec)
   k_gas_boxes<<<(n + kLbvhBlock - 1) / kLbvhBlock, kLbvhBlock, 0, st>>>(verts, triangle_leaves(rec), n, R.lo, R.hi, R.centreBox);
   ctx->kernelLaunches += 2;
   RTC_CUDA(cudaGetLastError());
-  if (int rc = lbvh_rebuild_tail(ctx, R)) return rc;
+  if (int rc = lbvh_rebuild_tail(ctx, R, n)) return rc;
   k_gas_bounds<<<1, 1, 0, st>>>(R.boxLo, R.boxHi, rec.refit.box);
   ctx->kernelLaunches++;
   RTC_CUDA(cudaGetLastError());

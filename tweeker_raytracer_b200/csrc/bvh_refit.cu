@@ -6,8 +6,10 @@
 //                                                   to arrive processes the parent), re-quantised through bvh_rules.h
 //   instance records                 k_instance_gather  one record per written instance: its matrix (device memory: the
 //   (rtc_ias_build,                                     caller's for rtc_ias_update_device, staged by rtc_ias_update, the
-//    rtc_ias_update,                                    scene's own object->world rows for rtc_ias_build), the inverse, its
-//    rtc_ias_update_device)                             GAS's entry of the per-GAS table
+//    rtc_ias_update,                                    scene's own object->world rows for rtc_ias_build, the caller's
+//    rtc_ias_update_device,                             rtc_instance_desc records for rtc_ias_build_device), the inverse, its
+//    rtc_ias_build_device)                              GAS's entry of the per-GAS table (of a created scene: the context's
+//                                                       table, indexed by handle; the records written are selected here)
 //                                    k_instance_bounds, k_instance_finish: the padded world box, the traversal and shading rows
 //   instance-level refit             k_refit_nodes over the instance level (rtc_ias_build builds its nodes on the host instead,
 //   (the updates)                                   over the boxes the records hold)
@@ -146,6 +148,7 @@ struct InstanceUpdate
   float    inverse[12];            // world -> object (invert_3x4)
   GasUpdateInput gas;              // its GAS's entry of the per-GAS table
   uint32_t instance, pad;
+  int32_t  materialIndex, lightIndex;   // rtc_ias_build_device: the record's (written with the GAS's indices)
 };
 
 // ---- instance level: tight world bounds of every instance from its transformed vertices -------------------------
@@ -154,9 +157,11 @@ struct InstanceUpdate
 // corners of the GAS box, which is loose for rotated instances (a torus rotated by 45 degrees: +40 % per axis) and made
 // rays enter instances they cannot hit; an instance entry costs about three node visits.  One CTA per instance now
 // transforms every vertex of the instance's GAS and reduces min/max.
+// numUp: the records k_instance_gather selected on the device (created scenes; the grid is their upper bound), or null
 __global__ void __launch_bounds__(kB)
-k_instance_bounds(const InstanceUpdate* __restrict__ up, PrimBox* __restrict__ out)
+k_instance_bounds(const InstanceUpdate* __restrict__ up, PrimBox* __restrict__ out, const uint32_t* __restrict__ numUp)
 {
+  if (numUp && blockIdx.x >= *numUp) return;
   const InstanceUpdate& I = up[blockIdx.x];
   const GasUpdateInput& g = I.gas;
   float lo[3] = { FLT_MAX, FLT_MAX, FLT_MAX }, hi[3] = { -FLT_MAX, -FLT_MAX, -FLT_MAX };
@@ -198,10 +203,63 @@ struct GatherParams
   uint32_t numCandidates, first, count, stride;
   const uint8_t* transforms;       // the object->world matrices of instances first .. first + count - 1, `stride` bytes apart
   const float4* o2w;               // the scene's current object->world rows (3 per instance)
-  const uint32_t* gasSlot;         // instance -> its entry of `gas`
+  uint32_t* gasSlot;               // instance -> its entry of `gas` (written from the records by rtc_ias_build_device)
   const GasUpdateInput* gas;
   InstanceUpdate* up;
+  // created scenes (null otherwise): thread j looks at instance j < numCandidates and appends the records it writes to `up`,
+  // counting them in words[kCandidateWord]
+  uint32_t* words;
+  const uint8_t* records;          // rtc_ias_build_device: rtc_instance_desc of instance i at records + i * stride
+  uint32_t numGas;                 // handles in `gas` (the context's table)
+  const uint64_t* gasGen;          // per handle: the GAS's generation
+  uint64_t* instGen;               // per instance: the generation its record was written at
+  uint32_t* gasRefs;               // per handle: instances referencing it (rtc_ias_build_device)
+  const void* emptyGas;            // the geometry of a rejected record: one empty node
 };
+
+// A created scene's instance j: whether its record is written and, if so, its matrix, GAS entry and (build) material.
+__device__ __forceinline__ bool gather_created(const GatherParams& P, uint32_t i, InstanceUpdate& u)
+{
+  uint32_t h;
+  if (P.records)
+  {
+    const uint8_t* r = P.records + (size_t)i * P.stride;
+    const uint32_t* w = reinterpret_cast<const uint32_t*>(r);
+    for (int k = 0; k < 12; ++k) u.transform[k] = __uint_as_float(w[k]);
+    h = w[13];
+    if (w[12] != i || h >= P.numGas || P.gas[h].nodes == nullptr) { h = kRejectedInstance; atomicAdd(P.words + kRejectedWord, 1u); }
+    else { atomicAdd(P.gasRefs + h, 1u); P.instGen[i] = P.gasGen[h]; }
+    P.gasSlot[i] = h;
+    u.materialIndex = (int32_t)w[14]; u.lightIndex = (int32_t)w[15];
+  }
+  else
+  {
+    h = P.gasSlot[i];
+    const bool changed = h != kRejectedInstance && P.gasGen[h] != P.instGen[i];
+    if (i - P.first >= P.count && !changed) return false;
+    if (changed) P.instGen[i] = P.gasGen[h];
+    if (i - P.first < P.count)
+    {
+      const float* t = reinterpret_cast<const float*>(P.transforms + (size_t)(i - P.first) * P.stride);
+      for (int k = 0; k < 12; ++k) u.transform[k] = t[k];
+    }
+    else
+      for (int r = 0; r < 3; ++r)
+      {
+        const float4 v = P.o2w[3u * (size_t)i + r];
+        u.transform[4 * r] = v.x; u.transform[4 * r + 1] = v.y; u.transform[4 * r + 2] = v.z; u.transform[4 * r + 3] = v.w;
+      }
+    u.materialIndex = 0; u.lightIndex = 0;
+  }
+  if (h != kRejectedInstance) u.gas = P.gas[h];
+  else
+  {
+    // an empty GAS: a point box at the origin, and nothing to hit if a ray enters it
+    u.gas = GasUpdateInput{};
+    u.gas.nodes = P.emptyGas; u.gas.tris = static_cast<const uint8_t*>(P.emptyGas) + sizeof(Node8); u.gas.emptyGas = 1u;
+  }
+  return true;
+}
 
 // One thread per candidate: its matrix (new from `transforms`, or the current one), the inverse (bvh_rules.h, the bits of the
 // host's invert_3x4: this file is compiled with -fmad=false) and its GAS's table entry, as the records the two kernels below read.
@@ -210,8 +268,16 @@ k_instance_gather(const GatherParams P)
 {
   const uint32_t j = blockIdx.x * blockDim.x + threadIdx.x;
   if (j >= P.numCandidates) return;
-  const uint32_t i = P.candidates ? P.candidates[j] : P.first + j;
   InstanceUpdate u;
+  if (P.words)
+  {
+    if (!gather_created(P, j, u)) return;
+    invert_3x4(u.transform, u.inverse);
+    u.instance = j; u.pad = 0u;
+    P.up[atomicAdd(P.words + kCandidateWord, 1u)] = u;
+    return;
+  }
+  const uint32_t i = P.candidates ? P.candidates[j] : P.first + j;
   if (i - P.first < P.count)                            // unsigned: first <= i < first + count
   {
     const float* t = reinterpret_cast<const float*>(P.transforms + (size_t)(i - P.first) * P.stride);
@@ -233,13 +299,14 @@ k_instance_gather(const GatherParams P)
 
 // One thread per written instance: the padded box (instance_box_finish, bvh_rules.h), the instance's 64 B traversal record
 // (world->object rows 0..2, row 3 = {GAS nodes, GAS triangles}) and its rows of the shading tables (object->world, vertex
-// attributes).
+// attributes; with `material` also the GAS's indices and the record's material and light).  numUp as in k_instance_bounds.
 __global__ void __launch_bounds__(128)
-k_instance_finish(const InstanceUpdate* __restrict__ up, uint32_t count, const PrimBox* __restrict__ exact, int tight,
-                  PrimBox* __restrict__ instBoxes, float4* __restrict__ instances, float4* __restrict__ o2w, rt_GeometryInstanceData* __restrict__ gi)
+k_instance_finish(const InstanceUpdate* __restrict__ up, uint32_t count, const uint32_t* __restrict__ numUp, const PrimBox* __restrict__ exact,
+                  int tight, int material, PrimBox* __restrict__ instBoxes, float4* __restrict__ instances, float4* __restrict__ o2w,
+                  rt_GeometryInstanceData* __restrict__ gi)
 {
   const uint32_t i = blockIdx.x * blockDim.x + threadIdx.x;
-  if (i >= count) return;
+  if (i >= (numUp ? *numUp : count)) return;
   const InstanceUpdate& u = up[i];
   const GasUpdateInput& g = u.gas;
   float gas[6];
@@ -256,6 +323,7 @@ k_instance_finish(const InstanceUpdate* __restrict__ up, uint32_t count, const P
   }
   *reinterpret_cast<ulonglong2*>(instances + 4u * inst + 3) = make_ulonglong2((uintptr_t)g.nodes, (uintptr_t)g.tris);
   gi[inst].attributes = g.attributes;
+  if (material) { gi[inst].indices = g.indices; gi[inst].materialIndex = u.materialIndex; gi[inst].lightIndex = u.lightIndex; }
 }
 
 // pooled: from the stream-ordered pool (the instance level: its updates never allocate with a call that may block)
@@ -338,6 +406,7 @@ int write_instance_records_gpu(rtc_context* ctx, SceneRecord& s, const uint8_t* 
   P.candidates = candidates.empty() ? nullptr : d_list;
   P.numCandidates = m; P.first = first; P.count = count; P.stride = strideBytes; P.transforms = transforms;
   P.o2w = static_cast<const float4*>(s.d_o2w); P.gasSlot = s.d_instGasSlot; P.gas = d_gas;
+  P.words = nullptr; P.records = nullptr; P.numGas = 0; P.gasGen = nullptr; P.instGen = nullptr; P.gasRefs = nullptr; P.emptyGas = nullptr;
   cudaError_t e = cudaMemcpyAsync(d_gas, gas.data(), gasBytes, cudaMemcpyHostToDevice, ctx->stream);
   if (e == cudaSuccess && listBytes) e = cudaMemcpyAsync(d_list, candidates.data(), listBytes, cudaMemcpyHostToDevice, ctx->stream);
   if (e == cudaSuccess)
@@ -348,19 +417,62 @@ int write_instance_records_gpu(rtc_context* ctx, SceneRecord& s, const uint8_t* 
   }
   if (e == cudaSuccess && tight)
   {
-    k_instance_bounds<<<m, kB, 0, ctx->stream>>>(P.up, d_exact);
+    k_instance_bounds<<<m, kB, 0, ctx->stream>>>(P.up, d_exact, nullptr);
     ctx->kernelLaunches++;
     e = cudaGetLastError();
   }
   if (e == cudaSuccess)
   {
-    k_instance_finish<<<(m + 127) / 128, 128, 0, ctx->stream>>>(P.up, m, d_exact, tight ? 1 : 0, s.d_instBoxes, static_cast<float4*>(s.d_instances),
-                                                                static_cast<float4*>(s.d_o2w), static_cast<rt_GeometryInstanceData*>(s.d_geomInst));
+    k_instance_finish<<<(m + 127) / 128, 128, 0, ctx->stream>>>(P.up, m, nullptr, d_exact, tight ? 1 : 0, 0, s.d_instBoxes,
+                                                                static_cast<float4*>(s.d_instances), static_cast<float4*>(s.d_o2w),
+                                                                static_cast<rt_GeometryInstanceData*>(s.d_geomInst));
     ctx->kernelLaunches++;
     e = cudaGetLastError();
   }
   cudaFreeAsync(d, ctx->stream);
   if (e != cudaSuccess) return rtc_set_error(__FILE__, __LINE__, "write_instance_records_gpu", (int)e, cudaGetErrorString(e));
+  return 0;
+}
+
+int write_created_records_gpu(rtc_context* ctx, SceneRecord& s, const uint8_t* records, const uint8_t* transforms, uint32_t strideBytes,
+                              uint32_t first, uint32_t count, bool tight)
+{
+  const uint32_t m = s.desc.numInstances;          // every instance may be written: the device selects them
+  if (m == 0) return 0;
+  const size_t upBytes = m * sizeof(InstanceUpdate);
+  uint8_t* d = nullptr;
+  RTC_CUDA(cudaMallocAsync((void**)&d, upBytes + m * sizeof(PrimBox), ctx->stream));
+  GatherParams P;
+  P.candidates = nullptr; P.numCandidates = m; P.first = first; P.count = count; P.stride = strideBytes; P.transforms = transforms;
+  P.o2w = static_cast<const float4*>(s.d_o2w); P.gasSlot = s.d_instGasSlot; P.gas = ctx->d_gasTable;
+  P.up = reinterpret_cast<InstanceUpdate*>(d);
+  P.words = s.d_words; P.records = records; P.numGas = (uint32_t)ctx->gas.size(); P.gasGen = ctx->d_gasGen; P.instGen = s.d_instGen;
+  P.gasRefs = s.d_gasRefs; P.emptyGas = s.d_emptyGas;
+  PrimBox* d_exact = reinterpret_cast<PrimBox*>(d + upBytes);
+  const uint32_t* numUp = s.d_words + kCandidateWord;
+  cudaError_t e = cudaMemsetAsync(s.d_words + kCandidateWord, 0, sizeof(uint32_t), ctx->stream);
+  if (e == cudaSuccess)
+  {
+    k_instance_gather<<<(m + 127) / 128, 128, 0, ctx->stream>>>(P);
+    ctx->kernelLaunches++;
+    e = cudaGetLastError();
+  }
+  if (e == cudaSuccess && tight)
+  {
+    k_instance_bounds<<<m, kB, 0, ctx->stream>>>(P.up, d_exact, numUp);
+    ctx->kernelLaunches++;
+    e = cudaGetLastError();
+  }
+  if (e == cudaSuccess)
+  {
+    k_instance_finish<<<(m + 127) / 128, 128, 0, ctx->stream>>>(P.up, m, numUp, d_exact, tight ? 1 : 0, records ? 1 : 0, s.d_instBoxes,
+                                                                static_cast<float4*>(s.d_instances), static_cast<float4*>(s.d_o2w),
+                                                                static_cast<rt_GeometryInstanceData*>(s.d_geomInst));
+    ctx->kernelLaunches++;
+    e = cudaGetLastError();
+  }
+  cudaFreeAsync(d, ctx->stream);
+  if (e != cudaSuccess) return rtc_set_error(__FILE__, __LINE__, "write_created_records_gpu", (int)e, cudaGetErrorString(e));
   return 0;
 }
 

@@ -35,7 +35,8 @@ namespace {
 
 constexpr int kCollapseBlock = 128;
 constexpr int kScanThreads = 256;
-// words of LbvhRebuild::counters; kInput (two words) is the caller's: the GAS rebuild keeps the vertex buffer of the call there
+// words of LbvhRebuild::counters; kInput (two words) is the caller's: the GAS rebuild keeps the vertex buffer of the call there,
+// the instance level the primitive count of the call (a created scene's count changes from build to build)
 enum { kNodeCount = 0, kLeafCount = 1, kWorkCount = 2 /* two: ping-pong */, kLevelNodeBase = 4, kLevelLeafBase = 5, kInput = 6, kNumCounters = 8 };
 
 struct CollapseArgs
@@ -81,8 +82,8 @@ __device__ __forceinline__ void collapse_begin(float* __restrict__ centreBox, ui
 }
 
 // One thread per work item (binary node, wide node index) of the level: the wide node without its childBase / triBase, its
-// slots' binary nodes, and the exclusive scan of (inner children, leaf slots) within the block.
-__device__ __forceinline__ void collapse_pick(const CollapseArgs& A, const int2* __restrict__ work, const uint32_t* __restrict__ workCount)
+// slots' binary nodes, and the exclusive scan of (inner children, leaf slots) within the block.  n: the primitives of this build.
+__device__ __forceinline__ void collapse_pick(const CollapseArgs& A, int n, const int2* __restrict__ work, const uint32_t* __restrict__ workCount)
 {
   const uint32_t count = *workCount;
   if (blockIdx.x * kCollapseBlock >= count) return;             // the whole block: no thread reaches the scan
@@ -94,7 +95,7 @@ __device__ __forceinline__ void collapse_pick(const CollapseArgs& A, const int2*
     int kidAt[8];
     union { Node8 n; uint4 v[5]; } node;
     uint32_t numInner, numLeaves;
-    lbvh_instance_node(item.x, A.n,
+    lbvh_instance_node(item.x, n,
                        [&](int id, float lo[3], float hi[3]) {
                          const float4 a = A.boxLo[id], b = A.boxHi[id];
                          lo[0] = a.x; lo[1] = a.y; lo[2] = a.z; hi[0] = b.x; hi[1] = b.y; hi[2] = b.z;
@@ -148,7 +149,7 @@ __device__ __forceinline__ void collapse_scan(const CollapseArgs& A, const uint3
 // child and a zero arrival counter for the refit (bvh_refit.cu).  leaf(slot, p) writes leaf slot `slot`, which holds the
 // primitive at sorted position p.
 template <class Leaf>
-__device__ __forceinline__ void collapse_emit(const CollapseArgs& A, const int2* __restrict__ work, const uint32_t* __restrict__ workCount,
+__device__ __forceinline__ void collapse_emit(const CollapseArgs& A, int n, const int2* __restrict__ work, const uint32_t* __restrict__ workCount,
                                               int2* __restrict__ nextWork, const Leaf& leaf)
 {
   const uint32_t w = blockIdx.x * kCollapseBlock + threadIdx.x;
@@ -163,7 +164,7 @@ __device__ __forceinline__ void collapse_emit(const CollapseArgs& A, const int2*
   {
     const int kid = A.kidAt[8u * (size_t)w + s];
     if (kid < 0) continue;
-    if (kid >= A.n - 1) { leaf(triBase + numLeaves, (uint32_t)(kid - (A.n - 1))); ++numLeaves; }
+    if (kid >= n - 1) { leaf(triBase + numLeaves, (uint32_t)(kid - (n - 1))); ++numLeaves; }
     else
     {
       nextWork[innerOff + inner] = make_int2(kid, (int)(childBase + inner));
@@ -182,7 +183,7 @@ __device__ __forceinline__ void collapse_emit(const CollapseArgs& A, const int2*
 // Everything one structure's rebuilds use, allocated by the first (free_lbvh_rebuild releases it).
 struct LbvhRebuild
 {
-  uint32_t n = 0, capacity = 0;                 // primitives, wide nodes the node array holds
+  uint32_t n = 0, capacity = 0;                 // primitives the arrays hold (at most), wide nodes the node array holds
   void* base = nullptr;
   void* nodes = nullptr; RefitScratch refit;     // the structure's new node array and refit scratch until setup has succeeded
   float4 *lo = nullptr, *hi = nullptr, *boxLo = nullptr, *boxHi = nullptr;
@@ -246,7 +247,7 @@ int lbvh_rebuild_alloc(rtc_context* ctx, LbvhRebuild& R, uint32_t n, uint32_t* l
   R.sortTemp = b + oSort;
   {
     // which buffer the sort leaves its result in depends only on n and the key bits: found once (over the still unwritten
-    // arrays), the collapse graph captures it
+    // arrays), the collapse graph captures it; a build of fewer primitives copies its result there (lbvh_rebuild_tail)
     cub::DoubleBuffer<unsigned long long> k(R.keys, R.keysAlt);
     cub::DoubleBuffer<uint32_t> v(R.order, R.orderAlt);
     RTC_CUDA(cub::DeviceRadixSort::SortPairs(R.sortTemp, R.sortBytes, k, v, (int)n, 0, 63, ctx->stream));
@@ -288,11 +289,10 @@ int build_collapse_graph(rtc_context* ctx, LbvhRebuild& R, const Level& level)
   return 0;
 }
 
-// Every step after the primitive boxes (R.lo, R.hi, R.centreBox): Morton codes, the sort, the radix tree, the fit and the
-// collapse graph, all enqueued on ctx->stream.
-int lbvh_rebuild_tail(rtc_context* ctx, LbvhRebuild& R)
+// Every step after the primitive boxes (R.lo, R.hi, R.centreBox) of n <= R.n primitives: Morton codes, the sort, the radix
+// tree, the fit and the collapse graph, all enqueued on ctx->stream.
+int lbvh_rebuild_tail(rtc_context* ctx, LbvhRebuild& R, uint32_t n)
 {
-  const uint32_t n = R.n;
   cudaStream_t st = ctx->stream;
   const unsigned gridN = (n + kLbvhBlock - 1) / kLbvhBlock;
   k_morton<<<gridN, kLbvhBlock, 0, st>>>(R.lo, R.hi, n, R.centreBox, R.keys, R.order);
@@ -301,8 +301,16 @@ int lbvh_rebuild_tail(rtc_context* ctx, LbvhRebuild& R)
   {
     cub::DoubleBuffer<unsigned long long> k(R.keys, R.keysAlt);
     cub::DoubleBuffer<uint32_t> v(R.order, R.orderAlt);
+    if (n != R.n)
+    {
+      size_t bytes = 0;
+      RTC_CUDA(cub::DeviceRadixSort::SortPairs(nullptr, bytes, k, v, (int)n, 0, 63, st));
+      if (bytes > R.sortBytes) RTC_FAIL("radix sort needs more temporary storage for fewer items (internal error)");
+    }
     RTC_CUDA(cub::DeviceRadixSort::SortPairs(R.sortTemp, R.sortBytes, k, v, (int)n, 0, 63, st));
-    if (k.Current() != R.sortedKeys || v.Current() != R.sortedOrder) RTC_FAIL("radix sort changed its output buffer (internal error)");
+    // the sort's output buffer depends on n: the captured kernels read the one found for R.n
+    if (k.Current() != R.sortedKeys) RTC_CUDA(cudaMemcpyAsync((void*)R.sortedKeys, k.Current(), (size_t)n * 8u, cudaMemcpyDeviceToDevice, st));
+    if (v.Current() != R.sortedOrder) RTC_CUDA(cudaMemcpyAsync((void*)R.sortedOrder, v.Current(), (size_t)n * 4u, cudaMemcpyDeviceToDevice, st));
   }
   if (n > 1)
   {

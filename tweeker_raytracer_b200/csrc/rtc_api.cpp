@@ -4,6 +4,7 @@
 // rays, hits or pixels ends in a kernel launch on the context's stream.
 #include "rtc_internal.h"
 
+#include <algorithm>
 #include <chrono>
 #include <cmath>
 #include <cstdio>
@@ -33,18 +34,30 @@ void free_scene(SceneRecord* s, cudaStream_t stream)
 {
   cudaFree(s->d_desc); cudaFree(s->d_tlasNodes); cudaFree(s->d_instances); cudaFree(s->d_tlasLeaves); cudaFree(s->d_o2w); cudaFree(s->d_geomInst); cudaFree(s->d_instFlags);
   cudaFree(s->d_instBoxes); cudaFree(s->d_instGasSlot); free_refit_scratch(s->refit, stream); free_lbvh_rebuild(s->rebuild);
+  cudaFree(s->d_instGen); cudaFree(s->d_words); cudaFree(s->d_emptyGas);
+  if (s->d_gasRefs) cudaFreeAsync(s->d_gasRefs, stream);
   delete s;
 }
 
 constexpr const char* kDestroyedGas = "a GAS of this scene was destroyed";
 constexpr const char* kStaleScene = "a GAS of this scene was refitted after the scene was built or updated: call rtc_ias_update on the scene first";
+constexpr const char* kStaleCreatedScene = "a GAS of the context was refitted or rebuilt after this scene of rtc_ias_create was built or updated: "
+                                           "call rtc_ias_update on the scene first";
 
 // Why the scene cannot be traced, or nullptr.  A GAS it instances was destroyed: its nodes and triangles are freed, and the
 // scene's instance records still point at them.  Or (unless `refitAllowed`, for the instance updates, which cure it) the scene is
 // stale: a GAS was refitted after the scene was built or last updated, so its instance boxes and instance level no longer
 // bound the triangles, and its shading table may point at a vertex buffer the caller has since freed.
+// A created scene does not know on the host which GAS it references: it is stale after a refit or rebuild of any GAS of the
+// context (conservative; the update then recomputes exactly the instances whose GAS changed), and rtc_gas_destroy marks it when
+// its last build references the handle.
 const char* scene_unusable(const rtc_context* ctx, const SceneRecord* s, bool refitAllowed = false)
 {
+  if (s->created)
+  {
+    if (s->gasDestroyed) return kDestroyedGas;
+    return (s->gasEpoch != ctx->gasEpoch && !refitAllowed) ? kStaleCreatedScene : nullptr;
+  }
   bool stale = false;
   for (const std::pair<uint32_t, uint64_t>& g : s->gasGeneration)
   {
@@ -83,22 +96,61 @@ int sync_gas_node_count(rtc_context* ctx, uint32_t gas)
   return 0;
 }
 
-// The per-GAS table of the scene's instance records, in gasGeneration order.  A refitted GAS's bounds are read on the device.
+// One GAS as its instance records read it.  A refitted GAS's bounds are read on the device; a destroyed one has null nodes.
+GasUpdateInput gas_entry(const GasRecord& g)
+{
+  GasUpdateInput u;
+  u.nodes = g.d_nodes; u.tris = g.d_tris;
+  u.verts = reinterpret_cast<const uint8_t*>((uintptr_t)g.attributes); u.stride = g.strideBytes; u.numVerts = g.numTris ? g.numVerts : 0u;
+  u.gasBox = g.boundsOnDevice ? g.refit.box : nullptr;
+  for (int c = 0; c < 3; ++c) { u.gasLoHi[c] = g.lo[c]; u.gasLoHi[3 + c] = g.hi[c]; }
+  u.attributes = g.attributes;
+  u.emptyGas = g.numTris == 0 ? 1u : 0u; u.pad = 0u;
+  u.indices = g.indices;
+  return u;
+}
+
+// The per-GAS table of the scene's instance records, in gasGeneration order.
 std::vector<GasUpdateInput> gas_update_inputs(const rtc_context* ctx, const SceneRecord* s)
 {
   std::vector<GasUpdateInput> gas(s->gasGeneration.size());
-  for (size_t k = 0; k < gas.size(); ++k)
-  {
-    const GasRecord& g = ctx->gas[s->gasGeneration[k].first];
-    GasUpdateInput& u = gas[k];
-    u.nodes = g.d_nodes; u.tris = g.d_tris;
-    u.verts = reinterpret_cast<const uint8_t*>((uintptr_t)g.attributes); u.stride = g.strideBytes; u.numVerts = g.numTris ? g.numVerts : 0u;
-    u.gasBox = g.boundsOnDevice ? g.refit.box : nullptr;
-    for (int c = 0; c < 3; ++c) { u.gasLoHi[c] = g.lo[c]; u.gasLoHi[3 + c] = g.hi[c]; }
-    u.attributes = g.attributes;
-    u.emptyGas = g.numTris == 0 ? 1u : 0u; u.pad = 0u;
-  }
+  for (size_t k = 0; k < gas.size(); ++k) gas[k] = gas_entry(ctx->gas[s->gasGeneration[k].first]);
   return gas;
+}
+
+// Writes GAS h's entry and generation into the context's device GAS table, stream-ordered; a handle past the table grows it from
+// the pool behind the stream (work already enqueued keeps reading the old table until it is freed behind it).
+int write_gas_table(rtc_context* ctx, uint32_t h)
+{
+  if (h >= ctx->gasTableCapacity)
+  {
+    const uint32_t cap = std::max(std::max(64u, h + 1u), 2u * ctx->gasTableCapacity);
+    GasUpdateInput* table = nullptr;
+    uint64_t* gen = nullptr;
+    RTC_CUDA(cudaMallocAsync((void**)&table, (size_t)cap * sizeof(GasUpdateInput), ctx->stream));
+    const cudaError_t e = cudaMallocAsync((void**)&gen, (size_t)cap * sizeof(uint64_t), ctx->stream);
+    if (e != cudaSuccess) { cudaFreeAsync(table, ctx->stream); return rtc_set_error(__FILE__, __LINE__, "cudaMallocAsync(GAS table)", (int)e, cudaGetErrorString(e)); }
+    if (ctx->gasTableCapacity)
+    {
+      RTC_CUDA(cudaMemcpyAsync(table, ctx->d_gasTable, (size_t)ctx->gasTableCapacity * sizeof(GasUpdateInput), cudaMemcpyDeviceToDevice, ctx->stream));
+      RTC_CUDA(cudaMemcpyAsync(gen, ctx->d_gasGen, (size_t)ctx->gasTableCapacity * sizeof(uint64_t), cudaMemcpyDeviceToDevice, ctx->stream));
+      cudaFreeAsync(ctx->d_gasTable, ctx->stream);
+      cudaFreeAsync(ctx->d_gasGen, ctx->stream);
+    }
+    ctx->d_gasTable = table; ctx->d_gasGen = gen; ctx->gasTableCapacity = cap;
+  }
+  const GasRecord& g = ctx->gas[h];
+  const GasUpdateInput entry = gas_entry(g);
+  RTC_CUDA(cudaMemcpyAsync(ctx->d_gasTable + h, &entry, sizeof(entry), cudaMemcpyHostToDevice, ctx->stream));
+  RTC_CUDA(cudaMemcpyAsync(ctx->d_gasGen + h, &g.generation, sizeof(uint64_t), cudaMemcpyHostToDevice, ctx->stream));
+  return 0;
+}
+
+// instances of a created scene are at most its capacity; flags of positions past the instance count wait for a later build
+void count_cutout(SceneRecord* s)
+{
+  s->numCutout = 0;
+  for (uint32_t i = 0; i < s->desc.numInstances && i < s->instFlags.size(); ++i) if (s->instFlags[i] & RTC_INSTANCE_CUTOUT) s->numCutout++;
 }
 
 // rtc_ias_update and rtc_ias_update_device (arguments checked): instance first + i takes the matrix at transforms + i * strideBytes
@@ -106,6 +158,17 @@ std::vector<GasUpdateInput> gas_update_inputs(const rtc_context* ctx, const Scen
 // -- no other: the vertex buffer of a GAS that was not refitted may already hold positions its boxes do not bound yet.
 int update_instances(rtc_context* ctx, SceneRecord* s, uint32_t first, uint32_t count, const uint8_t* transforms, uint32_t strideBytes)
 {
+  if (s->created)
+  {
+    // the candidates are selected on the device (the range, and the instances whose GAS's generation changed)
+    if (s->desc.numInstances)
+    {
+      if (int rc = write_created_records_gpu(ctx, *s, nullptr, transforms, strideBytes, first, count, instance_bounds_tight())) return rc;
+      if (int rc = refit_instance_level_gpu(ctx, *s)) return rc;
+    }
+    s->gasEpoch = ctx->gasEpoch;
+    return 0;
+  }
   std::vector<uint8_t> refitted(ctx->gas.size(), 0u);
   bool anyRefitted = false;
   for (const std::pair<uint32_t, uint64_t>& g : s->gasGeneration)
@@ -249,6 +312,8 @@ int rtc_context_destroy(rtc_context* ctx)
   if (ctx->wf.base) cudaFree(ctx->wf.base);
   if (ctx->wf.cutBase) cudaFree(ctx->wf.cutBase);
   for (void* t : ctx->textures) cudaFree(t);
+  cudaFree(ctx->d_gasTable);
+  cudaFree(ctx->d_gasGen);
   cudaFree(ctx->d_stats);
   cudaFree(ctx->d_launchCounts);
   cudaFree(ctx->d_cursor);
@@ -435,7 +500,7 @@ int rtc_gas_build(rtc_context* ctx, uint64_t attributes, uint32_t strideBytes, u
   rec.buildMs = now_ms() - t0;
   ctx->gas.push_back(rec);
   *gas = (uint32_t)(ctx->gas.size() - 1);
-  return 0;
+  return write_gas_table(ctx, *gas);
 }
 
 int rtc_gas_destroy(rtc_context* ctx, uint32_t gas)
@@ -444,10 +509,18 @@ int rtc_gas_destroy(rtc_context* ctx, uint32_t gas)
   RTC_CUDA(cudaSetDevice(ctx->device));
   RTC_CUDA(cudaStreamSynchronize(ctx->stream));
   GasRecord& g = ctx->gas[gas];
+  // created scenes whose last build references the handle (the device's reference counts, read now that the stream is drained)
+  for (SceneRecord* s : ctx->scenes)
+    if (s->created && gas < s->gasRefsCount && g.d_nodes)
+    {
+      uint32_t refs = 0;
+      RTC_CUDA(cudaMemcpy(&refs, s->d_gasRefs + gas, sizeof(refs), cudaMemcpyDeviceToHost));
+      if (refs) s->gasDestroyed = true;
+    }
   cudaFree(g.d_nodes); cudaFree(g.d_tris); free_refit_scratch(g.refit, ctx->stream); free_lbvh_rebuild(g.rebuild);
   g.d_nodes = nullptr; g.d_tris = nullptr; g.numNodes = 0; g.numTris = 0; g.boundsOnDevice = false;
   g.rebuild = nullptr; g.d_numNodes = nullptr;
-  return 0;
+  return write_gas_table(ctx, gas);
 }
 
 int rtc_gas_refit(rtc_context* ctx, uint32_t gas, uint64_t attributes)
@@ -457,7 +530,9 @@ int rtc_gas_refit(rtc_context* ctx, uint32_t gas, uint64_t attributes)
   GasRecord& g = ctx->gas[gas];
   if (attributes) g.attributes = attributes;
   g.generation++;
-  return refit_gas_gpu(ctx, g);
+  ctx->gasEpoch++;
+  if (int rc = refit_gas_gpu(ctx, g)) return rc;
+  return write_gas_table(ctx, gas);
 }
 
 int rtc_gas_rebuild(rtc_context* ctx, uint32_t gas, uint64_t attributes)
@@ -467,7 +542,9 @@ int rtc_gas_rebuild(rtc_context* ctx, uint32_t gas, uint64_t attributes)
   GasRecord& g = ctx->gas[gas];
   if (attributes) g.attributes = attributes;
   g.generation++;
-  return rebuild_gas_gpu(ctx, g);
+  ctx->gasEpoch++;
+  if (int rc = rebuild_gas_gpu(ctx, g)) return rc;
+  return write_gas_table(ctx, gas);
 }
 
 // ------------------------------------------------------------------------------------------------
@@ -616,12 +693,124 @@ int rtc_ias_rebuild(rtc_context* ctx, uint64_t topObject)
   return rebuild_instances_gpu(ctx, *s);
 }
 
+// A created scene's GAS totals from the device's per-handle reference counts.  Synchronises the stream.
+int sync_created_scene_totals(rtc_context* ctx, SceneRecord* s)
+{
+  std::vector<uint32_t> refs(s->gasRefsCount);
+  RTC_CUDA(cudaStreamSynchronize(ctx->stream));
+  if (!refs.empty()) RTC_CUDA(cudaMemcpy(refs.data(), s->d_gasRefs, refs.size() * sizeof(uint32_t), cudaMemcpyDeviceToHost));
+  s->numGas = 0; s->totalNodes = s->desc.numTlasNodes; s->totalTris = 0; s->gasBuildMs = 0.0;
+  for (uint32_t h = 0; h < refs.size(); ++h)
+  {
+    if (!refs[h] || !ctx->gas[h].d_nodes) continue;
+    if (int rc = sync_gas_node_count(ctx, h)) return rc;
+    const GasRecord& g = ctx->gas[h];
+    s->numGas++; s->totalNodes += g.numNodes; s->totalTris += g.numTris; s->gasBuildMs += g.buildMs;
+  }
+  return 0;
+}
+
+int rtc_ias_create(rtc_context* ctx, uint32_t capacity, uint64_t* topObject)
+{
+  if (!topObject) RTC_FAIL("topObject is null");
+  RTC_CUDA(cudaSetDevice(ctx->device));
+  SceneRecord* s = new SceneRecord();
+  s->created = true;
+  s->capacity = capacity;
+  s->instFlags.assign(capacity, 0u);
+  const size_t cap = capacity ? capacity : 1u;
+  cudaError_t e = cudaSuccess;
+  auto alloc = [&](void** dst, size_t bytes) { if (e == cudaSuccess) e = cudaMalloc(dst, bytes); };
+  alloc((void**)&s->d_desc, sizeof(SceneDesc));
+  alloc(&s->d_instances, cap * 4u * sizeof(float4));
+  alloc(&s->d_tlasLeaves, cap * sizeof(uint32_t));
+  alloc(&s->d_o2w, cap * 3u * sizeof(float4));
+  alloc(&s->d_geomInst, cap * sizeof(rt_GeometryInstanceData));
+  alloc(&s->d_instFlags, cap * sizeof(uint32_t));
+  alloc((void**)&s->d_instBoxes, cap * sizeof(PrimBox));
+  alloc((void**)&s->d_instGasSlot, cap * sizeof(uint32_t));
+  alloc((void**)&s->d_instGen, cap * sizeof(uint64_t));
+  alloc((void**)&s->d_words, kSceneWords * sizeof(uint32_t));
+  alloc(&s->d_emptyGas, sizeof(Node8) + 3u * sizeof(float4));
+  // the empty GAS of rejected records: every slot of its root empty (imask 0, meta 0)
+  if (e == cudaSuccess) e = cudaMemsetAsync(s->d_emptyGas, 0, sizeof(Node8) + 3u * sizeof(float4), ctx->stream);
+  if (e == cudaSuccess) e = cudaMemsetAsync(s->d_instFlags, 0, cap * sizeof(uint32_t), ctx->stream);
+  if (e == cudaSuccess) e = cudaMemsetAsync(s->d_words, 0, kSceneWords * sizeof(uint32_t), ctx->stream);
+  if (e != cudaSuccess) { free_scene(s, ctx->stream); return rtc_set_error(__FILE__, __LINE__, "rtc_ias_create", (int)e, cudaGetErrorString(e)); }
+  s->desc.instFlags = (const uint32_t*)s->d_instFlags;
+  s->desc.tlasLeaves = (const uint32_t*)s->d_tlasLeaves;
+  s->desc.instances = (const float4*)s->d_instances;
+  s->desc.objectToWorld = (const float4*)s->d_o2w;
+  s->desc.geomInst = (const rt_GeometryInstanceData*)s->d_geomInst;
+  s->desc.numInstances = 0; s->desc.numTlasLeaves = 0; s->desc.numTlasNodes = 1;
+  // the node array, refit scratch, LBVH arrays and collapse graph for the capacity; the one empty root node of no instances
+  if (int rc = create_instance_level_gpu(ctx, *s, capacity)) { cudaStreamSynchronize(ctx->stream); free_scene(s, ctx->stream); return rc; }
+  e = cudaMemcpyAsync(s->d_desc, &s->desc, sizeof(SceneDesc), cudaMemcpyHostToDevice, ctx->stream);
+  if (e == cudaSuccess) e = cudaStreamSynchronize(ctx->stream);
+  if (e != cudaSuccess) { free_scene(s, ctx->stream); return rtc_set_error(__FILE__, __LINE__, "rtc_ias_create", (int)e, cudaGetErrorString(e)); }
+  s->totalNodes = 1;
+  s->gasEpoch = ctx->gasEpoch;
+  ctx->scenes.push_back(s);
+  *topObject = (uint64_t)(uintptr_t)s->d_desc;
+  return 0;
+}
+
+int rtc_ias_build_device(rtc_context* ctx, uint64_t topObject, uint64_t instances, uint32_t strideBytes, uint32_t numInstances)
+{
+  SceneRecord* s = find_scene(ctx, topObject);
+  if (!s) RTC_FAIL("unknown topObject");
+  if (!s->created) RTC_FAIL("rtc_ias_build_device needs a scene of rtc_ias_create (this one was built by rtc_ias_build)");
+  if (numInstances > s->capacity) RTC_FAIL("numInstances exceeds the scene's capacity");
+  if (numInstances && !instances) RTC_FAIL("instances is null");
+  if (numInstances && (instances & 3u)) RTC_FAIL("instances is not 4-byte aligned");
+  if (numInstances && (strideBytes < 64 || (strideBytes & 3u))) RTC_FAIL("strideBytes must be a multiple of 4 and at least 64");
+  RTC_CUDA(cudaSetDevice(ctx->device));
+  const double t0 = now_ms();
+  // the per-handle reference counts cover every handle of the context (pooled, grown behind the stream)
+  const uint32_t numGas = (uint32_t)ctx->gas.size();
+  if (numGas > s->gasRefsCapacity)
+  {
+    if (s->d_gasRefs) RTC_CUDA(cudaFreeAsync(s->d_gasRefs, ctx->stream));
+    s->d_gasRefs = nullptr; s->gasRefsCapacity = 0; s->gasRefsCount = 0;
+    const uint32_t cap = std::max(numGas, ctx->gasTableCapacity);
+    RTC_CUDA(cudaMallocAsync((void**)&s->d_gasRefs, (size_t)cap * sizeof(uint32_t), ctx->stream));
+    s->gasRefsCapacity = cap;
+  }
+  s->gasRefsCount = numGas;
+  if (numGas) RTC_CUDA(cudaMemsetAsync(s->d_gasRefs, 0, (size_t)numGas * sizeof(uint32_t), ctx->stream));
+  RTC_CUDA(cudaMemsetAsync(s->d_words + kRejectedWord, 0, sizeof(uint32_t), ctx->stream));
+  s->desc.numInstances = numInstances;
+  s->desc.numTlasLeaves = numInstances;
+  RTC_CUDA(cudaMemcpyAsync(s->d_desc, &s->desc, sizeof(SceneDesc), cudaMemcpyHostToDevice, ctx->stream));
+  if (int rc = write_created_records_gpu(ctx, *s, reinterpret_cast<const uint8_t*>((uintptr_t)instances), nullptr, strideBytes, 0u, 0u,
+                                         instance_bounds_tight())) return rc;
+  if (int rc = rebuild_instances_gpu(ctx, *s)) return rc;
+  count_cutout(s);
+  s->gasEpoch = ctx->gasEpoch;
+  s->gasDestroyed = false;
+  s->iasBuildMs = now_ms() - t0;
+  return 0;
+}
+
+int rtc_scene_rejected_instances(rtc_context* ctx, uint64_t topObject, uint32_t* count)
+{
+  SceneRecord* s = find_scene(ctx, topObject);
+  if (!s) RTC_FAIL("unknown topObject");
+  if (!count) RTC_FAIL("count is null");
+  if (!s->created) RTC_FAIL("not a scene of rtc_ias_create");
+  RTC_CUDA(cudaSetDevice(ctx->device));
+  RTC_CUDA(cudaMemcpyAsync(count, s->d_words + kRejectedWord, sizeof(uint32_t), cudaMemcpyDeviceToHost, ctx->stream));
+  RTC_CUDA(cudaStreamSynchronize(ctx->stream));
+  return 0;
+}
+
 int rtc_scene_info_get(rtc_context* ctx, uint64_t topObject, rtc_scene_info* info)
 {
   SceneRecord* s = find_scene(ctx, topObject);
   if (!s) RTC_FAIL("unknown topObject");
   RTC_CUDA(cudaSetDevice(ctx->device));
   if (int rc = sync_tlas_node_count(ctx, s)) return rc;
+  if (s->created) { if (int rc = sync_created_scene_totals(ctx, s)) return rc; }
   for (const std::pair<uint32_t, uint64_t>& g : s->gasGeneration) if (int rc = sync_gas_node_count(ctx, g.first)) return rc;
   std::memset(info, 0, sizeof(*info));
   info->numNodes = s->totalNodes; info->numTris = s->totalTris; info->numInstances = s->desc.numInstances;
@@ -649,13 +838,13 @@ int rtc_scene_set_instance_flags(rtc_context* ctx, uint64_t topObject, uint32_t 
 {
   SceneRecord* s = find_scene(ctx, topObject);
   if (!s) RTC_FAIL("unknown topObject");
-  if ((uint64_t)first + count > s->desc.numInstances) RTC_FAIL("instance range out of bounds");
+  // a created scene's flags belong to positions up to its capacity and persist across its builds
+  if ((uint64_t)first + count > (s->created ? s->capacity : s->desc.numInstances)) RTC_FAIL("instance range out of bounds");
   if (count == 0) return 0;
   if (!flags) RTC_FAIL("flags is null");
   RTC_CUDA(cudaSetDevice(ctx->device));
   for (uint32_t i = 0; i < count; ++i) s->instFlags[first + i] = flags[i];
-  s->numCutout = 0;
-  for (uint32_t f : s->instFlags) if (f & RTC_INSTANCE_CUTOUT) s->numCutout++;
+  count_cutout(s);
   // stream-ordered behind the launches already enqueued; `flags` may be reused by the caller at once (pageable source: staged copy)
   RTC_CUDA(cudaMemcpyAsync((uint32_t*)s->d_instFlags + first, &s->instFlags[first], (size_t)count * 4u, cudaMemcpyHostToDevice, ctx->stream));
   return 0;
@@ -713,7 +902,9 @@ int rtc_scene_export(rtc_context* ctx, uint64_t topObject, void* tlasNodes, uint
   // world->object rows 0..2 of each 64-byte instance record, where the updates computed them
   if (worldToObject && s->desc.numInstances)
     RTC_CUDA(cudaMemcpy2D(worldToObject, 48, s->d_instances, 64, 48, s->desc.numInstances, cudaMemcpyDeviceToHost));
-  if (instanceGas) std::memcpy(instanceGas, s->instGas.data(), s->instGas.size() * sizeof(uint32_t));
+  if (instanceGas && s->created && s->desc.numInstances)
+    RTC_CUDA(cudaMemcpy(instanceGas, s->d_instGasSlot, (size_t)s->desc.numInstances * sizeof(uint32_t), cudaMemcpyDeviceToHost));
+  else if (instanceGas) std::memcpy(instanceGas, s->instGas.data(), s->instGas.size() * sizeof(uint32_t));
   return 0;
 }
 

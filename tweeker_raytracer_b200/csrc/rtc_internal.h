@@ -127,7 +127,21 @@ struct SceneRecord
   // rtc_ias_build, rtc_ias_update and rtc_ias_update_device write them there, rtc_scene_export and rtc_instance_inverse read them back.
   std::vector<uint32_t> instGas;           // GAS handle per instance
   std::vector<std::pair<uint32_t, uint64_t>> gasGeneration;   // each distinct GAS and its generation at the last build / update
-  uint32_t* d_instGasSlot = nullptr;       // per instance: the position of its GAS in gasGeneration (the instance records' per-GAS table)
+  // per instance: the position of its GAS in gasGeneration (the instance records' per-GAS table); in a created scene its GAS handle
+  // (an index of the context's GAS table), or kRejectedInstance
+  uint32_t* d_instGasSlot = nullptr;
+  // rtc_ias_create / rtc_ias_build_device: the instance set lives on the device, in arrays sized for `capacity`.  instGas and
+  // gasGeneration stay empty; the device holds what they hold for a built scene.
+  bool     created = false;
+  uint32_t capacity = 0;
+  uint64_t* d_instGen = nullptr;           // per instance: its GAS's generation when its record was written
+  uint32_t* d_words = nullptr;             // [kRejectedWord] records the last build rejected, [kCandidateWord] records written by a call
+  uint32_t* d_gasRefs = nullptr;           // per GAS handle: instances of the last build that reference it (pooled)
+  uint32_t  gasRefsCount = 0;              // handles d_gasRefs covers (the context's GAS count at the last build)
+  uint32_t  gasRefsCapacity = 0;
+  void*     d_emptyGas = nullptr;          // an empty GAS root node (and room for its triangles): the geometry of a rejected record
+  uint64_t  gasEpoch = 0;                  // rtc_context::gasEpoch at the last build / update: a created scene is stale when it differs
+  bool      gasDestroyed = false;          // rtc_gas_destroy of a handle the last build references
   PrimBox* d_instBoxes = nullptr;          // the padded world box of every instance (leaf boxes of the instance level)
   RefitScratch refit;
   // rtc_ias_rebuild (bvh_build_ias_gpu.cu): its arrays, made by the first rebuild, and from then on the instance level's node count
@@ -216,6 +230,12 @@ struct rtc_context
   ScheduleTuner tuner;                            // picks traceSchedule by timing one batch with each (kernels_shade.cu, "schedule tuner")
   void*  cutoutGraph = nullptr;                   // CutoutGraph (kernels_shade.cu): the device-side loop of the ordered any-hit rounds
   uint64_t cutoutGraphBuilds = 0;                 // graph pairs captured since the last rtc_stats_reset (rtc_stats)
+  // The device GAS table, indexed by handle: the instance records of created scenes read it.  Kept up to date on the stream by
+  // rtc_gas_build, rtc_gas_refit, rtc_gas_rebuild and rtc_gas_destroy (a destroyed GAS has null nodes); grown from the pool.
+  struct GasUpdateInput* d_gasTable = nullptr;
+  uint64_t* d_gasGen = nullptr;                   // per handle: GasRecord::generation
+  uint32_t gasTableCapacity = 0;
+  uint64_t gasEpoch = 0;                          // refits and rebuilds of any GAS of the context
 };
 
 // work counters of one traversal kernel: {nodes, tris, insts, rays}
@@ -245,7 +265,11 @@ struct GasUpdateInput
   float    gasLoHi[6];
   uint64_t attributes;             // rt_GeometryInstanceData::attributes
   uint32_t emptyGas, pad;
+  uint64_t indices;                // rt_GeometryInstanceData::indices (written by the builds of created scenes)
 };
+// d_instGasSlot of a created scene for a record rtc_ias_build_device rejected
+constexpr uint32_t kRejectedInstance = 0xffffffffu;
+enum { kRejectedWord = 0, kCandidateWord = 1, kSceneWords = 2 };
 // The records of the candidate instances (rtc_ias_build: every instance; rtc_ias_update, rtc_ias_update_device: the recomputed
 // ones): candidate j is instance candidates[j], or first + j when `candidates` is empty.  Instance i in [first, first + count)
 // takes the object->world matrix at transforms + (i - first) * strideBytes (device-readable memory, read when the stream gets
@@ -254,6 +278,13 @@ struct GasUpdateInput
 // stream-ordered pool.
 int write_instance_records_gpu(rtc_context* ctx, SceneRecord& s, const uint8_t* transforms, uint32_t strideBytes, uint32_t first,
                                uint32_t count, const std::vector<uint32_t>& candidates, const std::vector<GasUpdateInput>& gas, bool tight);
+// The same kernels for a created scene, over the context's GAS table, with the candidates selected on the device.  records
+// non-null (rtc_ias_build_device): every instance i < s.desc.numInstances takes the rtc_instance_desc at records + i * strideBytes,
+// which is validated; its GAS handle, generation, shading-table row and the per-handle reference counts are written, rejected
+// records counted.  records null (the updates): the instances of [first, first + count) take the matrices at transforms, and every
+// instance whose GAS's generation changed is recomputed with its current one.
+int write_created_records_gpu(rtc_context* ctx, SceneRecord& s, const uint8_t* records, const uint8_t* transforms, uint32_t strideBytes,
+                              uint32_t first, uint32_t count, bool tight);
 // The updates' refit of the instance level's nodes over s.d_instBoxes; a scene's first refit allocates its scratch from the
 // stream-ordered pool.
 int refit_instance_level_gpu(rtc_context* ctx, SceneRecord& s);
@@ -263,6 +294,8 @@ void free_refit_scratch(RefitScratch& r, cudaStream_t stream);
 // bvh_build_ias_gpu.cu: a new LBVH topology of the instance level over s.d_instBoxes, in place and stream-ordered; the first call
 // on a scene allocates (and synchronises once), later calls never block the host
 int rebuild_instances_gpu(rtc_context* ctx, SceneRecord& s);
+// rtc_ias_create: the rebuild's arrays for `capacity` instances, set up at once (synchronises); the scene starts with no instance
+int create_instance_level_gpu(rtc_context* ctx, SceneRecord& s, uint32_t capacity);
 // bvh_build_gas_rebuild_gpu.cu: the same for a geometry, over the triangles of rec.attributes / rec.indices; writes the triangle
 // records in leaf order and the root box into rec.refit.box[0..5]
 int rebuild_gas_gpu(rtc_context* ctx, GasRecord& rec);
