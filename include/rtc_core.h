@@ -121,7 +121,10 @@ int rtc_host_alloc(rtc_context* ctx, uint64_t bytes, void** ptr);               
 int rtc_host_free(rtc_context* ctx, void* ptr);
 
 /* attributes: device pointer to vertex records, position = 3 floats at offset 0, strideBytes apart
- * (48 for TriangleAttributes); indices: device pointer to numTris uint32 triplets. */
+ * (48 for TriangleAttributes); indices: device pointer to numTris uint32 triplets.
+ * Inactive inputs (every build, refit, rebuild and update below; DESIGN.md section 3): a triangle with a vertex coordinate that
+ * is NaN, +-inf or beyond B = 2^126 in magnitude, and an instance whose transform has such an entry or whose transformed vertices
+ * reach beyond B, are never hit and bound nothing; every other triangle and instance gives exactly the brute-force hits. */
 int rtc_gas_build(rtc_context* ctx, uint64_t attributes, uint32_t strideBytes, uint32_t numVerts,
                   uint64_t indices, uint32_t numTris, uint32_t buildFlags, uint32_t* gas);
 /* Builds the instance level, the per-instance tables and returns SystemData::topObject. */

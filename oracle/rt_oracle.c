@@ -11,6 +11,7 @@
 #include "rt_oracle.h"
 #include "rt_portable_math.h"
 
+#include <float.h>
 #include <math.h>
 #include <pthread.h>
 #include <stdlib.h>
@@ -124,6 +125,7 @@ typedef struct {
   int   material;
   int   light;
   aabb  world;
+  int   active;    /* 0: inactive (tri_active's comment): no ray hits the instance */
 } instance;
 
 struct orc_scene {
@@ -342,6 +344,22 @@ static void build_rec(build_ctx* c, uint32_t nodeIdx, uint32_t first, uint32_t c
   build_rec(c, left + 1, mid, first + count - mid);
 }
 
+/* Inactive inputs (DESIGN.md section 3), with the bound B = 2^126 of the product's quantised boxes: a triangle with a vertex
+ * coordinate that is NaN, infinite or beyond B is never hit and bounds nothing (the oracle's BVH gives it an empty box and both
+ * traversal modes skip it); so is an instance whose transform has an entry that is not finite, or whose geometry's in-range
+ * vertices, transformed, reach beyond B. */
+static int in_range(float x) { return fabsf(x) <= 0x1p126f; }
+
+static int tri_active(const geometry* g, uint32_t t)
+{
+  for (int c = 0; c < 3; ++c)
+  {
+    const rt_float3 v = g->attrs[g->indices[3 * t + c]].vertex;
+    if (!in_range(v.x) || !in_range(v.y) || !in_range(v.z)) return 0;
+  }
+  return 1;
+}
+
 static void bvh_build(bvh* t, const aabb* primBoxes, uint32_t n)
 {
   bvh_free(t);
@@ -367,6 +385,7 @@ void orc_scene_commit(orc_scene* s)
     for (uint32_t t = 0; t < g->numTris; ++t)
     {
       box_empty(&pb[t]);
+      if (!tri_active(g, t)) { for (int a = 0; a < 3; ++a) { pb[t].lo[a] = FLT_MAX; pb[t].hi[a] = -FLT_MAX; } continue; }
       for (int k = 0; k < 3; ++k)
       {
         const rt_float3 v = g->attrs[g->indices[3 * t + k]].vertex;
@@ -400,7 +419,28 @@ void orc_scene_commit(orc_scene* s)
         if (hi > in->world.hi[r]) in->world.hi[r] = hi;
       }
     }
-    if (s->geoms[in->geometry].numTris == 0) { for (int k = 0; k < 3; ++k) { in->world.lo[k] = 0.0f; in->world.hi[k] = 0.0f; } }
+    if (s->geoms[in->geometry].numTris == 0 || !(gb->lo[0] <= gb->hi[0]))
+      for (int k = 0; k < 3; ++k) { in->world.lo[k] = 0.0f; in->world.hi[k] = 0.0f; }
+    in->active = 1;
+    for (int k = 0; k < 12; ++k) in->active &= in_range(in->m[k]);
+    if (in->active && s->geoms[in->geometry].numTris && gb->lo[0] <= gb->hi[0])
+    {
+      /* the exact world bounds of the geometry's in-range vertices (one fmaf chain per row) must lie within B */
+      const geometry* g = &s->geoms[in->geometry];
+      for (uint32_t v = 0; v < g->numVerts; ++v)
+      {
+        const float p[3] = { g->attrs[v].vertex.x, g->attrs[v].vertex.y, g->attrs[v].vertex.z };
+        if (!in_range(p[0]) || !in_range(p[1]) || !in_range(p[2])) continue;
+        for (int r = 0; r < 3; ++r)
+          in->active &= in_range(fmaf(in->m[4 * r], p[0], fmaf(in->m[4 * r + 1], p[1], fmaf(in->m[4 * r + 2], p[2], in->m[4 * r + 3]))));
+      }
+    }
+    if (!in->active) for (int k = 0; k < 3; ++k) { in->world.lo[k] = 0.0f; in->world.hi[k] = 0.0f; }
+    else for (int k = 0; k < 3; ++k)            /* overflowing pads of the oracle's own (looser) box: keep its BVH finite */
+    {
+      if (!isfinite(in->world.lo[k])) in->world.lo[k] = -FLT_MAX;
+      if (!isfinite(in->world.hi[k])) in->world.hi[k] = FLT_MAX;
+    }
     ib[ii] = in->world;
   }
   bvh_build(&s->top, ib, (uint32_t)s->numInsts);
@@ -541,7 +581,7 @@ static int trace_instance(const orc_scene* s, uint32_t ii, const float o[3], con
 {
   const instance* in = &s->insts[ii];
   const geometry* g = &s->geoms[in->geometry];
-  if (g->numTris == 0) return 0;
+  if (g->numTris == 0 || !in->active) return 0;
   oray r; to_object(in->inv, o, d, &r);
   if (st) st->instancesEntered++;
   const float *v0, *v1, *v2; float t, u, v;
@@ -549,6 +589,7 @@ static int trace_instance(const orc_scene* s, uint32_t ii, const float o[3], con
   {
     for (uint32_t p = 0; p < g->numTris; ++p)
     {
+      if (!tri_active(g, p)) continue;
       tri_verts(g, p, &v0, &v1, &v2);
       if (st) st->trisTested++;
       if (tri_test(&r, v0, v1, v2, &t, &u, &v))
@@ -571,6 +612,7 @@ static int trace_instance(const orc_scene* s, uint32_t ii, const float o[3], con
       for (uint32_t i = n->left; i < n->left + n->count; ++i)
       {
         const uint32_t p = g->tree.prims[i];
+        if (!tri_active(g, p)) continue;
         tri_verts(g, p, &v0, &v1, &v2);
         if (st) st->trisTested++;
         if (tri_test(&r, v0, v1, v2, &t, &u, &v))

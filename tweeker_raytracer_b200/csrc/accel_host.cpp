@@ -26,13 +26,16 @@ bool gas_assemble_host(const uint8_t* verts, uint32_t strideBytes, uint32_t numV
   {
     PrimBox& b = boxes[t];
     for (int k = 0; k < 3; ++k) { b.lo[k] = std::numeric_limits<float>::infinity(); b.hi[k] = -b.lo[k]; }
+    bool active = true;
     for (int c = 0; c < 3; ++c)
     {
       const uint32_t vi = idx[3u * t + c];
       if (vi >= numVerts) return false;
       const float* p = vertex(vi);
+      active = active && rules_in_range3(p);
       for (int k = 0; k < 3; ++k) { b.lo[k] = std::fmin(b.lo[k], p[k]); b.hi[k] = std::fmax(b.hi[k], p[k]); }
     }
+    if (!active) rules_empty_box(b.lo, b.hi);
   }
   // triangles per leaf child of the host SAH build.  2: geometry scene 2526 -> 2545 Msamples/s, Cornell box 809 -> 820 against
   // leaves of up to 3; 1 is better only for the instanced scene (355 -> 368) and loses 2 % elsewhere.  RTC_HOST_LEAF_MAX overrides.
@@ -43,13 +46,7 @@ bool gas_assemble_host(const uint8_t* verts, uint32_t strideBytes, uint32_t numV
   for (uint32_t s = 0; s < numTris; ++s)
   {
     const uint32_t prim = bvh.primOrder[s];
-    for (int c = 0; c < 3; ++c)
-    {
-      const float* p = vertex(idx[3u * prim + c]);
-      float w = 0.0f;
-      if (c == 0) std::memcpy(&w, &prim, 4);
-      tris[3u * (size_t)s + c] = make_float4(p[0], p[1], p[2], w);
-    }
+    rules_tri_record(vertex(idx[3u * prim]), vertex(idx[3u * prim + 1]), vertex(idx[3u * prim + 2]), prim, &tris[3u * (size_t)s]);
   }
   return true;
 }
@@ -63,6 +60,7 @@ void instance_bounds_host(const float transform[12], const uint8_t* verts, uint3
   for (uint32_t v = 0; v < numVerts; ++v)
   {
     const float* p = reinterpret_cast<const float*>(verts + (size_t)v * strideBytes);
+    if (!rules_in_range3(p)) continue;         // only inactive triangles use it
     for (int r = 0; r < 3; ++r)
     {
       const float* m = transform + 4 * r;
@@ -183,24 +181,21 @@ int rtc_host_gas_refit(rtc_host_accel* accel, const void* attributes, uint32_t s
   for (uint32_t s = 0; s < accel->numTris; ++s)
   {
     const uint32_t prim = accel->bvh.primOrder[s];
-    for (int c = 0; c < 3; ++c)
-    {
-      const float* p = reinterpret_cast<const float*>(verts + (size_t)accel->indices[3u * prim + c] * strideBytes);
-      float4& r = accel->tris[3u * (size_t)s + c];
-      r.x = p[0]; r.y = p[1]; r.z = p[2];
-    }
+    auto vertex = [&](int c) { return reinterpret_cast<const float*>(verts + (size_t)accel->indices[3u * prim + c] * strideBytes); };
+    rules_tri_record(vertex(0), vertex(1), vertex(2), prim, &accel->tris[3u * (size_t)s]);
   }
   if (accel->numTris == 0) return 0;
   const std::vector<float4>& tris = accel->tris;
   refit_host(accel->bvh, [&](uint32_t first, uint32_t count, float lo[3], float hi[3]) {
     for (int k = 0; k < 3; ++k) { lo[k] = INFINITY; hi[k] = -INFINITY; }
     for (uint32_t t = first; t < first + count; ++t)
+    {
+      float x[3][3];
+      for (int c = 0; c < 3; ++c) { const float4& v = tris[3u * (size_t)t + c]; x[c][0] = v.x; x[c][1] = v.y; x[c][2] = v.z; }
+      if (!rules_in_range3(x[0]) || !rules_in_range3(x[1]) || !rules_in_range3(x[2])) continue;     // inactive triangle
       for (int c = 0; c < 3; ++c)
-      {
-        const float4& v = tris[3u * (size_t)t + c];
-        const float x[3] = { v.x, v.y, v.z };
-        for (int k = 0; k < 3; ++k) { lo[k] = x[k] < lo[k] ? x[k] : lo[k]; hi[k] = hi[k] < x[k] ? x[k] : hi[k]; }
-      }
+        for (int k = 0; k < 3; ++k) { lo[k] = x[c][k] < lo[k] ? x[c][k] : lo[k]; hi[k] = hi[k] < x[c][k] ? x[c][k] : hi[k]; }
+    }
   });
   return 0;
 }
@@ -241,6 +236,7 @@ static void lbvh_rebuild_host(const std::vector<PrimBox>& boxes, WideBvh& out)
     const PrimBox& b = boxes[i];
     lo[i] = make_float4(b.lo[0], b.lo[1], b.lo[2], 0.0f);
     hi[i] = make_float4(b.hi[0], b.hi[1], b.hi[2], 0.0f);
+    if (rules_box_empty(b.lo, b.hi)) continue;          // an inactive primitive's centre stays out of the frame
     for (int k = 0; k < 3; ++k)
     {
       const float c = 0.5f * (b.lo[k] + b.hi[k]);
@@ -332,23 +328,20 @@ int rtc_host_gas_rebuild(rtc_host_accel* accel, const void* attributes, uint32_t
   {
     PrimBox& b = boxes[t];
     for (int k = 0; k < 3; ++k) { b.lo[k] = FLT_MAX; b.hi[k] = -FLT_MAX; }
+    bool active = true;
     for (int c = 0; c < 3; ++c)
     {
       const float* p = vertex(t, c);
+      active = active && rules_in_range3(p);
       for (int k = 0; k < 3; ++k) { b.lo[k] = std::fmin(b.lo[k], p[k]); b.hi[k] = std::fmax(b.hi[k], p[k]); }
     }
+    if (!active) rules_empty_box(b.lo, b.hi);
   }
   lbvh_rebuild_host(boxes, accel->bvh);
   for (uint32_t s = 0; s < n; ++s)
   {
     const uint32_t prim = accel->bvh.primOrder[s];
-    for (int c = 0; c < 3; ++c)
-    {
-      const float* p = vertex(prim, c);
-      float w = 0.0f;
-      if (c == 0) std::memcpy(&w, &prim, 4);
-      accel->tris[3u * (size_t)s + c] = make_float4(p[0], p[1], p[2], w);
-    }
+    rules_tri_record(vertex(prim, 0), vertex(prim, 1), vertex(prim, 2), prim, &accel->tris[3u * (size_t)s]);
   }
   return 0;
 }

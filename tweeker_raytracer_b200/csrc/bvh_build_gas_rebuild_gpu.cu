@@ -42,16 +42,20 @@ k_gas_boxes(const uint8_t* __restrict__ verts, const TriangleLeaves L, uint32_t 
   if (t < n)
   {
     float bLo[3] = { FLT_MAX, FLT_MAX, FLT_MAX }, bHi[3] = { -FLT_MAX, -FLT_MAX, -FLT_MAX };
+    bool active = true;
     for (int c = 0; c < 3; ++c)
     {
       const uint32_t vi = __ldg(L.idx + 3u * (size_t)t + c);
       if (vi >= L.numVerts) continue;                   // indices are the build's, which checked them
       const float* p = reinterpret_cast<const float*>(verts + (size_t)vi * L.stride);
-      for (int k = 0; k < 3; ++k) { const float v = __ldg(p + k); bLo[k] = fminf(bLo[k], v); bHi[k] = fmaxf(bHi[k], v); }
+      const float x[3] = { __ldg(p), __ldg(p + 1), __ldg(p + 2) };
+      active = active && rules_in_range3(x);
+      for (int k = 0; k < 3; ++k) { bLo[k] = fminf(bLo[k], x[k]); bHi[k] = fmaxf(bHi[k], x[k]); }
     }
+    if (!active) rules_empty_box(bLo, bHi);
     lo[t] = make_float4(bLo[0], bLo[1], bLo[2], 0.0f);
     hi[t] = make_float4(bHi[0], bHi[1], bHi[2], 0.0f);
-    for (int k = 0; k < 3; ++k) { cLo[k] = 0.5f * (bLo[k] + bHi[k]); cHi[k] = cLo[k]; }
+    if (active) for (int k = 0; k < 3; ++k) { cLo[k] = 0.5f * (bLo[k] + bHi[k]); cHi[k] = cLo[k]; }
   }
   lbvh_reduce_centre_box(cLo, cHi, centreBox);
 }
@@ -90,14 +94,18 @@ k_gas_emit(const CollapseArgs A, const TriangleLeaves L, const int2* __restrict_
   collapse_emit(A, A.n, work, workCount, nextWork, [&](uint32_t slot, uint32_t p) {
     const uint8_t* verts = rebuild_verts(A);
     const uint32_t prim = A.order[p];
-    float4* out = L.tris + 3u * (size_t)slot;
+    float x[3][3];
     for (int c = 0; c < 3; ++c)
     {
       const uint32_t vi = __ldg(L.idx + 3u * (size_t)prim + c);
-      if (vi >= L.numVerts) continue;
+      if (vi >= L.numVerts) return;                     // indices are the build's, which checked them
       const float* v = reinterpret_cast<const float*>(verts + (size_t)vi * L.stride);
-      out[c] = make_float4(__ldg(v), __ldg(v + 1), __ldg(v + 2), c == 0 ? __uint_as_float(prim) : 0.0f);
+      x[c][0] = __ldg(v); x[c][1] = __ldg(v + 1); x[c][2] = __ldg(v + 2);
     }
+    float4 rec[3];
+    rules_tri_record(x[0], x[1], x[2], prim, rec);
+    float4* out = L.tris + 3u * (size_t)slot;
+    for (int c = 0; c < 3; ++c) out[c] = rec[c];
   });
 }
 

@@ -51,13 +51,17 @@ k_tri_bounds(const uint8_t* __restrict__ verts, uint32_t stride, const uint32_t*
   float lo[3] = { FLT_MAX, FLT_MAX, FLT_MAX }, hi[3] = { -FLT_MAX, -FLT_MAX, -FLT_MAX };
   if (t < n)
   {
+    bool active = true;
     for (int c = 0; c < 3; ++c)
     {
       const uint32_t vi = __ldg(idx + 3u * (size_t)t + c);
       if (vi >= numVerts) { atomicExch(badIndex, 1u); continue; }
       const float* p = reinterpret_cast<const float*>(verts + (size_t)vi * stride);
-      for (int k = 0; k < 3; ++k) { const float v = __ldg(p + k); lo[k] = fminf(lo[k], v); hi[k] = fmaxf(hi[k], v); }
+      const float x[3] = { __ldg(p), __ldg(p + 1), __ldg(p + 2) };
+      active = active && rules_in_range3(x);
+      for (int k = 0; k < 3; ++k) { lo[k] = fminf(lo[k], x[k]); hi[k] = fmaxf(hi[k], x[k]); }
     }
+    if (!active) rules_empty_box(lo, hi);               // inactive triangle: empty box, outside the scene box
     triLo[t] = make_float4(lo[0], lo[1], lo[2], 0.0f);
     triHi[t] = make_float4(hi[0], hi[1], hi[2], 0.0f);
   }
@@ -220,12 +224,16 @@ k_collapse_level(const CollapseParams P, const int2* __restrict__ work, uint32_t
       {
         const uint32_t prim = P.order[first + i];
         float4* out = P.tris + (size_t)(node.triBase + triOffset + (uint32_t)i) * 3u;
+        float x[3][3];
         for (int c = 0; c < 3; ++c)
         {
           const uint32_t vi = __ldg(P.idx + 3u * (size_t)prim + c);
           const float* v = reinterpret_cast<const float*>(P.verts + (size_t)vi * P.stride);
-          out[c] = make_float4(__ldg(v), __ldg(v + 1), __ldg(v + 2), c == 0 ? __uint_as_float(prim) : 0.0f);
+          x[c][0] = __ldg(v); x[c][1] = __ldg(v + 1); x[c][2] = __ldg(v + 2);
         }
+        float4 rec[3];
+        rules_tri_record(x[0], x[1], x[2], prim, rec);
+        for (int c = 0; c < 3; ++c) out[c] = rec[c];
       }
       triOffset += (uint32_t)cnt;
     }

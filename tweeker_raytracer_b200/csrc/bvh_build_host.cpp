@@ -23,6 +23,7 @@ struct Box
   void grow(const float* l, const float* h) { for (int k = 0; k < 3; ++k) { lo[k] = std::min(lo[k], l[k]); hi[k] = std::max(hi[k], h[k]); } }
   float halfArea() const
   {
+    if (rules_box_empty(lo, hi)) return 0.0f;       // only inactive primitives (bvh_rules.h): nothing to intersect
     const float dx = hi[0] - lo[0], dy = hi[1] - lo[1], dz = hi[2] - lo[2];
     return dx * dy + dy * dz + dz * dx;
   }
@@ -37,6 +38,14 @@ struct BinNode
 
 constexpr int kBins = 32;
 constexpr uint32_t kLeafMax = 3;    // a leaf child of a wide node carries 1..3 primitives (3 bits of meta)
+
+// SAH bin of a centre; clamped in float before the conversion, because centres of boxes near the float limit overflow to
+// infinity and the conversion of a NaN or an out-of-range value is undefined
+inline int bin_of(float centre, float lo, float scale)
+{
+  const float f = (centre - lo) * scale;
+  return f >= (float)(kBins - 1) ? kBins - 1 : (f > 0.0f ? (int)f : 0);
+}
 
 struct Builder
 {
@@ -73,8 +82,7 @@ struct Builder
       for (uint32_t i = first; i < first + count; ++i)
       {
         const PrimBox& p = prims[order[i]];
-        int b = (int)((0.5f * (p.lo[axis] + p.hi[axis]) - cbox.lo[axis]) * scale);
-        b = std::min(std::max(b, 0), kBins - 1);
+        const int b = bin_of(0.5f * (p.lo[axis] + p.hi[axis]), cbox.lo[axis], scale);
         bb[b].grow(p.lo, p.hi); bc[b]++;
       }
       float rightArea[kBins]; uint32_t rightCount[kBins]; Box acc; acc.clear(); uint32_t n = 0;
@@ -107,9 +115,7 @@ struct Builder
       const float clo = cbox.lo[bestAxis];
       auto it = std::partition(order.begin() + first, order.begin() + first + count, [&](uint32_t pi) {
         const PrimBox& p = prims[pi];
-        int b = (int)((0.5f * (p.lo[bestAxis] + p.hi[bestAxis]) - clo) * scale);
-        b = std::min(std::max(b, 0), kBins - 1);
-        return b <= bestSplit;
+        return bin_of(0.5f * (p.lo[bestAxis] + p.hi[bestAxis]), clo, scale) <= bestSplit;
       });
       mid = (uint32_t)(it - order.begin());
       if (mid == first || mid == first + count) mid = first + count / 2;
@@ -245,7 +251,7 @@ struct Emitter
     {
       int bi = -1, bs = -1; float bc = -std::numeric_limits<float>::infinity();
       for (int i = 0; i < n; ++i) if (!kidDone[i])
-        for (int s = 0; s < 8; ++s) if (!slotUsed[s] && cost[i][s] > bc) { bc = cost[i][s]; bi = i; bs = s; }
+        for (int s = 0; s < 8; ++s) if (!slotUsed[s] && (cost[i][s] > bc || bi < 0)) { bc = cost[i][s]; bi = i; bs = s; }
       slotOf[bi] = bs; slotUsed[bs] = true; kidDone[bi] = true;
     }
     int kidAt[8]; for (int s = 0; s < 8; ++s) kidAt[s] = -1;

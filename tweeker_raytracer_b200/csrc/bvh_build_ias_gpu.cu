@@ -31,7 +31,8 @@ k_ias_boxes(const PrimBox* __restrict__ boxes, uint32_t n, float4* __restrict__ 
     const PrimBox b = boxes[t];
     lo[t] = make_float4(b.lo[0], b.lo[1], b.lo[2], 0.0f);
     hi[t] = make_float4(b.hi[0], b.hi[1], b.hi[2], 0.0f);
-    for (int k = 0; k < 3; ++k) { cLo[k] = 0.5f * (b.lo[k] + b.hi[k]); cHi[k] = cLo[k]; }
+    if (!rules_box_empty(b.lo, b.hi))                  // an inactive instance's centre stays out of the frame
+      for (int k = 0; k < 3; ++k) { cLo[k] = 0.5f * (b.lo[k] + b.hi[k]); cHi[k] = cLo[k]; }
   }
   lbvh_reduce_centre_box(cLo, cHi, centreBox);
 }

@@ -52,13 +52,17 @@ k_refit_tris(float4* __restrict__ tris, uint32_t numTris, const uint8_t* __restr
   if (t >= numTris) return;
   float4* rec = tris + 3u * (size_t)t;
   const uint32_t prim = __float_as_uint(rec[0].w);
+  float x[3][3];
   for (int c = 0; c < 3; ++c)
   {
     const uint32_t vi = __ldg(idx + 3u * (size_t)prim + c);
-    if (vi >= numVerts) continue;                       // indices are the build's, which checked them
+    if (vi >= numVerts) return;                         // indices are the build's, which checked them
     const float* p = reinterpret_cast<const float*>(verts + (size_t)vi * stride);
-    rec[c] = make_float4(__ldg(p), __ldg(p + 1), __ldg(p + 2), c == 0 ? __uint_as_float(prim) : 0.0f);
+    x[c][0] = __ldg(p); x[c][1] = __ldg(p + 1); x[c][2] = __ldg(p + 2);
   }
+  float4 r[3];
+  rules_tri_record(x[0], x[1], x[2], prim, r);
+  for (int c = 0; c < 3; ++c) rec[c] = r[c];
 }
 
 struct RefitParams
@@ -79,12 +83,15 @@ __device__ void refit_one(const RefitParams& P, uint32_t idx)
     {
       if (P.tris)
       {
+        float x[3][3];
         for (int c = 0; c < 3; ++c)
         {
           const float4 v = P.tris[3u * (size_t)t + c];
-          const float x[3] = { v.x, v.y, v.z };
-          for (int k = 0; k < 3; ++k) { lo[k] = x[k] < lo[k] ? x[k] : lo[k]; hi[k] = hi[k] < x[k] ? x[k] : hi[k]; }
+          x[c][0] = v.x; x[c][1] = v.y; x[c][2] = v.z;
         }
+        if (!rules_in_range3(x[0]) || !rules_in_range3(x[1]) || !rules_in_range3(x[2])) continue;     // inactive triangle
+        for (int c = 0; c < 3; ++c)
+          for (int k = 0; k < 3; ++k) { lo[k] = x[c][k] < lo[k] ? x[c][k] : lo[k]; hi[k] = hi[k] < x[c][k] ? x[c][k] : hi[k]; }
       }
       else
       {
@@ -169,6 +176,7 @@ k_instance_bounds(const InstanceUpdate* __restrict__ up, PrimBox* __restrict__ o
   {
     const float* p = reinterpret_cast<const float*>(g.verts + (size_t)v * g.stride);
     const float x = p[0], y = p[1], z = p[2];
+    if (!rules_in_range(x) || !rules_in_range(y) || !rules_in_range(z)) continue;      // only inactive triangles use it
 #pragma unroll
     for (int r = 0; r < 3; ++r)
     {

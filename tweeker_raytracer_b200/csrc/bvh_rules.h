@@ -30,6 +30,40 @@ RTC_HD float rules_pow2f(int e)
   return f;
 }
 
+// Inactive inputs (DESIGN.md section 3).  B = 2^126: coordinates of magnitude up to B keep every node extent within the
+// 254 grid steps of 2^120 that quantise_node can represent, so finite inputs up to B are exact.  A triangle with a vertex
+// coordinate that is NaN, infinite or beyond B, and an instance whose transform has a non-finite entry or whose world bounds
+// reach beyond B, is inactive: its box is the empty box lo = FLT_MAX, hi = -FLT_MAX (centre 0, so the builders' binning and
+// Morton codes stay finite; unions skip it and quantise_node gives it an empty slot), and an inactive triangle's leaf record
+// holds NaN for v0 (rules_tri_record), so the triangle test never reports it when it shares a leaf with active ones.
+#define RTC_COORD_BOUND 0x1p126f
+
+RTC_HD bool rules_in_range(float x) { return fabsf(x) <= RTC_COORD_BOUND; }      // false for NaN, +-inf and beyond B
+
+RTC_HD bool rules_in_range3(const float* p) { return rules_in_range(p[0]) && rules_in_range(p[1]) && rules_in_range(p[2]); }
+
+RTC_HD void rules_empty_box(float lo[3], float hi[3])
+{
+  for (int k = 0; k < 3; ++k) { lo[k] = 3.402823466e38f; hi[k] = -3.402823466e38f; }
+}
+
+// The leaf record of a triangle (v0.xyz | primitive id bits, v1.xyz | 0, v2.xyz | 0).  An inactive triangle's v0 is NaN: that
+// makes two edge functions, the determinant and t NaN in the triangle test, so it is never reported.
+RTC_HD void rules_tri_record(const float* v0, const float* v1, const float* v2, uint32_t prim, float4 rec[3])
+{
+  const bool active = rules_in_range3(v0) && rules_in_range3(v1) && rules_in_range3(v2);
+  float w;
+  memcpy(&w, &prim, 4);
+  rec[0] = active ? make_float4(v0[0], v0[1], v0[2], w) : make_float4(__builtin_nanf(""), __builtin_nanf(""), __builtin_nanf(""), w);
+  rec[1] = make_float4(v1[0], v1[1], v1[2], 0.0f);
+  rec[2] = make_float4(v2[0], v2[1], v2[2], 0.0f);
+}
+
+RTC_HD bool rules_box_empty(const float lo[3], const float hi[3])
+{
+  return !(lo[0] <= hi[0] && lo[1] <= hi[1] && lo[2] <= hi[2]);
+}
+
 // World->object matrix of an instance.  DEFINED here (OptiX computed it inside optixAccelBuild,
 // Device.cpp:1478, read back by closesthit.cu:49-52): adjugate / determinant of the upper 3x3 in double,
 // rounded once to float; translation -(Minv * t) in double.  The oracle states the same definition.
@@ -55,19 +89,33 @@ RTC_HD void invert_3x4(const float m[12], float out[12])
 
 // Quantisation frame and conservative planes of one wide node.  child(s, lo, hi) yields the float box of the child in slot s for
 // every slot set in `occupied`; the frame is derived from the union of those boxes, which is returned in nodeLo / nodeHi.
-// Writes p, e, qlo, qhi; empty slots get qlo = 255, qhi = 0.  imask, childBase, triBase and meta are left alone.
+// Writes p, e, qlo, qhi; empty slots and slots whose box is empty (rules_box_empty) get qlo = 255, qhi = 0 and stay out of the
+// node box.  When every box is empty the node box is empty (lo = INFINITY, hi = -INFINITY) and the frame is p = 0, e = 0.
+// imask, childBase, triBase and meta are left alone.
 // Per axis: grid step 2^e with (hi - p) <= 254 steps, origin p a sixteenth of a step below the box, so every child plane keeps
 // slack on the grid (see DESIGN.md "conservative boxes").
 template <class ChildBox>
 RTC_HD void quantise_node(uint32_t occupied, const ChildBox& child, Node8& node, float nodeLo[3], float nodeHi[3])
 {
   for (int k = 0; k < 3; ++k) { nodeLo[k] = INFINITY; nodeHi[k] = -INFINITY; }
+  uint32_t live = 0;
   for (int s = 0; s < 8; ++s)
   {
     if (!(occupied & (1u << s))) continue;
     float lo[3], hi[3];
     child(s, lo, hi);
+    if (rules_box_empty(lo, hi)) continue;
+    live |= 1u << s;
     for (int k = 0; k < 3; ++k) { nodeLo[k] = lo[k] < nodeLo[k] ? lo[k] : nodeLo[k]; nodeHi[k] = nodeHi[k] < hi[k] ? hi[k] : nodeHi[k]; }
+  }
+  occupied = live;
+  if (!occupied)
+  {
+    node.px = node.py = node.pz = 0.0f;
+    node.ex = node.ey = node.ez = 127;
+    uint8_t* q[6] = { node.qlox, node.qloy, node.qloz, node.qhix, node.qhiy, node.qhiz };
+    for (int k = 0; k < 6; ++k) for (int s = 0; s < 8; ++s) q[k][s] = k < 3 ? 255 : 0;
+    return;
   }
   float maxExt = 0.0f;
   for (int k = 0; k < 3; ++k) { const float d = nodeHi[k] - nodeLo[k]; maxExt = maxExt < d ? d : maxExt; }
@@ -131,17 +179,26 @@ RTC_HD void refit_node(Node8& node, const LeafBox& leafBox, const InnerBox& inne
 // The box the instance level is built over.  tight: b holds the exact bounds of the transformed vertices on entry and is padded
 // -- the object-space ray is a ROUNDED transform of the world ray, so a hit found in object space may lie a few ulps outside
 // the exact world-space box.  Otherwise b becomes the padded bounds of the eight transformed corners of the GAS box (the
-// round-1 bounds, looser for rotated instances).  Instances of an empty GAS get a point box at the origin.
+// round-1 bounds, looser for rotated instances).  Instances of an empty GAS, or of one whose triangles are all inactive, get a
+// point box at the origin.  An instance whose transform has a non-finite entry, or whose world bounds reach beyond B (tight: the
+// exact bounds on entry; otherwise the padded corner box), is inactive: it gets the empty box, which no ray enters.
 RTC_HD void instance_box_finish(const float transform[12], const float gasLo[3], const float gasHi[3], bool tight, bool emptyGas, PrimBox& b)
 {
+  bool active = true;
+  for (int k = 0; k < 12; ++k) active = active && rules_in_range(transform[k]);
+  if (!active) { rules_empty_box(b.lo, b.hi); return; }
+  if (emptyGas || rules_box_empty(gasLo, gasHi)) { for (int k = 0; k < 3; ++k) { b.lo[k] = 0.0f; b.hi[k] = 0.0f; } return; }
   const double ext = fabs((double)gasHi[0] - gasLo[0]) + fabs((double)gasHi[1] - gasLo[1]) + fabs((double)gasHi[2] - gasLo[2]);
   if (tight)
   {
+    if (!rules_in_range3(b.lo) || !rules_in_range3(b.hi)) { rules_empty_box(b.lo, b.hi); return; }
     for (int r = 0; r < 3; ++r)
     {
       const float* m = &transform[4 * r];
       const double scale = fabs((double)m[0]) + fabs((double)m[1]) + fabs((double)m[2]);
-      const double padLo = (fabs((double)b.lo[r]) + ext * scale) * 1.0e-5, padHi = (fabs((double)b.hi[r]) + ext * scale) * 1.0e-5;
+      // the pad is capped at 2^116 so that exact bounds within B stay finite however large ext * scale is
+      const double padLo = fmin((fabs((double)b.lo[r]) + ext * scale) * 1.0e-5, 0x1p116);
+      const double padHi = fmin((fabs((double)b.hi[r]) + ext * scale) * 1.0e-5, 0x1p116);
       b.lo[r] = nextafterf((float)((double)b.lo[r] - padLo), -INFINITY);
       b.hi[r] = nextafterf((float)((double)b.hi[r] + padHi), INFINITY);
     }
@@ -163,8 +220,8 @@ RTC_HD void instance_box_finish(const float transform[12], const float gasLo[3],
         b.lo[r] = fminf(b.lo[r], lo); b.hi[r] = fmaxf(b.hi[r], hi);
       }
     }
+    if (!rules_in_range3(b.lo) || !rules_in_range3(b.hi)) rules_empty_box(b.lo, b.hi);
   }
-  if (emptyGas) { for (int k = 0; k < 3; ++k) { b.lo[k] = 0.0f; b.hi[k] = 0.0f; } }
 }
 
 // ---- LBVH (Karras 2012) ---------------------------------------------------------------------------------------------------------

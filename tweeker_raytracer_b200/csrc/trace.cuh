@@ -181,25 +181,39 @@ __device__ __forceinline__ float quant_i2f(uint32_t w)
   return (float)((w >> (8u * I)) & 0xffu);
 }
 
+// 1/d of one axis saturated at 2^112 / gridStep (eb = the biased exponent of the grid step), so that |adj| <= 2^112 and the
+// bias term 32768 * adj stays finite.  Saturation scales that axis's plane distances t by one factor s < 1, which keeps the
+// near plane conservative; the far plane of a hit child keeps at least step / 64 of slack, so its scaled t stays >= 2^106,
+// above every tmax < 2^100 (DESIGN.md section 3).  Unsaturated (grid steps up to 2^32 for any ray) the bits are unchanged.
+// A plane origin term (p - o) / d that still overflows means the whole node lies more than 2^16 steps to one side of the
+// origin, and the resulting +-inf culls exactly the boxes that lie entirely behind the origin or beyond tmax.
+__device__ __forceinline__ float sat_idir(float id, uint32_t eb)
+{
+  const uint32_t raw = 0xB7000000u - (eb << 23);      // bits of 2^(112 - e) = 2^(239 - eb)
+  const float lim = __uint_as_float(raw < 0x7F000000u ? raw : 0x7F000000u);   // at most 2^127
+  return fminf(fmaxf(id, -lim), lim);
+}
+
 // Tests the 8 quantised child boxes of one node.  Returns bit s set when the box in slot s is hit.
 // opaqueZero: a value that is always 0 but that the compiler cannot prove to be (bit 31 of a child index).
 __device__ __forceinline__ uint32_t node_test(const BoxRay& b, const uint4 n0, const uint4 n2, const uint4 n3, const uint4 n4,
                                               float tmin, float tlimit, uint32_t opaqueZero)
 {
   const uint32_t e = n0.w;
-  const float adjx = __uint_as_float((e & 0xffu) << 23) * b.idx;
-  const float adjy = __uint_as_float(((e >> 8) & 0xffu) << 23) * b.idy;
-  const float adjz = __uint_as_float(((e >> 16) & 0xffu) << 23) * b.idz;
-  const float orgx = fmaf(-32768.0f, adjx, (__uint_as_float(n0.x) - b.ox) * b.idx);
+  const float idx = sat_idir(b.idx, e & 0xffu), idy = sat_idir(b.idy, (e >> 8) & 0xffu), idz = sat_idir(b.idz, (e >> 16) & 0xffu);
+  const float adjx = __uint_as_float((e & 0xffu) << 23) * idx;
+  const float adjy = __uint_as_float(((e >> 8) & 0xffu) << 23) * idy;
+  const float adjz = __uint_as_float(((e >> 16) & 0xffu) << 23) * idz;
+  const float orgx = fmaf(-32768.0f, adjx, (__uint_as_float(n0.x) - b.ox) * idx);
 #if RTC_I2F_AXES >= 2
-  const float orgy = (__uint_as_float(n0.y) - b.oy) * b.idy;
+  const float orgy = (__uint_as_float(n0.y) - b.oy) * idy;
 #else
-  const float orgy = fmaf(-32768.0f, adjy, (__uint_as_float(n0.y) - b.oy) * b.idy);
+  const float orgy = fmaf(-32768.0f, adjy, (__uint_as_float(n0.y) - b.oy) * idy);
 #endif
 #if RTC_I2F_AXES >= 1
-  const float orgz = (__uint_as_float(n0.z) - b.oz) * b.idz;            // z planes: plain q through I2F, no bias to cancel
+  const float orgz = (__uint_as_float(n0.z) - b.oz) * idz;              // z planes: plain q through I2F, no bias to cancel
 #else
-  const float orgz = fmaf(-32768.0f, adjz, (__uint_as_float(n0.z) - b.oz) * b.idz);
+  const float orgz = fmaf(-32768.0f, adjz, (__uint_as_float(n0.z) - b.oz) * idz);
 #endif
   // near/far plane words per axis, selected by the direction sign
   // layout: n2 = qlox[0..3], qlox[4..7], qloy[0..3], qloy[4..7]; n3 = qloz, qhix; n4 = qhiy, qhiz
