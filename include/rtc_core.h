@@ -187,6 +187,45 @@ int rtc_ias_rebuild(rtc_context* ctx, uint64_t topObject);
  */
 int rtc_gas_rebuild(rtc_context* ctx, uint32_t gas, uint64_t attributes);
 /*
+ * Geometry whose triangle set lives on the device (optixAccelBuild over OPTIX_BUILD_INPUT_TYPE_TRIANGLES with inputs in device
+ * memory, called every frame into the same output buffers): meshes whose triangle count or connectivity changes from frame to
+ * frame -- isosurfaces, fracture, level of detail, streamed terrain tiles -- without a host stall and without a new handle.
+ *
+ * rtc_gas_create: a GAS with room for `capacity` triangles (0 is treated as 1) and no triangle yet (the nodes and bounds
+ *   rtc_gas_build writes for numTris == 0: every ray misses it).  Allocates everything its builds will use -- a node array for
+ *   capacity + 16 nodes, 48 B of triangle records per triangle, refit scratch, the LBVH arrays and the collapse graph -- and
+ *   synchronises once.  The handle works wherever one of rtc_gas_build does (rtc_ias_build, records of rtc_ias_build_device,
+ *   rtc_gas_refit, rtc_gas_rebuild, rtc_gas_info, rtc_gas_export, rtc_gas_destroy).
+ * rtc_gas_build_device: replaces the GAS's whole triangle set with numTris <= capacity triangles (uint3 index triplets at
+ *   `indices`) over numVerts vertex records of strideBytes bytes at `attributes` (the position is their first 12 bytes), and
+ *   builds a new LBVH over them in place: same handle, same node array.
+ *   - Stream order: vertices and indices are read ON THE CONTEXT STREAM, when the stream reaches the call, as rtc_ias_build_device
+ *     reads its records.  Never synchronises the host; allocates only from the stream-ordered pool.  Work enqueued before sees the
+ *     old triangles, work enqueued after sees the new ones.
+ *   - Ownership: `attributes` and `indices` become the GAS's buffers, as if rtc_gas_build had been given them: shading reads
+ *     them, rtc_gas_refit(gas, 0) and rtc_gas_rebuild(gas, 0) work on them.  Keep them alive and unchanged (apart from refits)
+ *     until the next build or rtc_gas_destroy.  numVerts and numTris may differ from call to call.
+ *   - Bad indices: an index >= numVerts reads the vertex (NaN, NaN, NaN), so its triangle is inactive (never hit, bounds
+ *     nothing, NaN in v0 of its record), and is counted for rtc_gas_rejected_triangles.  No index makes a kernel read outside
+ *     [attributes, attributes + numVerts * strideBytes).
+ *   - Result bytes: nodes and triangle records equal rtc_host_gas_build + rtc_host_gas_rebuild(accel, NULL) over the same
+ *     triangles, with every out-of-range index replaced by the index of one NaN vertex appended to the vertices.  Two builds of
+ *     the same input give the same bytes, whatever the GAS held before.
+ *   - Staleness: as after rtc_gas_rebuild, every scene that instances the GAS is stale until rtc_ias_update or
+ *     rtc_ias_build_device runs on it; launches and rtc_trace_* on it are refused until then.
+ *   - Refused (synchronously, nothing enqueued, the GAS unchanged): an unknown or destroyed handle, a GAS of rtc_gas_build,
+ *     numTris > capacity, a stride below 12 or not a multiple of 4, `attributes` or `indices` not 4-byte aligned, null buffers
+ *     with numTris > 0.
+ *   rtc_gas_info, rtc_gas_export and rtc_scene_info_get report the current triangle count.
+ * rtc_gas_rejected_triangles: the triangles with an out-of-range index in the last build of the GAS (0 for a GAS of
+ *   rtc_gas_build, which refuses such indices).  Synchronises.
+ * Detect the feature by these exports (rtc_version is unchanged).
+ */
+int rtc_gas_create(rtc_context* ctx, uint32_t capacity, uint32_t* gas);
+int rtc_gas_build_device(rtc_context* ctx, uint32_t gas, uint64_t attributes, uint32_t strideBytes, uint32_t numVerts,
+                         uint64_t indices, uint32_t numTris);
+int rtc_gas_rejected_triangles(rtc_context* ctx, uint32_t gas, uint32_t* count);
+/*
  * Scenes whose instance set lives on the device (optixAccelBuild over OPTIX_BUILD_INPUT_TYPE_INSTANCES, called every frame into
  * the same buffers): spawn and despawn objects, swap an instance's GAS (level of detail, a broken variant) or reassign its
  * material without a host stall and without a new topObject.

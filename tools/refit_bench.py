@@ -24,6 +24,13 @@
     (device ms between events, and host ms of the call and its synchronisation), against rtc_ias_build of the same records and,
     for the counts a scene of rtc_ias_build can hold, rtc_ias_update_device + rtc_ias_rebuild; incoherent closest-hit Mrays/s of
     the created and the built scene after each, whose hits are checked to be equal in the same run.
+  * --device-geometry: the traded soups above, built into one GAS of rtc_gas_create by rtc_gas_build_device from vertices and
+    indices already in device memory: device ms between events and host ms of the call alone (its enqueue), against
+    rtc_gas_build(RTC_BUILD_DEFAULT) host wall ms and rtc_gas_rebuild device ms of the same triangles; the device memory the
+    created GAS holds per triangle of capacity; incoherent closest-hit Mrays/s of the result against the default build (the host
+    SAH builder below 2^20 triangles), whose hits are checked to be equal in the same run; a count that changes between calls
+    (0.9 n, n, 0.1 n into capacity n); and a build of n / 100 triangles into capacity n against the same build into a GAS of
+    capacity n / 100 (the collapse graph's grids are sized for the capacity).
 Builds are timed on the host clock (they end in a synchronisation); refits, updates and traces between CUDA events on the
 context stream, each the median of `repeats` runs after one warm-up.
 """
@@ -177,6 +184,70 @@ def soup_runs(ctx, n, nrays, repeats):
     ctx.scene_destroy(top)
     ctx.gas_destroy(gas)
     for p in (d_v, d_i, d_rays, d_hits, d_hits2, d_hits3):
+        ctx.free(p)
+
+
+def device_geometry_runs(ctx, n, nrays, repeats):
+    verts = bench.soup_numpy(n)
+    verts = verts.reshape(n, 9)[np.random.default_rng(3).permutation(n)].reshape(-1, 3)        # the traded soup
+    idx = np.arange(3 * n, dtype=np.uint32)
+    d_v, d_i = ctx.malloc(verts.nbytes), ctx.malloc(idx.nbytes)
+    ctx.upload(d_v, verts)
+    ctx.upload(d_i, idx)
+    del verts, idx
+    inst = np.zeros(1, dtype=core.INSTANCE_DTYPE)
+    inst[0]["transform"] = [1, 0, 0, 0, 0, 1, 0, 0, 0, 0, 1, 0]
+    default_ms = wall(ctx, lambda: ctx.gas_destroy(ctx.gas_build(d_v, 12, 3 * n, d_i, n)), 3)
+    built = ctx.gas_build(d_v, 12, 3 * n, d_i, n)
+    ctx.gas_rebuild(built)                                                  # the first rebuild allocates
+    rebuild_ms = timed(ctx, lambda: ctx.gas_rebuild(built), repeats)
+    ctx.gas_destroy(built)
+    ctx.synchronize()
+    free0 = mem_free()
+    g = ctx.gas_create(n)
+    resident = free0 - mem_free()
+    device_ms = timed(ctx, lambda: ctx.gas_build_device(g, d_v, 12, 3 * n, d_i, n), repeats)
+    call_ms = []
+    for _ in range(repeats):
+        ctx.synchronize()
+        t0 = time.perf_counter()
+        ctx.gas_build_device(g, d_v, 12, 3 * n, d_i, n)
+        call_ms.append((time.perf_counter() - t0) * 1e3)
+    inst[0]["gas"] = g
+    top = ctx.ias_build(inst)
+    default = ctx.gas_build(d_v, 12, 3 * n, d_i, n)
+    inst[0]["gas"] = default
+    default_top = ctx.ias_build(inst)
+    rays = bench.rays_numpy(nrays, "incoh", "closest")
+    d_rays, d_hits, d_hits2 = ctx.malloc(rays.nbytes), ctx.malloc(20 * nrays), ctx.malloc(20 * nrays)
+    ctx.upload(d_rays, rays)
+    del rays
+    created_rate = mrays(ctx, top, d_rays, nrays, d_hits, repeats)
+    default_rate = mrays(ctx, default_top, d_rays, nrays, d_hits2, repeats)
+    a = ctx.download(d_hits, np.uint8, 20 * nrays)
+    b = ctx.download(d_hits2, np.uint8, 20 * nrays)
+    emit(what="gas_build_device", triangles=n, build_device_ms=device_ms, build_device_call_host_ms=float(np.median(call_ms)),
+         gas_rebuild_ms=rebuild_ms, gas_build_default_wall_ms=default_ms,
+         default_builder="host_sah" if n <= (1 << 20) else "gpu_lbvh", resident_bytes_of_create=resident,
+         resident_bytes_per_triangle_of_capacity=resident / n, rays=nrays, created_mrays=created_rate, default_mrays=default_rate,
+         created_over_default=created_rate / default_rate, hits_equal=bool(np.array_equal(a, b)))
+    ctx.scene_destroy(top)
+    ctx.scene_destroy(default_top)
+    ctx.gas_destroy(default)
+    # a count that changes from call to call, into the same GAS
+    counts = [(9 * n) // 10, n, n // 10]
+    ms = [timed(ctx, lambda: ctx.gas_build_device(g, d_v, 12, 3 * n, d_i, m), repeats) for m in counts]
+    emit(what="gas_build_device_changing_count", capacity=n, triangles=counts, build_device_ms=ms)
+    # n / 100 triangles into capacity n, against a GAS whose capacity is n / 100
+    m = max(1, n // 100)
+    big_ms = timed(ctx, lambda: ctx.gas_build_device(g, d_v, 12, 3 * n, d_i, m), repeats)
+    small = ctx.gas_create(m)
+    small_ms = timed(ctx, lambda: ctx.gas_build_device(small, d_v, 12, 3 * n, d_i, m), repeats)
+    emit(what="gas_build_device_small_in_large", capacity=n, triangles=m, build_device_ms=big_ms, capacity_equal_ms=small_ms,
+         idle_capacity_ms=big_ms - small_ms)
+    ctx.gas_destroy(small)
+    ctx.gas_destroy(g)
+    for p in (d_v, d_i, d_rays, d_hits, d_hits2):
         ctx.free(p)
 
 
@@ -392,6 +463,7 @@ def main():
     ap.add_argument("--no-instances", action="store_true")
     ap.add_argument("--many-instances", default="1M", help="instance count of the small-instance scene (0: skip)")
     ap.add_argument("--changing-instances", default="10001,1M", help="capacities of the changing instance sets (0: skip)")
+    ap.add_argument("--device-geometry", default="", help="triangle counts of the rtc_gas_build_device runs, e.g. 1M,10M,100M")
     args = ap.parse_args()
     scale = {"K": 10 ** 3, "M": 10 ** 6}
     count = lambda s: int(float(s[:-1]) * scale[s[-1]]) if s[-1] in scale else int(s)    # noqa: E731
@@ -401,6 +473,8 @@ def main():
     with core.Context(0) as ctx:
         for s in filter(None, args.sizes.split(",")):
             soup_runs(ctx, count(s), count(args.rays), args.repeats)
+        for s in filter(None, args.device_geometry.split(",")):
+            device_geometry_runs(ctx, count(s), count(args.rays), args.repeats)
         if not args.no_instances:
             instance_runs(ctx, count(args.rays), args.repeats)
             if count(args.many_instances):

@@ -38,6 +38,7 @@ SYMBOLS = [
     "rtc_ias_rebuild", "rtc_host_ias_rebuild", "rtc_ias_update_device",
     "rtc_gas_rebuild", "rtc_host_gas_rebuild",
     "rtc_ias_create", "rtc_ias_build_device", "rtc_scene_rejected_instances",
+    "rtc_gas_create", "rtc_gas_build_device", "rtc_gas_rejected_triangles",
 ]
 
 MATH_FUNCTIONS = ["sin", "cos", "atan", "atan2", "acos", "exp", "log", "pow", "div", "sqrt", "muladd"]     # enum rtc_math_fn
@@ -113,6 +114,9 @@ def lib():
         L.rtc_ias_create.argtypes = [C.c_void_p, C.c_uint32, C.POINTER(C.c_uint64)]
         L.rtc_ias_build_device.argtypes = [C.c_void_p, C.c_uint64, C.c_uint64, C.c_uint32, C.c_uint32]
         L.rtc_scene_rejected_instances.argtypes = [C.c_void_p, C.c_uint64, C.POINTER(C.c_uint32)]
+        L.rtc_gas_create.argtypes = [C.c_void_p, C.c_uint32, C.POINTER(C.c_uint32)]
+        L.rtc_gas_build_device.argtypes = [C.c_void_p, C.c_uint32, C.c_uint64, C.c_uint32, C.c_uint32, C.c_uint64, C.c_uint32]
+        L.rtc_gas_rejected_triangles.argtypes = [C.c_void_p, C.c_uint32, C.POINTER(C.c_uint32)]
         L.rtc_scene_info_get.argtypes = [C.c_void_p, C.c_uint64, C.POINTER(SceneInfo)]
         L.rtc_scene_destroy.argtypes = [C.c_void_p, C.c_uint64]
         L.rtc_scene_set_instance_flags.argtypes = [C.c_void_p, C.c_uint64, C.c_uint32, C.c_uint32, C.c_void_p]
@@ -251,35 +255,76 @@ def host_scene_refit_export(geometries, instances, new_attributes, new_transform
     return export, info
 
 
+def _nan_padded(attrs):
+    """vertex records as bytes [n + 1, stride] with one record appended whose position is (NaN, NaN, NaN): the vertex an
+    out-of-range index of rtc_gas_build_device reads"""
+    attrs, stride = _vertex_records(attrs)
+    rows = attrs.view(np.uint8).reshape(len(attrs), stride)
+    pad = np.zeros((1, stride), dtype=np.uint8)
+    pad[0, :12] = np.full(3, np.nan, dtype=np.float32).view(np.uint8)
+    return np.ascontiguousarray(np.concatenate([rows, pad])), stride
+
+
+def _host_gas_build_device(L, attrs, idx):
+    """the twin of rtc_gas_build_device: rtc_host_gas_build + rtc_host_gas_rebuild over the vertices with one NaN vertex appended,
+    which every index >= the vertex count is replaced by"""
+    n = len(np.ascontiguousarray(attrs))
+    padded, stride = _nan_padded(attrs)
+    idx = np.array(idx, dtype=np.uint32).reshape(-1, 3)
+    idx[idx >= n] = n
+    h = C.c_void_p()
+    _check(L.rtc_host_gas_build(padded.ctypes.data_as(C.c_void_p), stride, n + 1, idx.ctypes.data_as(C.c_void_p), len(idx), C.byref(h)))
+    rc = L.rtc_host_gas_rebuild(h, None, 0)
+    if rc != 0:
+        L.rtc_host_accel_destroy(h)
+        _check(rc)
+    return h
+
+
 def host_scene_rebuild_export(geometries, instances, steps):
     """host_scene_export of the scene built from (geometries, instances), then taken WITHOUT a GPU through `steps`, in order:
     "rebuild" (rtc_host_ias_rebuild, the twin of rtc_ias_rebuild), ("gas_rebuild", g, attributes) (rtc_host_gas_rebuild, the
-    twin of rtc_gas_rebuild of geometry g: attributes = its new vertex records, or None for its current positions) or
-    (new_attributes, new_transforms), a refit as in host_scene_refit_export (rtc_gas_refit of the geometries given, then
-    rtc_ias_update of every instance).  A device program of rtc_gas_rebuild / rtc_gas_refit calls followed by rtc_ias_update is
+    twin of rtc_gas_rebuild of geometry g: attributes = its new vertex records, or None for its current positions),
+    ("gas_build_device", g, attributes, indices) (the twin of rtc_gas_build_device of geometry g: its triangle set becomes
+    (attributes, indices), out-of-range indices included) or (new_attributes, new_transforms), a refit as in
+    host_scene_refit_export (rtc_gas_refit of the geometries given, then rtc_ias_update of every instance).  A device program of
+    rtc_gas_build_device / rtc_gas_rebuild / rtc_gas_refit calls followed by rtc_ias_update is ("gas_build_device", ...) and
     ("gas_rebuild", ...) steps and then one refit step that refits the other geometries."""
     L = lib()
     accels, info = [], {}
+    padded = set()              # geometries replaced by a gas_build_device step: their twin holds one NaN vertex more
     try:
         top, inst_gas = _host_build(L, geometries, instances, accels)
         accels.append(top)
         handles = (C.c_void_p * max(len(inst_gas), 1))(*[accels[int(g)] for g in inst_gas])
+
+        def records(g, attrs):
+            return _nan_padded(attrs) if g in padded else _vertex_records(attrs)
+
         for step in steps:
             if isinstance(step, str) and step == "rebuild":
                 _check(L.rtc_host_ias_rebuild(top))
+                continue
+            if isinstance(step, tuple) and len(step) == 4 and step[0] == "gas_build_device":
+                _, g, attrs, idx = step
+                h = _host_gas_build_device(L, attrs, idx)
+                L.rtc_host_accel_destroy(accels[g])
+                accels[g] = h
+                padded.add(g)
+                handles = (C.c_void_p * max(len(inst_gas), 1))(*[accels[int(k)] for k in inst_gas])
                 continue
             if isinstance(step, tuple) and len(step) == 3 and step[0] == "gas_rebuild":
                 _, g, attrs = step
                 if attrs is None:
                     _check(L.rtc_host_gas_rebuild(accels[g], None, 0))
                 else:
-                    attrs, stride = _vertex_records(attrs)
+                    attrs, stride = records(g, attrs)
                     _check(L.rtc_host_gas_rebuild(accels[g], attrs.ctypes.data_as(C.c_void_p), stride))
                 continue
             new_attributes, new_transforms = step
             for g, attrs in enumerate(new_attributes):
                 if attrs is not None:
-                    attrs, stride = _vertex_records(attrs)
+                    attrs, stride = records(g, attrs)
                     _check(L.rtc_host_gas_refit(accels[g], attrs.ctypes.data_as(C.c_void_p), stride))
             transforms = np.ascontiguousarray(new_transforms, dtype=np.float32).reshape(len(inst_gas), 12)
             _check(L.rtc_host_ias_refit(top, transforms.ctypes.data_as(C.c_void_p), C.cast(handles, C.c_void_p), len(inst_gas)))
@@ -384,6 +429,26 @@ class Context:
         d_attributes = new records of the build's stride), on the device and in place (the handle stays valid).  Asynchronous,
         except for the first rebuild of a GAS.  Every scene instancing it must then get ias_update before it is traced."""
         _check(self.L.rtc_gas_rebuild(self.h, gas, int(d_attributes)))
+
+    def gas_create(self, capacity):
+        """rtc_gas_create: a GAS without triangles (every ray misses it) with room for `capacity` triangles, whose triangle set
+        gas_build_device replaces in place.  Synchronises once."""
+        g = C.c_uint32(0)
+        _check(self.L.rtc_gas_create(self.h, int(capacity), C.byref(g)))
+        return g.value
+
+    def gas_build_device(self, gas, d_attributes, stride, num_verts, d_indices, num_tris):
+        """rtc_gas_build_device: the GAS's triangles become the num_tris index triplets at the device address d_indices over the
+        num_verts vertex records (stride bytes each) at d_attributes (ints, e.g. tensor.data_ptr()), built on the device in place.
+        Both buffers are read on the context stream when the build runs and become the GAS's own, as in gas_build: keep them alive.
+        Never blocks the host.  Every scene instancing the GAS must then get ias_update (or ias_build_device) before it is traced."""
+        _check(self.L.rtc_gas_build_device(self.h, int(gas), int(d_attributes), int(stride), int(num_verts), int(d_indices), int(num_tris)))
+
+    def gas_rejected_triangles(self, gas):
+        """rtc_gas_rejected_triangles: triangles of the last gas_build_device with an index >= num_verts (synchronises)."""
+        n = C.c_uint32(0)
+        _check(self.L.rtc_gas_rejected_triangles(self.h, int(gas), C.byref(n)))
+        return n.value
 
     def ias_update(self, top, transforms, first=0):
         """rtc_ias_update: transforms [count, 12] (object -> world) of instances first .. first + count - 1 (count may be 0: only

@@ -56,7 +56,11 @@ k_refit_tris(float4* __restrict__ tris, uint32_t numTris, const uint8_t* __restr
   for (int c = 0; c < 3; ++c)
   {
     const uint32_t vi = __ldg(idx + 3u * (size_t)prim + c);
-    if (vi >= numVerts) return;                         // indices are the build's, which checked them
+    if (vi >= numVerts)                                 // only rtc_gas_build_device leaves such an index: an inactive triangle
+    {
+      x[c][0] = x[c][1] = x[c][2] = __uint_as_float(kMissingVertexBits);
+      continue;
+    }
     const float* p = reinterpret_cast<const float*>(verts + (size_t)vi * stride);
     x[c][0] = __ldg(p); x[c][1] = __ldg(p + 1); x[c][2] = __ldg(p + 2);
   }
@@ -306,8 +310,9 @@ k_instance_gather(const GatherParams P)
 }
 
 // One thread per written instance: the padded box (instance_box_finish, bvh_rules.h), the instance's 64 B traversal record
-// (world->object rows 0..2, row 3 = {GAS nodes, GAS triangles}) and its rows of the shading tables (object->world, vertex
-// attributes; with `material` also the GAS's indices and the record's material and light).  numUp as in k_instance_bounds.
+// (world->object rows 0..2, row 3 = {GAS nodes, GAS triangles}) and its rows of the shading tables (object->world, the GAS's
+// vertex attributes and indices -- rtc_gas_build_device replaces both; with `material` also the record's material and light).
+// numUp as in k_instance_bounds.
 __global__ void __launch_bounds__(128)
 k_instance_finish(const InstanceUpdate* __restrict__ up, uint32_t count, const uint32_t* __restrict__ numUp, const PrimBox* __restrict__ exact,
                   int tight, int material, PrimBox* __restrict__ instBoxes, float4* __restrict__ instances, float4* __restrict__ o2w,
@@ -331,7 +336,8 @@ k_instance_finish(const InstanceUpdate* __restrict__ up, uint32_t count, const u
   }
   *reinterpret_cast<ulonglong2*>(instances + 4u * inst + 3) = make_ulonglong2((uintptr_t)g.nodes, (uintptr_t)g.tris);
   gi[inst].attributes = g.attributes;
-  if (material) { gi[inst].indices = g.indices; gi[inst].materialIndex = u.materialIndex; gi[inst].lightIndex = u.lightIndex; }
+  gi[inst].indices = g.indices;
+  if (material) { gi[inst].materialIndex = u.materialIndex; gi[inst].lightIndex = u.lightIndex; }
 }
 
 // pooled: from the stream-ordered pool (the instance level: its updates never allocate with a call that may block)

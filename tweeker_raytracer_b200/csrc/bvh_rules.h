@@ -59,6 +59,10 @@ RTC_HD void rules_tri_record(const float* v0, const float* v1, const float* v2, 
   rec[2] = make_float4(v2[0], v2[1], v2[2], 0.0f);
 }
 
+// The position an index past the vertex records reads in rtc_gas_build_device (and the refit and rebuild of its GAS): (NaN, NaN,
+// NaN), the quiet NaN of rules_tri_record, so its triangle is inactive.  The host twin appends one such vertex instead.
+constexpr uint32_t kMissingVertexBits = 0x7fc00000u;
+
 RTC_HD bool rules_box_empty(const float lo[3], const float hi[3])
 {
   return !(lo[0] <= hi[0] && lo[1] <= hi[1] && lo[2] <= hi[2]);

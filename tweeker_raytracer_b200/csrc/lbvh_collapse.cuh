@@ -1,6 +1,7 @@
 // lbvh_collapse.cuh -- the device LBVH rebuild both levels share: one primitive per leaf slot, deterministic bytes, and no host
-// synchronisation after the first call.  bvh_build_ias_gpu.cu (rtc_ias_rebuild, instance leaves) and bvh_build_gas_rebuild_gpu.cu
-// (rtc_gas_rebuild, triangle leaves) wrap the device bodies below in their own kernels and hand them the leaf write.
+// synchronisation after the first call.  bvh_build_ias_gpu.cu (rtc_ias_rebuild, rtc_ias_build_device: instance leaves) and
+// bvh_build_gas_rebuild_gpu.cu (rtc_gas_rebuild, rtc_gas_build_device: triangle leaves) wrap the device bodies below in their own
+// kernels and hand them the leaf write.
 //
 //   primitive boxes and the exact min / max of their centres                     the caller's kernel, lbvh_reduce_centre_box
 //   63-bit Morton codes, stable radix sort (key, then index)                      k_morton, cub::DeviceRadixSort    (lbvh.cuh)
@@ -35,13 +36,13 @@ namespace {
 
 constexpr int kCollapseBlock = 128;
 constexpr int kScanThreads = 256;
-// words of LbvhRebuild::counters; kInput (two words) is the caller's: the GAS rebuild keeps the vertex buffer of the call there,
-// the instance level the primitive count of the call (a created scene's count changes from build to build)
-enum { kNodeCount = 0, kLeafCount = 1, kWorkCount = 2 /* two: ping-pong */, kLevelNodeBase = 4, kLevelLeafBase = 5, kInput = 6, kNumCounters = 8 };
+// words of LbvhRebuild::counters; from kInput on they hold the inputs of the call, which the collapse graph (captured once) reads:
+// counters[kInput] is the primitive count of the call (a created structure's count changes from build to build), the words
+// after it are the caller's (a geometry keeps its vertex and index buffers there, bvh_build_gas_rebuild_gpu.cu)
+enum { kNodeCount = 0, kLeafCount = 1, kWorkCount = 2 /* two: ping-pong */, kLevelNodeBase = 4, kLevelLeafBase = 5, kInput = 6, kNumCounters = 14 };
 
 struct CollapseArgs
 {
-  int n;
   const int2* child; const float4* boxLo; const float4* boxHi;
   const uint32_t* order;          // sorted position -> primitive
   uint4* nodes; uint32_t* leaves; // leaves: the instance level's leaf slots (null for a geometry, whose leaf write is its own)
@@ -254,7 +255,7 @@ int lbvh_rebuild_alloc(rtc_context* ctx, LbvhRebuild& R, uint32_t n, uint32_t* l
     R.sortedKeys = k.Current(); R.sortedOrder = v.Current();
   }
   CollapseArgs& A = R.args;
-  A.n = (int)n; A.child = R.child; A.boxLo = R.boxLo; A.boxHi = R.boxHi; A.order = R.sortedOrder;
+  A.child = R.child; A.boxLo = R.boxLo; A.boxHi = R.boxHi; A.order = R.sortedOrder;
   A.nodes = static_cast<uint4*>(R.nodes); A.leaves = leaves;
   A.parent = R.refit.parent; A.arrivals = R.refit.arrivals;
   A.kidAt = reinterpret_cast<int*>(b + oKidAt); A.local = reinterpret_cast<uint32_t*>(b + oLocal);

@@ -519,7 +519,7 @@ int rtc_gas_destroy(rtc_context* ctx, uint32_t gas)
     }
   cudaFree(g.d_nodes); cudaFree(g.d_tris); free_refit_scratch(g.refit, ctx->stream); free_lbvh_rebuild(g.rebuild);
   g.d_nodes = nullptr; g.d_tris = nullptr; g.numNodes = 0; g.numTris = 0; g.boundsOnDevice = false;
-  g.rebuild = nullptr; g.d_numNodes = nullptr;
+  g.rebuild = nullptr; g.d_numNodes = nullptr; g.d_rejected = nullptr; g.capacity = 0;
   return write_gas_table(ctx, gas);
 }
 
@@ -545,6 +545,72 @@ int rtc_gas_rebuild(rtc_context* ctx, uint32_t gas, uint64_t attributes)
   ctx->gasEpoch++;
   if (int rc = rebuild_gas_gpu(ctx, g)) return rc;
   return write_gas_table(ctx, gas);
+}
+
+// A GAS whose triangle set rtc_gas_build_device replaces in place: node array, triangle records, refit scratch, LBVH arrays and
+// collapse graph for `capacity` triangles, allocated now; no triangle yet (the empty node of rtc_gas_build for none).
+int rtc_gas_create(rtc_context* ctx, uint32_t capacity, uint32_t* gas)
+{
+  if (!gas) RTC_FAIL("gas is null");
+  RTC_CUDA(cudaSetDevice(ctx->device));
+  const double t0 = now_ms();
+  GasRecord rec;
+  rec.capacity = capacity ? capacity : 1u;
+  rec.strideBytes = 12;
+  rec.builder = RTC_BUILD_GPU_LBVH;
+  RTC_CUDA(cudaMalloc(&rec.d_tris, (size_t)rec.capacity * 3u * sizeof(float4)));
+  int rc = create_gas_gpu(ctx, rec, rec.capacity);
+  if (rc == 0) { const cudaError_t e = cudaStreamSynchronize(ctx->stream); if (e != cudaSuccess) rc = rtc_set_error(__FILE__, __LINE__, "rtc_gas_create", (int)e, cudaGetErrorString(e)); }
+  if (rc)
+  {
+    cudaStreamSynchronize(ctx->stream);
+    cudaFree(rec.d_nodes); cudaFree(rec.d_tris); free_refit_scratch(rec.refit, ctx->stream); free_lbvh_rebuild(rec.rebuild);
+    cudaGetLastError();
+    return rc;
+  }
+  rec.numNodes = 1;
+  rec.buildMs = now_ms() - t0;
+  ctx->gas.push_back(rec);
+  *gas = (uint32_t)(ctx->gas.size() - 1);
+  return write_gas_table(ctx, *gas);
+}
+
+int rtc_gas_build_device(rtc_context* ctx, uint32_t gas, uint64_t attributes, uint32_t strideBytes, uint32_t numVerts,
+                         uint64_t indices, uint32_t numTris)
+{
+  if (gas >= ctx->gas.size() || ctx->gas[gas].d_nodes == nullptr) RTC_FAIL("bad gas handle");
+  GasRecord& g = ctx->gas[gas];
+  if (!g.capacity) RTC_FAIL("rtc_gas_build_device needs a GAS of rtc_gas_create (this one was built by rtc_gas_build)");
+  if (numTris > g.capacity) RTC_FAIL("numTris exceeds the GAS's capacity");
+  if (strideBytes < 12 || (strideBytes & 3u)) RTC_FAIL("vertex stride must be a multiple of 4 and at least 12");
+  if (attributes & 3u) RTC_FAIL("attributes is not 4-byte aligned");
+  if (indices & 3u) RTC_FAIL("indices is not 4-byte aligned");
+  if (numTris && (!attributes || !indices)) RTC_FAIL("attributes or indices is null");
+  RTC_CUDA(cudaSetDevice(ctx->device));
+  const double t0 = now_ms();
+  // the triangle totals of the scenes of rtc_ias_build that instance it (created scenes count theirs from the GAS records)
+  for (SceneRecord* s : ctx->scenes)
+    for (const std::pair<uint32_t, uint64_t>& e : s->gasGeneration)
+      if (e.first == gas) s->totalTris = s->totalTris - g.numTris + numTris;
+  g.attributes = attributes; g.indices = indices; g.strideBytes = strideBytes; g.numVerts = numVerts; g.numTris = numTris;
+  g.generation++;
+  ctx->gasEpoch++;
+  if (int rc = rebuild_gas_gpu(ctx, g)) return rc;
+  g.buildMs = now_ms() - t0;
+  return write_gas_table(ctx, gas);
+}
+
+int rtc_gas_rejected_triangles(rtc_context* ctx, uint32_t gas, uint32_t* count)
+{
+  if (gas >= ctx->gas.size() || ctx->gas[gas].d_nodes == nullptr) RTC_FAIL("bad gas handle");
+  if (!count) RTC_FAIL("count is null");
+  *count = 0;
+  const GasRecord& g = ctx->gas[gas];
+  if (!g.d_rejected || !g.numTris) return 0;      // rtc_gas_build checked every index
+  RTC_CUDA(cudaSetDevice(ctx->device));
+  RTC_CUDA(cudaMemcpyAsync(count, g.d_rejected, sizeof(uint32_t), cudaMemcpyDeviceToHost, ctx->stream));
+  RTC_CUDA(cudaStreamSynchronize(ctx->stream));
+  return 0;
 }
 
 // ------------------------------------------------------------------------------------------------

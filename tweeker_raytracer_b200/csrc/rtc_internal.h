@@ -106,13 +106,17 @@ struct GasRecord
   uint32_t strideBytes = 0, numVerts = 0;
   double   buildMs = 0.0;
   int      builder = 0;                    // RTC_BUILD_HOST_SAH or RTC_BUILD_GPU_LBVH
-  uint64_t generation = 0;                 // rtc_gas_refit / rtc_gas_rebuild count: scenes built / updated at an older generation are stale
+  uint64_t generation = 0;                 // rtc_gas_refit / rtc_gas_rebuild / rtc_gas_build_device count: scenes built / updated at an older generation are stale
   RefitScratch refit;
   bool     boundsOnDevice = false;         // lo / hi are stale: the refitted or rebuilt bounds are refit.box[0..5] on the device
   // rtc_gas_rebuild (bvh_build_gas_rebuild_gpu.cu): its arrays, made by the first rebuild, and from then on the node count on the
-  // device -- numNodes is then only brought up to date by sync_gas_node_count (rtc_api.cpp)
+  // device -- numNodes is then only brought up to date by sync_gas_node_count (rtc_api.cpp) -- and the triangles the last build
+  // rejected (rtc_gas_rejected_triangles)
   LbvhRebuild* rebuild = nullptr;
   const uint32_t* d_numNodes = nullptr;
+  const uint32_t* d_rejected = nullptr;
+  // rtc_gas_create: the triangles its arrays hold (the most rtc_gas_build_device accepts); 0 for a GAS of rtc_gas_build
+  uint32_t capacity = 0;
 };
 
 struct SceneRecord
@@ -231,7 +235,7 @@ struct rtc_context
   void*  cutoutGraph = nullptr;                   // CutoutGraph (kernels_shade.cu): the device-side loop of the ordered any-hit rounds
   uint64_t cutoutGraphBuilds = 0;                 // graph pairs captured since the last rtc_stats_reset (rtc_stats)
   // The device GAS table, indexed by handle: the instance records of created scenes read it.  Kept up to date on the stream by
-  // rtc_gas_build, rtc_gas_refit, rtc_gas_rebuild and rtc_gas_destroy (a destroyed GAS has null nodes); grown from the pool.
+  // rtc_gas_build, rtc_gas_create, rtc_gas_build_device, rtc_gas_refit, rtc_gas_rebuild and rtc_gas_destroy (a destroyed GAS has null nodes); grown from the pool.
   struct GasUpdateInput* d_gasTable = nullptr;
   uint64_t* d_gasGen = nullptr;                   // per handle: GasRecord::generation
   uint32_t gasTableCapacity = 0;
@@ -265,7 +269,7 @@ struct GasUpdateInput
   float    gasLoHi[6];
   uint64_t attributes;             // rt_GeometryInstanceData::attributes
   uint32_t emptyGas, pad;
-  uint64_t indices;                // rt_GeometryInstanceData::indices (written by the builds of created scenes)
+  uint64_t indices;                // rt_GeometryInstanceData::indices
 };
 // d_instGasSlot of a created scene for a record rtc_ias_build_device rejected
 constexpr uint32_t kRejectedInstance = 0xffffffffu;
@@ -296,9 +300,12 @@ void free_refit_scratch(RefitScratch& r, cudaStream_t stream);
 int rebuild_instances_gpu(rtc_context* ctx, SceneRecord& s);
 // rtc_ias_create: the rebuild's arrays for `capacity` instances, set up at once (synchronises); the scene starts with no instance
 int create_instance_level_gpu(rtc_context* ctx, SceneRecord& s, uint32_t capacity);
-// bvh_build_gas_rebuild_gpu.cu: the same for a geometry, over the triangles of rec.attributes / rec.indices; writes the triangle
-// records in leaf order and the root box into rec.refit.box[0..5]
+// bvh_build_gas_rebuild_gpu.cu: the same for a geometry, over the rec.numTris triangles of rec.attributes / rec.indices (an index
+// >= rec.numVerts reads a NaN vertex); writes the triangle records in leaf order and the root box into rec.refit.box[0..5]
 int rebuild_gas_gpu(rtc_context* ctx, GasRecord& rec);
+// rtc_gas_create: the rebuild's arrays for `capacity` triangles (rec.d_tris already holds them), set up at once (synchronises);
+// the GAS starts with rec.numTris == 0
+int create_gas_gpu(rtc_context* ctx, GasRecord& rec, uint32_t capacity);
 // the wide nodes a rebuilt node array holds: every wide node but the root has a sibling-group parent, so one-primitive leaves give
 // < n + 16 (the same bound as build_gas_gpu's)
 inline uint32_t ias_rebuild_capacity(uint32_t numPrims) { return numPrims + 16u; }
