@@ -403,6 +403,36 @@ int rtc_trace_closest(rtc_context* ctx, uint64_t topObject, uint64_t rays, uint6
 int rtc_trace_any(rtc_context* ctx, uint64_t topObject, uint64_t rays, uint64_t numRays, uint64_t occluded);
 /* Same traversal as rtc_trace_closest (anyHit = 0) / rtc_trace_any (anyHit = 1) with work counters; synchronous. */
 int rtc_trace_count(rtc_context* ctx, uint64_t topObject, uint64_t rays, uint64_t numRays, int anyHit, rtc_trace_counts* out);
+/*
+ * Visibility masks and face culling of the ray queries (OptixInstance::visibilityMask, the visibilityMask argument of optixTrace,
+ * OPTIX_RAY_FLAG_CULL_{BACK,FRONT}_FACING_TRIANGLES).
+ *   - Instance masks are 8 bits; every instance starts at 0xFF.  rtc_scene_set_instance_masks sets masks[i] on instance
+ *     first + i, stream-ordered on the context stream like rtc_scene_set_instance_flags; `masks` may be reused on return.  In a
+ *     scene of rtc_ias_create the masks belong to positions up to the capacity and persist across rtc_ias_build_device, like
+ *     flags.  rtc_ias_update, rtc_ias_update_device and rtc_ias_rebuild never touch them.
+ *   - Mask test: a ray of mask m never enters an instance of mask k with (k & m) == 0, and nothing of that instance is hit.  In
+ *     the counters of rtc_trace_count_ex such an instance is not entered; the instance-level node visits that found it count.
+ *   - Facing is decided in the instance's object space: a hit is front-facing when dot((v1 - v0) x (v2 - v0), d) < 0, d the
+ *     object-space ray direction.  A mirrored instance (transform of negative determinant) therefore culls the opposite
+ *     world-space side.  A culled candidate is not a hit: the closest-hit query goes on to the next candidate, the any-hit query
+ *     does not stop.  Both flags together cull every triangle.
+ *   - rtc_trace_closest, rtc_trace_any and rtc_trace_count are the _ex calls with (0xFF, 0).
+ *   - Refused (synchronously, nothing enqueued): visibilityMask > 0xFF, unknown rayFlags bits, and what the plain calls refuse
+ *     (an unknown or unusable scene, more than 2^32 rays); for the setter an unknown scene, first + count out of range, or null
+ *     masks with count > 0.
+ *   - Rendering does not evaluate masks: while an instance mask of a scene is not 0xFF, rtc_launch / rtc_launch_ex on that scene
+ *     fail, and they work again once the masks are 0xFF.
+ * Detect the feature by these exports (rtc_version is unchanged).
+ */
+#define RTC_RAY_CULL_BACK_FACING   1u
+#define RTC_RAY_CULL_FRONT_FACING  2u
+int rtc_scene_set_instance_masks(rtc_context* ctx, uint64_t topObject, uint32_t first, uint32_t count, const uint8_t* masks);
+int rtc_trace_closest_ex(rtc_context* ctx, uint64_t topObject, uint64_t rays, uint64_t numRays, uint64_t hits,
+                         uint32_t visibilityMask, uint32_t rayFlags);
+int rtc_trace_any_ex(rtc_context* ctx, uint64_t topObject, uint64_t rays, uint64_t numRays, uint64_t occluded,
+                     uint32_t visibilityMask, uint32_t rayFlags);
+int rtc_trace_count_ex(rtc_context* ctx, uint64_t topObject, uint64_t rays, uint64_t numRays, int anyHit,
+                       uint32_t visibilityMask, uint32_t rayFlags, rtc_trace_counts* out);
 /* Primary rays of one iteration, one rtc_ray per launch index (skipped indices get tmax = -1). */
 int rtc_generate_primary(rtc_context* ctx, const rt_SystemData* sys, uint32_t launchWidth, uint32_t launchHeight,
                          int iteration, uint64_t rays);

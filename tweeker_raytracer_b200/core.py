@@ -39,6 +39,7 @@ SYMBOLS = [
     "rtc_gas_rebuild", "rtc_host_gas_rebuild",
     "rtc_ias_create", "rtc_ias_build_device", "rtc_scene_rejected_instances",
     "rtc_gas_create", "rtc_gas_build_device", "rtc_gas_rejected_triangles",
+    "rtc_scene_set_instance_masks", "rtc_trace_closest_ex", "rtc_trace_any_ex", "rtc_trace_count_ex",
 ]
 
 MATH_FUNCTIONS = ["sin", "cos", "atan", "atan2", "acos", "exp", "log", "pow", "div", "sqrt", "muladd"]     # enum rtc_math_fn
@@ -60,6 +61,7 @@ class TraceCounts(C.Structure):
 
 
 SCHEDULE_GROUP, SCHEDULE_ONE_TRI, SCHEDULE_TWO_TRI = 0, 1, 2
+RAY_CULL_BACK_FACING, RAY_CULL_FRONT_FACING = 1, 2      # rayFlags of rtc_trace_*_ex
 SCHEDULE_NAMES = ["group", "one_tri", "two_tri"]
 
 
@@ -135,6 +137,10 @@ def lib():
         L.rtc_trace_closest.argtypes = [C.c_void_p, C.c_uint64, C.c_uint64, C.c_uint64, C.c_uint64]
         L.rtc_trace_any.argtypes = [C.c_void_p, C.c_uint64, C.c_uint64, C.c_uint64, C.c_uint64]
         L.rtc_trace_count.argtypes = [C.c_void_p, C.c_uint64, C.c_uint64, C.c_uint64, C.c_int, C.POINTER(TraceCounts)]
+        L.rtc_scene_set_instance_masks.argtypes = [C.c_void_p, C.c_uint64, C.c_uint32, C.c_uint32, C.c_void_p]
+        L.rtc_trace_closest_ex.argtypes = [C.c_void_p, C.c_uint64, C.c_uint64, C.c_uint64, C.c_uint64, C.c_uint32, C.c_uint32]
+        L.rtc_trace_any_ex.argtypes = [C.c_void_p, C.c_uint64, C.c_uint64, C.c_uint64, C.c_uint64, C.c_uint32, C.c_uint32]
+        L.rtc_trace_count_ex.argtypes = [C.c_void_p, C.c_uint64, C.c_uint64, C.c_uint64, C.c_int, C.c_uint32, C.c_uint32, C.POINTER(TraceCounts)]
         L.rtc_generate_primary.argtypes = [C.c_void_p, C.c_void_p, C.c_uint32, C.c_uint32, C.c_int, C.c_uint64]
         L.rtc_composite.argtypes = [C.c_void_p, C.c_void_p]
         L.rtc_tonemap.argtypes = [C.c_void_p, C.c_void_p, C.c_uint64, C.c_uint64, C.c_uint64]
@@ -508,6 +514,11 @@ class Context:
         f = np.ascontiguousarray(flags, dtype=np.uint32)
         _check(self.L.rtc_scene_set_instance_flags(self.h, int(top), first, len(f), f.ctypes.data_as(C.c_void_p)))
 
+    def set_instance_masks(self, top, first, masks):
+        """8-bit visibility masks of instances first .. first + len(masks) - 1 (rtc_scene_set_instance_masks; 0xFF by default)."""
+        m = np.ascontiguousarray(masks, dtype=np.uint8)
+        _check(self.L.rtc_scene_set_instance_masks(self.h, int(top), first, len(m), m.ctypes.data_as(C.c_void_p)))
+
     def set_albedo_textures(self, top, enable):
         _check(self.L.rtc_scene_set_albedo_textures(self.h, int(top), 1 if enable else 0))
 
@@ -612,15 +623,25 @@ class Context:
         _check(self.L.rtc_profile_get(self.h, C.byref(p)))
         return {name: (p.ms[i], p.launches[i]) for i, name in enumerate(KERNEL_CLASSES)}
 
-    def trace_closest(self, top, d_rays, n, d_hits):
-        _check(self.L.rtc_trace_closest(self.h, int(top), int(d_rays), int(n), int(d_hits)))
+    # mask: the ray's visibility mask, flags: RAY_CULL_*; the _ex exports are called only when either is not the default
+    def trace_closest(self, top, d_rays, n, d_hits, mask=0xFF, flags=0):
+        if mask == 0xFF and flags == 0:
+            _check(self.L.rtc_trace_closest(self.h, int(top), int(d_rays), int(n), int(d_hits)))
+        else:
+            _check(self.L.rtc_trace_closest_ex(self.h, int(top), int(d_rays), int(n), int(d_hits), int(mask), int(flags)))
 
-    def trace_any(self, top, d_rays, n, d_occluded):
-        _check(self.L.rtc_trace_any(self.h, int(top), int(d_rays), int(n), int(d_occluded)))
+    def trace_any(self, top, d_rays, n, d_occluded, mask=0xFF, flags=0):
+        if mask == 0xFF and flags == 0:
+            _check(self.L.rtc_trace_any(self.h, int(top), int(d_rays), int(n), int(d_occluded)))
+        else:
+            _check(self.L.rtc_trace_any_ex(self.h, int(top), int(d_rays), int(n), int(d_occluded), int(mask), int(flags)))
 
-    def trace_count(self, top, d_rays, n, any_hit=False):
+    def trace_count(self, top, d_rays, n, any_hit=False, mask=0xFF, flags=0):
         out = TraceCounts()
-        _check(self.L.rtc_trace_count(self.h, int(top), int(d_rays), int(n), 1 if any_hit else 0, C.byref(out)))
+        if mask == 0xFF and flags == 0:
+            _check(self.L.rtc_trace_count(self.h, int(top), int(d_rays), int(n), 1 if any_hit else 0, C.byref(out)))
+        else:
+            _check(self.L.rtc_trace_count_ex(self.h, int(top), int(d_rays), int(n), 1 if any_hit else 0, int(mask), int(flags), C.byref(out)))
         return out
 
     def generate_primary(self, sys, launch_width, launch_height, iteration, d_rays):
@@ -641,23 +662,23 @@ class Context:
         _check(self.L.rtc_stats_reset(self.h))
 
     # convenience for host-resident ray sets
-    def trace_closest_host(self, top, rays):
+    def trace_closest_host(self, top, rays, mask=0xFF, flags=0):
         rays = np.ascontiguousarray(rays, dtype=RAY_DTYPE)
         d_r = self.to_device(rays)
         d_h = self.malloc(max(len(rays) * HIT_DTYPE.itemsize, 16))
         try:
-            self.trace_closest(top, d_r, len(rays), d_h)
+            self.trace_closest(top, d_r, len(rays), d_h, mask=mask, flags=flags)
             return self.download(d_h, HIT_DTYPE, len(rays))
         finally:
             self.free(d_r)
             self.free(d_h)
 
-    def trace_any_host(self, top, rays):
+    def trace_any_host(self, top, rays, mask=0xFF, flags=0):
         rays = np.ascontiguousarray(rays, dtype=RAY_DTYPE)
         d_r = self.to_device(rays)
         d_o = self.malloc(max(len(rays) * 4, 16))
         try:
-            self.trace_any(top, d_r, len(rays), d_o)
+            self.trace_any(top, d_r, len(rays), d_o, mask=mask, flags=flags)
             return self.download(d_o, np.uint32, len(rays))
         finally:
             self.free(d_r)

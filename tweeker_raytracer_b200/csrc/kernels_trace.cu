@@ -158,6 +158,35 @@ int launch_k_trace(rtc_context* ctx, const SceneDesc* scene, const Policy& p, ui
   return 0;
 }
 
+// The filtered traversal of rtc_trace_*_ex (trace.cuh FILTER): the mask and cull flags are a kernel parameter, the same for every
+// lane.  The query kernels only: rendering refuses scenes with masks.
+template <bool ANY, bool COUNT, class Policy, int TRICAP = 0>
+__global__ void __launch_bounds__(kTraceBlock, RTC_TRACE_MIN_BLOCKS)
+k_trace_filtered(const SceneDesc sc, const Policy policy, const TraceFilter filt, uint32_t n, uint32_t* __restrict__ cursor,
+                 unsigned long long* __restrict__ counts)
+{
+  __shared__ uint2 smem[RTC_SM_STACK * kTraceBlock + (RTC_SM_RAY_WORDS * kTraceBlock + 1) / 2];
+  trace_stream<ANY, COUNT, kTraceBlock, false, TRICAP, const Policy, true>(sc, n, cursor, policy, smem, counts, filt);
+}
+
+// the schedules of launch_k_trace: the counting kernels keep the one schedule
+template <bool ANY, bool COUNT, class Policy>
+int launch_k_trace_filtered(rtc_context* ctx, const SceneDesc* scene, const Policy& p, const TraceFilter& f, uint32_t n, unsigned long long* counts)
+{
+  const unsigned grid = ctx->numSMs * RTC_TRACE_MIN_BLOCKS;
+  if constexpr (COUNT)
+    k_trace_filtered<ANY, true, Policy><<<grid, kTraceBlock, 0, ctx->stream>>>(*scene, p, f, n, ctx->d_cursor, counts);
+  else if (ctx->traceSchedule == RTC_SCHEDULE_ONE_TRI)
+    k_trace_filtered<ANY, false, Policy, 1><<<grid, kTraceBlock, 0, ctx->stream>>>(*scene, p, f, n, ctx->d_cursor, counts);
+  else if (ctx->traceSchedule == RTC_SCHEDULE_TWO_TRI)
+    k_trace_filtered<ANY, false, Policy, 2><<<grid, kTraceBlock, 0, ctx->stream>>>(*scene, p, f, n, ctx->d_cursor, counts);
+  else
+    k_trace_filtered<ANY, false, Policy><<<grid, kTraceBlock, 0, ctx->stream>>>(*scene, p, f, n, ctx->d_cursor, counts);
+  ctx->kernelLaunches++;
+  RTC_CUDA(cudaGetLastError());
+  return 0;
+}
+
 } // namespace
 
 // With lazy module loading a kernel is loaded at its first launch; the schedule tuner must not time that.
@@ -197,6 +226,23 @@ int launch_trace_count(rtc_context* ctx, const SceneDesc* scene, const rtc_ray* 
   QueryCount p = { reinterpret_cast<const float4*>(rays) };
   if (anyHit) return launch_k_trace<true, true, QueryCount, false>(ctx, scene, p, (uint32_t)n, nullptr, ctx->d_cursor, d_counts);
   return launch_k_trace<false, true, QueryCount, false>(ctx, scene, p, (uint32_t)n, nullptr, ctx->d_cursor, d_counts);
+}
+
+int launch_trace_filtered(rtc_context* ctx, const SceneDesc* scene, const uint8_t* masks, uint32_t rayMask, uint32_t cullFlags, int query,
+                          const rtc_ray* rays, uint64_t n, void* out, unsigned long long* d_counts)
+{
+  if (n == 0) return 0;
+  if (n > 0xfffffff0ull) RTC_FAIL("more than 2^32 rays in one call");
+  RTC_CUDA(cudaMemsetAsync(ctx->d_cursor, 0, sizeof(uint32_t), ctx->stream));
+  const TraceFilter f = { masks, rayMask, cullFlags };
+  const float4* r = reinterpret_cast<const float4*>(rays);
+  switch (query)
+  {
+  case 0: { QueryClosest p = { r, static_cast<rtc_hit*>(out) }; return launch_k_trace_filtered<false, false, QueryClosest>(ctx, scene, p, f, (uint32_t)n, nullptr); }
+  case 1: { QueryAny p = { r, static_cast<uint32_t*>(out) }; return launch_k_trace_filtered<true, false, QueryAny>(ctx, scene, p, f, (uint32_t)n, nullptr); }
+  case 2: { QueryCount p = { r }; return launch_k_trace_filtered<false, true, QueryCount>(ctx, scene, p, f, (uint32_t)n, d_counts); }
+  default: { QueryCount p = { r }; return launch_k_trace_filtered<true, true, QueryCount>(ctx, scene, p, f, (uint32_t)n, d_counts); }
+  }
 }
 
 int launch_extend(rtc_context* ctx, const SceneDesc* scene, const WavefrontBuffers& wf, const uint32_t* queue, const uint32_t* count,

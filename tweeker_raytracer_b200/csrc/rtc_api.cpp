@@ -33,6 +33,7 @@ SceneRecord* find_scene(rtc_context* ctx, uint64_t topObject)
 void free_scene(SceneRecord* s, cudaStream_t stream)
 {
   cudaFree(s->d_desc); cudaFree(s->d_tlasNodes); cudaFree(s->d_instances); cudaFree(s->d_tlasLeaves); cudaFree(s->d_o2w); cudaFree(s->d_geomInst); cudaFree(s->d_instFlags);
+  cudaFree(s->d_instMasks);
   cudaFree(s->d_instBoxes); cudaFree(s->d_instGasSlot); free_refit_scratch(s->refit, stream); free_lbvh_rebuild(s->rebuild);
   cudaFree(s->d_instGen); cudaFree(s->d_words); cudaFree(s->d_emptyGas);
   if (s->d_gasRefs) cudaFreeAsync(s->d_gasRefs, stream);
@@ -152,6 +153,16 @@ void count_cutout(SceneRecord* s)
   s->numCutout = 0;
   for (uint32_t i = 0; i < s->desc.numInstances && i < s->instFlags.size(); ++i) if (s->instFlags[i] & RTC_INSTANCE_CUTOUT) s->numCutout++;
 }
+
+// the same for the visibility masks: instances whose mask is not 0xFF
+void count_masked(SceneRecord* s)
+{
+  s->numMasked = 0;
+  for (uint32_t i = 0; i < s->desc.numInstances && i < s->instMasks.size(); ++i) if (s->instMasks[i] != 0xFFu) s->numMasked++;
+}
+
+constexpr const char* kMaskedScene = "an instance mask of this scene is not 0xFF, and the renderer does not evaluate instance masks: "
+                                     "reset the masks with rtc_scene_set_instance_masks, or trace the scene with rtc_trace_*_ex";
 
 // rtc_ias_update and rtc_ias_update_device (arguments checked): instance first + i takes the matrix at transforms + i * strideBytes
 // (device-readable).  Recomputes exactly the instances of the range and those of every GAS refitted since the last build / update
@@ -649,6 +660,7 @@ int rtc_ias_build(rtc_context* ctx, const rtc_instance_desc* instances, uint32_t
   std::vector<uint32_t> slot(numInstances);
   for (uint32_t i = 0; i < numInstances; ++i) slot[i] = (uint32_t)std::distance(distinct.begin(), distinct.find(rec->instGas[i]));
   rec->instFlags.assign(numInstances, 0u);
+  rec->instMasks.assign(numInstances, 0xFFu);
 
   auto alloc = [](void** dst, size_t bytes) { return cudaMalloc(dst, bytes ? bytes : 16); };
   // stream-ordered: the kernels that write the instance records read what is staged here
@@ -662,6 +674,7 @@ int rtc_ias_build(rtc_context* ctx, const rtc_instance_desc* instances, uint32_t
   if (e == cudaSuccess) e = upload(&rec->d_o2w, o2w.data(), o2w.size() * sizeof(float4));
   if (e == cudaSuccess) e = upload(&rec->d_geomInst, gi.data(), gi.size() * sizeof(rt_GeometryInstanceData));
   if (e == cudaSuccess) e = upload(&rec->d_instFlags, rec->instFlags.data(), rec->instFlags.size() * 4u);
+  if (e == cudaSuccess) e = upload(&rec->d_instMasks, rec->instMasks.data(), rec->instMasks.size());
   if (e == cudaSuccess) e = alloc((void**)&rec->d_instBoxes, (size_t)numInstances * sizeof(PrimBox));
   if (e == cudaSuccess) e = upload((void**)&rec->d_instGasSlot, slot.data(), slot.size() * 4u);
   if (e != cudaSuccess) { free_scene(rec, ctx->stream); return rtc_set_error(__FILE__, __LINE__, "rtc_ias_build upload", (int)e, cudaGetErrorString(e)); }
@@ -784,6 +797,7 @@ int rtc_ias_create(rtc_context* ctx, uint32_t capacity, uint64_t* topObject)
   s->created = true;
   s->capacity = capacity;
   s->instFlags.assign(capacity, 0u);
+  s->instMasks.assign(capacity, 0xFFu);
   const size_t cap = capacity ? capacity : 1u;
   cudaError_t e = cudaSuccess;
   auto alloc = [&](void** dst, size_t bytes) { if (e == cudaSuccess) e = cudaMalloc(dst, bytes); };
@@ -793,6 +807,7 @@ int rtc_ias_create(rtc_context* ctx, uint32_t capacity, uint64_t* topObject)
   alloc(&s->d_o2w, cap * 3u * sizeof(float4));
   alloc(&s->d_geomInst, cap * sizeof(rt_GeometryInstanceData));
   alloc(&s->d_instFlags, cap * sizeof(uint32_t));
+  alloc(&s->d_instMasks, cap);
   alloc((void**)&s->d_instBoxes, cap * sizeof(PrimBox));
   alloc((void**)&s->d_instGasSlot, cap * sizeof(uint32_t));
   alloc((void**)&s->d_instGen, cap * sizeof(uint64_t));
@@ -801,6 +816,7 @@ int rtc_ias_create(rtc_context* ctx, uint32_t capacity, uint64_t* topObject)
   // the empty GAS of rejected records: every slot of its root empty (imask 0, meta 0)
   if (e == cudaSuccess) e = cudaMemsetAsync(s->d_emptyGas, 0, sizeof(Node8) + 3u * sizeof(float4), ctx->stream);
   if (e == cudaSuccess) e = cudaMemsetAsync(s->d_instFlags, 0, cap * sizeof(uint32_t), ctx->stream);
+  if (e == cudaSuccess) e = cudaMemsetAsync(s->d_instMasks, 0xFF, cap, ctx->stream);
   if (e == cudaSuccess) e = cudaMemsetAsync(s->d_words, 0, kSceneWords * sizeof(uint32_t), ctx->stream);
   if (e != cudaSuccess) { free_scene(s, ctx->stream); return rtc_set_error(__FILE__, __LINE__, "rtc_ias_create", (int)e, cudaGetErrorString(e)); }
   s->desc.instFlags = (const uint32_t*)s->d_instFlags;
@@ -852,6 +868,7 @@ int rtc_ias_build_device(rtc_context* ctx, uint64_t topObject, uint64_t instance
                                          instance_bounds_tight())) return rc;
   if (int rc = rebuild_instances_gpu(ctx, *s)) return rc;
   count_cutout(s);
+  count_masked(s);
   s->gasEpoch = ctx->gasEpoch;
   s->gasDestroyed = false;
   s->iasBuildMs = now_ms() - t0;
@@ -913,6 +930,22 @@ int rtc_scene_set_instance_flags(rtc_context* ctx, uint64_t topObject, uint32_t 
   count_cutout(s);
   // stream-ordered behind the launches already enqueued; `flags` may be reused by the caller at once (pageable source: staged copy)
   RTC_CUDA(cudaMemcpyAsync((uint32_t*)s->d_instFlags + first, &s->instFlags[first], (size_t)count * 4u, cudaMemcpyHostToDevice, ctx->stream));
+  return 0;
+}
+
+// Per-instance visibility masks (OptixInstance::visibilityMask); the rules of rtc_scene_set_instance_flags.
+int rtc_scene_set_instance_masks(rtc_context* ctx, uint64_t topObject, uint32_t first, uint32_t count, const uint8_t* masks)
+{
+  SceneRecord* s = find_scene(ctx, topObject);
+  if (!s) RTC_FAIL("unknown topObject");
+  if ((uint64_t)first + count > (s->created ? s->capacity : s->desc.numInstances)) RTC_FAIL("instance range out of bounds");
+  if (count == 0) return 0;
+  if (!masks) RTC_FAIL("masks is null");
+  RTC_CUDA(cudaSetDevice(ctx->device));
+  for (uint32_t i = 0; i < count; ++i) s->instMasks[first + i] = masks[i];
+  count_masked(s);
+  // stream-ordered behind the launches already enqueued, from the host copy (pageable: staged before cudaMemcpyAsync returns)
+  RTC_CUDA(cudaMemcpyAsync((uint8_t*)s->d_instMasks + first, &s->instMasks[first], count, cudaMemcpyHostToDevice, ctx->stream));
   return 0;
 }
 
@@ -1020,7 +1053,11 @@ int rtc_launch(rtc_context* ctx, const rt_SystemData* sys, uint32_t launchWidth,
   if (raygen != RTC_RAYGEN_FULL_FRAME && raygen != RTC_RAYGEN_LOCAL_COPY) RTC_FAIL("bad raygen selector");
   if (miss < RT_MISS_NULL || miss > RT_MISS_SPHERE) RTC_FAIL("bad miss selector");
   if (miss == RT_MISS_SPHERE && (sys->envTexture == 0 || sys->envCDF_U == 0 || sys->envCDF_V == 0)) RTC_FAIL("miss 2 needs envTexture/envCDF_U/envCDF_V");
-  if (const SceneRecord* s = find_scene(ctx, sys->topObject)) { if (const char* why = scene_unusable(ctx, s)) RTC_FAIL(why); }
+  if (const SceneRecord* s = find_scene(ctx, sys->topObject))
+  {
+    if (const char* why = scene_unusable(ctx, s)) RTC_FAIL(why);
+    if (s->numMasked) RTC_FAIL(kMaskedScene);
+  }
   RTC_CUDA(cudaSetDevice(ctx->device));
   return launch_wavefront(ctx, *sys, launchWidth, launchHeight, raygen, miss, iterationFirst, iterationCount, iterationFirst, false);
 }
@@ -1033,7 +1070,11 @@ int rtc_launch_ex(rtc_context* ctx, const rt_SystemData* sys, uint32_t launchWid
   if (miss < RT_MISS_NULL || miss > RT_MISS_SPHERE) RTC_FAIL("bad miss selector");
   if (miss == RT_MISS_SPHERE && (sys->envTexture == 0 || sys->envCDF_U == 0 || sys->envCDF_V == 0)) RTC_FAIL("miss 2 needs envTexture/envCDF_U/envCDF_V");
   if (accumulationFirst < 0) RTC_FAIL("accumulationFirst < 0");
-  if (const SceneRecord* s = find_scene(ctx, sys->topObject)) { if (const char* why = scene_unusable(ctx, s)) RTC_FAIL(why); }
+  if (const SceneRecord* s = find_scene(ctx, sys->topObject))
+  {
+    if (const char* why = scene_unusable(ctx, s)) RTC_FAIL(why);
+    if (s->numMasked) RTC_FAIL(kMaskedScene);
+  }
   RTC_CUDA(cudaSetDevice(ctx->device));
   return launch_wavefront(ctx, *sys, launchWidth, launchHeight, raygen, miss, iterationFirst, iterationCount, accumulationFirst, countWork != 0);
 }
@@ -1141,47 +1182,81 @@ int rtc_profile_get(rtc_context* ctx, rtc_profile* out)
   return 0;
 }
 
-int rtc_trace_closest(rtc_context* ctx, uint64_t topObject, uint64_t rays, uint64_t numRays, uint64_t hits)
+// The ray queries.  The plain kernels serve every call whose filter cannot reject anything: ray mask 0xFF, no cull flag and every
+// instance mask 0xFF (rtc_trace_closest / _any / _count on a scene without masks, which keep launching exactly what they did).
+// Otherwise the filtered kernels run.  query: 0 closest, 1 any.
+static int trace_query(rtc_context* ctx, uint64_t topObject, uint64_t rays, uint64_t numRays, uint64_t out, uint32_t visibilityMask,
+                       uint32_t rayFlags, int query)
 {
+  if (visibilityMask > 0xFFu) RTC_FAIL("visibilityMask has bits above 0xFF");
+  if (rayFlags & ~(RTC_RAY_CULL_BACK_FACING | RTC_RAY_CULL_FRONT_FACING)) RTC_FAIL("unknown rayFlags bits");
   SceneRecord* s = find_scene(ctx, topObject);
   if (!s) RTC_FAIL("unknown topObject");
   if (const char* why = scene_unusable(ctx, s)) RTC_FAIL(why);
+  if (numRays > 0xfffffff0ull) RTC_FAIL("more than 2^32 rays in one call");
   RTC_CUDA(cudaSetDevice(ctx->device));
+  const bool plain = visibilityMask == 0xFFu && rayFlags == 0u && s->numMasked == 0u;
   RTC_CUDA(cudaEventRecord(ctx->evA, ctx->stream));
-  if (int rc = launch_trace_closest(ctx, &s->desc, (const rtc_ray*)(uintptr_t)rays, numRays, (rtc_hit*)(uintptr_t)hits)) return rc;
+  int rc = 0;
+  if (plain && query == 0) rc = launch_trace_closest(ctx, &s->desc, (const rtc_ray*)(uintptr_t)rays, numRays, (rtc_hit*)(uintptr_t)out);
+  else if (plain)          rc = launch_trace_any(ctx, &s->desc, (const rtc_ray*)(uintptr_t)rays, numRays, (uint32_t*)(uintptr_t)out);
+  else rc = launch_trace_filtered(ctx, &s->desc, (const uint8_t*)s->d_instMasks, visibilityMask, rayFlags, query,
+                                  (const rtc_ray*)(uintptr_t)rays, numRays, (void*)(uintptr_t)out, nullptr);
+  if (rc) return rc;
   RTC_CUDA(cudaEventRecord(ctx->evB, ctx->stream));
   ctx->traceTimed = true;
   return 0;
+}
+
+int rtc_trace_closest(rtc_context* ctx, uint64_t topObject, uint64_t rays, uint64_t numRays, uint64_t hits)
+{
+  return trace_query(ctx, topObject, rays, numRays, hits, 0xFFu, 0u, 0);
 }
 
 int rtc_trace_any(rtc_context* ctx, uint64_t topObject, uint64_t rays, uint64_t numRays, uint64_t occluded)
 {
-  SceneRecord* s = find_scene(ctx, topObject);
-  if (!s) RTC_FAIL("unknown topObject");
-  if (const char* why = scene_unusable(ctx, s)) RTC_FAIL(why);
-  RTC_CUDA(cudaSetDevice(ctx->device));
-  RTC_CUDA(cudaEventRecord(ctx->evA, ctx->stream));
-  if (int rc = launch_trace_any(ctx, &s->desc, (const rtc_ray*)(uintptr_t)rays, numRays, (uint32_t*)(uintptr_t)occluded)) return rc;
-  RTC_CUDA(cudaEventRecord(ctx->evB, ctx->stream));
-  ctx->traceTimed = true;
-  return 0;
+  return trace_query(ctx, topObject, rays, numRays, occluded, 0xFFu, 0u, 1);
 }
 
-int rtc_trace_count(rtc_context* ctx, uint64_t topObject, uint64_t rays, uint64_t numRays, int anyHit, rtc_trace_counts* out)
+int rtc_trace_closest_ex(rtc_context* ctx, uint64_t topObject, uint64_t rays, uint64_t numRays, uint64_t hits,
+                         uint32_t visibilityMask, uint32_t rayFlags)
 {
+  return trace_query(ctx, topObject, rays, numRays, hits, visibilityMask, rayFlags, 0);
+}
+
+int rtc_trace_any_ex(rtc_context* ctx, uint64_t topObject, uint64_t rays, uint64_t numRays, uint64_t occluded,
+                     uint32_t visibilityMask, uint32_t rayFlags)
+{
+  return trace_query(ctx, topObject, rays, numRays, occluded, visibilityMask, rayFlags, 1);
+}
+
+int rtc_trace_count_ex(rtc_context* ctx, uint64_t topObject, uint64_t rays, uint64_t numRays, int anyHit,
+                       uint32_t visibilityMask, uint32_t rayFlags, rtc_trace_counts* out)
+{
+  if (visibilityMask > 0xFFu) RTC_FAIL("visibilityMask has bits above 0xFF");
+  if (rayFlags & ~(RTC_RAY_CULL_BACK_FACING | RTC_RAY_CULL_FRONT_FACING)) RTC_FAIL("unknown rayFlags bits");
   SceneRecord* s = find_scene(ctx, topObject);
   if (!s) RTC_FAIL("unknown topObject");
   if (!out) RTC_FAIL("out is null");
   if (const char* why = scene_unusable(ctx, s)) RTC_FAIL(why);
+  if (numRays > 0xfffffff0ull) RTC_FAIL("more than 2^32 rays in one call");
   RTC_CUDA(cudaSetDevice(ctx->device));
+  const bool plain = visibilityMask == 0xFFu && rayFlags == 0u && s->numMasked == 0u;
   unsigned long long* d = ctx->d_launchCounts + 2 * kTraceCountWords;
   RTC_CUDA(cudaMemsetAsync(d, 0, kTraceCountWords * sizeof(uint64_t), ctx->stream));
-  if (int rc = launch_trace_count(ctx, &s->desc, (const rtc_ray*)(uintptr_t)rays, numRays, anyHit, d)) return rc;
+  if (plain) { if (int rc = launch_trace_count(ctx, &s->desc, (const rtc_ray*)(uintptr_t)rays, numRays, anyHit, d)) return rc; }
+  else if (int rc = launch_trace_filtered(ctx, &s->desc, (const uint8_t*)s->d_instMasks, visibilityMask, rayFlags, anyHit ? 3 : 2,
+                                          (const rtc_ray*)(uintptr_t)rays, numRays, nullptr, d)) return rc;
   uint64_t h[4];
   RTC_CUDA(cudaMemcpyAsync(h, d, sizeof(h), cudaMemcpyDeviceToHost, ctx->stream));
   RTC_CUDA(cudaStreamSynchronize(ctx->stream));
   out->nodes = h[0]; out->tris = h[1]; out->instances = h[2]; out->rays = h[3];
   return 0;
+}
+
+int rtc_trace_count(rtc_context* ctx, uint64_t topObject, uint64_t rays, uint64_t numRays, int anyHit, rtc_trace_counts* out)
+{
+  return rtc_trace_count_ex(ctx, topObject, rays, numRays, anyHit, 0xFFu, 0u, out);
 }
 
 int rtc_generate_primary(rtc_context* ctx, const rt_SystemData* sys, uint32_t launchWidth, uint32_t launchHeight,

@@ -126,6 +126,11 @@ struct SceneRecord
   void *d_tlasNodes = nullptr, *d_instances = nullptr, *d_tlasLeaves = nullptr, *d_o2w = nullptr, *d_geomInst = nullptr, *d_instFlags = nullptr;
   std::vector<uint32_t> instFlags;         // host copy of the per-instance flags
   uint32_t numCutout = 0;                  // instances using the cutout hit records: > 0 selects the ordered any-hit path
+  // per-instance visibility masks (rtc_scene_set_instance_masks; uint8 per instance, 0xFF by default) and the instances whose mask
+  // is not 0xFF: > 0 sends every ray query to the filtered kernels and makes rtc_launch refuse the scene
+  void*    d_instMasks = nullptr;
+  std::vector<uint8_t> instMasks;
+  uint32_t numMasked = 0;
   bool     albedoTextures = false;         // MaterialDefinition.textureAlbedo may be non-zero: selects the textured shade kernels
   // The current object->world and world->object matrices live on the device only (d_o2w, d_instances): the instance records of
   // rtc_ias_build, rtc_ias_update and rtc_ias_update_device write them there, rtc_scene_export and rtc_instance_inverse read them back.
@@ -321,6 +326,10 @@ int launch_trace_closest(rtc_context* ctx, const SceneDesc* d_scene, const rtc_r
 int launch_trace_any(rtc_context* ctx, const SceneDesc* d_scene, const rtc_ray* rays, uint64_t n, uint32_t* occluded);
 // counting variant: adds {nodes popped, triangles tested, instances entered, rays} to d_counts[0..3]
 int launch_trace_count(rtc_context* ctx, const SceneDesc* d_scene, const rtc_ray* rays, uint64_t n, int anyHit, unsigned long long* d_counts);
+// the same three queries through the filtered traversal (rtc_trace_*_ex): instance masks (device, one byte per instance), the ray
+// mask and the RTC_RAY_CULL_* flags.  query: 0 closest (out = rtc_hit*), 1 any (out = uint32_t*), 2 / 3 counting closest / any
+int launch_trace_filtered(rtc_context* ctx, const SceneDesc* d_scene, const uint8_t* masks, uint32_t rayMask, uint32_t cullFlags, int query,
+                          const rtc_ray* rays, uint64_t n, void* out, unsigned long long* d_counts);
 // cursor: zero-initialised device counter the persistent warps hand rays out from (one per launch)
 int launch_extend(rtc_context* ctx, const SceneDesc* d_scene, const WavefrontBuffers& wf, const uint32_t* queue, const uint32_t* count,
                   uint32_t* cursor, bool countWork);

@@ -263,6 +263,15 @@ __device__ __forceinline__ uint32_t xor_permute8(uint32_t h, uint32_t x)
 // Per-ray work counters of the counting variant (the algorithmic-bytes figure of DESIGN.md section 5).
 struct TraceCounts { uint32_t nodes, tris, insts; };
 
+// Launch-uniform filter of the FILTER variant (rtc_trace_*_ex): a kernel parameter, read from the constant bank where it is
+// tested.  An instance whose mask shares no bit with rayMask is never entered; cullFlags (RTC_RAY_CULL_*) drop triangle
+// candidates by the sign of the watertight test's det, which is > 0 exactly for front-facing hits (DESIGN.md section 3).
+struct TraceFilter
+{
+  const uint8_t* masks;      // per instance
+  uint32_t rayMask, cullFlags;
+};
+
 #define RTC_SM_STACK 8        // traversal stack entries per thread kept in shared memory
 #if RTC_RESTORE_WORLD
 #define RTC_SM_RAY_WORDS 15   // float columns per thread behind the stack (Traversal::smRay)
@@ -287,7 +296,9 @@ __device__ unsigned int RTC_STACK_OVERFLOW_COUNTER = 0;
 // enumerate the candidates of a ray in that order.
 // TRICAP > 0 (rtc_context::traceSchedule, RTC_SCHEDULE_ONE_TRI / RTC_SCHEDULE_TWO_TRI): a step tests at most TRICAP triangles and a
 // lane with more pending skips its node visit until they are done; see step().  0: every triangle of the leaves a node visit found.
-template <bool ANY, bool COUNT, int BLOCK, bool SKIP = false, int TRICAP = RTC_ONE_TRI_PER_STEP>
+// FILTER = true (rtc_trace_*_ex): the TraceFilter passed to step() / leaf_phase() masks instances and culls triangles by facing;
+// with FILTER = false the filter argument is never read and the generated code is that of the plain traversal.
+template <bool ANY, bool COUNT, int BLOCK, bool SKIP = false, int TRICAP = RTC_ONE_TRI_PER_STEP, bool FILTER = false>
 struct Traversal
 {
   float skipT; uint32_t skipInst, skipPrim;       // SKIP only
@@ -398,7 +409,7 @@ struct Traversal
   }
 
   // returns false when the ray is finished (ANY: first hit)
-  __device__ __forceinline__ bool leaf_phase(const SceneDesc& sc)
+  __device__ __forceinline__ bool leaf_phase(const SceneDesc& sc, const TraceFilter& filt = TraceFilter())
   {
     int tested = 0;      // TRICAP > 1 only
     while (triGroup.y)
@@ -409,6 +420,7 @@ struct Traversal
       {
         // instance-level leaf: enter the instance
         const uint32_t inst = __ldg(sc.tlasLeaves + triGroup.x + idx);
+        if (FILTER && !(__ldg(filt.masks + inst) & filt.rayMask)) continue;      // masked out: not entered, next leaf bit
         if (triGroup.y) push(triGroup);
         if (nodeGroup.y & 0xff000000u) push(nodeGroup);
         const float4* ip = sc.instances + (size_t)inst * 4u;
@@ -439,7 +451,9 @@ struct Traversal
         const float4 v0 = __ldg(tp), v1 = __ldg(tp + 1), v2 = __ldg(tp + 2);
         if (COUNT) counts.tris++;
         float t, det, V, W;
-        if (tri_test(orr, br.ox, br.oy, br.oz, v0, v1, v2, t, det, V, W) && t > tmin)
+        // FILTER: det > 0 is a front-facing candidate; a culled one is not a hit (and still counts towards TRICAP)
+        if (tri_test(orr, br.ox, br.oy, br.oz, v0, v1, v2, t, det, V, W) &&
+            (!FILTER || !(filt.cullFlags & (det > 0.0f ? RTC_RAY_CULL_FRONT_FACING : RTC_RAY_CULL_BACK_FACING))) && t > tmin)
         {
           const uint32_t prim = __float_as_uint(v0.w);
           if (SKIP && !(t > skipT || (t == skipT && (curInst > skipInst || (curInst == skipInst && prim > skipPrim))))) continue;
@@ -488,7 +502,7 @@ struct Traversal
   }
 
   // returns true while the ray needs more steps
-  __device__ __forceinline__ bool step(const SceneDesc& sc)
+  __device__ __forceinline__ bool step(const SceneDesc& sc, const TraceFilter& filt = TraceFilter())
   {
     if (TRICAP > 0)
     {
@@ -501,12 +515,12 @@ struct Traversal
       // Built after the last GPU session of round 2 and therefore never enabled blindly: the library times one batch with each
       // schedule and keeps a capped one only where it is faster (kernels_shade.cu, "schedule tuner").
       if (!(blasBase >= 0 && has_leaves())) node_phase();
-      if (!leaf_phase(sc)) return false;
+      if (!leaf_phase(sc, filt)) return false;
       if (blasBase >= 0 && has_leaves()) return true;
       return advance(sc);
     }
     node_phase();
-    if (!leaf_phase(sc)) return false;
+    if (!leaf_phase(sc, filt)) return false;
     return advance(sc);
   }
 };
@@ -515,11 +529,12 @@ struct Traversal
 // global cursor (one atomicAdd per warp and refill), so short rays do not leave their lanes idle while the longest ray of
 // the warp finishes.  Policy (stateless) supplies load(i, org, dir, tag) -> bool (false: skip this
 // index; tag = the policy's per-ray word, e.g. the path id), store(tag, hit) and, for SKIP kernels, skip_key(tag, t, inst, prim).
-template <bool ANY, bool COUNT, int BLOCK, bool SKIP, int TRICAP = RTC_ONE_TRI_PER_STEP, class Policy>
+// FILTER: the traversal reads `filt` (a kernel parameter of the caller); otherwise it is never read.
+template <bool ANY, bool COUNT, int BLOCK, bool SKIP, int TRICAP = RTC_ONE_TRI_PER_STEP, class Policy, bool FILTER = false>
 __device__ __forceinline__ void trace_stream(const SceneDesc& sc, uint32_t n, uint32_t* __restrict__ cursor, Policy& policy, uint2* smem,
-                                             unsigned long long* __restrict__ countsOut)
+                                             unsigned long long* __restrict__ countsOut, const TraceFilter& filt = TraceFilter())
 {
-  Traversal<ANY, COUNT, BLOCK, SKIP, TRICAP> tr;
+  Traversal<ANY, COUNT, BLOCK, SKIP, TRICAP, FILTER> tr;
   uint2 overflow[RTC_LM_STACK];
   tr.smStack = smem + threadIdx.x;
   tr.smRay = reinterpret_cast<float*>(smem + RTC_SM_STACK * BLOCK) + threadIdx.x;
@@ -570,7 +585,7 @@ __device__ __forceinline__ void trace_stream(const SceneDesc& sc, uint32_t n, ui
       const uint32_t nHeld = (uint32_t)__popc(heldLanes), nActive = (uint32_t)__popc(activeLanes);
       if (nHeld >= RTC_LEAF_THRESHOLD || nHeld * 4u >= nActive)
       {
-        if (held) running = tr.leaf_phase(sc);
+        if (held) running = tr.leaf_phase(sc, filt);
       }
     }
     if (running && !tr.has_leaves()) running = tr.advance(sc);
@@ -583,7 +598,7 @@ __device__ __forceinline__ void trace_stream(const SceneDesc& sc, uint32_t n, ui
 #else
     if (active)
     {
-      if (!tr.step(sc))
+      if (!tr.step(sc, filt))
       {
         policy.store(tag, tr.result());
         if (COUNT) { cNodes += tr.counts.nodes; cTris += tr.counts.tris; cInsts += tr.counts.insts; cRays++; }
