@@ -14,6 +14,7 @@
 // the primary-ray extend kernel generates its rays with the shading arithmetic of this translation unit (see ExtendPrimary)
 #define RTC_STACK_OVERFLOW_COUNTER g_rtcStackOverflowsPrimary
 #include "trace.cuh"
+#include "primary_lists.cuh"
 #include "schedule_tuner.h"
 
 #include <cstdlib>
@@ -25,8 +26,9 @@ constexpr int kBlock = 256;
 constexpr uint32_t kNoPixel = 0xffffffffu;
 constexpr uint32_t kDeadPath = 0xfffffffeu;           // hitInst of a launch index that falls outside the image (fused primary path)
 // device counters of one batch: [0..63] extend counts per depth, [64..127] shadow counts, [128..191] extend cursors,
-// [192..255] connect cursors, [256 + 8 d + c] paths of shade class c at depth d
-constexpr uint32_t kNumCounters = 256 + 64 * 8;
+// [192..255] connect cursors, [256 + 8 d + c] paths of shade class c at depth d, [kOverflowTiles] tiles whose list overflowed
+constexpr uint32_t kOverflowTiles = 256 + 64 * 8;
+constexpr uint32_t kNumCounters = kOverflowTiles + 1;
 constexpr uint32_t kPendingRR = 0x80000000u;          // misc.y bit: Russian roulette postponed until the shadow ray is resolved
 constexpr uint32_t kDepthMask = 0x0000ffffu;
 constexpr uint64_t kMaxPathsInFlight = 64ull << 20;   // 64 Mi paths x 320 B of wavefront state = 21 GB of the 180 GB HBM
@@ -202,23 +204,25 @@ k_generate(const __grid_constant__ WfArgs a, uint32_t* __restrict__ queue, uint3
 struct ExtendPrimary
 {
   WfArgs a;
-  __device__ __forceinline__ bool load(uint32_t i, float4& o, float4& d, uint32_t& path) const
+  // the primary ray of `path`; false (and hitInst = kDeadPath) for a launch index outside the image
+  __device__ __forceinline__ bool load_path(uint32_t path, float4& o, float4& d) const
   {
-    path = i;
     const uint32_t pixelsPerIter = a.launchWidth * a.launchHeight;
-    const uint32_t it = i / pixelsPerIter, idx = i - it * pixelsPerIter;
+    const uint32_t it = path / pixelsPerIter, idx = path - it * pixelsPerIter;
     uint32_t x, y;
     launch_xy(idx, a.launchWidth, a.launchHeight, x, y);
     uint32_t seed = 0, col = 0; float3 pos, wi;
     if (!start_path(a.sys, a.launchWidth, x, y, a.iterFirst + (int)it, seed, pos, wi, col))
     {
-      a.wf.hitInst[i] = kDeadPath;
+      a.wf.hitInst[path] = kDeadPath;
       return false;
     }
     o = make_float4(pos.x, pos.y, pos.z, a.sys.sceneEpsilon);
     d = make_float4(wi.x, wi.y, wi.z, RT_DEFAULT_MAX);
     return true;
   }
+  __device__ __forceinline__ uint32_t count(uint32_t n) const { return n; }
+  __device__ __forceinline__ bool load(uint32_t i, float4& o, float4& d, uint32_t& path) const { path = i; return load_path(i, o, d); }
   __device__ __forceinline__ void store(uint32_t path, const TraceHit& h) const
   {
     __stcs(a.wf.hit + path, make_float4(h.t, h.u, h.v, __uint_as_float(h.prim)));
@@ -226,14 +230,67 @@ struct ExtendPrimary
   }
 };
 
+// The paths of the tiles whose candidate list overflowed (tile lists, primary_lists.cuh): ray i is lane i % 32 of warp-sized
+// group i / 32, and the groups run through the batch's iterations of one listed tile before the next tile.
+struct ExtendPrimaryTiles : ExtendPrimary
+{
+  const uint32_t* tiles; const uint32_t* numTiles;
+  __device__ __forceinline__ uint32_t count(uint32_t) const { return *numTiles * 32u * (uint32_t)a.iterCount; }
+  __device__ __forceinline__ bool load(uint32_t i, float4& o, float4& d, uint32_t& path) const
+  {
+    const uint32_t group = i >> 5, slot = group / (uint32_t)a.iterCount, it = group - slot * (uint32_t)a.iterCount;
+    path = it * (a.launchWidth * a.launchHeight) + tiles[slot] * 32u + (i & 31u);
+    return load_path(path, o, d);
+  }
+};
+
 constexpr int kPrimaryBlock = 128;
 
-template <bool COUNT, int TRICAP = 0>
+template <bool COUNT, int TRICAP = 0, class Policy = ExtendPrimary>
 __global__ void __launch_bounds__(kPrimaryBlock, RTC_TRACE_MIN_BLOCKS)
-k_extend_primary(const SceneDesc sc, const ExtendPrimary policy, uint32_t n, uint32_t* __restrict__ cursor, unsigned long long* __restrict__ counts)
+k_extend_primary(const SceneDesc sc, const Policy policy, uint32_t n, uint32_t* __restrict__ cursor, unsigned long long* __restrict__ counts)
 {
   __shared__ uint2 smem[RTC_SM_STACK * kPrimaryBlock + (RTC_SM_RAY_WORDS * kPrimaryBlock + 1) / 2];
-  trace_stream<false, COUNT, kPrimaryBlock, false, TRICAP>(sc, n, cursor, policy, smem, counts);
+  trace_stream<false, COUNT, kPrimaryBlock, false, TRICAP>(sc, policy.count(n), cursor, policy, smem, counts);
+}
+
+// ---- tile lists of a pinhole launch (primary_lists.cuh) --------------------------------------------------------------------
+// One thread per 8x4 tile: the tile's candidate list from the camera on the device (so a camera uploaded on the stream is
+// seen), its count, and the overflowed tiles appended to `overflow`.
+constexpr int kListBlock = 128;
+constexpr uint64_t kMinListTiles = 1u << 15;          // launches with fewer tiles, and scenes with more instances, keep the traversal
+constexpr uint32_t kMaxListInstances = 1024;
+
+__global__ void __launch_bounds__(kListBlock, 1)
+k_build_tile_lists(const __grid_constant__ WfArgs a, const SceneDesc sc, uint2* __restrict__ lists, uint32_t* __restrict__ counts,
+                   uint32_t* __restrict__ overflow, uint32_t* __restrict__ numOverflow)
+{
+  const uint32_t tilesPerRow = a.launchWidth >> 3, tiles = tilesPerRow * (a.launchHeight >> 2);
+  const uint32_t tile = blockIdx.x * blockDim.x + threadIdx.x;
+  if (tile >= tiles) return;
+  const uint32_t ty = tile / tilesPerRow, tx = tile - ty * tilesPerRow;
+  float P[3], n[4][3], c[3];
+  const uint32_t count = tile_planes(a.sys, tx << 3, ty << 2, P, n, c) ? build_tile_list(sc, P, n, c, lists + (size_t)tile * kTileListK) : kTileOverflow;
+  counts[tile] = count;
+  if (count == kTileOverflow) overflow[atomicAdd(numOverflow, 1u)] = tile;
+}
+
+// The list pass: one warp per (tile, iteration), the iterations of a tile on consecutive warps.  A listed tile's 32 paths get
+// their closest hit from trace_tile_list, stored as ExtendPrimary::store does; an overflowed tile is left to k_extend_primary.
+__global__ void __launch_bounds__(kListBlock)
+k_extend_listed(const __grid_constant__ WfArgs a, const SceneDesc sc, const uint2* __restrict__ lists, const uint32_t* __restrict__ counts)
+{
+  const uint32_t tiles = (a.launchWidth >> 3) * (a.launchHeight >> 2);
+  const uint32_t group = (blockIdx.x * blockDim.x + threadIdx.x) >> 5;
+  if (group >= tiles * (uint32_t)a.iterCount) return;
+  const uint32_t tile = group / (uint32_t)a.iterCount, it = group - tile * (uint32_t)a.iterCount;
+  const uint32_t count = counts[tile];
+  if (count == kTileOverflow) return;
+  const ExtendPrimary p = { a };
+  const uint32_t path = it * (a.launchWidth * a.launchHeight) + tile * 32u + (threadIdx.x & 31u);
+  float4 o, d;
+  if (!p.load_path(path, o, d)) return;
+  p.store(path, trace_tile_list(sc, lists + (size_t)tile * kTileListK, count, o, d));
 }
 
 __device__ __forceinline__ float3 xf_vector(const float4 r0, const float4 r1, const float4 r2, float3 v)
@@ -859,6 +916,7 @@ int ensure_wavefront(rtc_context* ctx, uint64_t capacity, bool* outOfMemory)
     release_cutout_graph(ctx);
     RTC_CUDA(cudaFree(wf.base));
     if (wf.cutBase) RTC_CUDA(cudaFree(wf.cutBase));
+    if (wf.tileBase) RTC_CUDA(cudaFree(wf.tileBase));
     wf = WavefrontBuffers();
   }
   // one allocation, carved into 256-byte aligned SoA arrays
@@ -980,6 +1038,25 @@ int ensure_cutout_buffers(rtc_context* ctx, uint64_t capacity)
   char* b = static_cast<char*>(base);
   wf.cutBase = base; wf.cutCapacity = capacity;
   wf.cutQueue[0] = (uint32_t*)b; wf.cutQueue[1] = (uint32_t*)(b + q); wf.cutCounters = (uint32_t*)(b + 2 * q);
+  return 0;
+}
+
+// the tile lists of a launch of `tiles` 8x4 tiles (WavefrontBuffers::tileLists)
+int ensure_tile_lists(rtc_context* ctx, uint64_t tiles)
+{
+  WavefrontBuffers& wf = ctx->wf;
+  if (wf.tileCapacity >= tiles) return 0;
+  if (wf.tileBase)
+  {
+    RTC_CUDA(cudaStreamSynchronize(ctx->stream));
+    RTC_CUDA(cudaFree(wf.tileBase)); wf.tileBase = nullptr; wf.tileCapacity = 0;
+  }
+  const uint64_t lists = (8 * kTileListK * tiles + 255u) & ~(uint64_t)255u, words = (4 * tiles + 255u) & ~(uint64_t)255u;
+  void* base = nullptr;
+  RTC_CUDA(cudaMalloc(&base, lists + 2 * words));
+  char* b = static_cast<char*>(base);
+  wf.tileBase = base; wf.tileCapacity = tiles;
+  wf.tileLists = (uint2*)b; wf.tileCounts = (uint32_t*)(b + lists); wf.overflowTiles = (uint32_t*)(b + lists + words);
   return 0;
 }
 
@@ -1156,6 +1233,8 @@ void preload_capped_kernels()
   cudaFuncAttributes attr;
   cudaFuncGetAttributes(&attr, k_extend_primary<false, 1>);
   cudaFuncGetAttributes(&attr, k_extend_primary<false, 2>);
+  cudaFuncGetAttributes(&attr, k_extend_primary<false, 1, ExtendPrimaryTiles>);
+  cudaFuncGetAttributes(&attr, k_extend_primary<false, 2, ExtendPrimaryTiles>);
   preload_capped_trace_kernels();
   cudaGetLastError();
 }
@@ -1198,6 +1277,14 @@ int launch_wavefront(rtc_context* ctx, const rt_SystemData& sys, uint32_t w, uin
   const bool cutout = scene->numCutout > 0;
   const bool tex = cutout || scene->albedoTextures;
   if (cutout) { if (int rc = ensure_cutout_buffers(ctx, pixels * perBatch)) return rc; }
+  // Tile lists for the depth-0 extend (primary_lists.cuh): the pinhole lens (every primary ray of a tile starts at cam.P and
+  // points into the tile's pixel rectangle), a launch that tiles, no tile distribution over devices.  The counting launch keeps
+  // the traversal: its per-ray work counters are what it measures.  Measured on a B200 (DESIGN.md section 3), the lists lose
+  // below about a megapixel (the Cornell box at 512x512, 8 192 tiles: -0.4 %) and with thousands of instances (10 000 instances:
+  // -0.9 %, most tiles overflow): there the build and the two extra launches cost more than the lists save.
+  const bool listed = !tex && 0 < maxDepth && !countWork && sys.lensShader == RT_LENS_PINHOLE && ((w & 7u) | (h & 3u)) == 0u &&
+                      !(sys.distribution && 1 < sys.deviceCount) && pixels / 32u >= kMinListTiles && scene->desc.numInstances <= kMaxListInstances;
+  if (listed) { if (int rc = ensure_tile_lists(ctx, pixels / 32u)) return rc; }
 
   const int gridShade = ctx->numSMs * 16;     // swept (tools/sweep_shade_block.sh): 8 -> 16 CTAs of 256 per SM in the grid, +0.8 %; the CTA size itself is flat from 128 to 512
   for (int done = 0; done < iterCount; done += (int)perBatch)
@@ -1224,7 +1311,27 @@ int launch_wavefront(rtc_context* ctx, const rt_SystemData& sys, uint32_t w, uin
     for (int d = 0; d < maxDepth; ++d)
     {
       const bool primary = fused && d == 0;
-      if (primary)
+      if (primary && listed)
+      {
+        // tile lists: build, list pass over the listed tiles, the traversal over the overflowed ones (primary_lists.cuh)
+        if (int rc = profile_begin(ctx, RTC_KERNEL_EXTEND)) return rc;
+        const uint32_t tiles = (uint32_t)(pixels / 32u);
+        const WavefrontBuffers& wf = ctx->wf;
+        k_build_tile_lists<<<(tiles + kListBlock - 1) / kListBlock, kListBlock, 0, ctx->stream>>>(a, scene->desc, wf.tileLists, wf.tileCounts,
+                                                                                                   wf.overflowTiles, cnt + kOverflowTiles);
+        const uint64_t listThreads = (uint64_t)tiles * (uint64_t)batch * 32u;
+        k_extend_listed<<<(unsigned)((listThreads + kListBlock - 1) / kListBlock), kListBlock, 0, ctx->stream>>>(a, scene->desc, wf.tileLists, wf.tileCounts);
+        ExtendPrimaryTiles policy;
+        policy.a = a; policy.tiles = wf.overflowTiles; policy.numTiles = cnt + kOverflowTiles;
+        const int gridTrace = ctx->numSMs * RTC_TRACE_MIN_BLOCKS;
+        if (ctx->traceSchedule == RTC_SCHEDULE_ONE_TRI) k_extend_primary<false, 1, ExtendPrimaryTiles><<<gridTrace, kPrimaryBlock, 0, ctx->stream>>>(scene->desc, policy, 0u, cnt + 128, nullptr);
+        else if (ctx->traceSchedule == RTC_SCHEDULE_TWO_TRI) k_extend_primary<false, 2, ExtendPrimaryTiles><<<gridTrace, kPrimaryBlock, 0, ctx->stream>>>(scene->desc, policy, 0u, cnt + 128, nullptr);
+        else           k_extend_primary<false, 0, ExtendPrimaryTiles><<<gridTrace, kPrimaryBlock, 0, ctx->stream>>>(scene->desc, policy, 0u, cnt + 128, nullptr);
+        ctx->kernelLaunches += 3;
+        RTC_CUDA(cudaGetLastError());
+        if (int rc = profile_end(ctx)) return rc;
+      }
+      else if (primary)
       {
         if (int rc = profile_begin(ctx, RTC_KERNEL_EXTEND)) return rc;
         ExtendPrimary policy = { a };

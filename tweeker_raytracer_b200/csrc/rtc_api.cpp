@@ -322,6 +322,7 @@ int rtc_context_destroy(rtc_context* ctx)
   for (GasRecord& g : ctx->gas) { cudaFree(g.d_nodes); cudaFree(g.d_tris); free_refit_scratch(g.refit, ctx->stream); free_lbvh_rebuild(g.rebuild); }
   if (ctx->wf.base) cudaFree(ctx->wf.base);
   if (ctx->wf.cutBase) cudaFree(ctx->wf.cutBase);
+  if (ctx->wf.tileBase) cudaFree(ctx->wf.tileBase);
   for (void* t : ctx->textures) cudaFree(t);
   cudaFree(ctx->d_gasTable);
   cudaFree(ctx->d_gasGen);

@@ -185,6 +185,12 @@ struct WavefrontBuffers
   uint32_t *cutCounters = nullptr;
   uint64_t cutCapacity = 0;
   void* cutBase = nullptr;
+  // candidate lists of the primary rays of a pinhole launch (primary_lists.cuh), per 8x4 tile: the list, its count, and the
+  // tiles whose list overflowed; sized by the tile count, allocated on first use
+  uint2* tileLists = nullptr;
+  uint32_t *tileCounts = nullptr, *overflowTiles = nullptr;
+  uint64_t tileCapacity = 0;
+  void* tileBase = nullptr;
 };
 
 // RTC_SCHEDULE_GROUP / RTC_SCHEDULE_ONE_TRI / RTC_SCHEDULE_TWO_TRI (rtc_core.h): how the lane-owned traversal driver times its triangle tests

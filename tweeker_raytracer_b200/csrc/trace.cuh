@@ -120,6 +120,29 @@ __device__ __forceinline__ bool tri_test(const ObjRay& r, float ox, float oy, fl
   return true;
 }
 
+// Instance entry: the world ray (wo, wd) in the instance's object space through its world->object rows r0..r2, and the shear
+// constants of the watertight test.  (oox, ooy, ooz) is the origin tri_test takes.  The traversal and the primary-ray list pass
+// (primary_lists.cuh) both call this, so their object-space rays agree to the bit.
+__device__ __forceinline__ void enter_instance(const float4 r0, const float4 r1, const float4 r2, float wox, float woy, float woz,
+                                               float wdx, float wdy, float wdz, ObjRay& orr, float& oox, float& ooy, float& ooz)
+{
+  oox = __fmaf_rn(r0.x, wox, __fmaf_rn(r0.y, woy, __fmaf_rn(r0.z, woz, r0.w)));
+  ooy = __fmaf_rn(r1.x, wox, __fmaf_rn(r1.y, woy, __fmaf_rn(r1.z, woz, r1.w)));
+  ooz = __fmaf_rn(r2.x, wox, __fmaf_rn(r2.y, woy, __fmaf_rn(r2.z, woz, r2.w)));
+  orr.dx = __fmaf_rn(r0.x, wdx, __fmaf_rn(r0.y, wdy, __fmul_rn(r0.z, wdz)));
+  orr.dy = __fmaf_rn(r1.x, wdx, __fmaf_rn(r1.y, wdy, __fmul_rn(r1.z, wdz)));
+  orr.dz = __fmaf_rn(r2.x, wdx, __fmaf_rn(r2.y, wdy, __fmul_rn(r2.z, wdz)));
+  shear_setup(orr);
+}
+
+// The closest-hit order: a candidate (t, inst, prim) that passed tri_test and t > tmin replaces the best hit so far when it is
+// smaller in (t, instance, primitive); the first one when t < tlimit.  hitInst == 0xffffffff: nothing found yet.  A total order,
+// so the result does not depend on the order in which candidates are tested.
+__device__ __forceinline__ bool closer_hit(float t, uint32_t inst, uint32_t prim, float hitT, uint32_t hitInst, uint32_t hitPrim, float tlimit)
+{
+  return hitInst != 0xffffffffu ? (t < hitT || (t == hitT && (inst < hitInst || (inst == hitInst && prim < hitPrim)))) : (t < tlimit);
+}
+
 // Per-space constants of the box test.
 struct BoxRay
 {
@@ -140,7 +163,8 @@ __device__ __forceinline__ float fast_rcp(float d)
   float r;
   asm("rcp.approx.ftz.f32 %0, %1;" : "=f"(r) : "f"(d));
   return r;
-#else      // host build: rcp.approx has no portable definition; the host harness only instantiates EXACT = true
+#else      // host build: rcp.approx has no portable definition, so the IEEE reciprocal stands in (the traversal's host harness
+          // instantiates EXACT = true; the tile frustum of primary_lists.cuh, which only has to be conservative, takes EXACT = false)
   return 1.0f / d;
 #endif
 }
@@ -426,15 +450,9 @@ struct Traversal
         const float4* ip = sc.instances + (size_t)inst * 4u;
         const float4 r0 = __ldg(ip), r1 = __ldg(ip + 1), r2 = __ldg(ip + 2), r3 = __ldg(ip + 3);
         if (COUNT) counts.insts++;
-        const float wox = smRay[0], woy = smRay[BLOCK], woz = smRay[2 * BLOCK];
-        const float wdx = smRay[3 * BLOCK], wdy = smRay[4 * BLOCK], wdz = smRay[5 * BLOCK];
-        const float oox = __fmaf_rn(r0.x, wox, __fmaf_rn(r0.y, woy, __fmaf_rn(r0.z, woz, r0.w)));
-        const float ooy = __fmaf_rn(r1.x, wox, __fmaf_rn(r1.y, woy, __fmaf_rn(r1.z, woz, r1.w)));
-        const float ooz = __fmaf_rn(r2.x, wox, __fmaf_rn(r2.y, woy, __fmaf_rn(r2.z, woz, r2.w)));
-        orr.dx = __fmaf_rn(r0.x, wdx, __fmaf_rn(r0.y, wdy, __fmul_rn(r0.z, wdz)));
-        orr.dy = __fmaf_rn(r1.x, wdx, __fmaf_rn(r1.y, wdy, __fmul_rn(r1.z, wdz)));
-        orr.dz = __fmaf_rn(r2.x, wdx, __fmaf_rn(r2.y, wdy, __fmul_rn(r2.z, wdz)));
-        shear_setup(orr);
+        float oox, ooy, ooz;
+        enter_instance(r0, r1, r2, smRay[0], smRay[BLOCK], smRay[2 * BLOCK], smRay[3 * BLOCK], smRay[4 * BLOCK], smRay[5 * BLOCK],
+                       orr, oox, ooy, ooz);
         box_setup<COUNT>(br, oox, ooy, ooz, orr.dx, orr.dy, orr.dz);
         curInst = inst;
         blasBase = sp;
@@ -463,9 +481,7 @@ struct Traversal
           }
           else
           {
-            const bool better = found() ? (t < hitT || (t == hitT && (curInst < hitInst || (curInst == hitInst && prim < hitPrim))))
-                                      : (t < tlimit);
-            if (better)
+            if (closer_hit(t, curInst, prim, hitT, hitInst, hitPrim, tlimit))
             {
               tlimit = t;
               hitT = t; hitInst = curInst; hitPrim = prim;
