@@ -398,7 +398,9 @@ typedef struct {
 int rtc_profile_enable(rtc_context* ctx, int enable);          /* enabling resets the accumulated profile */
 int rtc_profile_get(rtc_context* ctx, rtc_profile* out);        /* synchronises the stream */
 
-/* Ray queries against a built scene; rays/hits/occluded are device pointers.  occluded: one uint32 per ray. */
+/* Ray queries against a built scene; rays/hits/occluded are device pointers.  occluded: one uint32 per ray.
+ * The same queries from the caller's own CUDA kernels, one ray per call with its own mask and flags: include/rtc_device.cuh
+ * (rtc_device_trace_closest / rtc_device_trace_any on topObject), whose comment is their contract. */
 int rtc_trace_closest(rtc_context* ctx, uint64_t topObject, uint64_t rays, uint64_t numRays, uint64_t hits);
 int rtc_trace_any(rtc_context* ctx, uint64_t topObject, uint64_t rays, uint64_t numRays, uint64_t occluded);
 /* Same traversal as rtc_trace_closest (anyHit = 0) / rtc_trace_any (anyHit = 1) with work counters; synchronous. */

@@ -7,6 +7,7 @@
 #include <algorithm>
 #include <chrono>
 #include <cmath>
+#include <cstddef>
 #include <cstdio>
 #include <cstdlib>
 #include <cstring>
@@ -66,6 +67,38 @@ const char* scene_unusable(const rtc_context* ctx, const SceneRecord* s, bool re
     stale = stale || ctx->gas[g.first].generation != g.second;
   }
   return (stale && !refitAllowed) ? kStaleScene : nullptr;
+}
+
+// The device record behind the SceneDesc (SceneDeviceRecord), written whole when the scene is made.  Stream-ordered; the source
+// is pageable, so it is staged before cudaMemcpyAsync returns.
+int write_device_record(rtc_context* ctx, SceneRecord* s)
+{
+  SceneDeviceRecord r;
+  r.instMasks = static_cast<const uint8_t*>(s->d_instMasks);
+  r.usable = s->usableWritten = scene_unusable(ctx, s) ? 0u : 1u;
+  r.abi = kSceneDeviceAbi;
+  RTC_CUDA(cudaMemcpyAsync(reinterpret_cast<uint8_t*>(s->d_desc) + kSceneDeviceRecordOffset, &r, sizeof(r), cudaMemcpyHostToDevice, ctx->stream));
+  return 0;
+}
+
+// The record's `usable` word follows scene_unusable in stream order: after every call that can change the answer, one 4-byte copy
+// on the context stream when it differs from the last value written.  A device-side query (include/rtc_device.cuh) cannot be
+// refused on the host, and the instance records of an unusable scene may point at GAS nodes a rebuild or a destroy has freed.
+int write_usable(rtc_context* ctx, SceneRecord* s)
+{
+  const uint32_t usable = scene_unusable(ctx, s) ? 0u : 1u;
+  if (usable == s->usableWritten) return 0;
+  s->usableWritten = usable;
+  RTC_CUDA(cudaMemcpyAsync(reinterpret_cast<uint8_t*>(s->d_desc) + kSceneDeviceRecordOffset + offsetof(SceneDeviceRecord, usable),
+                           &s->usableWritten, sizeof(uint32_t), cudaMemcpyHostToDevice, ctx->stream));
+  return 0;
+}
+
+// GAS refits, rebuilds, device builds and destroys: every scene that references the GAS, and every created scene, may change
+int write_usable_all(rtc_context* ctx)
+{
+  for (SceneRecord* s : ctx->scenes) if (int rc = write_usable(ctx, s)) return rc;
+  return 0;
 }
 
 // After rtc_ias_rebuild the instance level's node count is only on the device: bring the host copy (desc.numTlasNodes and the
@@ -532,6 +565,7 @@ int rtc_gas_destroy(rtc_context* ctx, uint32_t gas)
   cudaFree(g.d_nodes); cudaFree(g.d_tris); free_refit_scratch(g.refit, ctx->stream); free_lbvh_rebuild(g.rebuild);
   g.d_nodes = nullptr; g.d_tris = nullptr; g.numNodes = 0; g.numTris = 0; g.boundsOnDevice = false;
   g.rebuild = nullptr; g.d_numNodes = nullptr; g.d_rejected = nullptr; g.capacity = 0;
+  if (int rc = write_usable_all(ctx)) return rc;
   return write_gas_table(ctx, gas);
 }
 
@@ -543,6 +577,7 @@ int rtc_gas_refit(rtc_context* ctx, uint32_t gas, uint64_t attributes)
   if (attributes) g.attributes = attributes;
   g.generation++;
   ctx->gasEpoch++;
+  if (int rc = write_usable_all(ctx)) return rc;
   if (int rc = refit_gas_gpu(ctx, g)) return rc;
   return write_gas_table(ctx, gas);
 }
@@ -555,6 +590,7 @@ int rtc_gas_rebuild(rtc_context* ctx, uint32_t gas, uint64_t attributes)
   if (attributes) g.attributes = attributes;
   g.generation++;
   ctx->gasEpoch++;
+  if (int rc = write_usable_all(ctx)) return rc;
   if (int rc = rebuild_gas_gpu(ctx, g)) return rc;
   return write_gas_table(ctx, gas);
 }
@@ -607,6 +643,7 @@ int rtc_gas_build_device(rtc_context* ctx, uint32_t gas, uint64_t attributes, ui
   g.attributes = attributes; g.indices = indices; g.strideBytes = strideBytes; g.numVerts = numVerts; g.numTris = numTris;
   g.generation++;
   ctx->gasEpoch++;
+  if (int rc = write_usable_all(ctx)) return rc;
   if (int rc = rebuild_gas_gpu(ctx, g)) return rc;
   g.buildMs = now_ms() - t0;
   return write_gas_table(ctx, gas);
@@ -708,8 +745,10 @@ int rtc_ias_build(rtc_context* ctx, const rtc_instance_desc* instances, uint32_t
   rec->desc.numInstances = numInstances;
   rec->desc.numTlasNodes = (uint32_t)bvh.nodes.size();
   rec->desc.numTlasLeaves = (uint32_t)bvh.primOrder.size();
-  if (e == cudaSuccess) e = upload((void**)&rec->d_desc, &rec->desc, sizeof(SceneDesc));
+  if (e == cudaSuccess) e = alloc((void**)&rec->d_desc, kSceneDeviceRecordOffset + sizeof(SceneDeviceRecord));
+  if (e == cudaSuccess) e = cudaMemcpyAsync(rec->d_desc, &rec->desc, sizeof(SceneDesc), cudaMemcpyHostToDevice, ctx->stream);
   if (e != cudaSuccess) { free_scene(rec, ctx->stream); return rtc_set_error(__FILE__, __LINE__, "rtc_ias_build upload", (int)e, cudaGetErrorString(e)); }
+  if (int rc = write_device_record(ctx, rec)) { free_scene(rec, ctx->stream); return rc; }
   rec->totalNodes += bvh.nodes.size();
   rec->iasBuildMs = now_ms() - t0;
   ctx->scenes.push_back(rec);
@@ -748,7 +787,7 @@ int rtc_ias_update(rtc_context* ctx, uint64_t topObject, uint32_t first, uint32_
   }
   const int rc = update_instances(ctx, s, first, count, staged, 48u);
   if (staged) cudaFreeAsync(staged, ctx->stream);
-  return rc;
+  return rc ? rc : write_usable(ctx, s);
 }
 
 int rtc_ias_update_device(rtc_context* ctx, uint64_t topObject, uint32_t first, uint32_t count, uint64_t transforms, uint32_t strideBytes)
@@ -761,7 +800,8 @@ int rtc_ias_update_device(rtc_context* ctx, uint64_t topObject, uint32_t first, 
   if (strideBytes < 48 || (strideBytes & 3u)) RTC_FAIL("strideBytes must be a multiple of 4 and at least 48");
   if (const char* why = scene_unusable(ctx, s, true)) RTC_FAIL(why);
   RTC_CUDA(cudaSetDevice(ctx->device));
-  return update_instances(ctx, s, first, count, reinterpret_cast<const uint8_t*>((uintptr_t)transforms), strideBytes);
+  if (int rc = update_instances(ctx, s, first, count, reinterpret_cast<const uint8_t*>((uintptr_t)transforms), strideBytes)) return rc;
+  return write_usable(ctx, s);
 }
 
 int rtc_ias_rebuild(rtc_context* ctx, uint64_t topObject)
@@ -770,7 +810,8 @@ int rtc_ias_rebuild(rtc_context* ctx, uint64_t topObject)
   if (!s) RTC_FAIL("unknown topObject");
   if (const char* why = scene_unusable(ctx, s)) RTC_FAIL(why);
   RTC_CUDA(cudaSetDevice(ctx->device));
-  return rebuild_instances_gpu(ctx, *s);
+  if (int rc = rebuild_instances_gpu(ctx, *s)) return rc;
+  return write_usable(ctx, s);
 }
 
 // A created scene's GAS totals from the device's per-handle reference counts.  Synchronises the stream.
@@ -802,7 +843,7 @@ int rtc_ias_create(rtc_context* ctx, uint32_t capacity, uint64_t* topObject)
   const size_t cap = capacity ? capacity : 1u;
   cudaError_t e = cudaSuccess;
   auto alloc = [&](void** dst, size_t bytes) { if (e == cudaSuccess) e = cudaMalloc(dst, bytes); };
-  alloc((void**)&s->d_desc, sizeof(SceneDesc));
+  alloc((void**)&s->d_desc, kSceneDeviceRecordOffset + sizeof(SceneDeviceRecord));
   alloc(&s->d_instances, cap * 4u * sizeof(float4));
   alloc(&s->d_tlasLeaves, cap * sizeof(uint32_t));
   alloc(&s->d_o2w, cap * 3u * sizeof(float4));
@@ -828,11 +869,13 @@ int rtc_ias_create(rtc_context* ctx, uint32_t capacity, uint64_t* topObject)
   s->desc.numInstances = 0; s->desc.numTlasLeaves = 0; s->desc.numTlasNodes = 1;
   // the node array, refit scratch, LBVH arrays and collapse graph for the capacity; the one empty root node of no instances
   if (int rc = create_instance_level_gpu(ctx, *s, capacity)) { cudaStreamSynchronize(ctx->stream); free_scene(s, ctx->stream); return rc; }
+  s->gasEpoch = ctx->gasEpoch;
   e = cudaMemcpyAsync(s->d_desc, &s->desc, sizeof(SceneDesc), cudaMemcpyHostToDevice, ctx->stream);
+  if (e == cudaSuccess)
+    if (int rc = write_device_record(ctx, s)) { cudaStreamSynchronize(ctx->stream); free_scene(s, ctx->stream); return rc; }
   if (e == cudaSuccess) e = cudaStreamSynchronize(ctx->stream);
   if (e != cudaSuccess) { free_scene(s, ctx->stream); return rtc_set_error(__FILE__, __LINE__, "rtc_ias_create", (int)e, cudaGetErrorString(e)); }
   s->totalNodes = 1;
-  s->gasEpoch = ctx->gasEpoch;
   ctx->scenes.push_back(s);
   *topObject = (uint64_t)(uintptr_t)s->d_desc;
   return 0;
@@ -873,7 +916,7 @@ int rtc_ias_build_device(rtc_context* ctx, uint64_t topObject, uint64_t instance
   s->gasEpoch = ctx->gasEpoch;
   s->gasDestroyed = false;
   s->iasBuildMs = now_ms() - t0;
-  return 0;
+  return write_usable(ctx, s);
 }
 
 int rtc_scene_rejected_instances(rtc_context* ctx, uint64_t topObject, uint32_t* count)

@@ -57,6 +57,21 @@ struct SceneDesc
   uint32_t        pad0;
 };
 
+// What the device-side queries of include/rtc_device.cuh read behind the SceneDesc: the allocation topObject points at holds this
+// record at kSceneDeviceRecordOffset.  The kernels of the library never read it (they get the SceneDesc by value).
+//   instMasks: SceneRecord::d_instMasks (never null)
+//   usable   : 1 while scene_unusable(ctx, s) == nullptr as the context stream reaches each point (rtc_api.cpp write_usable)
+//   abi      : kSceneDeviceAbi of the library that wrote it; the header compares it with its own
+struct SceneDeviceRecord
+{
+  const uint8_t* instMasks;
+  uint32_t       usable;
+  uint32_t       abi;
+};
+constexpr size_t kSceneDeviceRecordOffset = (sizeof(SceneDesc) + 15u) & ~(size_t)15u;
+constexpr uint32_t kSceneDeviceAbi = 0x52544401u;      // "RTD" 1
+static_assert(sizeof(SceneDeviceRecord) == 16, "the device record is 16 bytes");
+
 // Host-side result of a BVH build over generic primitive boxes.
 struct WideBvh
 {
@@ -122,7 +137,8 @@ struct GasRecord
 struct SceneRecord
 {
   SceneDesc desc{};          // host copy
-  SceneDesc* d_desc = nullptr;
+  SceneDesc* d_desc = nullptr;             // followed by the SceneDeviceRecord at kSceneDeviceRecordOffset
+  uint32_t usableWritten = 1;              // SceneDeviceRecord::usable as the last write enqueued on the stream left it
   void *d_tlasNodes = nullptr, *d_instances = nullptr, *d_tlasLeaves = nullptr, *d_o2w = nullptr, *d_geomInst = nullptr, *d_instFlags = nullptr;
   std::vector<uint32_t> instFlags;         // host copy of the per-instance flags
   uint32_t numCutout = 0;                  // instances using the cutout hit records: > 0 selects the ordered any-hit path

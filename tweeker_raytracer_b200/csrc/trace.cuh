@@ -307,10 +307,15 @@ struct TraceFilter
 // Rays whose traversal stack ran out of its 40 entries (the dropped subtree may hide a hit).  Never non-zero for the 8-wide
 // trees this library builds; exported through rtc_stats so that a violation is loud instead of a silently wrong image.
 // (one counter per translation unit that instantiates the traversal: kernels_trace.cu and kernels_shade.cu)
+// RTC_STACK_OVERFLOW_STORAGE `static` makes the counter local to the translation unit, so that several of them can include
+// this header and still device-link (include/rtc_device.cuh).
 #ifndef RTC_STACK_OVERFLOW_COUNTER
 #define RTC_STACK_OVERFLOW_COUNTER g_rtcStackOverflows
 #endif
-__device__ unsigned int RTC_STACK_OVERFLOW_COUNTER = 0;
+#ifndef RTC_STACK_OVERFLOW_STORAGE
+#define RTC_STACK_OVERFLOW_STORAGE
+#endif
+RTC_STACK_OVERFLOW_STORAGE __device__ unsigned int RTC_STACK_OVERFLOW_COUNTER = 0;
 
 // One ray's traversal as a resumable state machine: begin() once, then step() until it returns false.
 // A step visits one wide node (or pops a postponed leaf group) and tests the triangles / enters the instance it yields.
