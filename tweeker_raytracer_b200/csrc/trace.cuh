@@ -10,6 +10,8 @@
 // The box test is only required to be conservative and is free to use contracted arithmetic.
 #pragma once
 
+#include <type_traits>
+
 #include "rtc_internal.h"
 
 #ifndef RTC_I2F_AXES
@@ -296,6 +298,9 @@ struct TraceFilter
   uint32_t rayMask, cullFlags;
 };
 
+// ANYHIT of Traversal: no any-hit callback (every kernel of the library, and rtc_device_trace_closest / _any).
+struct TraceNoAnyHit {};
+
 #define RTC_SM_STACK 8        // traversal stack entries per thread kept in shared memory
 #if RTC_RESTORE_WORLD
 #define RTC_SM_RAY_WORDS 15   // float columns per thread behind the stack (Traversal::smRay)
@@ -327,9 +332,17 @@ RTC_STACK_OVERFLOW_STORAGE __device__ unsigned int RTC_STACK_OVERFLOW_COUNTER = 
 // lane with more pending skips its node visit until they are done; see step().  0: every triangle of the leaves a node visit found.
 // FILTER = true (rtc_trace_*_ex): the TraceFilter passed to step() / leaf_phase() masks instances and culls triangles by facing;
 // with FILTER = false the filter argument is never read and the generated code is that of the plain traversal.
-template <bool ANY, bool COUNT, int BLOCK, bool SKIP = false, int TRICAP = RTC_ONE_TRI_PER_STEP, bool FILTER = false>
+// ANYHIT (the any-hit callbacks of include/rtc_device.cuh): a candidate that passed tri_test, the cull flags, t > tmin and the
+// ANY / closer_hit condition is offered to (*anyHit)(t, det, V, W, inst, prim) before it becomes the hit: 0 ignores it, 2 accepts
+// it and ends the ray, anything else accepts it (the ANY query ends on every accept).  With TraceNoAnyHit the argument is never
+// read and the generated code is that of the traversal without it.
+template <bool ANY, bool COUNT, int BLOCK, bool SKIP = false, int TRICAP = RTC_ONE_TRI_PER_STEP, bool FILTER = false, class ANYHIT = TraceNoAnyHit>
 struct Traversal
 {
+  static constexpr bool HAS_ANYHIT = !std::is_same<ANYHIT, TraceNoAnyHit>::value;
+  // ignore is a `continue` in leaf_phase: it would not count towards the triangle cap, and SKIP / COUNT have no callback use
+  static_assert(!HAS_ANYHIT || (!SKIP && !COUNT && TRICAP == 0 && FILTER), "any-hit callbacks run in the uncapped filtered traversal only");
+
   float skipT; uint32_t skipInst, skipPrim;       // SKIP only
   // World ray origin/direction (needed only when an instance is entered or left) and the barycentric numerators of the
   // best hit (written once per accepted hit) live in shared memory, column-major like the stack: nine registers less,
@@ -437,8 +450,8 @@ struct Traversal
     }
   }
 
-  // returns false when the ray is finished (ANY: first hit)
-  __device__ __forceinline__ bool leaf_phase(const SceneDesc& sc, const TraceFilter& filt = TraceFilter())
+  // returns false when the ray is finished (ANY: first hit; ANYHIT: first accept of ANY, accept-and-end)
+  __device__ __forceinline__ bool leaf_phase(const SceneDesc& sc, const TraceFilter& filt = TraceFilter(), ANYHIT* anyHit = nullptr)
   {
     int tested = 0;      // TRICAP > 1 only
     while (triGroup.y)
@@ -479,6 +492,22 @@ struct Traversal
             (!FILTER || !(filt.cullFlags & (det > 0.0f ? RTC_RAY_CULL_FRONT_FACING : RTC_RAY_CULL_BACK_FACING))) && t > tmin)
         {
           const uint32_t prim = __float_as_uint(v0.w);
+          if constexpr (HAS_ANYHIT)
+          {
+            // Only a candidate that would become the hit is offered; ignore keeps tlimit, so the box tests stay conservative
+            // for every candidate the callback has not seen yet.
+            if (ANY ? t < tlimit : closer_hit(t, curInst, prim, hitT, hitInst, hitPrim, tlimit))
+            {
+              const int decision = (*anyHit)(t, det, V, W, curInst, prim);
+              if (decision == 0) continue;
+              hitT = t; hitInst = curInst; hitPrim = prim;
+              if (ANY) return false;
+              tlimit = t;
+              smRay[6 * BLOCK] = V; smRay[7 * BLOCK] = W; smRay[8 * BLOCK] = det;
+              if (decision == 2) return false;
+            }
+            continue;
+          }
           if (SKIP && !(t > skipT || (t == skipT && (curInst > skipInst || (curInst == skipInst && prim > skipPrim))))) continue;
           if (ANY)
           {
@@ -523,7 +552,7 @@ struct Traversal
   }
 
   // returns true while the ray needs more steps
-  __device__ __forceinline__ bool step(const SceneDesc& sc, const TraceFilter& filt = TraceFilter())
+  __device__ __forceinline__ bool step(const SceneDesc& sc, const TraceFilter& filt = TraceFilter(), ANYHIT* anyHit = nullptr)
   {
     if (TRICAP > 0)
     {
@@ -536,12 +565,12 @@ struct Traversal
       // Built after the last GPU session of round 2 and therefore never enabled blindly: the library times one batch with each
       // schedule and keeps a capped one only where it is faster (kernels_shade.cu, "schedule tuner").
       if (!(blasBase >= 0 && has_leaves())) node_phase();
-      if (!leaf_phase(sc, filt)) return false;
+      if (!leaf_phase(sc, filt, anyHit)) return false;
       if (blasBase >= 0 && has_leaves()) return true;
       return advance(sc);
     }
     node_phase();
-    if (!leaf_phase(sc, filt)) return false;
+    if (!leaf_phase(sc, filt, anyHit)) return false;
     return advance(sc);
   }
 };
